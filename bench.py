@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- feature updates / s of the OrcVIO filter-update hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[3], "stress frame"): one frozen frame with a 30-clone window
@@ -81,6 +81,14 @@ WORKLOAD = f"stress frame: {N_CLONES}-clone window, {N_FEATURES} features, max_t
 def make_frame(seed, n_feat=N_FEATURES):
     from orcvio_b200 import synth
     return synth.stress_snapshot(N_CLONES, n_feat, MAX_TRACK, seed=seed)
+
+
+def dump_outputs(path, out):
+    """What a caller of the frame update receives (posterior P, delta_x, per-feature status and gamma, updated clones),
+    one float64 .npy per array, so that two builds can be compared output for output on the same seeded frame."""
+    os.makedirs(path, exist_ok=True)
+    for name in ("P", "delta_x", "status", "gamma", "clones"):
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(out[name], dtype=np.float64))
 
 
 def algorithmic_bytes(snap, status, stage):
@@ -480,7 +488,13 @@ def main():
     ap.add_argument("--mc-traj", type=int, default=1024)
     ap.add_argument("--mc-frames", type=int, default=200)
     ap.add_argument("--mc-feats", type=int, default=150)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed frame update computed in its last step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -540,6 +554,10 @@ def main():
     launches = fr.kernel_launches() - l0
     barrier()
     t_val = torch.tensor([dev_us * 1e-6], dtype=torch.float64, device=dev)
+    if args.dump_outputs and rank == 0:
+        # fetch() replays the chain once with the download queued; every run restores the frame's inputs first, so
+        # this is exactly what the last timed step computed
+        dump_outputs(args.dump_outputs, fr.fetch())
 
     # ---- e2e: host buffers through the C ABI, wall clock around synchronous calls
     for _ in range(args.warmup):

@@ -5,8 +5,6 @@ The key set and the values are those read by OrcVIO::loadParameters
 config/kitti_odom.yaml (the table in SURVEY.md A.2).  They are kept here as Python
 dictionaries and written out as OpenCV-YAML (`%YAML:1.0`, `!!opencv-matrix`) so that
 both the product's C++ reader and cv2.FileStorage (oracle) parse the same file.
-tests/test_abi_cpu.py checks these dictionaries against the reference's yaml files
-whenever /root/reference is mounted.
 """
 import copy
 
