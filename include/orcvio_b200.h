@@ -170,6 +170,14 @@ int orcvio_batch_process(orcvio_batch* b, const double* t_img, const OrcvioFeatu
 int orcvio_batch_replay(orcvio_batch* b, int n_frames, const double* t_img, const OrcvioFeature* const* feats,
                         const int* feat_off, const OrcvioImu* const* imu, const int* n_imu, double imu_window,
                         double* poses_out, int* ok_out);
+/* orcvio_batch_replay that also records what filter consistency needs.  state17_out: n_filters x n_frames x 17 = t (the
+ * IMU state's own time), p (3), q xyzw (4), v (3), bg (3), ba (3) after every frame.  cov15_out: n_filters x n_frames x
+ * 225, the leading 15 x 15 block of the covariance (error state [theta, v, p, b_g, b_a], row-major) after every frame,
+ * captured on the device and downloaded once at the end of the call.  Either may be NULL; with both NULL this is
+ * orcvio_batch_replay. */
+int orcvio_batch_replay_states(orcvio_batch* b, int n_frames, const double* t_img, const OrcvioFeature* const* feats,
+                               const int* feat_off, const OrcvioImu* const* imu, const int* n_imu, double imu_window,
+                               double* poses_out, int* ok_out, double* state17_out, double* cov15_out);
 /* Object pose initialisation, first step (ObjectFeatureInitializer::single_object_initialization without RANSAC,
  * src/obj/ObjectFeatureInitializer.cpp:99-111): findTransform (:265-341) -- similarity fit of the mean-shape keypoints
  * onto the triangulated ones, scale from the polyline lengths, rotation by Kabsch -- and, with se2_flag,
@@ -219,6 +227,20 @@ int orcvio_lm_known_answer(int which, double* x_out, int* status, int* nfev, int
  * (deg), mean position error (m), position RMSE (m) and final position error (m) -> out4 (n_traj x 4).  Poses are
  * n_traj x n_frames x 7 (p, q xyzw, Hamilton), host pointers. */
 int orcvio_trajectory_metrics(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, double* out4);
+/* NEES of a batch of filter runs against their truth, on the device.  est17 / gt17: n_traj x n_frames x 17 (layout of
+ * state17_out), cov15: n_traj x n_frames x 225 (cov15_out), host pointers.  flags: bit0 use_larvio, bit1
+ * use_left_perturbation (the orientation error is Log(R R_est^T) if either is set, else Log(R_est^T R); v, p and the
+ * biases are true - estimate).  nees8_out (n_traj x n_frames x 8): NEES of theta (dof 3), v (3), p (3), pose [theta, p]
+ * (6), navigation [theta, v, p] (9), full IMU state (15), then |dtheta| in degrees and |dp| in metres; NaN when the
+ * 15 x 15 block is not positive definite or an input is not finite.  summary9_out (n_frames x 9, may be NULL): per frame
+ * over the valid trajectories, the ANEES of the six blocks, the RMS orientation error (deg), the RMS position error (m)
+ * and the number of valid trajectories (fixed-order reduction: the same rows give the same bits).  The 95 % bounds of
+ * the ANEES of a block of dof d over N runs are orcvio_chi2_quantile(0.025 | 0.975, N d) / N. */
+int orcvio_trajectory_nees(const double* est17, const double* gt17, const double* cov15, int n_traj, int n_frames,
+                           int flags, double* nees8_out, double* summary9_out);
+/* summary9_out of orcvio_trajectory_nees from NEES rows alone (n_traj x n_frames x 8), e.g. rows gathered from several
+ * ranks: the same kernel, so the same rows give the same bits as the summary of orcvio_trajectory_nees. */
+int orcvio_nees_summary(const double* nees8, int n_traj, int n_frames, double* summary9_out);
 /* The reference's KITTI-style relative error (python_scripts/trajectory_eval/traj_eval.py:61-90 -> the vendored
  * rpg_trajectory_evaluation: compute_trajectory_errors.py:10-67, trajectory.py:341-377, 309-339) for a batch of
  * trajectories on the device: for every sub-trajectory length the pairs (start, first pose closest to start + length

@@ -83,7 +83,10 @@ def lib():
     L.orcvio_batch_process.argtypes = [vp, dp, vp, ip, vp, ip, ip, ip]
     L.orcvio_batch_get_state.argtypes = [vp, C.c_int, C.POINTER(OrcvioState)]
     L.orcvio_batch_replay.argtypes = [vp, C.c_int, dp, vp, ip, vp, ip, C.c_double, dp, ip]
+    L.orcvio_batch_replay_states.argtypes = [vp, C.c_int, dp, vp, ip, vp, ip, C.c_double, dp, ip, dp, dp]
     L.orcvio_trajectory_metrics.argtypes = [dp, dp, C.c_int, C.c_int, dp]
+    L.orcvio_trajectory_nees.argtypes = [dp, dp, dp, C.c_int, C.c_int, C.c_int, dp, dp]
+    L.orcvio_nees_summary.argtypes = [dp, C.c_int, C.c_int, dp]
     L.orcvio_get_tcw.argtypes = [vp, dp, dp]
     L.orcvio_set_pose_log.argtypes = [vp, C.c_char_p]
     L.orcvio_batch_get_cov.argtypes = [vp, C.c_int, dp, C.c_int, ip]
@@ -395,10 +398,8 @@ class Batch:
             raise RuntimeError(f"orcvio_batch_process failed: {rc}")
         return used, pub
 
-    def replay(self, t_img, feats, feat_off, imus, imu_window=0.02):
-        """Whole-sequence replay (orcvio_batch_replay).  t_img (n, F); feats: list of n struct arrays (all frames of a
-        filter concatenated); feat_off (n, F + 1); imus: list of n struct arrays.  Returns (poses (n, F, 7), ok (n,)).
-        The call releases the GIL: several batches replay concurrently from Python threads."""
+    def _replay_args(self, t_img, feats, feat_off, imus, imu_window):
+        """(n, F, the inputs of orcvio_batch_replay[_states] up to imu_window); the arrays stay referenced by the tuple."""
         t_img = np.ascontiguousarray(t_img, dtype=np.float64)
         n, F = t_img.shape
         assert n == self.n
@@ -406,13 +407,33 @@ class Batch:
         fptr = (C.c_void_p * n)(*[f.ctypes.data for f in feats])
         iptr = (C.c_void_p * n)(*[m.ctypes.data for m in imus])
         n_imu = np.array([len(m) for m in imus], dtype=np.int32)
+        return n, F, (F, _dp(t_img), fptr, _ip(feat_off), iptr, _ip(n_imu), float(imu_window))
+
+    def replay(self, t_img, feats, feat_off, imus, imu_window=0.02):
+        """Whole-sequence replay (orcvio_batch_replay).  t_img (n, F); feats: list of n struct arrays (all frames of a
+        filter concatenated); feat_off (n, F + 1); imus: list of n struct arrays.  Returns (poses (n, F, 7), ok (n,)).
+        The call releases the GIL: several batches replay concurrently from Python threads."""
+        n, F, args = self._replay_args(t_img, feats, feat_off, imus, imu_window)
         poses = np.zeros((n, F, 7))
         ok = np.zeros(n, dtype=np.int32)
-        rc = self._L.orcvio_batch_replay(self._h, F, _dp(t_img), fptr, _ip(feat_off), iptr, _ip(n_imu), float(imu_window),
-                                         _dp(poses), _ip(ok))
+        rc = self._L.orcvio_batch_replay(self._h, *args, _dp(poses), _ip(ok))
         if rc != 0:
             raise RuntimeError(f"orcvio_batch_replay failed: {rc}")
         return poses, ok
+
+    def replay_states(self, t_img, feats, feat_off, imus, imu_window=0.02, states=True, cov=True):
+        """replay() that also records, after every frame, the IMU state (n, F, 17: t, p, q xyzw, v, bg, ba) and the
+        leading 15 x 15 block of the covariance (n, F, 15, 15; error state [theta, v, p, b_g, b_a]), captured on the
+        device (orcvio_batch_replay_states).  Returns (poses, ok, states, cov15); a record not asked for is None."""
+        n, F, args = self._replay_args(t_img, feats, feat_off, imus, imu_window)
+        poses = np.zeros((n, F, 7))
+        ok = np.zeros(n, dtype=np.int32)
+        st = np.zeros((n, F, 17)) if states else None
+        cv = np.zeros((n, F, 15, 15)) if cov else None
+        rc = self._L.orcvio_batch_replay_states(self._h, *args, _dp(poses), _ip(ok), _dp(st), _dp(cv))
+        if rc != 0:
+            raise RuntimeError(f"orcvio_batch_replay_states failed: {rc}")
+        return poses, ok, st, cv
 
     def state(self, i):
         s = OrcvioState()
@@ -707,6 +728,51 @@ def trajectory_metrics(est_pose7, gt_pose7):
     if rc != 0:
         raise RuntimeError(f"orcvio_trajectory_metrics failed: {rc}")
     return out
+
+
+NEES_BLOCKS = (("theta", 3), ("v", 3), ("p", 3), ("pose", 6), ("nav", 9), ("full", 15))
+
+
+def nees_flags(cfg):
+    """The orientation-error convention of a configuration: bit0 use_larvio_flag, bit1 use_left_perturbation_flag."""
+    return (1 if int(cfg.get("use_larvio_flag", 0)) else 0) | (2 if int(cfg.get("use_left_perturbation_flag", 0)) else 0)
+
+
+def trajectory_nees(est17, gt17, cov15, flags):
+    """NEES of filter runs against their truth on the device (orcvio_trajectory_nees).  est17 / gt17 (n, F, 17) state
+    records (t, p, q xyzw, v, bg, ba), cov15 (n, F, 15, 15), flags: bit0 use_larvio, bit1 use_left_perturbation.
+    Returns (nees (n, F, 8): NEES theta, v, p, pose, nav, full, |dtheta| deg, |dp| m -- NaN rows where the block is not
+    positive definite or an input is not finite;  summary (F, 9): per frame ANEES of the six blocks, RMS orientation error
+    (deg), RMS position error (m), number of valid trajectories)."""
+    e = np.ascontiguousarray(est17, dtype=np.float64)
+    g = np.ascontiguousarray(gt17, dtype=np.float64)
+    c = np.ascontiguousarray(cov15, dtype=np.float64)
+    assert e.shape == g.shape and e.ndim == 3 and e.shape[2] == 17 and c.size == e.shape[0] * e.shape[1] * 225
+    n, F = e.shape[:2]
+    nees = np.zeros((n, F, 8))
+    summ = np.zeros((F, 9))
+    rc = lib().orcvio_trajectory_nees(_dp(e), _dp(g), _dp(c), n, F, int(flags), _dp(nees), _dp(summ))
+    if rc != 0:
+        raise RuntimeError(f"orcvio_trajectory_nees failed: {rc}")
+    return nees, summ
+
+
+def nees_summary(nees):
+    """The per-frame summary of trajectory_nees from NEES rows alone (orcvio_nees_summary, the same kernel)."""
+    r = np.ascontiguousarray(nees, dtype=np.float64)
+    assert r.ndim == 3 and r.shape[2] == 8
+    summ = np.zeros((r.shape[1], 9))
+    rc = lib().orcvio_nees_summary(_dp(r), r.shape[0], r.shape[1], _dp(summ))
+    if rc != 0:
+        raise RuntimeError(f"orcvio_nees_summary failed: {rc}")
+    return summ
+
+
+def anees_bounds(n, dof, p=0.95):
+    """Two-sided `p` bounds of the ANEES of a dof-dimensional block averaged over n runs:
+    chi2_quantile((1 -+ p) / 2, n dof) / n."""
+    a = (1.0 - p) / 2.0
+    return chi2_quantile(a, n * dof) / n, chi2_quantile(1.0 - a, n * dof) / n
 
 
 def trajectory_align_ate(est_pose7, gt_pose7, method="sim3"):

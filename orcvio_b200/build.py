@@ -32,6 +32,7 @@ SOURCES = {
     "ekf_kernel.cu": [],
     "hybrid_kernel.cu": [],
     "metrics_kernel.cu": [],
+    "consistency_kernel.cu": [],
     "kabsch_kernel.cu": [],
     "objlm_kernel.cu": [],
     "lm.cpp": [],

@@ -346,6 +346,7 @@ Batch::~Batch() {
   if (blob_early_.pinned) cudaFreeHost(blob_early_.pinned);
   cudaFree(dLs_); cudaFree(dTileRows_); cudaFree(dFilterRows_); cudaFree(dSyrkCnt_);
   if (dZuptDec_) cudaFree(dZuptDec_);
+  if (dCovHist_) cudaFree(dCovHist_);
   if (dZuptInfo_) cudaFree(dZuptInfo_);
   if (hZuptDec_) cudaFreeHost(hZuptDec_);
   if (hZuptInfo_) cudaFreeHost(hZuptInfo_);
@@ -1007,8 +1008,34 @@ static thread_local SecProf g_sp;
 // drive several batches from as many host threads).  poses_out: n_filters x n_frames x 7, the IMU pose after every
 // frame (position, quaternion x y z w: one line of the reference's state_est_geo_feat.txt log, src/orcvio.cpp:643-645);
 // ok_out[i] = 0 when some frame of filter i was not published.
+//
+// state17_out (n_filters x n_frames x 17: IM_TIME, p, q xyzw, v, b_g, b_a) comes from the host mirror like poses_out.
+// cov15_out (n_filters x n_frames x 225) is captured on the device: after frame f, k_capture_imu_cov copies the leading
+// 15 x 15 block of every filter's P into dCovHist_[i, f], and the history comes down once at the end.  The capture is
+// queued on stream_ behind the whole frame.  Every kernel that writes P runs on stream_ (propagation, augmentation,
+// ZUPT, k_compact_cov, k_reanchor, both update chains -- k_pinfo / k_apply_dx -- with the hybrid post kernels, k_remove;
+// the initial covariance is a memset + copy on stream_), and the side stream stream2_ only reads P (k_chol_prior,
+// k_imu_factor) and is joined to stream_ (ev_join_, ev_ls_) before the update writes it.  The next frame's P writers
+// are queued on stream_ after the capture, and its side-stream work forks from stream_ after it (ev_fork_): nothing
+// overwrites P before the capture has read it.
 int Batch::replay(int n_frames, const double* t_img, const OrcvioFeature* const* feats, const int* feat_off,
-                  const OrcvioImu* const* imu, const int* n_imu, double imu_window, double* poses_out, int* ok_out) {
+                  const OrcvioImu* const* imu, const int* n_imu, double imu_window, double* poses_out, int* ok_out,
+                  double* state17_out, double* cov15_out) {
+  if (cov15_out && n_frames > 0) {
+    const size_t need = (size_t)B_ * n_frames * 225;
+    if (need > covhist_cap_) {                           // grown ahead of the loop, never inside it
+      cudaSetDevice(dev_);
+      if (dCovHist_) cudaFree(dCovHist_);
+      dCovHist_ = nullptr;
+      covhist_cap_ = 0;
+      note_growth("covariance history", need * sizeof(double));
+      if (cudaMalloc(&dCovHist_, need * sizeof(double)) != cudaSuccess) {
+        dCovHist_ = nullptr;
+        return ORCVIO_ERR_CUDA;
+      }
+      covhist_cap_ = need;
+    }
+  }
   std::vector<const OrcvioFeature*> fp(B_);
   std::vector<const OrcvioImu*> ip(B_);
   std::vector<int> nf(B_), ni(B_), cursor(B_, 0), used(B_), pub(B_);
@@ -1041,7 +1068,28 @@ int Batch::replay(int n_frames, const double* t_img, const OrcvioFeature* const*
       double* o = poses_out + ((size_t)i * n_frames + f) * 7;
       for (int k = 0; k < 3; ++k) o[k] = im[IM_P + k];
       rotation_to_quat_xyzw(im + IM_R, o + 3);
+      if (state17_out) {
+        double* s = state17_out + ((size_t)i * n_frames + f) * 17;
+        s[0] = im[IM_TIME];
+        for (int k = 0; k < 7; ++k) s[1 + k] = o[k];
+        for (int k = 0; k < 3; ++k) {
+          s[8 + k] = im[IM_V + k];
+          s[11 + k] = im[IM_BG + k];
+          s[14 + k] = im[IM_BA + k];
+        }
+      }
     }
+    if (cov15_out) {
+      launch_capture_imu_cov(dP_, (size_t)ldp_ * ldp_, ldp_, B_, dCovHist_, n_frames, f, stream_);
+      ++launches_;
+    }
+  }
+  if (cov15_out && n_frames > 0) {
+    CK(cudaMemcpyAsync(cov15_out, dCovHist_, (size_t)B_ * n_frames * 225 * sizeof(double), cudaMemcpyDeviceToHost,
+                       stream_));
+    CK(cudaStreamSynchronize(stream_));
+    if (launch_error_count() > 0) { ok_ = false; err_ = "kernel launch failed"; }
+    if (!ok_) return ORCVIO_ERR_CUDA;
   }
   if (frame_prof && !frame_ms.empty()) {
     std::vector<double> v = frame_ms;

@@ -165,8 +165,10 @@ class Batch {
               const OrcvioImu* imu, const int* imu_off, int* imu_used, int* published);
   int process_ptrs(const double* t_img, const OrcvioFeature* const* feats, const int* n_feats,
                    const OrcvioImu* const* imu, const int* n_imu, int* imu_used, int* published);
+  // state17_out / cov15_out (either may be NULL): the IMU state and the leading 15 x 15 block of P after every frame
   int replay(int n_frames, const double* t_img, const OrcvioFeature* const* feats, const int* feat_off,
-             const OrcvioImu* const* imu, const int* n_imu, double imu_window, double* poses_out, int* ok_out);
+             const OrcvioImu* const* imu, const int* n_imu, double imu_window, double* poses_out, int* ok_out,
+             double* state17_out = nullptr, double* cov15_out = nullptr);
   int get_state(int i, OrcvioState* out);
   int get_cov(int i, double* P, int cap, int* D);
   int set_cov(int i, const double* P, int D);
@@ -316,6 +318,8 @@ class Batch {
   std::vector<double> chi2_host_;
   std::vector<double> chi2_zupt_host_;     // chi_squared_table_zupt (p = 0.95, :482-493)
   int* dZuptDec_ = nullptr; double* dZuptInfo_ = nullptr;
+  double* dCovHist_ = nullptr;         // replay with covariance capture: n_filters x n_frames x 225
+  size_t covhist_cap_ = 0;
   int* hZuptDec_ = nullptr; double* hZuptInfo_ = nullptr;
 
   void prereserve();

@@ -300,6 +300,14 @@ int orcvio_batch_replay(orcvio_batch* b, int n_frames, const double* t_img, cons
   return b->batch->replay(n_frames, t_img, feats, feat_off, imu, n_imu, imu_window, poses_out, ok_out);
 }
 
+int orcvio_batch_replay_states(orcvio_batch* b, int n_frames, const double* t_img, const OrcvioFeature* const* feats,
+                               const int* feat_off, const OrcvioImu* const* imu, const int* n_imu, double imu_window,
+                               double* poses_out, int* ok_out, double* state17_out, double* cov15_out) {
+  if (!b || n_frames < 0 || !t_img || !feats || !feat_off || !imu || !n_imu || !poses_out || !ok_out) return ORCVIO_ERR_ARG;
+  return b->batch->replay(n_frames, t_img, feats, feat_off, imu, n_imu, imu_window, poses_out, ok_out, state17_out,
+                          cov15_out);
+}
+
 int orcvio_object_kabsch_init(const double* mean_pts, const double* world_pts, const int* off, int n_obj, int se2_flag,
                               double* wTq16_out, int* ok_out) {
   return ob::kabsch_init(mean_pts, world_pts, off, n_obj, se2_flag, wTq16_out, ok_out);
@@ -335,6 +343,15 @@ int orcvio_lm_known_answer(int which, double* x_out, int* status, int* nfev, int
 int orcvio_trajectory_metrics(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, double* out4) {
   if (!est_pose7 || !gt_pose7 || !out4) return ORCVIO_ERR_ARG;
   return ob::trajectory_metrics(est_pose7, gt_pose7, n_traj, n_frames, out4);
+}
+
+int orcvio_trajectory_nees(const double* est17, const double* gt17, const double* cov15, int n_traj, int n_frames,
+                           int flags, double* nees8_out, double* summary9_out) {
+  return ob::trajectory_nees(est17, gt17, cov15, n_traj, n_frames, flags, nees8_out, summary9_out);
+}
+
+int orcvio_nees_summary(const double* nees8, int n_traj, int n_frames, double* summary9_out) {
+  return ob::nees_summary(nees8, n_traj, n_frames, summary9_out);
 }
 
 int orcvio_kitti_relative_error(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames,

@@ -329,6 +329,13 @@ int trajectory_metrics(const double* est_pose7, const double* gt_pose7, int n_tr
 int kitti_relative_error(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, const double* lengths,
                          int n_len, const double* scale, double* out4, double* trans_error_pct);
 int umeyama_ate(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, int known_scale, double* out15);
+// filter consistency (consistency_kernel.cu): the leading 15 x 15 block of every filter's P into hist[filter, frame]
+// (queued on the batch stream after a frame); NEES / ANEES of state records against the truth (host pointers)
+void launch_capture_imu_cov(const double* P, size_t p_stride, int ldp, int n_filters, double* hist, int n_frames,
+                            int frame, cudaStream_t s);
+int trajectory_nees(const double* est17, const double* gt17, const double* cov15, int n_traj, int n_frames, int flags,
+                    double* nees8, double* summary9);
+int nees_summary(const double* nees8, int n_traj, int n_frames, double* summary9);
 // findTransform (+ poseSE32SE2) for a batch of objects (kabsch_kernel.cu); host pointers
 int kabsch_init(const double* mean_pts, const double* world_pts, const int* off, int n_obj, int se2, double* wTq16, int* ok);
 // object state optimiser (objlm_kernel.cu); host pointers

@@ -82,10 +82,20 @@ def gt_poses(seqs, n_frames):
     return g
 
 
-def run_replay(cfg_path, seqs, traj_ids, n_threads=1):
+def truth_states(seqs, states):
+    """Ground truth of every sequence at its estimates' own state times (states[..., 0], an IMU stamp), in the layout of
+    the state records: (n, F, 17)."""
+    return np.stack([synth.truth_states(s["spec"], states[i, :, 0]) for i, s in enumerate(seqs)])
+
+
+def run_replay(cfg_path, seqs, traj_ids, n_threads=1, consistency=False):
     """The local trajectories, split into `n_threads` batches that replay concurrently from as many host threads (the
     host bookkeeping of a filter is serial code: the batches are what spreads it over the cores, and their kernels
-    overlap on the device).  Returns (records, dict(seconds, feature_updates, kernel_launches, poses))."""
+    overlap on the device).  Returns (records, dict(seconds, feature_updates, kernel_launches, poses)).
+
+    consistency: replay through Batch.replay_states instead (the IMU state and the leading 15 x 15 covariance block after
+    every frame, captured on the device) and add to the dict `states` (n, F, 17), `cov15` (n, F, 15, 15), `truth` (n, F,
+    17, at the states' own times), `nees` (n, F, 8) and `summary` (F, 9) of api.trajectory_nees over these trajectories."""
     import threading
     import time
     n = len(seqs)
@@ -102,11 +112,19 @@ def run_replay(cfg_path, seqs, traj_ids, n_threads=1):
         packs.append(pack_replay([seqs[i] for i in g], n_frames))
     poses = np.zeros((n, n_frames, 7))
     ok = np.zeros(n)
+    if consistency:
+        states = np.zeros((n, n_frames, 17))
+        cov15 = np.zeros((n, n_frames, 15, 15))
     errors = []
 
     def work(k):
         try:
-            p, o = batches[k].replay(*packs[k])
+            if consistency:
+                p, o, st, cv = batches[k].replay_states(*packs[k])
+                states[groups[k]] = st
+                cov15[groups[k]] = cv
+            else:
+                p, o = batches[k].replay(*packs[k])
             poses[groups[k]] = p
             ok[groups[k]] = o
         except Exception as e:       # surfaced after the join
@@ -128,6 +146,10 @@ def run_replay(cfg_path, seqs, traj_ids, n_threads=1):
         rec[i] = [traj_ids[i], n_frames, *poses[i, -1, :3], met[i, 1], fu / max(n, 1), ok[i]]
     info = dict(seconds=seconds, feature_updates=fu, kernel_launches=sum(b.kernel_launches() for b in batches),
                 poses=poses, metrics=met, n_frames=n_frames, n_batches=n_threads)
+    if consistency:
+        truth = truth_states(seqs, states)
+        nees, summary = api.trajectory_nees(states, truth, cov15, api.nees_flags(seqs[0]["cfg"]))
+        info.update(states=states, cov15=cov15, truth=truth, nees=nees, summary=summary)
     return rec, info
 
 
@@ -180,3 +202,33 @@ def gather_records(rec, n_traj, rank, world, device=None):
         a = a[a[:, 0] >= 0]
         out[a[:, 0].astype(int)] = a
     return out
+
+
+def gather_nees(nees, traj_ids, n_traj, rank, world, device=None):
+    """all_gather of the per-trajectory NEES rows (fixed size n_frames x 8 each, api.trajectory_nees); returns (n_traj,
+    n_frames, 8) ordered by trajectory id on every rank.  The summary over all trajectories is then
+    api.nees_summary(rows): the same rows in the same order, hence the same bits for every world size."""
+    nees = np.asarray(nees, dtype=np.float64)
+    n_frames = nees.shape[1]
+    width = 1 + n_frames * 8
+    rows = np.zeros((len(traj_ids), width))
+    rows[:, 0] = traj_ids
+    rows[:, 1:] = nees.reshape(len(traj_ids), -1)
+    if world == 1:
+        out = np.zeros((n_traj, width))
+        out[rows[:, 0].astype(int)] = rows
+        return out[:, 1:].reshape(n_traj, n_frames, 8)
+    import torch
+    import torch.distributed as dist
+    per = (n_traj + world - 1) // world
+    buf = torch.full((per, width), -1.0, dtype=torch.float64, device=device)
+    if len(rows):
+        buf[:len(rows)] = torch.as_tensor(rows, dtype=torch.float64, device=device)
+    parts = [torch.empty_like(buf) for _ in range(world)]
+    dist.all_gather(parts, buf)
+    out = np.zeros((n_traj, width))
+    for p in parts:
+        a = p.cpu().numpy()
+        a = a[a[:, 0] >= 0]
+        out[a[:, 0].astype(int)] = a
+    return out[:, 1:].reshape(n_traj, n_frames, 8)

@@ -145,6 +145,35 @@ def _extrinsics(cfg):
     return R_b2c, t_c_b
 
 
+def _trajectory(spec: SynthSpec, base):
+    """The analytic trajectory of a sequence (depends on the seed, the config's extrinsics and the stops only; draws
+    nothing from the random stream)."""
+    k = spec.seed
+    kind = "kitti" if spec.config == "kitti_odom" else "euroc"
+    R_b2c, _ = _extrinsics(base)
+    return Trajectory(kind=kind, speed=1.0 + 0.05 * ((k * 7) % 5), phase=0.37 * k,
+                      amp=1.0 + 0.03 * (k % 4), R_b2c=R_b2c, stops=tuple(spec.stops))
+
+
+def truth_states(spec: SynthSpec, times):
+    """Ground truth of the sequence `spec` at arbitrary times, as (len(times), 17) records in the layout of the filter's
+    state records: t, p (3), q xyzw (4), v (3), b_g (3), b_a (3) -- the biases are the spec's constant true biases.
+    At an image stamp p and q are exactly the sequence's `gt` entry."""
+    base = configs.make(spec.config, **spec.overrides)
+    traj = _trajectory(spec, base)
+    times = np.asarray(times, dtype=float).reshape(-1)
+    out = np.zeros((len(times), 17))
+    for i, t in enumerate(times):
+        p, R, v, _, _ = traj.kinematics(float(t))
+        out[i, 0] = t
+        out[i, 1:4] = p
+        out[i, 4:8] = _quat_xyzw(R)
+        out[i, 8:11] = v
+        out[i, 11:14] = spec.gyro_bias
+        out[i, 14:17] = spec.acc_bias
+    return out
+
+
 def make_sequence(spec: SynthSpec):
     """Returns dict(cfg, imu (n,7), frames [(t, feats (k,9))], gt [(t,p,q)], init)."""
     k = spec.seed
@@ -155,8 +184,7 @@ def make_sequence(spec: SynthSpec):
     img_dt = 1.0 / float(base["pub_frequency"])
     dt_imu = 1.0 / imu_rate
     R_b2c, t_c_b = _extrinsics(base)
-    traj = Trajectory(kind=kind, speed=1.0 + 0.05 * ((k * 7) % 5), phase=0.37 * k,
-                      amp=1.0 + 0.03 * (k % 4), R_b2c=R_b2c, stops=tuple(spec.stops))
+    traj = _trajectory(spec, base)
     fx, fy = base["intrinsics"]["fx"], base["intrinsics"]["fy"]
     cx, cy = base["intrinsics"]["cx"], base["intrinsics"]["cy"]
     x_min, x_max = -cx / fx, (base["resolution_width"] - cx) / fx
