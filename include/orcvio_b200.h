@@ -278,24 +278,23 @@ int orcvio_triangulate(const double* cam_R, const double* cam_t, int n_clones, c
                        int* out_status, int* out_iters, double* out_cost);
 
 /* Stages 1,2,4,5 on one frozen window ("stack -> compress -> update", SURVEY 8d):
- * triangulate every feature, Jacobian + nullspace + gate, QR compression, EKF update of
- * (state, P).  clone_R/clone_p: body poses; P: D x D with D = 22 + 6 n_clones.
- * flags: bit0 use_larvio, bit1 use_left_perturbation, bit2 discard_large_update.  Experimental
- * selectors: bit3 replaces the QR compression by the normal-equation (information) form (then
- * R_thin receives G = H^T H and r_thin receives b = H^T r; R^T R == G either way; NOT parity-safe
- * for ill-conditioned priors, see DESIGN.md), bit4 forces the CTA-level QR of qr_kernel.cu.
+ * triangulate every feature, Jacobian + nullspace + gate, compression in the whitened form,
+ * EKF update of (state, P).  clone_R/clone_p: body poses; P: D x D with D = 22 + 6 n_clones.
+ * flags: bit0 use_larvio, bit1 use_left_perturbation, bit2 discard_large_update; any other bit
+ * set is rejected with ORCVIO_ERR_ARG (the same flags, and the same check, for
+ * orcvio_measurement_jacobians and orcvio_frame_create, which returns NULL).
  * Outputs (any may be NULL): P_out, delta_x (D), status per feature (bit0 tri valid, bit1
- * gate pass), gamma per feature, positions, R_thin (6N x 6N column-major) and r_thin (6N),
- * updated clone poses (N x 12).  timings_us[8]: device time per stage measured with CUDA
- * events (tri, jac+gate, qr tiles, qr chain, update, total) when non-NULL. */
+ * gate pass), gamma per feature, positions, updated clone poses (N x 12).  timings_us[8]:
+ * device time per stage measured with CUDA events (tri, jac+gate, A = H' L, A^T A + Cholesky
+ * of W, posterior, total) when non-NULL. */
 int orcvio_snapshot_update(const double* clone_R, const double* clone_p, int n_clones,
                            const double* R_b2c, const double* t_c_b, const double* P_in,
                            const int* feat_off, const int* obs_clone, const double* obs_z, int n_feat,
                            int flags, double noise_feature_var, double chi2_p,
                            double translation_threshold, double cost_threshold,
                            double init_final_dist_threshold, double* P_out, double* delta_x,
-                           int* status, double* gamma, double* positions, double* R_thin,
-                           double* r_thin, double* clone_out, float* timings_us, int repeat);
+                           int* status, double* gamma, double* positions, double* clone_out,
+                           float* timings_us, int repeat);
 
 /* Persistent form of orcvio_snapshot_update for a stream of frames (no allocation per call):
  * the same stages 1,2,4,5 -- removeLostFeatures' "stack -> compress -> update" chain,

@@ -109,7 +109,7 @@ def lib():
                                      C.c_double, dp, ip, ip, dp]
     L.orcvio_snapshot_update.argtypes = [dp, dp, C.c_int, dp, dp, dp, ip, ip, dp, C.c_int, C.c_int,
                                          C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
-                                         dp, dp, ip, dp, dp, dp, dp, dp, C.POINTER(C.c_float), C.c_int]
+                                         dp, dp, ip, dp, dp, dp, C.POINTER(C.c_float), C.c_int]
     L.orcvio_measurement_jacobians.argtypes = [dp, dp, C.c_int, dp, dp, dp, ip, ip, dp, C.c_int, C.c_int,
                                                dp, dp, dp, dp]
     L.orcvio_object_residuals.argtypes = [dp, C.c_int, dp, dp, dp, C.c_int, dp, dp, C.c_int, dp, dp, dp,
@@ -884,16 +884,15 @@ def snapshot_update(snap, flags=0, noise_var=None, chi2_p=0.95, translation_thre
     obs_z = _f64(snap["obs_z"]).reshape(-1, 2)
     nf = len(feat_off) - 1
     out = dict(P=np.zeros((D, D), order="F"), delta_x=np.zeros(D), status=np.zeros(nf, dtype=np.int32),
-               gamma=np.zeros(nf), positions=np.zeros((nf, 3)), R_thin=np.zeros((6 * N, 6 * N), order="F"),
-               r_thin=np.zeros(6 * N), clones=np.zeros((N, 12)), timings_us=np.zeros(8, dtype=np.float32))
+               gamma=np.zeros(nf), positions=np.zeros((nf, 3)), clones=np.zeros((N, 12)),
+               timings_us=np.zeros(8, dtype=np.float32))
     if noise_var is None:
         noise_var = float(snap["cfg"]["noise_feature"]) ** 2
     rc = L.orcvio_snapshot_update(
         _dp(clone_R), _dp(clone_p), N, _dp(Rbc), _dp(tcb), _dp(P), _ip(feat_off), _ip(obs_clone), _dp(obs_z),
         nf, flags, noise_var, chi2_p, translation_threshold, cost_threshold, init_final_dist_threshold,
         _dp(out["P"]), _dp(out["delta_x"]), _ip(out["status"]), _dp(out["gamma"]), _dp(out["positions"]),
-        _dp(out["R_thin"]), _dp(out["r_thin"]), _dp(out["clones"]),
-        out["timings_us"].ctypes.data_as(C.POINTER(C.c_float)), repeat)
+        _dp(out["clones"]), out["timings_us"].ctypes.data_as(C.POINTER(C.c_float)), repeat)
     if rc != 0:
         raise RuntimeError(f"orcvio_snapshot_update failed: {rc}")
     return out

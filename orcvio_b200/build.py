@@ -22,8 +22,7 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relax
 SOURCES = {
     "tri_kernel.cu": ["--fmad=false"],
     "jac_kernel.cu": [],
-    "qr_kernel.cu": [],
-    "update_kernel.cu": [],
+    "project_kernel.cu": [],
     "info_kernel.cu": [],
     "peak_kernel.cu": [],
     "prop_kernel.cu": [],

@@ -187,7 +187,7 @@ class Batch {
 
   struct PhaseWork;
   // Stage-level entry on a frozen window (orcvio_triangulate / orcvio_measurement_jacobians /
-  // orcvio_snapshot_update): loads the window into filter 0 and runs tri -> jac -> qr -> update.
+  // orcvio_snapshot_update): loads the window into filter 0 and runs tri -> jac -> compression + update.
   struct SnapshotIO {
     const double* clone_R = nullptr; const double* clone_p = nullptr;   // body poses (or camera poses)
     bool poses_are_camera = false;
@@ -197,13 +197,12 @@ class Batch {
     const double* positions_in = nullptr;   // when given: skip triangulation, use these
     const int* feat_off = nullptr; const int* obs_clone = nullptr; const double* obs_z = nullptr;
     int n_feat = 0;
-    int stages = 0;                         // bit0 tri, bit1 jac+gate, bit2 qr+update
+    int stages = 0;                         // bit0 tri, bit1 jac+gate, bit2 compression+update
     bool early_prior = false;               // start k_chol_prior as soon as P is uploaded (end-to-end call)
     int repeat = 1;
     double* P_lead9 = nullptr;               // leading 9 x 9 block of the posterior (what getPpose / getPvel read)
     double* P_out = nullptr; double* delta_x = nullptr; int* status = nullptr; double* gamma = nullptr;
-    double* positions = nullptr; double* R_thin = nullptr; double* r_thin = nullptr;
-    double* clone_out = nullptr; float* timings_us = nullptr; int* iters = nullptr; double* cost = nullptr;
+    double* positions = nullptr; double* clone_out = nullptr; float* timings_us = nullptr; int* iters = nullptr; double* cost = nullptr;
     double* raw_Hx = nullptr; double* raw_He = nullptr; double* raw_Hf = nullptr; double* raw_r = nullptr;
   };
   int run_snapshot(const SnapshotIO& io);
@@ -224,8 +223,6 @@ class Batch {
   }
   void override_noise(double sigma2, double chi2_p);
   void override_flags(int flags) { flags_ = flags; }
-  void set_compress_qr(bool on) { compress_qr_ = on; }
-  bool compress_qr() const { return compress_qr_; }
 
   // stage 3, filter side (objects.cu)
   int construct_object_jacobians(int fi, const double* jac_sensor, int rows, const double* timestamps, int n_ts,
@@ -262,7 +259,6 @@ class Batch {
   std::vector<FilterHost> f_;
   cudaStream_t stream_ = nullptr, stream2_ = nullptr;
   cudaEvent_t ev_fork_ = nullptr, ev_join_ = nullptr, ev_ls_ = nullptr, ev_block_ = nullptr;
-  bool compress_qr_ = false;          // true: QR tiles + chain (qr_kernel.cu); false: whitened form (info_kernel.cu)
   double *dAmat_ = nullptr, *dPart_ = nullptr;
   size_t amat_cap_ = 0, part_cap_ = 0;
   double* dLs_ = nullptr;
@@ -275,15 +271,11 @@ class Batch {
   // device state
   double *dP_ = nullptr, *dImu_ = nullptr, *dClones_ = nullptr, *dFpos_ = nullptr;
   long long* dFgen_ = nullptr;
-  double *dR_ = nullptr, *dRthin_ = nullptr, *dT_ = nullptr, *dS_ = nullptr, *dYv_ = nullptr, *dDx_ = nullptr;
+  double *dT_ = nullptr, *dS_ = nullptr, *dYv_ = nullptr, *dDx_ = nullptr;
   double* dChi2_ = nullptr;
-  double* dFront_ = nullptr;
-  size_t front_stride_ = 0;
-  int* dErr_ = nullptr;
-  int* hErrPin_ = nullptr;             // pinned twin of dErr_
   // growable device scratch
-  double *dHblk_ = nullptr, *dRblk_ = nullptr, *dTileOut_ = nullptr;
-  size_t hblk_cap_ = 0, rblk_cap_ = 0, tileout_cap_ = 0;
+  double *dHblk_ = nullptr, *dRblk_ = nullptr;
+  size_t hblk_cap_ = 0, rblk_cap_ = 0;
   int* dStatus_ = nullptr;
   double* dGamma_ = nullptr;
   size_t cand_cap_ = 0;
@@ -325,7 +317,7 @@ class Batch {
   void prereserve();
   void wait_stream();
   void upload_blob();
-  void ensure_scratch(size_t n_cand, size_t hblk, size_t rblk, size_t tileout);
+  void ensure_scratch(size_t n_cand, size_t hblk, size_t rblk);
   void run_phase(PhaseWork& w, int phase);
   void stage_phase(PhaseWork& w);
   void stage_pack(PhaseWork& w);

@@ -416,9 +416,7 @@ static std::unique_ptr<Batch> make_snapshot_batch(int n_clones, int flags, doubl
   p.feature_translation_threshold = tthr;
   p.feature_cost_threshold = cthr;
   p.init_final_dist_threshold = ithr;
-  std::unique_ptr<Batch> b(new Batch(p, 1));
-  if (flags & 8) b->set_compress_qr(true);     // bit3: QR tiles + chain (qr_kernel.cu) instead of the whitened form
-  return b;
+  return std::unique_ptr<Batch>(new Batch(p, 1));
 }
 
 int orcvio_syrk_plan_probe(int arows, const int* jrow0, int n_clones, int cta_budget, int* out) {
@@ -467,8 +465,8 @@ int orcvio_snapshot_update(const double* clone_R, const double* clone_p, int n_c
                            const double* obs_z, int n_feat, int flags, double noise_feature_var, double chi2_p,
                            double translation_threshold, double cost_threshold,
                            double init_final_dist_threshold, double* P_out, double* delta_x, int* status,
-                           double* gamma, double* positions, double* R_thin, double* r_thin, double* clone_out,
-                           float* timings_us, int repeat) {
+                           double* gamma, double* positions, double* clone_out, float* timings_us, int repeat) {
+  if (flags & ~7) return ORCVIO_ERR_ARG;         // flag bits 0-2 only
   auto b = make_snapshot_batch(n_clones, flags, noise_feature_var, chi2_p, translation_threshold,
                                cost_threshold, init_final_dist_threshold);
   if (!b->ok()) return ORCVIO_ERR_NO_DEVICE;
@@ -478,7 +476,7 @@ int orcvio_snapshot_update(const double* clone_R, const double* clone_p, int n_c
   io.feat_off = feat_off; io.obs_clone = obs_clone; io.obs_z = obs_z; io.n_feat = n_feat;
   io.stages = 7; io.repeat = repeat;
   io.P_out = P_out; io.delta_x = delta_x; io.status = status; io.gamma = gamma; io.positions = positions;
-  io.R_thin = R_thin; io.r_thin = r_thin; io.clone_out = clone_out; io.timings_us = timings_us;
+  io.clone_out = clone_out; io.timings_us = timings_us;
   return b->run_snapshot(io);
 }
 
@@ -486,6 +484,7 @@ int orcvio_measurement_jacobians(const double* clone_R, const double* clone_p, i
                                  const double* t_c_b, const double* positions, const int* feat_off,
                                  const int* obs_clone, const double* obs_z, int n_feat, int flags, double* Hx,
                                  double* He, double* Hf, double* r) {
+  if (flags & ~7) return ORCVIO_ERR_ARG;         // flag bits 0-2 only
   auto b = make_snapshot_batch(n_clones, flags, 1.0, 0.95, -1.0, 1e300, 1e300);
   if (!b->ok()) return ORCVIO_ERR_NO_DEVICE;
   const int D = ORCVIO_LEG + 6 * n_clones;
@@ -513,7 +512,7 @@ struct orcvio_frame {
 orcvio_frame* orcvio_frame_create(int n_clones_cap, int flags, double noise_feature_var, double chi2_p,
                                   double translation_threshold, double cost_threshold,
                                   double init_final_dist_threshold) {
-  if (n_clones_cap < 1 || n_clones_cap > 31) return nullptr;
+  if (n_clones_cap < 1 || n_clones_cap > 31 || (flags & ~7)) return nullptr;
   orcvio_frame* f = new orcvio_frame();
   f->b = make_snapshot_batch(n_clones_cap, flags, noise_feature_var, chi2_p, translation_threshold,
                              cost_threshold, init_final_dist_threshold);

@@ -1,5 +1,5 @@
 // incrementState_IMUCam (reference src/orcvio.cpp:4468-4567) as a CTA-wide device routine shared by
-// every kernel that ends in a state increment (k_dx, k_apply_dx, k_zupt).
+// every kernel that ends in a state increment (k_pinfo, k_zupt).
 #pragma once
 #include "kernels.h"
 

@@ -1,4 +1,4 @@
-// Stages 4+5, default path -- measurement compression in the whitened ("A") form and the EKF
+// Stages 4+5 -- measurement compression in the whitened ("A") form and the EKF
 // update written around it.
 //
 // Reference: OrcVIO::measurementUpdate_msckf / measurementUpdate_hybrid
@@ -6,8 +6,8 @@
 // compressed with SuiteSparseQR to H_thin = (Q^T H).topRows, then
 //     S = H P H^T + s^2 I,  K = P H^T S^-1,  dx = K r,  P <- (I - K H) P,  P <- (P + P^T)/2.
 // On a GPU the QR is a chain of ~6N dependent Householder steps per clone block (pure latency:
-// qr_kernel.cu, kept as the selectable alternative, needs milliseconds on the stress frame).
-// This path produces the same posterior from massively parallel dense kernels:
+// milliseconds on the stress frame, DESIGN.md).  This file produces the same posterior from
+// massively parallel dense kernels:
 //   P = F F^T                 Cholesky of the prior in the order [clones | IMU]  (k_chol_prior,
 //                             on a second stream, overlapped with triangulation + Jacobians);
 //                             F_1 = first 6N columns, F_2 = the rest, L = F[clones, clones]
@@ -142,7 +142,7 @@ __device__ __forceinline__ int aform_stride(int W) {          // smallest stride
   return (k4 & 7) == 4 ? k4 : k4 + 4;
 }
 
-__global__ void __launch_bounds__(AF_THREADS, 3) k_aform(QrArgs a, const double* FT_all, size_t t_stride, int ldt,
+__global__ void __launch_bounds__(AF_THREADS, 3) k_aform(AformArgs a, const double* FT_all, size_t t_stride, int ldt,
                                                       double* Amat, int lda, int* tile_rows) {
   extern __shared__ double smem[];
   __shared__ int rowbase[256];
@@ -973,7 +973,7 @@ void launch_info_prior(const UpdArgs& u, const InfoBufs& ib, int max_N, cudaStre
   if (ib.ls_done) cudaEventRecord(ib.ls_done, s2);
 }
 
-void launch_info_update(const QrArgs& q, const UpdArgs& u, const InfoBufs& ib, int n_tiles, int max_tile_rows,
+void launch_info_update(const AformArgs& q, const UpdArgs& u, const InfoBufs& ib, int n_tiles, int max_tile_rows,
                         int max_w_blk, int max_N, cudaStream_t s, cudaStream_t s2, cudaEvent_t fork,
                         cudaEvent_t join, cudaEvent_t mid1, cudaEvent_t mid2, int* launches, bool prior_in_flight,
                         cudaEvent_t mid_syrk, cudaEvent_t prior_t0, cudaEvent_t prior_t1, int max_E,

@@ -96,14 +96,13 @@ struct JacArgs {
   double* raw_Hx; double* raw_He; double* raw_Hf; double* raw_r;
 };
 
-// Row tile of the stacked Jacobian, reduced to an upper-trapezoidal factor by one CTA.
+// Row tile of the stacked Jacobian: one CTA of k_aform forms its rows of the whitened matrix A.
 struct Tile {
   int filter;
   int cand_begin, cand_end;      // candidates (sorted by s_blk inside a filter)
   int rows;                      // rows if every candidate passes the gate
   int c0_blk, c1_blk;            // clone-block window [c0, c1)
-  int out_off;                   // offset (doubles) of its W x (W+1) output
-  int arow;                      // first row of this tile in the stacked A matrix (whitened form)
+  int arow;                      // first row of this tile in the stacked A matrix
 };
 
 struct FilterWork {              // per filter, per update
@@ -118,7 +117,7 @@ struct FilterWork {              // per filter, per update
   int dense_rows;                // dense rows behind the tiles' rows (hybrid mode: rows of the EKF-SLAM features)
 };
 
-struct QrArgs {
+struct AformArgs {               // inputs of k_aform: the gated rows of every tile
   const Cand* cand; const int* status;
   const int* status_f;                           // != nullptr: status by feature slot (direct-mode Jacobian pass)
   // direct mode (end-to-end frame call): no candidate records on the device at all -- order_f[c] is the feature
@@ -126,20 +125,16 @@ struct QrArgs {
   const int* order_f; const int* feat_off; const int* rowoff_f; const int* hblkoff_f; const int* sblk_f;
   const int* eblk_f;
   const double* hblk; const double* rblk;
-  const Tile* tiles; int n_tiles;
-  double* tile_out;
-  const FilterWork* fw; int n_filters;
-  double* Rm; double* rthin; size_t r_stride; int ldr;   // per-filter R (n x n) and r_thin
-  double* front_scratch; size_t front_stride;            // global fallback for wide fronts
-  int* err;                                              // device error flag (front overflow)
+  const Tile* tiles;
+  const FilterWork* fw;
 };
 
 struct UpdArgs {
   const FilterWork* fw; int n_filters;
   double* P; size_t p_stride; int ldp;
-  double* Rm; double* rthin; size_t r_stride; int ldr;
+  size_t r_stride; int ldr;                              // per-filter stride and ld of S
   double* T; double* S; size_t t_stride; int ldt;        // T: n x D, S: n x n (ld = ldr)
-  double* yv;                                            // L^-1 r_thin, per filter (ldr)
+  double* yv;                                            // C^-1 v, per filter (ldr)
   double* imu; double* clones; size_t clone_stride;
   double* dx; int lddx;                                  // delta_x log per filter
   int flags; double sigma2;
@@ -311,11 +306,7 @@ inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 
 void launch_triangulate(const TriArgs& a, cudaStream_t s);
 void launch_jac_gate(const JacArgs& small_list, const JacArgs& large_list, cudaStream_t s);
-void launch_qr(const QrArgs& a, size_t tile_smem_doubles, int max_w_blk, int max_n, cudaStream_t s,
-               int* launches, cudaEvent_t mid);
-void launch_update(const UpdArgs& a, int max_N, cudaStream_t s, int* launches);
-void launch_update_tail(const UpdArgs& a, int max_N, cudaStream_t s);   // k_trsm + k_apply_dx
-void launch_info_update(const QrArgs& q, const UpdArgs& u, const InfoBufs& ib, int n_tiles, int max_tile_rows,
+void launch_info_update(const AformArgs& q, const UpdArgs& u, const InfoBufs& ib, int n_tiles, int max_tile_rows,
                         int max_w_blk, int max_N, cudaStream_t s, cudaStream_t s2, cudaEvent_t fork,
                         cudaEvent_t join, cudaEvent_t mid1, cudaEvent_t mid2, int* launches,
                         bool prior_in_flight = false, cudaEvent_t mid_syrk = nullptr, cudaEvent_t prior_t0 = nullptr,
@@ -367,9 +358,8 @@ void launch_remove(const RemoveArgs& a, cudaStream_t s);
 void launch_zupt(const ZuptArgs& a, cudaStream_t s);
 
 // tile sizing shared by host tiler and kernels
-constexpr int QR_THREADS = 256;
-constexpr int QR_SMEM_BYTES = 200 * 1024;
-constexpr int AFORM_TILE_ROWS = 64;     // row cap of a tile of the whitened-form path
+constexpr int QR_THREADS = 256;         // CTA of k_project_dense; candidates per tile (k_aform's rowbase[256])
+constexpr int AFORM_TILE_ROWS = 64;     // row cap of a tile
 // Split-K plan of W = s^2 I + A^T A for ONE filter (k_syrk).  A^T A is computed as 64 x 64 tiles (I <= J) over
 // chunks of rows; column tile J of A is structurally zero above row jrow0[J] (features are sorted by first
 // clone and A = H' L with L lower triangular), so pair (I, J) only covers rows [jrow0[J], arows).  The plan
@@ -421,11 +411,6 @@ __host__ __device__ inline SyrkPlan syrk_plan(const FilterWork& fw, int cta_budg
   p.kc = kc;
   p.kcd = syrk_kcd(kc);
   return p;
-}
-inline int qr_tile_rows_cap(int w_cols) {                // rows that fit beside (w_cols+1) columns
-  int ld = w_cols + 2;
-  int cap = QR_SMEM_BYTES / 8 / ld;
-  return cap;
 }
 
 }  // namespace ob

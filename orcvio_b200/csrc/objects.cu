@@ -310,7 +310,7 @@ int Batch::object_update(int fi, const double* Hx, const double* Hf, const doubl
   UpdArgs ua{};
   ua.fw = dFw; ua.n_filters = 1;
   ua.P = dP_ + (size_t)fi * ldp_ * ldp_; ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
-  ua.Rm = dR_ + (size_t)fi * r_stride; ua.rthin = dRthin_ + (size_t)fi * ldr_; ua.r_stride = r_stride; ua.ldr = ldr_;
+  ua.r_stride = r_stride; ua.ldr = ldr_;
   ua.T = dT_ + (size_t)fi * nmax_ * ldt_; ua.S = dS_ + (size_t)fi * r_stride;
   ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
   ua.yv = dYv_ + (size_t)fi * ldr_;
@@ -445,7 +445,7 @@ int Batch::dense_update(const double* P_in, int D, const double* H, const double
   UpdArgs ua{};
   ua.fw = dFw.as<FilterWork>(); ua.n_filters = 1;
   ua.P = dP_; ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
-  ua.Rm = dR_; ua.rthin = dRthin_; ua.r_stride = r_stride; ua.ldr = ldr_;
+  ua.r_stride = r_stride; ua.ldr = ldr_;
   ua.T = dT_; ua.S = dS_; ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
   ua.yv = dYv_;
   ua.imu = dImu_; ua.clones = dClones_; ua.clone_stride = (size_t)Ncap_ * CL_STRIDE;

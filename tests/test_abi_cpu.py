@@ -62,6 +62,19 @@ def test_no_device_means_no_compute():
     assert vio.initialize() is False
 
 
+def test_frozen_window_entries_reject_unknown_flag_bits():
+    """Flag bits above bit 2 are refused before any device work, so a caller that sets one is not silently given the
+    default update."""
+    L = api.lib()
+    ERR_ARG = -2                                            # ORCVIO_ERR_ARG
+    for flags in (8, 16):
+        assert L.orcvio_snapshot_update(None, None, 10, None, None, None, None, None, None, 0, flags, 1e-4, 0.95,
+                                        -1.0, 1e-3, 100.0, None, None, None, None, None, None, None, 1) == ERR_ARG
+        assert L.orcvio_measurement_jacobians(None, None, 10, None, None, None, None, None, None, 0, flags,
+                                              None, None, None, None) == ERR_ARG
+        assert not L.orcvio_frame_create(10, flags, 1e-4, 0.95, -1.0, 1e-3, 100.0)
+
+
 def test_syrk_plan_covers_every_row_once_and_fits_the_budget():
     """Host logic of the staircase split-K plan (csrc/kernels.h syrk_plan), no device involved: every tile pair
     (I <= J) covers exactly the rows [jrow0[J], arows) in whole chunks of kc rows (kcd = 13/8 kc for a diagonal pair, which
