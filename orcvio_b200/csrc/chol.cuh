@@ -14,9 +14,12 @@
 //     of mma.m8n8k4 and -- with the k index of the MMA permuted to (even columns | odd columns), the same
 //     permutation on both operands -- its A / B operand: updates need no staging buffer at all;
 //   * warp 0 is the CHAIN warp.  In step q it factors the diagonal tile (q, q) (8-pivot L D L^T elimination, one
-//     row per lane), publishes the block, solves tile (q+1, q) against it and applies that panel to tile
-//     (q+1, q+1) with one MMA pair -- then goes on to step q+1.  It waits for exactly one tile per step, with a
-//     whole factorisation of slack;
+//     row per lane, every 8-lane segment redundantly) and publishes the block for the other warps.  Lanes 8..15
+//     then solve the rows of tile (q+1, q) in registers: the block's entries are the ones the elimination's
+//     shuffles already brought in, nothing is read back from shared memory.  The solved rows reach every lane by
+//     shuffles as the operand of the MMA pair that applies the panel to tile (q+1, q+1), and the updated tile is
+//     shuffled into row-per-lane form for step q+1 without a store and reload.  It waits for exactly one tile per
+//     step, with a whole factorisation of slack;
 //   * warp 4 is the FRONTIER warp (same scheduler as the chain warp, which is otherwise kept free of MMA
 //     work): in step q it solves tile (q+2, q) and brings tile (q+2, q+1) up to date with panel q -- the tile the
 //     chain warp needs one step later -- without waiting for anybody's bulk work;
@@ -100,8 +103,21 @@ __device__ __forceinline__ void chol_set_flag(volatile int* f, int v) {
   __syncwarp();
   if ((threadIdx.x & 31) == 0) *f = v;
 }
-// one row of a tile column against the published diagonal block: x <- x L_d^-T (update form: full ILP across
-// the remaining columns)
+// x <- x L_d^-T for one row held in registers (update form: full ILP across the remaining columns); dl = strictly
+// lower part of the factored diagonal block, di = 1 / its diagonal (0 for skipped pivots).  The chain warp and the
+// shared-memory row solve below both go through this, so they round alike.
+__device__ __forceinline__ void chol_solve_regs(double (&x)[CHB], const double (&dl)[CHB][CHB], const double (&di)[CHB],
+                                                int nb) {
+#pragma unroll
+  for (int c = 0; c < CHB; ++c) {
+    if (c >= nb) x[c] = 0.0;
+    x[c] *= di[c];
+#pragma unroll
+    for (int s = c + 1; s < CHB; ++s) x[s] -= x[c] * dl[s][c];
+  }
+}
+
+// one row of a tile column against the published diagonal block
 __device__ __forceinline__ void chol_solve_row(double* __restrict__ xt, const double (*dblk)[CHB], const double* dinv,
                                                int nb) {
   double dl[CHB][CHB], di[CHB];
@@ -126,13 +142,7 @@ __device__ __forceinline__ void chol_solve_row(double* __restrict__ xt, const do
     x[c] = t.x;
     x[c + 1] = t.y;
   }
-#pragma unroll
-  for (int c = 0; c < CHB; ++c) {
-    if (c >= nb) x[c] = 0.0;
-    x[c] *= di[c];
-#pragma unroll
-    for (int s = c + 1; s < CHB; ++s) x[s] -= x[c] * dl[s][c];
-  }
+  chol_solve_regs(x, dl, di, nb);
 #pragma unroll
   for (int c = 0; c < CHB; c += 2) *reinterpret_cast<double2*>(xt + c) = make_double2(x[c], x[c + 1]);
 }
@@ -214,19 +224,20 @@ __device__ void cta_cholesky(double* __restrict__ A, CholShared& cs, const doubl
   if (warp == 0) {
     // ------------------------------------------------ chain warp
     const int a = lane & 7;                                    // row of the diagonal tile (four redundant copies)
+    const bool solver = (lane >> 3) == 1;                      // lanes 8..15: row a of tile (q+1, q)
+    double d[CHB];                                             // row a of the diagonal tile; from step 1 on, the
+#pragma unroll                                                 // previous step leaves it here (it is never stored)
+    for (int b = 0; b < CHB; b += 2) {
+      const double2 t = *reinterpret_cast<const double2*>(A + a * 8 + b);
+      d[b] = t.x;
+      d[b + 1] = t.y;
+    }
     for (int q = 0; q < Tm; ++q) {
       const int k0 = q * CHB;
       const int nb = min(CHB, m - k0);
       const bool below = (q + 1 < Tr);
       if (PROF && lane == 0) prof[q * 8 + 0] = clock64();
       double* dt = A + (size_t)chol_tile(q, q, Tm) * 64 + a * 8;
-      double d[CHB];
-#pragma unroll
-      for (int b = 0; b < CHB; b += 2) {
-        const double2 t = *reinterpret_cast<const double2*>(dt + b);
-        d[b] = t.x;
-        d[b + 1] = t.y;
-      }
       // columns >= nb do not exist (last, partial block); rows nb..7 of the diagonal tile are then carried rows and
       // are eliminated along with the pivots
 #pragma unroll
@@ -237,7 +248,9 @@ __device__ void cta_cholesky(double* __restrict__ A, CholShared& cs, const doubl
       //   into w = u / pivot) -> FMA into the next pivot;
       // thresholds are preloaded, rejected pivots are handled by selects.  The 8 rsqrt that turn the
       // result into L = U D^-1/2 run afterwards, in parallel.
-      double thr[CHB], ivs[CHB];
+      // The shuffles of pivot c bring in column c of rows b > c in its final unscaled form: kept in dl, they give the
+      // strictly lower part of the factored block (the same products as the row scaling below) with no further traffic.
+      double thr[CHB], ivs[CHB], dl[CHB][CHB];
 #pragma unroll
       for (int c = 0; c < CHB; ++c) thr[c] = (tol != nullptr && c < nb) ? tol[k0 + c] : 0.0;
 #pragma unroll
@@ -257,6 +270,7 @@ __device__ void cta_cholesky(double* __restrict__ A, CholShared& cs, const doubl
 #pragma unroll
         for (int b = c + 1; b < CHB; ++b) {
           const double ub = __shfl_sync(0xffffffffu, u, b, 8);
+          dl[b][c] = ub;
           d[b] = fma(-w, ub, d[b]);                           // meaningful for rows below row b
         }
       }
@@ -266,7 +280,12 @@ __device__ void cta_cholesky(double* __restrict__ A, CholShared& cs, const doubl
         ivs[c] = (ivs[c] > 0.0) ? rs : 0.0;
         d[c] *= ivs[c];
       }
-      __syncwarp();   // lanes 8..31 hold redundant copies of the rows: their reads of the tile are done before it is rewritten
+      // the block as published in dblk: rows >= nb are zero
+#pragma unroll
+      for (int c = 0; c < CHB; ++c)
+#pragma unroll
+        for (int s = c + 1; s < CHB; ++s) dl[s][c] = (s < nb) ? dl[s][c] * ivs[c] : 0.0;
+      __syncwarp();   // lanes 8..31 hold redundant copies of the rows: their reads of tile (0, 0) are done before it is rewritten
       if (lane < CHB) {
         const bool tri = (a < nb);                             // triangle row: entries right of the diagonal are zeros
 #pragma unroll
@@ -288,19 +307,40 @@ __device__ void cta_cholesky(double* __restrict__ A, CholShared& cs, const doubl
         // tile (q+1, q): carries panels 0..q-1 once the frontier warp has finished its step q-1
         if (q > 0) chol_wait_flag(&cs.flag_w2, q);
         if (PROF && lane == 0) prof[q * 8 + 2] = clock64();
-        if (lane < CHB && CHB * (q + 1) + lane < mrows)
-          chol_solve_row(A + (size_t)chol_tile(q + 1, q, Tm) * 64 + lane * 8, cs.dblk[q & 1], cs.dinv[q & 1], nb);
+        double* xt = A + (size_t)chol_tile(q + 1, q, Tm) * 64 + a * 8;
+        double x[CHB];
+#pragma unroll
+        for (int c = 0; c < CHB; c += 2) {
+          const double2 t = solver ? *reinterpret_cast<const double2*>(xt + c) : make_double2(0.0, 0.0);
+          x[c] = t.x;
+          x[c + 1] = t.y;
+        }
+        if (solver && CHB * (q + 1) + a < mrows) {
+          chol_solve_regs(x, dl, ivs, nb);                     // ivs = the published dinv
+#pragma unroll
+          for (int c = 0; c < CHB; c += 2) *reinterpret_cast<double2*>(xt + c) = make_double2(x[c], x[c + 1]);
+        }
         chol_set_flag(&cs.flag_c2, q + 1);
         if (q + 1 < Tm) {
-          // tile (q+1, q+1) -= L(q+1, q) L(q+1, q)^T on top of its bulk update (panels < q, bulk step q-1)
+          // tile (q+1, q+1) -= L(q+1, q) L(q+1, q)^T on top of its bulk update (panels < q, bulk step q-1).  The
+          // operand chunk of this lane (row lane / 4, columns 2 (lane % 4) + 0, 1) comes from solver lane 8 + lane / 4.
+          double2 l = make_double2(0.0, 0.0);
+#pragma unroll
+          for (int j = 0; j < CHB / 2; ++j) {
+            const double lx = __shfl_sync(0xffffffffu, x[2 * j], CHB + (lane >> 2));
+            const double ly = __shfl_sync(0xffffffffu, x[2 * j + 1], CHB + (lane >> 2));
+            if ((lane & 3) == j) l = make_double2(lx, ly);
+          }
           if (q > 0) chol_wait_flag(&cs.flag_w3, q);
-          const double2 l = A2[(size_t)chol_tile(q + 1, q, Tm) * 32 + lane];
-          double2* cp = A2 + (size_t)chol_tile(q + 1, q + 1, Tm) * 32 + lane;
-          double2 cv = *cp;
+          double2 cv = A2[(size_t)chol_tile(q + 1, q + 1, Tm) * 32 + lane];
           dmma884(cv.x, cv.y, -l.x, l.x);
           dmma884(cv.x, cv.y, -l.y, l.y);
-          *cp = cv;
-          __syncwarp();
+          // row a of the updated tile for step q+1: its four chunks are in lanes 4a .. 4a+3
+#pragma unroll
+          for (int j = 0; j < CHB / 2; ++j) {
+            d[2 * j] = __shfl_sync(0xffffffffu, cv.x, 4 * a + j);
+            d[2 * j + 1] = __shfl_sync(0xffffffffu, cv.y, 4 * a + j);
+          }
         }
       }
       if (PROF && lane == 0) prof[q * 8 + 3] = clock64();
@@ -360,13 +400,16 @@ __device__ void cta_cholesky(double* __restrict__ A, CholShared& cs, const doubl
       }
       if (PROF && wtid == 0) prof[q * 8 + 6] = clock64();
       // ---- tile column q+2: bulk update with panels 0..q (left-looking; up to two tiles per pass and warp, two
-      // accumulators per tile so that the dependent MMA chain is a quarter of the k loop)
+      // accumulators per tile so that the dependent MMA chain is a quarter of the k loop).  Warp 0 takes only tile
+      // (q+2, q+2), which the chain warp waits for, and warp 1 only tile (q+3, q+2), which the frontier warp waits
+      // for; the other tiles go to warps 2..11.
       if (q + 2 < Tm) {
         const int tc = q + 2;
+        constexpr int NP = CHOL_BULK_WARPS - 2;
         chol_wait_flag(&cs.flag_f1, q + 1);                    // L(q+2, q): the B operand of the last k step
         const double2* pb = A2 + (size_t)chol_tile(tc, 0, Tm) * 32 + lane;
-        for (int t1 = tc + w; t1 < Tr; t1 += 2 * CHOL_BULK_WARPS) {
-          const int t2 = t1 + CHOL_BULK_WARPS;
+        for (int t1 = tc + w; t1 < Tr; t1 += (w < 2 ? Tr : 2 * NP)) {
+          const int t2 = w < 2 ? Tr : t1 + NP;
           double2* cp1 = A2 + (size_t)chol_tile(t1, tc, Tm) * 32 + lane;
           const double2* pa1 = A2 + (size_t)chol_tile(t1, 0, Tm) * 32 + lane;
           double2 c1 = *cp1, e1 = make_double2(0.0, 0.0);

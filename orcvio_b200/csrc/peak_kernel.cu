@@ -209,7 +209,7 @@ extern "C" int orcvio_chol_probe(int m, int nx, const double* A, const double* X
                                  long long* prof, int reps, float* us) {
   using namespace ob;
   if (m < 1 || m > ORCVIO_LEG + 6 * ORCVIO_MAX_OBS || nx < 0 || m + nx > CHOL_MAXR - 8 ||
-      chol_smem_doubles(m, nx) * sizeof(double) > 193 * 1024) return ORCVIO_ERR_ARG;
+      chol_smem_doubles(m, nx) * sizeof(double) > 225 * 1024) return ORCVIO_ERR_ARG;
   double *dA = nullptr, *dX = nullptr, *dL = nullptr, *dXs = nullptr;
   long long* dprof = nullptr;
   const size_t nA = (size_t)m * m, nX = (size_t)std::max(nx, 1) * m;
@@ -225,8 +225,8 @@ extern "C" int orcvio_chol_probe(int m, int nx, const double* A, const double* X
   const size_t smem = chol_smem_doubles(m, nx) * sizeof(double);
   auto kp = k_chol_probe<true>;
   auto kf = k_chol_probe<false>;
-  cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, 193 * 1024);
-  cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, 193 * 1024);
+  cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024);
+  cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024);
   kp<<<1, CHOL_THREADS, smem>>>(dA, dX, m, nx, dL, dXs, dprof);
   cudaEvent_t e0, e1;
   cudaEventCreate(&e0);
