@@ -303,7 +303,10 @@ int orcvio_snapshot_update(const double* clone_R, const double* clone_p, int n_c
  *                         host integration makes per frame;
  *   orcvio_frame_load / _run / _fetch : upload once, run the kernel chain `repeat` times on the
  *                         HBM-resident frame (each run restores the pristine window first),
- *                         device time in microseconds via CUDA events. */
+ *                         device time in microseconds via CUDA events.
+ * orcvio_frame_update and _update_pose_cov replace the resident frame: after them orcvio_frame_run
+ * and orcvio_frame_fetch return ORCVIO_ERR_ARG until the next successful orcvio_frame_load
+ * (orcvio_frame_fetch_last still returns the update's results). */
 typedef struct orcvio_frame orcvio_frame;
 orcvio_frame* orcvio_frame_create(int n_clones_cap, int flags, double noise_feature_var, double chi2_p,
                                   double translation_threshold, double cost_threshold,
@@ -324,8 +327,18 @@ int orcvio_frame_load(orcvio_frame* f, const double* clone_R, const double* clon
                       const double* R_b2c, const double* t_c_b, const double* P_in, const int* feat_off,
                       const int* obs_clone, const double* obs_z, int n_feat);
 int orcvio_frame_run(orcvio_frame* f, int repeat, float* total_us, float* stage_us6);
+/* Runs the resident chain once more, with the downloads queued, and returns its results. */
 int orcvio_frame_fetch(orcvio_frame* f, double* P_out, double* delta_x, int* status, double* gamma,
                        double* clone_out);
+/* The results the most recent orcvio_frame_run / _fetch / _update left on the device, as orcvio_frame_fetch
+ * returns them; it launches no kernel (a run that replays the CUDA graph downloads nothing, so this queues the
+ * copies and synchronises the frame's stream).  ORCVIO_ERR_ARG when f is NULL or nothing ran since the last
+ * orcvio_frame_load. */
+int orcvio_frame_fetch_last(orcvio_frame* f, double* P_out, double* delta_x, int* status, double* gamma,
+                            double* clone_out);
+/* CUDA-graph launches of the resident chain since the last orcvio_frame_load / _update (from the third
+ * orcvio_frame_run on, every run without stage times replays one graph); 0 when f is NULL. */
+long long orcvio_frame_graph_replays(orcvio_frame* f);
 long long orcvio_frame_kernel_launches(orcvio_frame* f);
 /* wall-clock split (us) of the last orcvio_frame_update: host work-list build + uploads, kernel launches,
  * wait + downloads, total -- explains the gap between the device-timed and the end-to-end figure */

@@ -130,6 +130,9 @@ def lib():
     L.orcvio_frame_load.argtypes = [vp, dp, dp, C.c_int, dp, dp, dp, ip, ip, dp, C.c_int]
     L.orcvio_frame_run.argtypes = [vp, C.c_int, fpt, fpt]
     L.orcvio_frame_fetch.argtypes = [vp, dp, dp, ip, dp, dp]
+    L.orcvio_frame_fetch_last.argtypes = [vp, dp, dp, ip, dp, dp]
+    L.orcvio_frame_graph_replays.restype = C.c_longlong
+    L.orcvio_frame_graph_replays.argtypes = [vp]
     L.orcvio_frame_kernel_launches.restype = C.c_longlong
     L.orcvio_frame_kernel_launches.argtypes = [vp]
     L.orcvio_frame_host_times.argtypes = [vp, C.POINTER(C.c_float)]
@@ -514,6 +517,7 @@ class Frame:
         if not isinstance(inp, dict) or "Rbc" not in inp:
             inp = self._inputs(inp)
         nf = len(inp["feat_off"]) - 1
+        self._keep = inp                     # (the shapes fetch_last returns)
         if out is None:
             out = self._outputs(inp["N"], nf)
         if not full_P:
@@ -575,6 +579,20 @@ class Frame:
         if rc != 0:
             raise RuntimeError(f"orcvio_frame_fetch failed: {rc}")
         return out
+
+    def fetch_last(self):
+        """What the last run (run, fetch or update) left on the device, without running the chain again."""
+        inp = self._keep
+        out = self._outputs(inp["N"], len(inp["feat_off"]) - 1)
+        rc = self._L.orcvio_frame_fetch_last(self._h, _dp(out["P"]), _dp(out["delta_x"]), _ip(out["status"]),
+                                             _dp(out["gamma"]), _dp(out["clones"]))
+        if rc != 0:
+            raise RuntimeError(f"orcvio_frame_fetch_last failed: {rc}")
+        return out
+
+    def graph_replays(self):
+        """CUDA-graph launches of the resident chain since the last load / update."""
+        return int(self._L.orcvio_frame_graph_replays(self._h))
 
     def kernel_launches(self):
         return int(self._L.orcvio_frame_kernel_launches(self._h))

@@ -2237,10 +2237,12 @@ struct Batch::SnapState {
   cudaGraphExec_t graph_exec = nullptr;
   int graph_launches = 0;          // kernels inside the graph
   int plain_runs = 0;              // uncaptured runs since the last prepare (the first ones grow the scratch buffers)
+  long long graph_replays = 0;     // launches of graph_exec since the last prepare
   void drop_graph() {
     if (graph_exec) cudaGraphExecDestroy(graph_exec);
     graph_exec = nullptr;
     plain_runs = 0;
+    graph_replays = 0;
   }
   ~SnapState() {
     drop_graph();
@@ -2652,6 +2654,7 @@ int Batch::snapshot_execute(bool download) {
                          !want_iters_ && !want_raw_;
   if (graphable && S.graph_exec) {
     CK(cudaGraphLaunch(S.graph_exec, stream_));
+    ++S.graph_replays;
     launches_ += S.graph_launches;
     S.by_feature = false;
     return ok_ ? ORCVIO_OK : ORCVIO_ERR_CUDA;
@@ -2684,6 +2687,7 @@ int Batch::snapshot_execute(bool download) {
     launches_ = launches_before;       // nothing has run yet: the capture only recorded the chain
     if (S.graph_exec) {
       CK(cudaGraphLaunch(S.graph_exec, stream_));
+      ++S.graph_replays;
       launches_ += S.graph_launches;
       return ok_ ? ORCVIO_OK : ORCVIO_ERR_CUDA;
     }
@@ -2774,6 +2778,21 @@ int Batch::snapshot_fetch(const SnapshotIO& io) {
   g_hp.done();
   return ok_ ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
+
+// Results of the most recent run as it left them on the device (a graph replay downloads nothing): queue the
+// per-candidate downloads from the buffers that run wrote, then the same fetch as after a downloading run.
+int Batch::snapshot_fetch_last(const SnapshotIO& io) {
+  if (!snap_) return ORCVIO_ERR_ARG;
+  const SnapState& S = *snap_;
+  const int nC = (int)S.w.cands.size();
+  if (nC > 0 && (io.status || io.gamma)) {
+    CK(cudaMemcpyAsync(hStatus_, S.by_feature ? dStatusF_ : dStatus_, sizeof(int) * nC, cudaMemcpyDeviceToHost, stream_));
+    CK(cudaMemcpyAsync(hGamma_, S.by_feature ? dGammaF_ : dGamma_, sizeof(double) * nC, cudaMemcpyDeviceToHost, stream_));
+  }
+  return snapshot_fetch(io);
+}
+
+long long Batch::snapshot_graph_replays() const { return snap_ ? snap_->graph_replays : 0; }
 
 // Per-stage device times (us) of the most recent snapshot_execute run with profiling on.
 void Batch::snapshot_stage_times(float* us6) {

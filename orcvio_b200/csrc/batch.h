@@ -211,6 +211,8 @@ class Batch {
   int snapshot_execute(bool download);
   int snapshot_execute_plain(bool download, bool prior_in_flight);
   int snapshot_fetch(const SnapshotIO& io);
+  int snapshot_fetch_last(const SnapshotIO& io);   // what the last run left on the device, nothing launched
+  long long snapshot_graph_replays() const;         // graph launches since the last snapshot_prepare
   void snapshot_stage_times(float* us6);
   float last_syrk_us() const { return last_syrk_us_; }     // k_syrk / k_chol_prior of the last profiled run
   float last_prior_us() const { return last_prior_us_; }

@@ -504,7 +504,8 @@ int orcvio_measurement_jacobians(const double* clone_R, const double* clone_p, i
 struct orcvio_frame {
   std::unique_ptr<Batch> b;
   cudaEvent_t e0 = nullptr, e1 = nullptr;
-  bool loaded = false;
+  bool loaded = false;                 // a frame is resident: orcvio_frame_run / _fetch may run its chain
+  bool has_result = false;             // a run since the last load / update left results for orcvio_frame_fetch_last
   float host_us[4] = {0, 0, 0, 0};     // last orcvio_frame_update: prepare, launch, wait+fetch, total (wall)
   float kern_us[2] = {0, 0};           // last profiled orcvio_frame_run: k_syrk, k_chol_prior (mean)
 };
@@ -551,6 +552,10 @@ int orcvio_frame_update(orcvio_frame* f, const double* clone_R, const double* cl
   Batch::SnapshotIO io = frame_io(clone_R, clone_p, n_clones, R_b2c, t_c_b, P_in, feat_off, obs_clone, obs_z, n_feat);
   io.P_out = P_out; io.delta_x = delta_x; io.status = status; io.gamma = gamma; io.clone_out = clone_out;
   io.early_prior = true;
+  // the end-to-end call keeps its work lists in the direct (per-feature) form, which the resident chain cannot run:
+  // orcvio_frame_run / _fetch need a new orcvio_frame_load
+  f->loaded = false;
+  f->has_result = false;
   using clk = std::chrono::steady_clock;
   auto us = [](clk::time_point a, clk::time_point b) {
     return (float)std::chrono::duration<double, std::micro>(b - a).count();
@@ -558,10 +563,10 @@ int orcvio_frame_update(orcvio_frame* f, const double* clone_R, const double* cl
   const auto t0 = clk::now();
   int rc = f->b->snapshot_prepare(io);
   if (rc != ORCVIO_OK) return rc;
-  f->loaded = true;
   const auto t1 = clk::now();
   rc = f->b->snapshot_execute(true);
   if (rc != ORCVIO_OK) return rc;
+  f->has_result = true;
   const auto t2 = clk::now();
   rc = f->b->snapshot_fetch(io);
   const auto t3 = clk::now();
@@ -577,11 +582,13 @@ int orcvio_frame_update_pose_cov(orcvio_frame* f, const double* clone_R, const d
   Batch::SnapshotIO io = frame_io(clone_R, clone_p, n_clones, R_b2c, t_c_b, P_in, feat_off, obs_clone, obs_z, n_feat);
   io.P_lead9 = P_lead9; io.delta_x = delta_x; io.status = status; io.gamma = gamma; io.clone_out = clone_out;
   io.early_prior = true;
+  f->loaded = false;                    // (as orcvio_frame_update)
+  f->has_result = false;
   int rc = f->b->snapshot_prepare(io);
   if (rc != ORCVIO_OK) return rc;
-  f->loaded = true;
   rc = f->b->snapshot_execute(true);
   if (rc != ORCVIO_OK) return rc;
+  f->has_result = true;
   return f->b->snapshot_fetch(io);
 }
 
@@ -603,6 +610,7 @@ int orcvio_frame_load(orcvio_frame* f, const double* clone_R, const double* clon
                       const int* obs_clone, const double* obs_z, int n_feat) {
   if (!f || !feat_off || !obs_clone || !obs_z || !clone_R || !clone_p) return ORCVIO_ERR_ARG;
   Batch::SnapshotIO io = frame_io(clone_R, clone_p, n_clones, R_b2c, t_c_b, P_in, feat_off, obs_clone, obs_z, n_feat);
+  f->has_result = false;
   int rc = f->b->snapshot_prepare(io);
   f->b->sync();
   f->loaded = (rc == ORCVIO_OK);
@@ -640,6 +648,7 @@ int orcvio_frame_run(orcvio_frame* f, int repeat, float* total_us, float* stage_
     if (total_us) *total_us = ms * 1000.f;
   }
   (void)l0;
+  f->has_result = b.ok();
   return b.ok() ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -650,8 +659,20 @@ int orcvio_frame_fetch(orcvio_frame* f, double* P_out, double* delta_x, int* sta
   io.P_out = P_out; io.delta_x = delta_x; io.status = status; io.gamma = gamma; io.clone_out = clone_out;
   // results of the last run: queue the per-candidate download that orcvio_frame_run skipped
   f->b->snapshot_execute(true);
-  return f->b->snapshot_fetch(io);
+  const int rc = f->b->snapshot_fetch(io);
+  f->has_result = (rc == ORCVIO_OK);
+  return rc;
 }
+
+int orcvio_frame_fetch_last(orcvio_frame* f, double* P_out, double* delta_x, int* status, double* gamma,
+                            double* clone_out) {
+  if (!f || !f->has_result) return ORCVIO_ERR_ARG;
+  Batch::SnapshotIO io;
+  io.P_out = P_out; io.delta_x = delta_x; io.status = status; io.gamma = gamma; io.clone_out = clone_out;
+  return f->b->snapshot_fetch_last(io);
+}
+
+long long orcvio_frame_graph_replays(orcvio_frame* f) { return f ? f->b->snapshot_graph_replays() : 0; }
 
 long long orcvio_frame_kernel_launches(orcvio_frame* f) { return f ? f->b->kernel_launches() : 0; }
 

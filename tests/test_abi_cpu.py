@@ -75,6 +75,18 @@ def test_frozen_window_entries_reject_unknown_flag_bits():
         assert not L.orcvio_frame_create(10, flags, 1e-4, 0.95, -1.0, 1e-3, 100.0)
 
 
+def test_frame_entries_reject_a_null_handle():
+    """The frame-handle readers answer a NULL handle without touching a device: fetch_last / fetch / run refuse it,
+    the replay and launch counters read 0."""
+    L = api.lib()
+    ERR_ARG = -2                                            # ORCVIO_ERR_ARG
+    assert L.orcvio_frame_fetch_last(None, None, None, None, None, None) == ERR_ARG
+    assert L.orcvio_frame_fetch(None, None, None, None, None, None) == ERR_ARG
+    assert L.orcvio_frame_run(None, 1, None, None) == ERR_ARG
+    assert L.orcvio_frame_graph_replays(None) == 0
+    assert L.orcvio_frame_kernel_launches(None) == 0
+
+
 def test_syrk_plan_covers_every_row_once_and_fits_the_budget():
     """Host logic of the staircase split-K plan (csrc/kernels.h syrk_plan), no device involved: every tile pair
     (I <= J) covers exactly the rows [jrow0[J], arows) in whole chunks of kc rows (kcd = 13/8 kc for a diagonal pair, which
