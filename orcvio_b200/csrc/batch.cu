@@ -183,7 +183,6 @@ Batch::Batch(const Params& p, int n) : p_(p), B_(n) {
   CK(cudaEventCreateWithFlags(&ev_fork_, cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&ev_join_, cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&ev_ls_, cudaEventDisableTiming));
-  if (env_int("ORCVIO_BLOCKING_SYNC", 0)) CK(cudaEventCreateWithFlags(&ev_block_, cudaEventDisableTiming | cudaEventBlockingSync));
   for (auto& e : ev_) CK(cudaEventCreate(&e));
   const size_t nB = (size_t)B_;
   CK(cudaMalloc(&dP_, nB * ldp_ * ldp_ * sizeof(double)));
@@ -239,8 +238,6 @@ Batch::Batch(const Params& p, int n) : p_(p), B_(n) {
     int dev = 0;
     cudaGetDevice(&dev);
     if (cudaDeviceGetAttribute(&n_sm_, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm_ < 1) n_sm_ = 148;
-    if (const char* e = std::getenv("ORCVIO_SYRK_WAVES")) syrk_waves_ = std::max(1, std::atoi(e));
-    syrk_group_ = std::max(1, env_int("ORCVIO_SYRK_GROUP", 8));
   }
   chi2_host_.assign(500, 0.0);
   for (int i = 1; i < 500; ++i) chi2_host_[i] = chi2_quantile(p_.chi_square_threshold_feat, i);
@@ -260,24 +257,12 @@ Batch::Batch(const Params& p, int n) : p_(p), B_(n) {
   CK(cudaMallocHost(&hClones_, nB * Ncap_ * CL_STRIDE * sizeof(double)));
   CK(cudaMallocHost(&hDx_, nB * ldp_ * sizeof(double)));
   std::memset(hImu_, 0, nB * IM_STRIDE * sizeof(double));
-  if (B_ > 1 || env_int("ORCVIO_PRERESERVE", 0)) prereserve();
+  if (B_ > 1) prereserve();
 }
 
 // Multi-trajectory batches: size the growable buffers for a typical frame up front.  Growing them later works (x 2
 // policy) but every growth is a cudaFree / cudaMallocHost, i.e. a device-wide synchronisation -- with several batches
 // replaying from as many host threads those stalls hit every thread at once.
-// End of a phase of process(): the host needs the downloaded results.  A single filter spins (lowest latency); the
-// batches of a multi-trajectory replay block on an event instead, so that a thread waiting for its kernels leaves its
-// core to the bookkeeping of another batch.
-void Batch::wait_stream() {
-  if (B_ > 1 && ev_block_) {
-    CK(cudaEventRecord(ev_block_, stream_));
-    CK(cudaEventSynchronize(ev_block_));
-  } else {
-    CK(cudaStreamSynchronize(stream_));
-  }
-}
-
 void Batch::prereserve() {
   const size_t nB = (size_t)B_;
   const size_t cands = nB * 192, rows = cands * 9, obs = cands * 6;
@@ -344,7 +329,6 @@ Batch::~Batch() {
   if (ev_fork_) cudaEventDestroy(ev_fork_);
   if (ev_join_) cudaEventDestroy(ev_join_);
   if (ev_ls_) cudaEventDestroy(ev_ls_);
-  if (ev_block_) cudaEventDestroy(ev_block_);
   if (stream2_) cudaStreamDestroy(stream2_);
   if (stream_up_) cudaStreamDestroy(stream_up_);
   if (ev_up_) cudaEventDestroy(ev_up_);
@@ -519,7 +503,7 @@ void Batch::stage_upload(PhaseWork& w) {
     CK(cudaMalloc(&dTileRows_, tilerows_cap_ * sizeof(int)));
   }
   int units = 1;
-  for (const FilterWork& f : w.fw) units = std::max(units, syrk_plan(f, n_sm_ * syrk_waves_).total);
+  for (const FilterWork& f : w.fw) units = std::max(units, syrk_plan(f, n_sm_).total);
   w.syrk_units = units;
   const size_t need_a = (w.arows_total + 16) * (size_t)ldr_;
   if (need_a > amat_cap_) {
@@ -713,7 +697,7 @@ void Batch::launch_phase(PhaseWork& w, bool download, bool prior_in_flight) {
     qa.fw = dFw;
     InfoBufs ib{};
     ib.Ls = dLs_; ib.Amat = dAmat_; ib.part = dPart_; ib.ls_done = ev_ls_;
-    ib.max_units = w.syrk_units; ib.cta_budget = n_sm_ * syrk_waves_; ib.group = syrk_group_; ib.syrk_cnt = dSyrkCnt_;
+    ib.max_units = w.syrk_units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_;
     ib.tile_rows = dTileRows_; ib.filter_rows = dFilterRows_;
     launch_info_update(qa, upd_args(dFw), ib, (int)w.tiles.size(), w.max_tile_rows, w.wmax_blk, w.maxN, stream_,
                        stream2_, ev_fork_, ev_join_, profiling_ ? e[3] : nullptr, profiling_ ? e[4] : nullptr, &nl,
@@ -1337,7 +1321,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     }
     // the blob is reused by the next phase: wait for the upload + kernels reading it
     g_sp.mark(2);
-    wait_stream();
+    CK(cudaStreamSynchronize(stream_));
     g_sp.mark(3);
     if (profiling_) {
       float ms = 0;
@@ -1562,7 +1546,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       launch_triangulate(ta, stream_);
       ++launches_;
       CK(cudaMemcpyAsync(hb->hSpecStatus, hb->dSpecStatus, nS * sizeof(int), cudaMemcpyDeviceToHost, stream_));
-      wait_stream();
+      CK(cudaStreamSynchronize(stream_));
     }
   }
   g_sp.mark(5);
@@ -1694,7 +1678,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
   }
   download_mirrors();
   g_sp.mark(7);
-  wait_stream();
+  CK(cudaStreamSynchronize(stream_));
   g_sp.mark(8);
   if (hybrid_) {
     hybrid_apply_gather(gather_tracks);
@@ -2015,7 +1999,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
   if (hybrid_) hybrid_queue_gather(gather_tracks);
   download_mirrors();
   g_sp.mark(10);
-  wait_stream();
+  CK(cudaStreamSynchronize(stream_));
   if (hybrid_) {
     hybrid_apply_gather(gather_tracks);
     if (!hyb_ok) { ok_ = false; err_ = "hybrid upload arena exhausted"; }
@@ -2649,9 +2633,8 @@ int Batch::snapshot_execute(bool download) {
   // Repeated runs on a resident frame (orcvio_frame_run: the device-timed loop) replay ONE CUDA graph holding the
   // restore copies and the whole two-stream kernel chain: the per-kernel launch latencies leave the critical path.
   // The first two runs after a prepare go the ordinary way (they grow scratch buffers and set function attributes).
-  static const int graph_env = env_int("ORCVIO_GRAPH", 1);
-  const bool graphable = graph_env && !download && !profiling_ && !prior_in_flight && !S.tri_early && !S.jac_early &&
-                         !want_iters_ && !want_raw_;
+  const bool graphable = !download && !profiling_ && !prior_in_flight && !S.tri_early && !S.jac_early && !want_iters_ &&
+                         !want_raw_;
   if (graphable && S.graph_exec) {
     CK(cudaGraphLaunch(S.graph_exec, stream_));
     ++S.graph_replays;

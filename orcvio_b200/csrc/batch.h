@@ -260,13 +260,13 @@ class Batch {
   int flags_ = 0;
   std::vector<FilterHost> f_;
   cudaStream_t stream_ = nullptr, stream2_ = nullptr;
-  cudaEvent_t ev_fork_ = nullptr, ev_join_ = nullptr, ev_ls_ = nullptr, ev_block_ = nullptr;
+  cudaEvent_t ev_fork_ = nullptr, ev_join_ = nullptr, ev_ls_ = nullptr;
   double *dAmat_ = nullptr, *dPart_ = nullptr;
   size_t amat_cap_ = 0, part_cap_ = 0;
   double* dLs_ = nullptr;
   int *dTileRows_ = nullptr, *dFilterRows_ = nullptr;
   unsigned int* dSyrkCnt_ = nullptr;   // split-K arrival counters of k_syrk
-  int n_sm_ = 148, syrk_waves_ = 1, syrk_group_ = 8;
+  int n_sm_ = 148;
   float last_syrk_us_ = 0.f, last_prior_us_ = 0.f;
   size_t tilerows_cap_ = 0;
   cudaEvent_t ev_[16];
@@ -317,7 +317,6 @@ class Batch {
   int* hZuptDec_ = nullptr; double* hZuptInfo_ = nullptr;
 
   void prereserve();
-  void wait_stream();
   void upload_blob();
   void ensure_scratch(size_t n_cand, size_t hblk, size_t rblk);
   void run_phase(PhaseWork& w, int phase);

@@ -155,12 +155,10 @@ __global__ void __launch_bounds__(AF_THREADS, 3) k_aform(AformArgs a, const doub
   const int tid = threadIdx.x, nt = blockDim.x;
   const int warp = tid >> 5, lane = tid & 31, nw = nt >> 5;
   const int nc = tl.cand_end - tl.cand_begin;      // host guarantees nc <= 256
-  pdl_launch_dependents();
   const int rows_ub = tl.rows;                     // <= AFORM_TILE_ROWS
   const int rows8 = (rows_ub + 7) & ~7;
   for (int e = tid; e < rows8 * Wp; e += nt) smem[e] = 0.0;
   if (tid < AFORM_TILE_ROWS) res[tid] = 0.0;
-  pdl_wait();                                      // above: host-built tile records; below: gate results, blocks, factor
   // ---- row bases of the gated candidates (block scan)
   int total = 0;
   for (int base = 0; base < nc; base += nt) {
@@ -323,8 +321,9 @@ constexpr int SY_T = SY_TILE, SY_KS = 32, SY_LD = 68;
 // Operand pipeline: SY_STAGES slabs of 32 rows x 64 columns of A (column tile I) and of column tile J (a diagonal pair:
 // 64 rows of its one tile), brought in by cp.async (LDGSTS, 16 bytes per copy, zero-fill past the end of the chunk) one
 // slab ahead of the MMAs; one __syncthreads per slab.  (A TMA variant -- one cp.async.bulk per slab row, mbarrier
-// producer warp -- was built and measured slower, and 64-row slabs for every unit change nothing: DESIGN.md.)
+// producer warp -- was built and measured slower; deeper rings and 64-row slabs for every unit change nothing: DESIGN.md.)
 constexpr int SY_THREADS = 256;
+constexpr int SY_STAGES = 2;
 constexpr int SY_STAGE_DOUBLES = 2 * SY_KS * SY_LD;
 
 __device__ __forceinline__ unsigned int smem_u32(const void* p) { return (unsigned int)__cvta_generic_to_shared(p); }
@@ -370,7 +369,6 @@ __constant__ unsigned char SY_DIAG_FRAG[8][5] = {
     {0x33, 0x34, 0x35, 0x36, 0x37}, {0x05, 0x06, 0x07, 0x77, 0xff}, {0x16, 0x17, 0x66, 0x67, 0xff},
     {0x27, 0x55, 0x56, 0x57, 0xff}, {0x44, 0x45, 0x46, 0x47, 0xff}};
 
-template <int SY_STAGES>
 __global__ void __launch_bounds__(SY_THREADS) k_syrk(UpdArgs a, const double* __restrict__ Amat, int lda, double* part,
                                                      int max_units, int cta_budget, int group, const Tile* tiles,
                                                      const int* tile_rows, int* filter_rows, unsigned int* counters,
@@ -380,8 +378,6 @@ __global__ void __launch_bounds__(SY_THREADS) k_syrk(UpdArgs a, const double* __
   const FilterWork fw = a.fw[fi];
   const int tid = threadIdx.x;
   const int unit = blockIdx.x;
-  pdl_launch_dependents();
-  pdl_wait();                                            // tile_rows and A are the previous kernel's output
   sy_stamp(unit, 0);
   if (unit == 0 && tid < 32) {                           // gated rows of this filter (k_pinfo skips P when 0): warp 0
     int rows = 0;
@@ -580,7 +576,7 @@ __global__ void __launch_bounds__(SY_THREADS) k_syrk(UpdArgs a, const double* __
     const int e0 = chunk * per, e1 = min(SY_T * SY_T, e0 + per);
     // same association as the two-level path below (chunks in order inside a group of gsz, then the group sums in
     // order), so a filter gives the same bits whichever of the two reductions its batch ends up with
-    int gsz = max(group, 1);
+    int gsz = group;
     if ((nchunks + gsz - 1) / gsz > SY_MAXG) gsz = (nchunks + SY_MAXG - 1) / SY_MAXG;
     const int ngroups = (nchunks + gsz - 1) / gsz;
     for (int e = e0 + tid; e < e1; e += 256) {
@@ -607,7 +603,7 @@ __global__ void __launch_bounds__(SY_THREADS) k_syrk(UpdArgs a, const double* __
     return;
   }
   // ---- level 1: the last chunk of a group sums the group (16 tile elements per thread)
-  int gsz = max(group, 1);
+  int gsz = group;
   if ((nchunks + gsz - 1) / gsz > SY_MAXG) gsz = (nchunks + SY_MAXG - 1) / SY_MAXG;
   const int ngroups = (nchunks + gsz - 1) / gsz;
   const int g = chunk / gsz;
@@ -720,10 +716,8 @@ __global__ void __launch_bounds__(CHOL_THREADS) k_chol_w_solve(UpdArgs a) {
   double* A = sm;
   const int Tm = (n + 7) >> 3;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();
   chol_init(A, cs, n, nx);
   __syncthreads();
-  pdl_wait();                                            // W (k_syrk) -- the tiles were zeroed while it was still running
   const int ldr = a.ldr, ldt0 = a.ldt;
   // triangle rows: W;  carried rows: row n + q = F_1[d0 + q][:] = FT[:][d0 + q];  last row: v = S[n][:]
   chol_load_rows(A, n, 0, n + nx, [&](int i, int j) -> const double* {
@@ -772,7 +766,6 @@ __global__ void __launch_bounds__(PI_THREADS) k_pinfo(UpdArgs a, const double* L
   if (!fw.active) return;
   const int n = fw.D - ORCVIO_LEG, D = fw.D, L = ORCVIO_LEG;
   const int tid = threadIdx.x;
-  pdl_wait();
   if (blockIdx.y == gridDim.y - 1) {
     if (blockIdx.x != 0) return;
     double* dxs = sm;
@@ -876,9 +869,7 @@ static void info_attrs() {
   cudaFuncSetAttribute(k_chol_w_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024);
   cudaFuncSetAttribute(k_pinfo, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
   cudaFuncSetAttribute(k_imu_factor, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-  cudaFuncSetAttribute(k_syrk<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * SY_STAGE_DOUBLES * (int)sizeof(double));
-  cudaFuncSetAttribute(k_syrk<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * SY_STAGE_DOUBLES * (int)sizeof(double));
-  cudaFuncSetAttribute(k_syrk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * SY_STAGE_DOUBLES * (int)sizeof(double));
+  cudaFuncSetAttribute(k_syrk, cudaFuncAttributeMaxDynamicSharedMemorySize, SY_STAGES * SY_STAGE_DOUBLES * (int)sizeof(double));
   check_launch("info attributes");
   attr = true;
 }
@@ -895,22 +886,14 @@ static void launch_syrk(const UpdArgs& u, const InfoBufs& ib, int B, const Tile*
     g_syrk_dbg_units = std::min(1024, std::max(ib.max_units, 1));
   }
   // the parallel slice reduction spins on the other chunks of a pair: only when every CTA of the grid is resident
-  static const int spin_env = env_int("ORCVIO_SYRK_SPIN", 1);
   int n_sm = 0, dev = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-  const int spin = (spin_env && (long long)gs.x * gs.y <= n_sm) ? 1 : 0;
-  static const int stages = env_int("ORCVIO_SYRK_STAGES", 2);
-  const size_t smem = (size_t)(stages == 4 ? 4 : stages == 3 ? 3 : 2) * SY_STAGE_DOUBLES * sizeof(double);
-  if (stages == 4)
-    launch_pdl(k_syrk<4>, gs, dim3(SY_THREADS), smem, s, u, ib.Amat, u.ldr, ib.part, ib.max_units, ib.cta_budget, ib.group,
-               tiles, ib.tile_rows, ib.filter_rows, ib.syrk_cnt, spin);
-  else if (stages == 3)
-    launch_pdl(k_syrk<3>, gs, dim3(SY_THREADS), smem, s, u, ib.Amat, u.ldr, ib.part, ib.max_units, ib.cta_budget, ib.group,
-               tiles, ib.tile_rows, ib.filter_rows, ib.syrk_cnt, spin);
-  else
-    launch_pdl(k_syrk<2>, gs, dim3(SY_THREADS), smem, s, u, ib.Amat, u.ldr, ib.part, ib.max_units, ib.cta_budget, ib.group,
-               tiles, ib.tile_rows, ib.filter_rows, ib.syrk_cnt, spin);
+  const int spin = ((long long)gs.x * gs.y <= n_sm) ? 1 : 0;
+  const size_t smem = (size_t)SY_STAGES * SY_STAGE_DOUBLES * sizeof(double);
+  // (SY_GROUP goes in as an argument: folded in as a constant, the reductions specialise and k_syrk spills more)
+  k_syrk<<<gs, SY_THREADS, smem, s>>>(u, ib.Amat, u.ldr, ib.part, ib.max_units, ib.cta_budget, SY_GROUP, tiles,
+                                       ib.tile_rows, ib.filter_rows, ib.syrk_cnt, spin);
   check_launch("k_syrk");
 }
 
@@ -919,8 +902,7 @@ static void launch_pinfo(const UpdArgs& u, const InfoBufs& ib, int nmax, int B, 
   const int g = (Dmax + PT - 1) / PT;
   dim3 g5(g, g + 1, B);                                  // last row of CTAs: the state increment
   const int n4 = (nmax + 3) & ~3;
-  launch_pdl(k_pinfo, g5, dim3(PI_THREADS), ((size_t)2 * n4 * PI_LD + 16 * 32 * 2) * sizeof(double), s, u, ib.Ls,
-             ib.filter_rows);
+  k_pinfo<<<g5, PI_THREADS, ((size_t)2 * n4 * PI_LD + 16 * 32 * 2) * sizeof(double), s>>>(u, ib.Ls, ib.filter_rows);
   check_launch("k_pinfo");
 }
 
@@ -942,7 +924,7 @@ void launch_info_dense_factor(const UpdArgs& u, const InfoBufs& ib, const double
   launch_syrk(u, ib, 1, nullptr, s);
   const size_t sm_w = chol_smem_doubles(n, CS + 1) * sizeof(double);
   dim3 gw((D + CS - 1) / CS, 1);
-  launch_pdl(k_chol_w_solve, gw, dim3(CHOL_THREADS), sm_w, s, u);
+  k_chol_w_solve<<<gw, CHOL_THREADS, sm_w, s>>>(u);
   check_launch("k_chol_w_solve");
 }
 
@@ -987,8 +969,8 @@ void launch_info_update(const AformArgs& q, const UpdArgs& u, const InfoBufs& ib
   if (n_tiles > 0) {
     const int rows8 = (std::max(max_tile_rows, 1) + 7) & ~7;
     const int wp = ((6 * max_w_blk + 3) & ~3) + 4;        // >= aform_stride(W) of every tile
-    launch_pdl(k_aform, dim3(n_tiles), dim3(AF_THREADS), (size_t)rows8 * wp * sizeof(double), s, q, u.T, u.t_stride,
-               u.ldt, ib.Amat, lda, ib.tile_rows);
+    k_aform<<<n_tiles, AF_THREADS, (size_t)rows8 * wp * sizeof(double), s>>>(q, u.T, u.t_stride, u.ldt, ib.Amat, lda,
+                                                                           ib.tile_rows);
     check_launch("k_aform");
   }
   if (hyb && max_dense > 0) {      // hybrid mode: the dense rows of the EKF-SLAM features, behind the tiles' rows
@@ -1003,7 +985,7 @@ void launch_info_update(const AformArgs& q, const UpdArgs& u, const InfoBufs& ib
   // k_chol_w_solve overwrites F_1 (u.T) with Y in place, and k_imu_factor on the side stream still reads the IMU
   // columns of F_1: it must be done first (it is, by tens of microseconds, unless other work delays the side stream)
   if (ib.ls_done) cudaStreamWaitEvent(s, ib.ls_done, 0);
-  launch_pdl(k_chol_w_solve, gw, dim3(CHOL_THREADS), sm_w, s, u);
+  k_chol_w_solve<<<gw, CHOL_THREADS, sm_w, s>>>(u);
   check_launch("k_chol_w_solve");
   if (mid2) cudaEventRecord(mid2, s);
   launch_pinfo(u, ib, nmax, B, s);

@@ -123,7 +123,7 @@ __global__ void __launch_bounds__(128, MINB) k_jac_gate(JacArgs a) {
   constexpr int LDQ = R2 + 1;
   constexpr int TEAM_DOUBLES = R2 * 6 + R2 * 3 + R2 + 4 + 3 * R2 * LDQ + R2;
   extern __shared__ double smem[];
-  pdl_launch_dependents();
+  pdl_launch_dependents();           // per-candidate overlap: the large-list grid may be scheduled behind this one
   const int teams_per_block = blockDim.x / TEAM;
   const int team = threadIdx.x / TEAM;
   const int lane = threadIdx.x % TEAM;
@@ -162,8 +162,6 @@ __global__ void __launch_bounds__(128, MINB) k_jac_gate(JacArgs a) {
       asm volatile("fence.acq_rel.gpu;" ::: "memory");
     }
     team_sync<TEAM>();
-  } else {
-    pdl_wait();
   }
   const int st_in = a.tri_status_f ? a.tri_status_f[cd.slot] : __ldcg(a.status + c);   // (L2: written by another SM moments ago)
   if (a.tri_status_f && lane == 0) a.status[c] = st_in;      // status by candidate, as the one-pass flow leaves it
@@ -385,21 +383,28 @@ static void launch_one(const JacArgs& a, cudaStream_t s) {
     attr_set = true;
   }
   int blocks = (a.n_list + tpb - 1) / tpb;
-  if (a.tri_done) launch_pdl_if(true, k_jac_gate<TEAM, MAXM, MINB>, dim3(blocks), dim3(threads), smem, s, a);
-  else launch_pdl(k_jac_gate<TEAM, MAXM, MINB>, dim3(blocks), dim3(threads), smem, s, a);
+  if (a.tri_done) {
+    // per-candidate overlap: programmatic stream serialisation lets the grid be scheduled while the previous kernel
+    // (k_triangulate, or the small-list k_jac_gate ahead of the large list) still runs; the flags order the data
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(blocks);
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    cudaLaunchKernelEx(&cfg, k_jac_gate<TEAM, MAXM, MINB>, a);
+  } else {
+    k_jac_gate<TEAM, MAXM, MINB><<<blocks, threads, smem, s>>>(a);
+  }
   check_launch("k_jac_gate");
 }
 
 void launch_jac_gate(const JacArgs& small_list, const JacArgs& large_list, cudaStream_t s) {
-  static const int minb = env_int("ORCVIO_JAC_MINB", 4);
-  switch (minb) {
-    case 2: launch_one<32, 8, 2>(small_list, s); break;
-    case 3: launch_one<32, 8, 3>(small_list, s); break;
-    case 5: launch_one<32, 8, 5>(small_list, s); break;
-    case 6: launch_one<32, 8, 6>(small_list, s); break;
-    case 8: launch_one<32, 8, 8>(small_list, s); break;
-    default: launch_one<32, 8, 4>(small_list, s); break;   // 128 registers, 4 CTAs per SM: fewest waves (measured)
-  }
+  launch_one<32, 8, 4>(small_list, s);   // 128 registers, 4 CTAs per SM: fewest waves (measured)
   launch_one<128, ORCVIO_MAX_OBS, 1>(large_list, s);
 }
 

@@ -145,7 +145,7 @@ struct InfoBufs {
   double* Ls;            // per filter 22 x 22 : IMU block factor given the clones
   double* Amat;          // stacked A = [r' | H' L], lda = ldr (residual in column 0)
   double* part;          // split-K partials of A^T A: [filter][work unit][64 x 64]
-  int max_units, cta_budget, group;        // part layout [filter][max_units]; SMs x waves; chunks per reduction group
+  int max_units, cta_budget;               // part layout [filter][max_units]; split-K budget (SMs, syrk_plan)
   unsigned int* syrk_cnt; // split-K arrival counters [filter][SY_MAXP][1 + SY_MAXG] (zero between launches)
   int* tile_rows;        // gated rows per tile
   int* filter_rows;      // gated rows per filter (0 -> posterior == prior, P is left untouched)
@@ -261,47 +261,13 @@ void launch_hybrid_gather(const int* filt, const int* slots, int n, const double
 // Records (and prints) a launch-configuration error; Batch polls launch_error_count().
 void check_launch(const char* name);
 int launch_error_count();
-int env_int(const char* name, int dflt);   // tuning knobs (ORCVIO_* environment variables)
+int env_int(const char* name, int dflt);   // diagnostics and the overlap threshold (ORCVIO_* environment variables)
 
-// Programmatic dependent launch (sm_90+): a kernel launched with launch_pdl() may be scheduled while the previous
-// kernel of its stream is still running (once every CTA of that kernel has called pdl_launch_dependents() or
-// exited); it runs its prologue (shared-memory zeroing, index arithmetic on host-provided lists) and then blocks in
-// pdl_wait() until the previous kernel has completed and its writes are visible.  Launched the ordinary way the two
-// device calls are no-ops.  Measured on the frame chain (B200, 2000 / 4096 features): no gain (207 -> 213 us, 252 -> 261 us),
-// so the attribute is OFF by default; ORCVIO_PDL=1 turns it on.
+// Programmatic dependent launch (sm_90+): once every CTA of a kernel has called this (or exited), the next kernel of
+// its stream, if launched with programmatic stream serialisation, may be scheduled.  Only the per-candidate overlap
+// uses that launch (k_jac_gate behind k_triangulate, jac_kernel.cu); behind an ordinary launch this is a no-op.
 #ifdef __CUDACC__
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-template <class... KArgs, class... Args>
-inline void launch_pdl_if(bool on, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
-                          Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = on ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-template <class... KArgs, class... Args>
-inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-  static const int pdl_on = env_int("ORCVIO_PDL", 0);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_on ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
 #endif
 
 void launch_triangulate(const TriArgs& a, cudaStream_t s);
@@ -364,9 +330,11 @@ constexpr int AFORM_TILE_ROWS = 64;     // row cap of a tile
 // chunks of rows; column tile J of A is structurally zero above row jrow0[J] (features are sorted by first
 // clone and A = H' L with L lower triangular), so pair (I, J) only covers rows [jrow0[J], arows).  The plan
 // picks the rows per chunk (multiple of 32, >= 128) so that the work units of all pairs fill `cta_budget`
-// (= SMs x waves).  A function of the filter alone: the chunking fixes the summation order, so a filter
+// (= SMs).  A function of the filter alone: the chunking fixes the summation order, so a filter
 // gives bit-identical results whether it runs alone or inside a batch.
-constexpr int SY_TILE = 64, SY_MAXT = 4, SY_MAXP = 10, SY_MAXG = 32;
+// The split-K reduction sums the chunks of a pair in groups of SY_GROUP (at most SY_MAXG groups), then the group
+// sums: the group size is part of W's summation tree, so changing it changes W's bits.
+constexpr int SY_TILE = 64, SY_MAXT = 4, SY_MAXP = 10, SY_MAXG = 32, SY_GROUP = 8;
 struct SyrkPlan {
   int kc, kcd, nt, npairs, total;   // rows per chunk of an off-diagonal / a diagonal pair
   int first[SY_MAXP + 1];        // first work unit of every pair (pair order: I outer, J >= I inner)

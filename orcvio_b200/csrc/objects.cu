@@ -290,7 +290,7 @@ int Batch::object_update(int fi, const double* Hx, const double* Hf, const doubl
   const int prow = rows - odim;
   FilterWork fw{};                                       // jrow0 = 0: a dense block has no staircase
   fw.N = N; fw.D = D; fw.active = 1; fw.arow0 = 0; fw.arows = prow;
-  const int units = syrk_plan(fw, n_sm_ * syrk_waves_).total;
+  const int units = syrk_plan(fw, n_sm_).total;
   const size_t need_a = ((size_t)prow + 16) * ldr_;
   if (need_a > amat_cap_) {
     if (dAmat_) cudaFree(dAmat_);
@@ -320,7 +320,7 @@ int Batch::object_update(int fi, const double* Hx, const double* Hf, const doubl
   ua.flags = flags_; ua.sigma2 = p_.feature_observation_noise;
   InfoBufs ib{};
   ib.Ls = dLs_ + (size_t)fi * ORCVIO_LEG * ORCVIO_LEG; ib.Amat = dAmat_; ib.part = dPart_;
-  ib.max_units = units; ib.cta_budget = n_sm_ * syrk_waves_; ib.group = syrk_group_; ib.syrk_cnt = dSyrkCnt_;
+  ib.max_units = units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_;
   ib.tile_rows = nullptr; ib.filter_rows = dFilterRows_ + fi;
   const double* Hp = dM + (size_t)odim * ld + odim;
   launch_info_dense_factor(ua, ib, Hp, ld, prow, n, stream_);
@@ -426,7 +426,7 @@ int Batch::dense_update(const double* P_in, int D, const double* H, const double
   FilterWork fw{};
   fw.N = 0;                                              // no clone poses behind this entry: dx is returned, not applied
   fw.D = D; fw.active = 1; fw.arow0 = 0; fw.arows = rows;
-  const int units = syrk_plan(fw, n_sm_ * syrk_waves_).total;
+  const int units = syrk_plan(fw, n_sm_).total;
   const size_t need_a = ((size_t)rows + 16) * ldr_;
   if (need_a > amat_cap_) {
     if (dAmat_) cudaFree(dAmat_);
@@ -453,7 +453,7 @@ int Batch::dense_update(const double* P_in, int D, const double* H, const double
   ua.flags = 0; ua.sigma2 = p_.feature_observation_noise;
   InfoBufs ib{};
   ib.Ls = dLs_; ib.Amat = dAmat_; ib.part = dPart_;
-  ib.max_units = units; ib.cta_budget = n_sm_ * syrk_waves_; ib.group = syrk_group_; ib.syrk_cnt = dSyrkCnt_;
+  ib.max_units = units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_;
   ib.tile_rows = nullptr; ib.filter_rows = dFilterRows_ + fi;
   CKO(cudaMemsetAsync(dImu_, 0, IM_STRIDE * sizeof(double), stream_));
   launch_info_dense_factor(ua, ib, dM.as<double>(), ld, rows, n, stream_);

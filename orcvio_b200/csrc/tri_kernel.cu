@@ -304,8 +304,8 @@ __device__ __forceinline__ bool check_motion(const double* clones, int first_clo
 // cand.filter selects the clone array / feature-position table of its filter.
 constexpr int TRI_WARPS = 4;
 
-// MINB = resident CTAs per SM the register allocation is held to (launch bound; chosen at run time by
-// tri_min_blocks(): the kernel is one LM latency chain per warp, so whole waves are what cost time).
+// MINB = resident CTAs per SM the register allocation is held to (launch bound; chosen from the grid size by
+// launch_triangulate(): the kernel is one LM latency chain per warp, so whole waves are what cost time).
 template <int MINB>
 __global__ void __launch_bounds__(32 * TRI_WARPS, MINB) k_triangulate(TriArgs a) {
   __shared__ double sm_all[TRI_WARPS][32 * TRI_SM_STRIDE];
@@ -403,15 +403,8 @@ void launch_triangulate(const TriArgs& a, cudaStream_t s) {
   int blocks = (a.n_cand + TRI_WARPS - 1) / TRI_WARPS;
   // 158 registers (3 CTAs per SM) is the fastest single wave; past two waves of that (measured at 4096 features)
   // the 128-register build with 4 CTAs per SM wins
-  static const int minb_env = env_int("ORCVIO_TRI_MINB", 0);
-  const int minb = minb_env ? minb_env : (blocks > 888 ? 4 : 3);
-  switch (minb) {
-    case 4: k_triangulate<4><<<blocks, 32 * TRI_WARPS, 0, s>>>(a); break;
-    case 5: k_triangulate<5><<<blocks, 32 * TRI_WARPS, 0, s>>>(a); break;
-    case 6: k_triangulate<6><<<blocks, 32 * TRI_WARPS, 0, s>>>(a); break;
-    case 8: k_triangulate<8><<<blocks, 32 * TRI_WARPS, 0, s>>>(a); break;
-    default: k_triangulate<3><<<blocks, 32 * TRI_WARPS, 0, s>>>(a); break;
-  }
+  if (blocks > 888) k_triangulate<4><<<blocks, 32 * TRI_WARPS, 0, s>>>(a);
+  else k_triangulate<3><<<blocks, 32 * TRI_WARPS, 0, s>>>(a);
   check_launch("k_triangulate");
 }
 

@@ -1,21 +1,16 @@
-"""Stage times (us) of the frozen stress frame for the current ORCVIO_* tuning environment.
+"""Stage times (us) of the frozen stress frame.
 
     python scripts/stage_times.py [--features 4096] [--repeat 30] [--flush]
-    python scripts/stage_times.py --sweep        # re-runs itself over the tuning knobs, one process each
 
-Prints one JSON line per run; used to pick launch bounds / split plans on the GPU box.
+Prints one JSON line: the mean device time per frame, the per-stage times and those of k_syrk / k_chol_prior.
 """
 import argparse
-import itertools
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-
-KNOBS = ["ORCVIO_TRI_MINB", "ORCVIO_JAC_MINB", "ORCVIO_SYRK_WAVES", "ORCVIO_SYRK_GROUP", "ORCVIO_TRI_CAP"]
 
 
 def one(n_feat, repeat, flush):
@@ -41,9 +36,8 @@ def one(n_feat, repeat, flush):
     kt = fr.kernel_times()
     st = {k: round(v, 1) for k, v in st.items()}
     st.update(syrk=round(kt["syrk"], 1), chol_prior=round(kt["chol_prior"], 1))
-    env = {k: os.environ[k] for k in KNOBS if k in os.environ}
     print(json.dumps(dict(features=n_feat, gated=int(((out["status"] & 2) != 0).sum()), us_per_frame=round(tot / repeat, 1),
-                          stages=st, env=env, chk=float(np.abs(out["delta_x"]).sum()))), flush=True)
+                          stages=st, chk=float(np.abs(out["delta_x"]).sum()))), flush=True)
 
 
 def main():
@@ -51,21 +45,8 @@ def main():
     ap.add_argument("--features", type=int, default=4096)
     ap.add_argument("--repeat", type=int, default=30)
     ap.add_argument("--flush", action="store_true")
-    ap.add_argument("--sweep", nargs="*", default=None, help="KNOB=v1,v2 ... (cartesian product)")
     args = ap.parse_args()
-    if args.sweep is None:
-        one(args.features, args.repeat, args.flush)
-        return
-    axes = []
-    for spec in args.sweep:
-        k, vs = spec.split("=")
-        axes.append([(k, v) for v in vs.split(",")])
-    for combo in itertools.product(*axes):
-        env = dict(os.environ)
-        env.update(dict(combo))
-        for nf in (2000, 4096):
-            cmd = [sys.executable, __file__, "--features", str(nf), "--repeat", str(args.repeat)] + (["--flush"] if args.flush else [])
-            subprocess.run(cmd, env=env, check=False)
+    one(args.features, args.repeat, args.flush)
 
 
 if __name__ == "__main__":
