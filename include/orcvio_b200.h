@@ -442,6 +442,9 @@ int orcvio_syrk_plan_probe(int arows, const int* jrow0, int n_clones, int cta_bu
 
 /* device / build info */
 int orcvio_device_count(void);
+/* bytes currently held by the library's device and pinned host buffers, summed over the process (either pointer may
+ * be NULL).  A buffer that only grows, such as the per-thread scratch of the object entries, is not counted. */
+int orcvio_device_bytes_held(long long* device, long long* pinned);
 /* select the CUDA device used by handles created afterwards on this thread (one process per GPU) */
 int orcvio_set_device(int device);
 const char* orcvio_version(void);

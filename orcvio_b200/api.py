@@ -100,6 +100,7 @@ def lib():
     L.orcvio_chi2_quantile.restype = C.c_double
     L.orcvio_chi2_quantile.argtypes = [C.c_double, C.c_int]
     L.orcvio_version.restype = C.c_char_p
+    L.orcvio_device_bytes_held.argtypes = [C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.orcvio_set_device.argtypes = [C.c_int]
     L.orcvio_fp64_peak.argtypes = [dp, dp]
     L.orcvio_latency_probe.argtypes = [dp]
@@ -978,6 +979,13 @@ def chol_probe(A, X=None, reps=10):
     if rc != 0:
         raise RuntimeError(f"orcvio_chol_probe failed: {rc}")
     return L, (Xs if X is not None else None), prof, us.value
+
+
+def device_bytes_held():
+    """(device, pinned) bytes held by the library's buffers, summed over the process."""
+    dev, pin = C.c_longlong(0), C.c_longlong(0)
+    lib().orcvio_device_bytes_held(C.byref(dev), C.byref(pin))
+    return dev.value, pin.value
 
 
 def chi2_quantile(p, dof):

@@ -36,6 +36,8 @@ namespace ob {
       ok_ = false;                                                                                \
     }                                                                                             \
   } while (0)
+// a failed allocation or growth of an owned buffer (devmem.h)
+#define CKA(ok) CK((ok) ? cudaSuccess : cudaErrorMemoryAllocation)
 
 struct Batch::PhaseWork {
   std::vector<Cand> cands;
@@ -90,44 +92,32 @@ struct Batch::PhaseWork {
 
 // Device / pinned buffers of the hybrid MSCKF / EKF-SLAM mode (allocated only when max_features_in_one_grid > 0).
 struct Batch::HybridBufs {
-  double* dSpecPos = nullptr;          // scratch position table of the speculative initializeInvParamPosition pass
-  long long* dSpecGen = nullptr;
-  double* dFinal = nullptr; size_t final_cap = 0;          // 3 per speculative candidate (anchor-frame solution)
-  int* dSpecStatus = nullptr; int* hSpecStatus = nullptr; size_t spec_cap = 0;
-  double* dHd = nullptr; size_t hd_cap = 0;                // dense rows, ldh = ldr
-  double *dH1 = nullptr, *dh2 = nullptr, *dr1 = nullptr, *dScratch = nullptr;
-  int *dEkfPass = nullptr, *dNewOk = nullptr, *dNNew = nullptr;
-  double* dEkfGamma = nullptr;
-  int* hEkfPass = nullptr; double* hEkfGamma = nullptr;    // pinned
-  double *dGather = nullptr, *hGather = nullptr; size_t gather_cap = 0;
+  DeviceBuf<double> dSpecPos;          // scratch position table of the speculative initializeInvParamPosition pass
+  DeviceBuf<long long> dSpecGen;
+  DeviceBuf<double> dFinal;            // 3 per speculative candidate (anchor-frame solution)
+  DeviceBuf<int> dSpecStatus; PinnedBuf<int> hSpecStatus;
+  DeviceBuf<double> dHd;               // dense rows, ldh = ldr
+  DeviceBuf<double> dH1, dh2, dr1, dScratch;
+  DeviceBuf<int> dEkfPass, dNewOk, dNNew;
+  DeviceBuf<double> dEkfGamma;
+  PinnedBuf<int> hEkfPass; PinnedBuf<double> hEkfGamma;
+  DeviceBuf<double> dGather; PinnedBuf<double> hGather;   // 6 per gathered feature
   // upload arena: sections are only appended between two synchronisations of the stream (reset after a sync), so a
   // queued copy never sees its pinned source rewritten; fixed capacity, so device pointers stay valid
-  char *pin = nullptr, *dev = nullptr; size_t cap = 0, used = 0;
+  PinnedBuf<char> pin; DeviceBuf<char> dev; size_t used = 0;
   template <class T>
   const T* put(const T* src, size_t n, cudaStream_t s, bool* ok) {
     const size_t off = (used + 255) & ~size_t(255), bytes = sizeof(T) * std::max<size_t>(n, 1);
-    if (off + bytes > cap) { *ok = false; return nullptr; }
-    if (n) std::memcpy(pin + off, src, sizeof(T) * n);
-    if (n && cudaMemcpyAsync(dev + off, pin + off, sizeof(T) * n, cudaMemcpyHostToDevice, s) != cudaSuccess) *ok = false;
+    if (off + bytes > dev.size()) { *ok = false; return nullptr; }
+    if (n) std::memcpy(pin.get() + off, src, sizeof(T) * n);
+    if (n && cudaMemcpyAsync(dev.get() + off, pin.get() + off, sizeof(T) * n, cudaMemcpyHostToDevice, s) != cudaSuccess)
+      *ok = false;
     used = off + bytes;
-    return reinterpret_cast<const T*>(dev + off);
+    return reinterpret_cast<const T*>(dev.get() + off);
   }
 };
 
-void Batch::HybridDeleter::operator()(HybridBufs* h) const {
-  if (!h) return;
-  cudaFree(h->dSpecPos); cudaFree(h->dSpecGen); cudaFree(h->dFinal); cudaFree(h->dSpecStatus);
-  if (h->hSpecStatus) cudaFreeHost(h->hSpecStatus);
-  cudaFree(h->dHd); cudaFree(h->dH1); cudaFree(h->dh2); cudaFree(h->dr1); cudaFree(h->dScratch);
-  cudaFree(h->dEkfPass); cudaFree(h->dNewOk); cudaFree(h->dNNew); cudaFree(h->dEkfGamma);
-  if (h->hEkfPass) cudaFreeHost(h->hEkfPass);
-  if (h->hEkfGamma) cudaFreeHost(h->hEkfGamma);
-  cudaFree(h->dGather);
-  if (h->hGather) cudaFreeHost(h->hGather);
-  cudaFree(h->dev);
-  if (h->pin) cudaFreeHost(h->pin);
-  delete h;
-}
+void Batch::HybridDeleter::operator()(HybridBufs* h) const { delete h; }
 
 Batch::Batch(const Params& p, int n) : p_(p), B_(n) {
   ok_ = true;
@@ -185,55 +175,54 @@ Batch::Batch(const Params& p, int n) : p_(p), B_(n) {
   CK(cudaEventCreateWithFlags(&ev_ls_, cudaEventDisableTiming));
   for (auto& e : ev_) CK(cudaEventCreate(&e));
   const size_t nB = (size_t)B_;
-  CK(cudaMalloc(&dP_, nB * ldp_ * ldp_ * sizeof(double)));
-  CK(cudaMemset(dP_, 0, nB * ldp_ * ldp_ * sizeof(double)));
-  CK(cudaMalloc(&dImu_, nB * IM_STRIDE * sizeof(double)));
-  CK(cudaMemset(dImu_, 0, nB * IM_STRIDE * sizeof(double)));
-  CK(cudaMalloc(&dClones_, nB * Ncap_ * CL_STRIDE * sizeof(double)));
-  CK(cudaMemset(dClones_, 0, nB * Ncap_ * CL_STRIDE * sizeof(double)));
-  CK(cudaMalloc(&dFpos_, nB * Fcap_ * FP_STRIDE * sizeof(double)));
-  CK(cudaMemset(dFpos_, 0, nB * Fcap_ * FP_STRIDE * sizeof(double)));
-  CK(cudaMalloc(&dFgen_, nB * Fcap_ * sizeof(long long)));
-  CK(cudaMemset(dFgen_, 0xFF, nB * Fcap_ * sizeof(long long)));
+  CKA(dP_.alloc(nB * ldp_ * ldp_));
+  CK(cudaMemset(dP_.get(), 0, dP_.bytes()));
+  CKA(dImu_.alloc(nB * IM_STRIDE));
+  CK(cudaMemset(dImu_.get(), 0, dImu_.bytes()));
+  CKA(dClones_.alloc(nB * Ncap_ * CL_STRIDE));
+  CK(cudaMemset(dClones_.get(), 0, dClones_.bytes()));
+  CKA(dFpos_.alloc(nB * Fcap_ * FP_STRIDE));
+  CK(cudaMemset(dFpos_.get(), 0, dFpos_.bytes()));
+  CKA(dFgen_.alloc(nB * Fcap_));
+  CK(cudaMemset(dFgen_.get(), 0xFF, dFgen_.bytes()));
   const int ncap = nmax_;
   if (hybrid_) {
-    CK(cudaMalloc(&dFidp_, nB * Fcap_ * FI_STRIDE * sizeof(double)));
-    CK(cudaMemset(dFidp_, 0, nB * Fcap_ * FI_STRIDE * sizeof(double)));
+    CKA(dFidp_.alloc(nB * Fcap_ * FI_STRIDE));
+    CK(cudaMemset(dFidp_.get(), 0, dFidp_.bytes()));
     hyb_.reset(new HybridBufs());
     HybridBufs& h = *hyb_;
-    CK(cudaMalloc(&h.dSpecPos, nB * Fcap_ * FP_STRIDE * sizeof(double)));
-    CK(cudaMemset(h.dSpecPos, 0, nB * Fcap_ * FP_STRIDE * sizeof(double)));
-    CK(cudaMalloc(&h.dSpecGen, nB * Fcap_ * sizeof(long long)));
-    CK(cudaMemset(h.dSpecGen, 0xFF, nB * Fcap_ * sizeof(long long)));
+    CKA(h.dSpecPos.alloc(nB * Fcap_ * FP_STRIDE));
+    CK(cudaMemset(h.dSpecPos.get(), 0, h.dSpecPos.bytes()));
+    CKA(h.dSpecGen.alloc(nB * Fcap_));
+    CK(cudaMemset(h.dSpecGen.get(), 0xFF, h.dSpecGen.bytes()));
     const size_t ne = nB * Emax_;
-    CK(cudaMalloc(&h.dH1, ne * ldr_ * sizeof(double)));
-    CK(cudaMalloc(&h.dh2, ne * sizeof(double)));
-    CK(cudaMalloc(&h.dr1, ne * sizeof(double)));
-    CK(cudaMalloc(&h.dScratch, nB * 64 * ldr_ * sizeof(double)));
-    CK(cudaMalloc(&h.dEkfPass, ne * sizeof(int)));
-    CK(cudaMalloc(&h.dEkfGamma, ne * sizeof(double)));
-    CK(cudaMalloc(&h.dNewOk, ne * sizeof(int)));
-    CK(cudaMalloc(&h.dNNew, nB * sizeof(int)));
-    CK(cudaMemset(h.dNNew, 0, nB * sizeof(int)));
-    CK(cudaMallocHost(&h.hEkfPass, ne * sizeof(int)));
-    CK(cudaMallocHost(&h.hEkfGamma, ne * sizeof(double)));
-    h.gather_cap = 2 * ne + 64;
-    CK(cudaMalloc(&h.dGather, h.gather_cap * 6 * sizeof(double)));
-    CK(cudaMallocHost(&h.hGather, h.gather_cap * 6 * sizeof(double)));
-    h.cap = (size_t)(2 << 20) + nB * (size_t)(64 << 10);
-    CK(cudaMalloc(&h.dev, h.cap));
-    CK(cudaMallocHost(&h.pin, h.cap));
+    CKA(h.dH1.alloc(ne * ldr_));
+    CKA(h.dh2.alloc(ne));
+    CKA(h.dr1.alloc(ne));
+    CKA(h.dScratch.alloc(nB * 64 * ldr_));
+    CKA(h.dEkfPass.alloc(ne));
+    CKA(h.dEkfGamma.alloc(ne));
+    CKA(h.dNewOk.alloc(ne));
+    CKA(h.dNNew.alloc(nB));
+    CK(cudaMemset(h.dNNew.get(), 0, h.dNNew.bytes()));
+    CKA(h.hEkfPass.alloc(ne));
+    CKA(h.hEkfGamma.alloc(ne));
+    CKA(h.dGather.alloc((2 * ne + 64) * 6));
+    CKA(h.hGather.alloc((2 * ne + 64) * 6));
+    const size_t cap = (size_t)(2 << 20) + nB * (size_t)(64 << 10);
+    CKA(h.dev.alloc(cap));
+    CKA(h.pin.alloc(cap));
   }
-  CK(cudaMalloc(&dS_, nB * (size_t)(ncap + 1) * ldr_ * sizeof(double)));
-  CK(cudaMalloc(&dYv_, nB * ldr_ * sizeof(double)));
-  CK(cudaMalloc(&dT_, nB * (size_t)ncap * ldt_ * sizeof(double)));
-  CK(cudaMalloc(&dDx_, nB * ldp_ * sizeof(double)));
-  CK(cudaMemset(dDx_, 0, nB * ldp_ * sizeof(double)));
-  CK(cudaMalloc(&dLs_, nB * ORCVIO_LEG * ORCVIO_LEG * sizeof(double)));
-  CK(cudaMalloc(&dFilterRows_, nB * sizeof(int)));
-  CK(cudaMemset(dFilterRows_, 0, nB * sizeof(int)));
-  CK(cudaMalloc(&dSyrkCnt_, nB * SY_MAXP * (SY_MAXG + 1) * sizeof(unsigned int)));
-  CK(cudaMemset(dSyrkCnt_, 0, nB * SY_MAXP * (SY_MAXG + 1) * sizeof(unsigned int)));
+  CKA(dS_.alloc(nB * (size_t)(ncap + 1) * ldr_));
+  CKA(dYv_.alloc(nB * ldr_));
+  CKA(dT_.alloc(nB * (size_t)ncap * ldt_));
+  CKA(dDx_.alloc(nB * ldp_));
+  CK(cudaMemset(dDx_.get(), 0, dDx_.bytes()));
+  CKA(dLs_.alloc(nB * ORCVIO_LEG * ORCVIO_LEG));
+  CKA(dFilterRows_.alloc(nB));
+  CK(cudaMemset(dFilterRows_.get(), 0, dFilterRows_.bytes()));
+  CKA(dSyrkCnt_.alloc(nB * SY_MAXP * (SY_MAXG + 1)));
+  CK(cudaMemset(dSyrkCnt_.get(), 0, dSyrkCnt_.bytes()));
   {
     int dev = 0;
     cudaGetDevice(&dev);
@@ -241,22 +230,22 @@ Batch::Batch(const Params& p, int n) : p_(p), B_(n) {
   }
   chi2_host_.assign(500, 0.0);
   for (int i = 1; i < 500; ++i) chi2_host_[i] = chi2_quantile(p_.chi_square_threshold_feat, i);
-  CK(cudaMalloc(&dChi2_, 500 * sizeof(double)));
-  CK(cudaMemcpy(dChi2_, chi2_host_.data(), 500 * sizeof(double), cudaMemcpyHostToDevice));
+  CKA(dChi2_.alloc(500));
+  CK(cudaMemcpy(dChi2_.get(), chi2_host_.data(), 500 * sizeof(double), cudaMemcpyHostToDevice));
   if (p_.if_ZUPT_valid) {
     chi2_zupt_host_.assign(500, 0.0);
     if (!p_.if_use_feature_zupt_flag)
       for (int i = 1; i < 500; ++i) chi2_zupt_host_[i] = chi2_quantile(0.95, i);
-    CK(cudaMalloc(&dZuptDec_, nB * sizeof(int)));
-    CK(cudaMalloc(&dZuptInfo_, nB * 2 * sizeof(double)));
-    CK(cudaMallocHost(&hZuptDec_, nB * sizeof(int)));
-    CK(cudaMallocHost(&hZuptInfo_, nB * 2 * sizeof(double)));
-    std::memset(hZuptDec_, 0, nB * sizeof(int));
+    CKA(dZuptDec_.alloc(nB));
+    CKA(dZuptInfo_.alloc(nB * 2));
+    CKA(hZuptDec_.alloc(nB));
+    CKA(hZuptInfo_.alloc(nB * 2));
+    if (hZuptDec_.get()) std::memset(hZuptDec_.get(), 0, hZuptDec_.bytes());
   }
-  CK(cudaMallocHost(&hImu_, nB * IM_STRIDE * sizeof(double)));
-  CK(cudaMallocHost(&hClones_, nB * Ncap_ * CL_STRIDE * sizeof(double)));
-  CK(cudaMallocHost(&hDx_, nB * ldp_ * sizeof(double)));
-  std::memset(hImu_, 0, nB * IM_STRIDE * sizeof(double));
+  CKA(hImu_.alloc(nB * IM_STRIDE));
+  CKA(hClones_.alloc(nB * Ncap_ * CL_STRIDE));
+  CKA(hDx_.alloc(nB * ldp_));
+  if (hImu_.get()) std::memset(hImu_.get(), 0, hImu_.bytes());
   if (B_ > 1) prereserve();
 }
 
@@ -268,63 +257,27 @@ void Batch::prereserve() {
   const size_t cands = nB * 192, rows = cands * 9, obs = cands * 6;
   ensure_scratch(cands, rows * 36, rows);
   const size_t tiles = nB * 48;
-  if (tiles > tilerows_cap_) {
-    tilerows_cap_ = tiles;
-    CK(cudaMalloc(&dTileRows_, tilerows_cap_ * sizeof(int)));
-  }
-  const size_t need_a = (rows + 64 * nB + 16) * (size_t)ldr_;
-  if (need_a > amat_cap_) {
-    amat_cap_ = need_a;
-    CK(cudaMalloc(&dAmat_, amat_cap_ * sizeof(double)));
-  }
+  CKA(dTileRows_.alloc(tiles));
+  CKA(dAmat_.alloc((rows + 64 * nB + 16) * (size_t)ldr_));
   // split-K partial tiles: up to ~18 work units per filter were seen on EuRoC-shaped frames (6 tile pairs x chunks of
   // >= 128 rows); 32 covers ~2500 stacked rows per filter without a growth in the middle of a replay
-  const size_t need_p = nB * 32 * 4096;
-  if (need_p > part_cap_) {
-    part_cap_ = need_p;
-    CK(cudaMalloc(&dPart_, part_cap_ * sizeof(double)));
-  }
+  CKA(dPart_.alloc(nB * 32 * 4096));
   const size_t blob_bytes = cands * sizeof(Cand) + obs * (sizeof(int) + 2 * sizeof(double)) + tiles * sizeof(Tile) +
                             nB * (sizeof(FilterWork) + 64) + cands * 2 * sizeof(int) + (size_t)(64 << 10);
-  blob_.ensure_pinned(blob_bytes);
-  if (blob_bytes > blob_.dev_cap) {
-    blob_.dev_cap = blob_bytes;
-    CK(cudaMalloc(&blob_.dev, blob_.dev_cap));
-  }
+  CKA(blob_.pinned.alloc(blob_bytes * 2 + 4096));
+  CKA(blob_.dev.alloc(blob_bytes));
   if (hybrid_) {
     HybridBufs& hb = *hyb_;
-    hb.hd_cap = nB * (size_t)(2 * Emax_ + 16 * 9) * ldr_;
-    CK(cudaMalloc(&hb.dHd, hb.hd_cap * sizeof(double)));
-    hb.spec_cap = nB * 64;
-    CK(cudaMalloc(&hb.dFinal, hb.spec_cap * 3 * sizeof(double)));
-    CK(cudaMalloc(&hb.dSpecStatus, hb.spec_cap * sizeof(int)));
-    CK(cudaMallocHost(&hb.hSpecStatus, hb.spec_cap * sizeof(int)));
+    CKA(hb.dHd.alloc(nB * (size_t)(2 * Emax_ + 16 * 9) * ldr_));
+    const size_t spec = nB * 64;
+    CKA(hb.dFinal.alloc(spec * 3));
+    CKA(hb.dSpecStatus.alloc(spec));
+    CKA(hb.hSpecStatus.alloc(spec));
   }
 }
 
 Batch::~Batch() {
-  cudaDeviceSynchronize();
-  cudaFree(dP_); cudaFree(dImu_); cudaFree(dClones_); cudaFree(dFpos_); cudaFree(dFgen_);
-  cudaFree(dS_); cudaFree(dYv_); cudaFree(dT_); cudaFree(dDx_); cudaFree(dChi2_);
-  cudaFree(dAmat_); cudaFree(dPart_);
-  cudaFree(dStatusF_); cudaFree(dGammaF_); cudaFree(dFidp_); cudaFree(dTriDone_);
-  if (blob_early2_.dev) cudaFree(blob_early2_.dev);
-  if (blob_early2_.pinned) cudaFreeHost(blob_early2_.pinned);
-  if (blob_early_.dev) cudaFree(blob_early_.dev);
-  if (blob_early_.pinned) cudaFreeHost(blob_early_.pinned);
-  cudaFree(dLs_); cudaFree(dTileRows_); cudaFree(dFilterRows_); cudaFree(dSyrkCnt_);
-  if (dZuptDec_) cudaFree(dZuptDec_);
-  if (dCovHist_) cudaFree(dCovHist_);
-  if (dZuptInfo_) cudaFree(dZuptInfo_);
-  if (hZuptDec_) cudaFreeHost(hZuptDec_);
-  if (hZuptInfo_) cudaFreeHost(hZuptInfo_);
-  cudaFree(dHblk_); cudaFree(dRblk_); cudaFree(dStatus_); cudaFree(dGamma_);
-  if (blob_.dev) cudaFree(blob_.dev);
-  if (blob_.pinned) cudaFreeHost(blob_.pinned);
-  cudaFreeHost(hImu_); cudaFreeHost(hClones_); cudaFreeHost(hDx_);
-  if (hDiag_) cudaFreeHost(hDiag_);
-  if (hStatus_) cudaFreeHost(hStatus_);
-  if (hGamma_) cudaFreeHost(hGamma_);
+  cudaDeviceSynchronize();             // before the buffers are released (members are destroyed after this body)
   for (auto& e : ev_) cudaEventDestroy(e);
   if (ev_fork_) cudaEventDestroy(ev_fork_);
   if (ev_join_) cudaEventDestroy(ev_join_);
@@ -353,7 +306,7 @@ void Batch::set_initial_state(int i, double t, const double* q, const double* p,
 // Write the initial IMU record and covariance of filter i (reference :514-523, :201-225).
 void Batch::init_filter_device(int i) {
   FilterHost& F = f_[i];
-  double* im = hImu_ + (size_t)i * IM_STRIDE;
+  double* im = hImu_.get() + (size_t)i * IM_STRIDE;
   std::memset(im, 0, IM_STRIDE * sizeof(double));
   quat_xyzw_to_R(F.init_q, im + IM_R);
   for (int k = 0; k < 3; ++k) {
@@ -370,75 +323,49 @@ void Batch::init_filter_device(int i) {
   // diagonal) -- a synchronous cudaMemcpy here runs on the legacy default stream, i.e. it waits for and blocks the
   // streams of EVERY batch of the process: with 16-32 replay threads initialising 64 filters each that was thousands of
   // device-wide serialisation points and first frames of up to 1.5 s (ORCVIO_HOST_PROF=3).
-  if (!hDiag_) {
-    CK(cudaMallocHost(&hDiag_, 16 * sizeof(double)));
+  if (!hDiag_.get()) {
+    CKA(hDiag_.alloc(16));
     const double v[5] = {p_.cov_orientation, p_.cov_velocity, p_.cov_position, p_.cov_gyro_bias, p_.cov_acc_bias};
-    for (int k = 0; k < 15; ++k) hDiag_[k] = v[k / 3];
-    hDiag_[15] = 0.0;
+    for (int k = 0; k < 15; ++k) hDiag_.get()[k] = v[k / 3];
+    hDiag_.get()[15] = 0.0;
   }
-  double* dPi = dP_ + (size_t)i * ldp_ * ldp_;
+  double* dPi = dP_.get() + (size_t)i * ldp_ * ldp_;
   CK(cudaMemsetAsync(dPi, 0, (size_t)ldp_ * ldp_ * sizeof(double), stream_));
-  CK(cudaMemcpy2DAsync(dPi, (size_t)(ldp_ + 1) * sizeof(double), hDiag_, sizeof(double), sizeof(double), 15,
+  CK(cudaMemcpy2DAsync(dPi, (size_t)(ldp_ + 1) * sizeof(double), hDiag_.get(), sizeof(double), sizeof(double), 15,
                        cudaMemcpyHostToDevice, stream_));
 }
 
-// ORCVIO_HOST_PROF=3: every growth of a device / pinned buffer after construction (a device-wide synchronisation that
-// stalls all the batches of the process) is reported
-static void note_growth(const char* what, size_t bytes) {
-  static const bool on = env_int("ORCVIO_HOST_PROF", 0) == 3;
-  if (on) std::fprintf(stderr, "[replay prof] growth: %s -> %.1f MB\n", what, bytes / 1048576.0);
+void Batch::ensure_scratch(size_t n_cand, size_t hblk, size_t rblk) {
+  CKA(dHblk_.grow(hblk, hblk * 2 + 1024, "hblk / rblk"));
+  CKA(dRblk_.grow(rblk, rblk * 2 + 1024, "hblk / rblk"));
+  CKA(dStatus_.grow(n_cand, n_cand * 2 + 1024, "candidate status"));
+  CKA(dGamma_.grow(n_cand, n_cand * 2 + 1024, "candidate gamma"));
+  CKA(hStatus_.grow(n_cand, n_cand * 2 + 1024, "candidate status (pinned)"));
+  CKA(hGamma_.grow(n_cand, n_cand * 2 + 1024, "candidate gamma (pinned)"));
 }
 
-void Batch::ensure_scratch(size_t n_cand, size_t hblk, size_t rblk) {
-  auto grow = [&](double*& ptr, size_t& cap, size_t need) {
-    if (need <= cap) return;
-    if (ptr) cudaFree(ptr);
-    cap = need * 2 + 1024;
-    note_growth("hblk / rblk", cap * sizeof(double));
-    CK(cudaMalloc(&ptr, cap * sizeof(double)));
-  };
-  grow(dHblk_, hblk_cap_, hblk);
-  grow(dRblk_, rblk_cap_, rblk);
-  if (n_cand > cand_cap_) {
-    if (dStatus_) cudaFree(dStatus_);
-    if (dGamma_) cudaFree(dGamma_);
-    cand_cap_ = n_cand * 2 + 1024;
-    note_growth("candidate status", cand_cap_ * 12);
-    CK(cudaMalloc(&dStatus_, cand_cap_ * sizeof(int)));
-    CK(cudaMalloc(&dGamma_, cand_cap_ * sizeof(double)));
-  }
-  if (n_cand > hcand_cap_) {
-    if (hStatus_) cudaFreeHost(hStatus_);
-    if (hGamma_) cudaFreeHost(hGamma_);
-    hcand_cap_ = n_cand * 2 + 1024;
-    note_growth("candidate status (pinned)", hcand_cap_ * 12);
-    CK(cudaMallocHost(&hStatus_, hcand_cap_ * sizeof(int)));
-    CK(cudaMallocHost(&hGamma_, hcand_cap_ * sizeof(double)));
-  }
+// A and the split-K partials of the update (x 2 growth)
+cudaError_t Batch::grow_update_scratch(size_t need_a, size_t need_p) {
+  const bool ok = dAmat_.grow(need_a, need_a * 2, "A") && dPart_.grow(need_p, need_p * 2, "split-K partials");
+  return ok ? cudaSuccess : cudaErrorMemoryAllocation;
 }
 
 void Batch::upload_blob() {
   if (blob_.used == 0) return;
-  if (blob_.used > blob_.dev_cap) {
-    if (blob_.dev) cudaFree(blob_.dev);
-    blob_.dev_cap = blob_.used * 2 + 4096;
-    note_growth("work-list blob", blob_.dev_cap);
-    CK(cudaMalloc(&blob_.dev, blob_.dev_cap));
-  }
   if (upload_on_side_stream_) {
     // kernels of this frame are already queued on stream_ (early triangulation / Jacobian pass): a copy on the
     // same stream would wait for them, so the blob goes up on its own stream and stream_ joins it afterwards
-    CK(cudaMemcpyAsync(blob_.dev, blob_.pinned, blob_.used, cudaMemcpyHostToDevice, stream_up_));
+    CK(blob_.upload(stream_up_));
     CK(cudaEventRecord(ev_up_, stream_up_));
     CK(cudaStreamWaitEvent(stream_, ev_up_, 0));
   } else {
-    CK(cudaMemcpyAsync(blob_.dev, blob_.pinned, blob_.used, cudaMemcpyHostToDevice, stream_));
+    CK(blob_.upload(stream_));
   }
 }
 
 void Batch::download_mirrors() {
-  CK(cudaMemcpyAsync(hImu_, dImu_, (size_t)B_ * IM_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-  CK(cudaMemcpyAsync(hClones_, dClones_, (size_t)B_ * Ncap_ * CL_STRIDE * sizeof(double),
+  CK(cudaMemcpyAsync(hImu_.get(), dImu_.get(), (size_t)B_ * IM_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  CK(cudaMemcpyAsync(hClones_.get(), dClones_.get(), (size_t)B_ * Ncap_ * CL_STRIDE * sizeof(double),
                      cudaMemcpyDeviceToHost, stream_));
 }
 
@@ -474,7 +401,7 @@ void Batch::stage_pack(PhaseWork& w) {
   const size_t o_s = blob_.reserve(sizeof(int) * std::max<size_t>(w.small_list.size(), 1));
   const size_t o_l = blob_.reserve(sizeof(int) * std::max<size_t>(w.large_list.size(), 1));
   const size_t o_x = blob_.reserve(sizeof(int) * std::max<size_t>(w.extra_ints.size(), 1));
-  char* h = blob_.pinned;
+  char* h = blob_.pinned.get();
   if (!w.extra_ints.empty()) std::memcpy(h + o_x, w.extra_ints.data(), sizeof(int) * w.extra_ints.size());
   if (nC && up_c) std::memcpy(h + o_c, w.cands.data(), sizeof(Cand) * nC);
   if (n_obs) {
@@ -496,38 +423,15 @@ void Batch::stage_upload(PhaseWork& w) {
                o_l = w.off[6], o_x = w.off[7];
   ensure_scratch(std::max(nC, 1), std::max<size_t>(w.hblk_total, 1), std::max<size_t>(w.rows_total, 1));
   // scratch of the update, grown outside any timed region
-  if (w.tiles.size() > tilerows_cap_) {
-    if (dTileRows_) cudaFree(dTileRows_);
-    tilerows_cap_ = w.tiles.size() * 2 + 64;
-    note_growth("tile rows", tilerows_cap_ * sizeof(int));
-    CK(cudaMalloc(&dTileRows_, tilerows_cap_ * sizeof(int)));
-  }
+  CKA(dTileRows_.grow(w.tiles.size(), w.tiles.size() * 2 + 64, "tile rows"));
   int units = 1;
   for (const FilterWork& f : w.fw) units = std::max(units, syrk_plan(f, n_sm_).total);
   w.syrk_units = units;
-  const size_t need_a = (w.arows_total + 16) * (size_t)ldr_;
-  if (need_a > amat_cap_) {
-    if (dAmat_) cudaFree(dAmat_);
-    amat_cap_ = need_a * 2;
-    note_growth("A", amat_cap_ * sizeof(double));
-    CK(cudaMalloc(&dAmat_, amat_cap_ * sizeof(double)));
-  }
-  const size_t need_p = (size_t)B_ * units * 4096;
-  if (need_p > part_cap_) {
-    if (dPart_) cudaFree(dPart_);
-    part_cap_ = need_p * 2;
-    note_growth("split-K partials", part_cap_ * sizeof(double));
-    CK(cudaMalloc(&dPart_, part_cap_ * sizeof(double)));
-  }
+  CK(grow_update_scratch((w.arows_total + 16) * (size_t)ldr_, (size_t)B_ * units * 4096));
   if (hybrid_ && w.hyb_phase >= 0) {
     HybridBufs& hb = *hyb_;
     const size_t need_h = (w.dense_total + 8) * (size_t)ldr_;
-    if (need_h > hb.hd_cap) {
-      if (hb.dHd) cudaFree(hb.dHd);
-      hb.hd_cap = need_h * 2;
-      note_growth("hybrid dense rows", hb.hd_cap * sizeof(double));
-      CK(cudaMalloc(&hb.dHd, hb.hd_cap * sizeof(double)));
-    }
+    CKA(hb.dHd.grow(need_h, need_h * 2, "hybrid dense rows"));
     bool okp = true;
     w.dHw = hb.put(w.hw.data(), w.hw.size(), stream_, &okp);
     w.dHfeats = hb.put(w.hfeats.data(), w.hfeats.size(), stream_, &okp);
@@ -535,7 +439,7 @@ void Batch::stage_upload(PhaseWork& w) {
     if (!okp) { ok_ = false; err_ = "hybrid upload arena exhausted"; }
   }
   upload_blob();
-  char* d = blob_.dev;
+  char* d = blob_.dev.get();
   w.dC = (const Cand*)(d + o_c);
   w.dOc = w.obs_preuploaded ? w.pre_dOc : (const int*)(d + o_oc);
   w.dOz = w.obs_preuploaded ? w.pre_dOz : (const double*)(d + o_oz);
@@ -554,12 +458,12 @@ void Batch::stage_phase(PhaseWork& w) {
 UpdArgs Batch::upd_args(const FilterWork* dFw) const {
   UpdArgs ua{};
   ua.fw = dFw; ua.n_filters = B_;
-  ua.P = dP_; ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
+  ua.P = dP_.get(); ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
   ua.r_stride = (size_t)(nmax_ + 1) * ldr_; ua.ldr = ldr_;
-  ua.T = dT_; ua.S = dS_; ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
-  ua.yv = dYv_;
-  ua.imu = dImu_; ua.clones = dClones_; ua.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-  ua.dx = dDx_; ua.lddx = ldp_;
+  ua.T = dT_.get(); ua.S = dS_.get(); ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
+  ua.yv = dYv_.get();
+  ua.imu = dImu_.get(); ua.clones = dClones_.get(); ua.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+  ua.dx = dDx_.get(); ua.lddx = ldp_;
   ua.flags = flags_; ua.sigma2 = p_.feature_observation_noise;
   return ua;
 }
@@ -568,17 +472,17 @@ HybArgs Batch::hyb_args(const PhaseWork& w) const {
   const HybridBufs& hb = *hyb_;
   HybArgs ha{};
   ha.hw = w.dHw; ha.n_filters = B_; ha.feats = w.dHfeats; ha.news = w.dHnews;
-  ha.clones = dClones_; ha.clone_stride = (size_t)Ncap_ * CL_STRIDE; ha.imu = dImu_;
-  ha.fpos = dFpos_; ha.fidp = dFidp_; ha.fcap = Fcap_;
-  ha.P = dP_; ha.p_stride = (size_t)ldp_ * ldp_; ha.ldp = ldp_;
+  ha.clones = dClones_.get(); ha.clone_stride = (size_t)Ncap_ * CL_STRIDE; ha.imu = dImu_.get();
+  ha.fpos = dFpos_.get(); ha.fidp = dFidp_.get(); ha.fcap = Fcap_;
+  ha.P = dP_.get(); ha.p_stride = (size_t)ldp_ * ldp_; ha.ldp = ldp_;
   ha.obs_clone = w.dOc; ha.obs_z = w.dOz;
-  ha.status = dStatus_;
+  ha.status = dStatus_.get();
   ha.sigma2 = p_.feature_observation_noise; ha.chi2_dof2 = chi2_host_[2];
-  ha.Hd = hb.dHd; ha.ldh = ldr_;
-  ha.H1 = hb.dH1; ha.h2 = hb.dh2; ha.r1 = hb.dr1; ha.new_cap = Emax_;
-  ha.scratch = hb.dScratch;
-  ha.ekf_pass = hb.dEkfPass; ha.ekf_gamma = hb.dEkfGamma; ha.new_ok = hb.dNewOk; ha.n_new = hb.dNNew;
-  ha.dx = dDx_; ha.lddx = ldp_;
+  ha.Hd = hb.dHd.get(); ha.ldh = ldr_;
+  ha.H1 = hb.dH1.get(); ha.h2 = hb.dh2.get(); ha.r1 = hb.dr1.get(); ha.new_cap = Emax_;
+  ha.scratch = hb.dScratch.get();
+  ha.ekf_pass = hb.dEkfPass.get(); ha.ekf_gamma = hb.dEkfGamma.get(); ha.new_ok = hb.dNewOk.get(); ha.n_new = hb.dNNew.get();
+  ha.dx = dDx_.get(); ha.lddx = ldp_;
   return ha;
 }
 
@@ -598,7 +502,7 @@ void Batch::launch_phase(PhaseWork& w, bool download, bool prior_in_flight) {
     // big CTA waits for an empty SM behind the first waves of k_triangulate
     CK(cudaEventRecord(ev_fork_, stream_));
     InfoBufs ib{};
-    ib.Ls = dLs_; ib.ls_done = ev_ls_;
+    ib.Ls = dLs_.get(); ib.ls_done = ev_ls_;
     launch_info_prior(upd_args(dFw), ib, w.maxN, stream2_, ev_fork_, ev_join_, profiling_ ? e[9] : nullptr,
                       profiling_ ? e[10] : nullptr, w.maxE);
     nl += 2;                               // k_chol_prior + k_imu_factor
@@ -607,21 +511,17 @@ void Batch::launch_phase(PhaseWork& w, bool download, bool prior_in_flight) {
   const bool hyb_on = hybrid_ && w.hyb_phase >= 0 && do_update;
   HybArgs ha{};
   if (hyb_on) ha = hyb_args(w);
-  if (want_iters_ && (size_t)nC > iters_cap_) {
-    if (dIters_) cudaFree(dIters_);
-    if (dCost_) cudaFree(dCost_);
-    iters_cap_ = (size_t)nC * 2 + 64;
-    CK(cudaMalloc(&dIters_, iters_cap_ * 2 * sizeof(int)));
-    CK(cudaMalloc(&dCost_, iters_cap_ * sizeof(double)));
+  if (want_iters_) {
+    const size_t cap = (size_t)nC * 2 + 64;
+    CKA(dIters_.grow((size_t)nC * 2, cap * 2, "triangulation iterations"));
+    CKA(dCost_.grow(nC, cap, "triangulation cost"));
   }
-  if (want_raw_ && w.n_obs() > raw_cap_) {
-    for (double** p : {&dRawHx_, &dRawHe_, &dRawHf_, &dRawR_})
-      if (*p) cudaFree(*p);
-    raw_cap_ = w.n_obs() * 2 + 64;
-    CK(cudaMalloc(&dRawHx_, raw_cap_ * 12 * sizeof(double)));
-    CK(cudaMalloc(&dRawHe_, raw_cap_ * 12 * sizeof(double)));
-    CK(cudaMalloc(&dRawHf_, raw_cap_ * 6 * sizeof(double)));
-    CK(cudaMalloc(&dRawR_, raw_cap_ * 2 * sizeof(double)));
+  if (want_raw_) {
+    const size_t n = w.n_obs(), cap = n * 2 + 64;
+    CKA(dRawHx_.grow(n * 12, cap * 12, "raw Jacobians"));
+    CKA(dRawHe_.grow(n * 12, cap * 12, "raw Jacobians"));
+    CKA(dRawHf_.grow(n * 6, cap * 6, "raw Jacobians"));
+    CKA(dRawR_.grow(n * 2, cap * 2, "raw residuals"));
   }
   // k_jac_gate follows k_triangulate candidate by candidate (completion flags + programmatic launch) instead of
   // waiting for the slowest LM chain of the whole grid; ORCVIO_TRI_OVERLAP=0 restores the grid-wide dependency
@@ -633,44 +533,42 @@ void Batch::launch_phase(PhaseWork& w, bool download, bool prior_in_flight) {
   const bool overlap = overlap_env && tri_here && !skip_jac_ && !jac_done_early_ && !want_iters_ && !want_raw_ &&
                        nC >= overlap_min;
   if (overlap) {
-    if ((size_t)nC > tridone_cap_) {
-      if (dTriDone_) cudaFree(dTriDone_);
-      tridone_cap_ = (size_t)nC * 2 + 1024;
-      CK(cudaMalloc(&dTriDone_, tridone_cap_ * sizeof(int)));
-      CK(cudaMemsetAsync(dTriDone_, 0, tridone_cap_ * sizeof(int), stream_));
+    if ((size_t)nC > dTriDone_.size()) {
+      CKA(dTriDone_.grow(nC, (size_t)nC * 2 + 1024, "triangulation flags"));
+      CK(cudaMemsetAsync(dTriDone_.get(), 0, dTriDone_.bytes(), stream_));
     }
     ++tri_epoch_;
     // (inside a graph the epoch is a baked-in constant: the flags are cleared by a node of the graph instead)
-    if (graph_capturing_) CK(cudaMemsetAsync(dTriDone_, 0, (size_t)nC * sizeof(int), stream_));
+    if (graph_capturing_) CK(cudaMemsetAsync(dTriDone_.get(), 0, (size_t)nC * sizeof(int), stream_));
   }
   if (tri_here) {
     TriArgs ta{};
-    ta.done = overlap ? dTriDone_ : nullptr; ta.epoch = tri_epoch_;
+    ta.done = overlap ? dTriDone_.get() : nullptr; ta.epoch = tri_epoch_;
     ta.cand = dC; ta.n_cand = nC;
-    ta.clones = dClones_; ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    ta.fpos = dFpos_; ta.fgen = dFgen_; ta.fcap = Fcap_;
+    ta.clones = dClones_.get(); ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+    ta.fpos = dFpos_.get(); ta.fgen = dFgen_.get(); ta.fcap = Fcap_;
     ta.obs_clone = dOc; ta.obs_z = dOz;
     ta.cfg = tricfg_;
-    ta.status = dStatus_;
-    ta.iters = want_iters_ ? dIters_ : nullptr;
-    ta.cost = want_iters_ ? dCost_ : nullptr;
+    ta.status = dStatus_.get();
+    ta.iters = want_iters_ ? dIters_.get() : nullptr;
+    ta.cost = want_iters_ ? dCost_.get() : nullptr;
     launch_triangulate(ta, stream_);
     ++nl;
   }
   if (profiling_ && !overlap) CK(cudaEventRecord(e[1], stream_));   // (an event between the two would serialise them)
   if (nC > 0 && !skip_jac_ && !jac_done_early_) {
     JacArgs ja{};
-    ja.tri_done = overlap ? dTriDone_ : nullptr; ja.tri_epoch = tri_epoch_;
+    ja.tri_done = overlap ? dTriDone_.get() : nullptr; ja.tri_epoch = tri_epoch_;
     ja.cand = dC;
-    ja.clones = dClones_; ja.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    ja.imu = dImu_; ja.fpos = dFpos_; ja.fcap = Fcap_;
-    ja.P = dP_; ja.p_stride = (size_t)ldp_ * ldp_; ja.ldp = ldp_;
+    ja.clones = dClones_.get(); ja.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+    ja.imu = dImu_.get(); ja.fpos = dFpos_.get(); ja.fcap = Fcap_;
+    ja.P = dP_.get(); ja.p_stride = (size_t)ldp_ * ldp_; ja.ldp = ldp_;
     ja.obs_clone = dOc; ja.obs_z = dOz;
-    ja.flags = flags_; ja.sigma2 = p_.feature_observation_noise; ja.chi2 = dChi2_;
-    ja.status = dStatus_; ja.gamma = dGamma_;
-    ja.hblk = dHblk_; ja.rblk = dRblk_;
-    if (want_raw_) { ja.raw_Hx = dRawHx_; ja.raw_He = dRawHe_; ja.raw_Hf = dRawHf_; ja.raw_r = dRawR_; }
-    ja.tri_status_f = tri_done_early_ ? dStatusF_ : nullptr;
+    ja.flags = flags_; ja.sigma2 = p_.feature_observation_noise; ja.chi2 = dChi2_.get();
+    ja.status = dStatus_.get(); ja.gamma = dGamma_.get();
+    ja.hblk = dHblk_.get(); ja.rblk = dRblk_.get();
+    if (want_raw_) { ja.raw_Hx = dRawHx_.get(); ja.raw_He = dRawHe_.get(); ja.raw_Hf = dRawHf_.get(); ja.raw_r = dRawR_.get(); }
+    ja.tri_status_f = tri_done_early_ ? dStatusF_.get() : nullptr;
     JacArgs js = ja, jl = ja;
     js.cand_list = dSmall; js.n_list = (int)w.small_list.size();
     jl.cand_list = dLarge; jl.n_list = (int)w.large_list.size();
@@ -685,20 +583,20 @@ void Batch::launch_phase(PhaseWork& w, bool download, bool prior_in_flight) {
   if (profiling_) CK(cudaEventRecord(e[2], stream_));
   if (do_update) {
     AformArgs qa{};
-    qa.cand = dC; qa.status = dStatus_;
-    qa.status_f = jac_done_early_ ? dStatusF_ : nullptr;
+    qa.cand = dC; qa.status = dStatus_.get();
+    qa.status_f = jac_done_early_ ? dStatusF_.get() : nullptr;
     if (jac_done_early_ && w.cands_stay_on_host) {
       qa.order_f = w.d_extra;
       qa.feat_off = dir_feat_off_; qa.rowoff_f = dir_rowoff_; qa.hblkoff_f = dir_hblkoff_;
       qa.sblk_f = dir_sblk_; qa.eblk_f = dir_eblk_;
     }
-    qa.hblk = dHblk_; qa.rblk = dRblk_;
+    qa.hblk = dHblk_.get(); qa.rblk = dRblk_.get();
     qa.tiles = dTiles;
     qa.fw = dFw;
     InfoBufs ib{};
-    ib.Ls = dLs_; ib.Amat = dAmat_; ib.part = dPart_; ib.ls_done = ev_ls_;
-    ib.max_units = w.syrk_units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_;
-    ib.tile_rows = dTileRows_; ib.filter_rows = dFilterRows_;
+    ib.Ls = dLs_.get(); ib.Amat = dAmat_.get(); ib.part = dPart_.get(); ib.ls_done = ev_ls_;
+    ib.max_units = w.syrk_units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_.get();
+    ib.tile_rows = dTileRows_.get(); ib.filter_rows = dFilterRows_.get();
     launch_info_update(qa, upd_args(dFw), ib, (int)w.tiles.size(), w.max_tile_rows, w.wmax_blk, w.maxN, stream_,
                        stream2_, ev_fork_, ev_join_, profiling_ ? e[3] : nullptr, profiling_ ? e[4] : nullptr, &nl,
                        prior_in_flight, profiling_ ? e[8] : nullptr, profiling_ ? e[9] : nullptr,
@@ -714,8 +612,8 @@ void Batch::launch_phase(PhaseWork& w, bool download, bool prior_in_flight) {
   tri_done_early_ = false;
   if (launch_error_count() > 0) { ok_ = false; err_ = "kernel launch failed"; }
   if (nC > 0 && download) {
-    CK(cudaMemcpyAsync(hStatus_, jac_done_early_ ? dStatusF_ : dStatus_, sizeof(int) * nC, cudaMemcpyDeviceToHost, stream_));
-    CK(cudaMemcpyAsync(hGamma_, jac_done_early_ ? dGammaF_ : dGamma_, sizeof(double) * nC, cudaMemcpyDeviceToHost, stream_));
+    CK(cudaMemcpyAsync(hStatus_.get(), jac_done_early_ ? dStatusF_.get() : dStatus_.get(), sizeof(int) * nC, cudaMemcpyDeviceToHost, stream_));
+    CK(cudaMemcpyAsync(hGamma_.get(), jac_done_early_ ? dGammaF_.get() : dGamma_.get(), sizeof(double) * nC, cudaMemcpyDeviceToHost, stream_));
   }
   jac_done_early_ = false;
 }
@@ -966,17 +864,9 @@ int Batch::replay(int n_frames, const double* t_img, const OrcvioFeature* const*
                   double* state17_out, double* cov15_out) {
   if (cov15_out && n_frames > 0) {
     const size_t need = (size_t)B_ * n_frames * 225;
-    if (need > covhist_cap_) {                           // grown ahead of the loop, never inside it
+    if (need > dCovHist_.size()) {                       // grown ahead of the loop, never inside it
       cudaSetDevice(dev_);
-      if (dCovHist_) cudaFree(dCovHist_);
-      dCovHist_ = nullptr;
-      covhist_cap_ = 0;
-      note_growth("covariance history", need * sizeof(double));
-      if (cudaMalloc(&dCovHist_, need * sizeof(double)) != cudaSuccess) {
-        dCovHist_ = nullptr;
-        return ORCVIO_ERR_CUDA;
-      }
-      covhist_cap_ = need;
+      if (!dCovHist_.grow(need, need, "covariance history")) return ORCVIO_ERR_CUDA;
     }
   }
   std::vector<const OrcvioFeature*> fp(B_);
@@ -1023,12 +913,12 @@ int Batch::replay(int n_frames, const double* t_img, const OrcvioFeature* const*
       }
     }
     if (cov15_out) {
-      launch_capture_imu_cov(dP_, (size_t)ldp_ * ldp_, ldp_, B_, dCovHist_, n_frames, f, stream_);
+      launch_capture_imu_cov(dP_.get(), (size_t)ldp_ * ldp_, ldp_, B_, dCovHist_.get(), n_frames, f, stream_);
       ++launches_;
     }
   }
   if (cov15_out && n_frames > 0) {
-    CK(cudaMemcpyAsync(cov15_out, dCovHist_, (size_t)B_ * n_frames * 225 * sizeof(double), cudaMemcpyDeviceToHost,
+    CK(cudaMemcpyAsync(cov15_out, dCovHist_.get(), (size_t)B_ * n_frames * 225 * sizeof(double), cudaMemcpyDeviceToHost,
                        stream_));
     CK(cudaStreamSynchronize(stream_));
     if (launch_error_count() > 0) { ok_ = false; err_ = "kernel launch failed"; }
@@ -1110,12 +1000,12 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       if (useful >= nimu) --useful;
       if (useful < 0) continue;
       init_filter_device(fi);
-      double* hm = hImu_ + (size_t)fi * IM_STRIDE;
+      double* hm = hImu_.get() + (size_t)fi * IM_STRIDE;
       for (int k = 0; k < 3; ++k) {
         hm[IM_GOLD + k] = im[useful].gyro[k];
         hm[IM_AOLD + k] = im[useful].acc[k];
       }
-      CK(cudaMemcpyAsync(dImu_ + (size_t)fi * IM_STRIDE, hm, IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
+      CK(cudaMemcpyAsync(dImu_.get() + (size_t)fi * IM_STRIDE, hm, IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
       need_imu_upload = true;
       prefix = useful;
       F.gravity_set = true;
@@ -1233,7 +1123,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     const size_t o_d = blob_.reserve(sizeof(int) * B_);
     const size_t o_n = blob_.reserve(sizeof(int) * B_);
     const size_t o_e = blob_.reserve(sizeof(int) * B_);
-    char* h = blob_.pinned;
+    char* h = blob_.pinned.get();
     std::memcpy(h + o_e, Evec.data(), sizeof(int) * B_);
     if (!samples.empty()) std::memcpy(h + o_s, samples.data(), sizeof(PropSample) * samples.size());
     std::memcpy(h + o_o, samp_off.data(), sizeof(int) * (B_ + 1));
@@ -1275,7 +1165,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       o_zm = blob_.reserve(sizeof(int) * B_);
       o_zn = blob_.reserve(sizeof(int) * B_);
       o_zc = blob_.reserve(sizeof(double) * B_);
-      h = blob_.pinned;
+      h = blob_.pinned.get();
       std::memcpy(h + o_zm, zmode.data(), sizeof(int) * B_);
       std::memcpy(h + o_zn, zN.data(), sizeof(int) * B_);
       std::memcpy(h + o_zc, zchk.data(), sizeof(double) * B_);
@@ -1283,38 +1173,38 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     upload_blob();
     if (profiling_) CK(cudaEventRecord(ev_[6], stream_));
     PropArgs pa{};
-    pa.P = dP_; pa.p_stride = (size_t)ldp_ * ldp_; pa.ldp = ldp_;
-    pa.imu = dImu_;
-    pa.samples = (const PropSample*)(blob_.dev + o_s);
-    pa.samp_off = (const int*)(blob_.dev + o_o);
-    pa.D = (const int*)(blob_.dev + o_d);
+    pa.P = dP_.get(); pa.p_stride = (size_t)ldp_ * ldp_; pa.ldp = ldp_;
+    pa.imu = dImu_.get();
+    pa.samples = (const PropSample*)(blob_.dev.get() + o_s);
+    pa.samp_off = (const int*)(blob_.dev.get() + o_o);
+    pa.D = (const int*)(blob_.dev.get() + o_d);
     pa.n_filters = B_; pa.flags = flags_;
     pa.qc[0] = p_.imu_gyro_noise; pa.qc[1] = p_.imu_acc_noise;
     pa.qc[2] = p_.imu_gyro_bias_noise; pa.qc[3] = p_.imu_acc_bias_noise;
     launch_propagate(pa, stream_);
     AugArgs aa{};
-    aa.P = dP_; aa.p_stride = pa.p_stride; aa.ldp = ldp_;
-    aa.imu = dImu_; aa.clones = dClones_; aa.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    aa.N = (const int*)(blob_.dev + o_n); aa.n_filters = B_;
-    aa.E = hybrid_ ? (const int*)(blob_.dev + o_e) : nullptr;
+    aa.P = dP_.get(); aa.p_stride = pa.p_stride; aa.ldp = ldp_;
+    aa.imu = dImu_.get(); aa.clones = dClones_.get(); aa.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+    aa.N = (const int*)(blob_.dev.get() + o_n); aa.n_filters = B_;
+    aa.E = hybrid_ ? (const int*)(blob_.dev.get() + o_e) : nullptr;
     launch_augment(aa, stream_);
     launches_ += 2;
     if (any_zupt) {
       ZuptArgs za{};
-      za.P = dP_; za.p_stride = pa.p_stride; za.ldp = ldp_;
-      za.imu = dImu_; za.clones = dClones_; za.clone_stride = aa.clone_stride;
+      za.P = dP_.get(); za.p_stride = pa.p_stride; za.ldp = ldp_;
+      za.imu = dImu_.get(); za.clones = dClones_.get(); za.clone_stride = aa.clone_stride;
       za.samples = pa.samples; za.samp_off = pa.samp_off;
-      za.N = (const int*)(blob_.dev + o_zn);
-      za.mode = (const int*)(blob_.dev + o_zm);
-      za.chi2_check = (const double*)(blob_.dev + o_zc);
-      za.decision = dZuptDec_; za.info = dZuptInfo_;
-      za.dx = dDx_; za.lddx = ldp_;
+      za.N = (const int*)(blob_.dev.get() + o_zn);
+      za.mode = (const int*)(blob_.dev.get() + o_zm);
+      za.chi2_check = (const double*)(blob_.dev.get() + o_zc);
+      za.decision = dZuptDec_.get(); za.info = dZuptInfo_.get();
+      za.dx = dDx_.get(); za.lddx = ldp_;
       za.n_filters = B_; za.flags = flags_;
       za.noise_v = p_.zupt_noise_v; za.noise_p = p_.zupt_noise_p; za.noise_q = p_.zupt_noise_q;
       launch_zupt(za, stream_);
       ++launches_;
-      CK(cudaMemcpyAsync(hZuptDec_, dZuptDec_, sizeof(int) * B_, cudaMemcpyDeviceToHost, stream_));
-      CK(cudaMemcpyAsync(hZuptInfo_, dZuptInfo_, sizeof(double) * 2 * B_, cudaMemcpyDeviceToHost, stream_));
+      CK(cudaMemcpyAsync(hZuptDec_.get(), dZuptDec_.get(), sizeof(int) * B_, cudaMemcpyDeviceToHost, stream_));
+      CK(cudaMemcpyAsync(hZuptInfo_.get(), dZuptInfo_.get(), sizeof(double) * 2 * B_, cudaMemcpyDeviceToHost, stream_));
     }
     if (profiling_) {
       CK(cudaEventRecord(ev_[7], stream_));
@@ -1332,9 +1222,9 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       for (int fi = 0; fi < B_; ++fi) {
         FilterHost& F = f_[fi];
         if (!F.active) continue;
-        F.if_zupt = hZuptDec_[fi] != 0;
-        F.zupt_chi2 = hZuptInfo_[2 * fi];
-        F.zupt_vnorm = hZuptInfo_[2 * fi + 1];
+        F.if_zupt = hZuptDec_.get()[fi] != 0;
+        F.zupt_chi2 = hZuptInfo_.get()[2 * fi];
+        F.zupt_vnorm = hZuptInfo_.get()[2 * fi + 1];
         F.stats.zupt = F.if_zupt ? 1 : 0;
         F.stats.zupt_chi2 = F.zupt_chi2;
         F.stats.zupt_vnorm = F.zupt_vnorm;
@@ -1459,7 +1349,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     if (any_compact) {
       const int* d_ni = hb->put(newidx.data(), newidx.size(), stream_, &hyb_ok);
       const int* d_do = hb->put(Dold.data(), Dold.size(), stream_, &hyb_ok);
-      if (hyb_ok) { launch_compact_cov(dP_, (size_t)ldp_ * ldp_, ldp_, d_ni, d_do, B_, stream_); ++launches_; }
+      if (hyb_ok) { launch_compact_cov(dP_.get(), (size_t)ldp_ * ldp_, ldp_, d_ni, d_do, B_, stream_); ++launches_; }
     }
   }
   auto grid_code = [&](const Track& tr) {   // :2286-2289 / :3841-3845 (the casts truncate toward zero)
@@ -1524,28 +1414,23 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
   std::vector<CommitRec> commits;
   if (hybrid_ && !wS.cands.empty()) {
     const size_t nS = wS.cands.size();
-    if (nS > hb->spec_cap) {
-      cudaFree(hb->dFinal); cudaFree(hb->dSpecStatus);
-      if (hb->hSpecStatus) cudaFreeHost(hb->hSpecStatus);
-      hb->spec_cap = nS * 2 + 64;
-      note_growth("speculative triangulation (device + pinned)", hb->spec_cap * 28);
-      CK(cudaMalloc(&hb->dFinal, hb->spec_cap * 3 * sizeof(double)));
-      CK(cudaMalloc(&hb->dSpecStatus, hb->spec_cap * sizeof(int)));
-      CK(cudaMallocHost(&hb->hSpecStatus, hb->spec_cap * sizeof(int)));
-    }
+    const size_t cap = nS * 2 + 64;
+    CKA(hb->dFinal.grow(nS * 3, cap * 3, "speculative triangulation"));
+    CKA(hb->dSpecStatus.grow(nS, cap, "speculative triangulation"));
+    CKA(hb->hSpecStatus.grow(nS, cap, "speculative triangulation (pinned)"));
     TriArgs ta{};
     ta.cand = hb->put(wS.cands.data(), nS, stream_, &hyb_ok); ta.n_cand = (int)nS;
-    ta.clones = dClones_; ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    ta.fpos = hb->dSpecPos; ta.fgen = hb->dSpecGen; ta.fcap = Fcap_;
+    ta.clones = dClones_.get(); ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+    ta.fpos = hb->dSpecPos.get(); ta.fgen = hb->dSpecGen.get(); ta.fcap = Fcap_;
     ta.obs_clone = hb->put(wS.obs_clone.data(), wS.obs_clone.size(), stream_, &hyb_ok);
     ta.obs_z = hb->put(wS.obs_z.data(), wS.obs_z.size(), stream_, &hyb_ok);
     ta.cfg = tricfg_;
-    ta.status = hb->dSpecStatus;
-    ta.final_pos = hb->dFinal;
+    ta.status = hb->dSpecStatus.get();
+    ta.final_pos = hb->dFinal.get();
     if (hyb_ok) {
       launch_triangulate(ta, stream_);
       ++launches_;
-      CK(cudaMemcpyAsync(hb->hSpecStatus, hb->dSpecStatus, nS * sizeof(int), cudaMemcpyDeviceToHost, stream_));
+      CK(cudaMemcpyAsync(hb->hSpecStatus.get(), hb->dSpecStatus.get(), nS * sizeof(int), cudaMemcpyDeviceToHost, stream_));
       CK(cudaStreamSynchronize(stream_));
     }
   }
@@ -1570,7 +1455,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
         if (!tr.ekf_feature) {
           tr.gen = pr.spec_gen;                                      // is_initialized = false
           tr.initialized = false;
-          if (!(hb->hSpecStatus[pr.spec] & ST_TRI_VALID)) continue;  // checkMotion / triangulation failed (:2297-2303)
+          if (!(hb->hSpecStatus.get()[pr.spec] & ST_TRI_VALID)) continue;  // checkMotion / triangulation failed (:2297-2303)
           tr.ekf_feature = true;
           tr.initialized = true;
           for (int k = (int)tr.obs.size() - 1; k >= 0; --k)          // anchor = the last camera used (feature.hpp:536)
@@ -1653,7 +1538,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
   if (hybrid_ && !commits.empty()) {
     const CommitRec* d_rec = hb->put(commits.data(), commits.size(), stream_, &hyb_ok);
     if (hyb_ok) {
-      launch_hybrid_commit(d_rec, (int)commits.size(), hb->dFinal, hb->dSpecPos, dFpos_, dFgen_, dFidp_, stream_);
+      launch_hybrid_commit(d_rec, (int)commits.size(), hb->dFinal.get(), hb->dSpecPos.get(), dFpos_.get(), dFgen_.get(), dFidp_.get(), stream_);
       ++launches_;
     }
   }
@@ -1672,8 +1557,8 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     }
     hybrid_queue_gather(gather_tracks);
     if (!wA.hfeats.empty()) {
-      CK(cudaMemcpyAsync(hb->hEkfPass, hb->dEkfPass, wA.hfeats.size() * sizeof(int), cudaMemcpyDeviceToHost, stream_));
-      CK(cudaMemcpyAsync(hb->hEkfGamma, hb->dEkfGamma, wA.hfeats.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+      CK(cudaMemcpyAsync(hb->hEkfPass.get(), hb->dEkfPass.get(), wA.hfeats.size() * sizeof(int), cudaMemcpyDeviceToHost, stream_));
+      CK(cudaMemcpyAsync(hb->hEkfGamma.get(), hb->dEkfGamma.get(), wA.hfeats.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
     }
   }
   download_mirrors();
@@ -1788,23 +1673,23 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     fw.active = 0;
     Nbefore[fi] = fw.N;
     if (!F.active) { Ebefore[fi] = (int)F.feature_states.size(); continue; }
-    std::memcpy(F.imu_mirror.data(), hImu_ + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
-    std::memcpy(F.clone_mirror.data(), hClones_ + (size_t)fi * Ncap_ * CL_STRIDE,
+    std::memcpy(F.imu_mirror.data(), hImu_.get() + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
+    std::memcpy(F.clone_mirror.data(), hClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE,
                 (size_t)Ncap_ * CL_STRIDE * sizeof(double));
     // results of phase A
     const int c0 = wA.cand_begin[fi], c1 = wA.cand_begin[fi + 1];
     for (int c = c0; c < c1; ++c) {
-      const int st = hStatus_[c];
+      const int st = hStatus_.get()[c];
       const CandInfo& ci = F.cinfo[0][c - c0];
       F.cstatus[0].push_back(st);
-      F.cgamma[0].push_back(hGamma_[c]);
+      F.cgamma[0].push_back(hGamma_.get()[c]);
       if (ci.kind == 3) {
         // candidate EKF-SLAM feature: in the state iff its MSCKF rows passed the gate (:2371-2411); a rejected one
         // keeps its inverse-depth record and waits outside the state
         const bool pass = (st & ST_GATE_PASS) != 0;
         F.log_new_ids.push_back(ci.id);
         F.log_new_ok.push_back(pass ? 1 : 0);
-        F.log_new_gamma.push_back(hGamma_[c]);
+        F.log_new_gamma.push_back(hGamma_.get()[c]);
         if (pass) {
           F.find_track(ci.id)->in_state = true;
           F.feature_states.push_back(ci.id);
@@ -1827,9 +1712,9 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       const HybWork& hw = wA.hw[fi];
       for (int i = 0; i < hw.E; ++i) {
         F.log_ekf_ids.push_back(F.feature_states[i]);
-        F.log_ekf_pass.push_back(hb->hEkfPass[hw.feat_begin + i]);
-        F.log_ekf_gamma.push_back(hb->hEkfGamma[hw.feat_begin + i]);
-        if (hb->hEkfPass[hw.feat_begin + i]) ++feature_updates_;
+        F.log_ekf_pass.push_back(hb->hEkfPass.get()[hw.feat_begin + i]);
+        F.log_ekf_gamma.push_back(hb->hEkfGamma.get()[hw.feat_begin + i]);
+        if (hb->hEkfPass.get()[hw.feat_begin + i]) ++feature_updates_;
       }
     }
     fw.D = L + 6 * fw.N + (int)F.feature_states.size();
@@ -1978,7 +1863,7 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     const ReanchorRec* d_rec = hb->put(reanchor.data(), reanchor.size(), stream_, &hyb_ok);
     const int* d_off = hb->put(reanchor_off.data(), reanchor_off.size(), stream_, &hyb_ok);
     if (hyb_ok) {
-      launch_reanchor(d_rec, d_off, B_, wB.dHw, dClones_, (size_t)Ncap_ * CL_STRIDE, dImu_, dFpos_, dFidp_, Fcap_, dP_,
+      launch_reanchor(d_rec, d_off, B_, wB.dHw, dClones_.get(), (size_t)Ncap_ * CL_STRIDE, dImu_.get(), dFpos_.get(), dFidp_.get(), Fcap_, dP_.get(),
                       (size_t)ldp_ * ldp_, ldp_, stream_);
       ++launches_;
     }
@@ -1989,8 +1874,8 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
   for (int v : rm_idx) any_rm |= (v >= 0);
   if (any_rm) {
     RemoveArgs ra{};
-    ra.P = dP_; ra.p_stride = (size_t)ldp_ * ldp_; ra.ldp = ldp_;
-    ra.clones = dClones_; ra.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+    ra.P = dP_.get(); ra.p_stride = (size_t)ldp_ * ldp_; ra.ldp = ldp_;
+    ra.clones = dClones_.get(); ra.clone_stride = (size_t)Ncap_ * CL_STRIDE;
     ra.rm = wB.d_extra; ra.N = wB.d_extra + 2 * B_; ra.n_filters = B_;
     ra.E = hybrid_ ? wB.d_extra + 3 * B_ : nullptr;
     launch_remove(ra, stream_);
@@ -2010,9 +1895,9 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     if (!F.active) continue;
     const int c0 = wB.cand_begin[fi], c1 = wB.cand_begin[fi + 1];
     for (int c = c0; c < c1; ++c) {
-      const int st = hStatus_[c];
+      const int st = hStatus_.get()[c];
       F.cstatus[1].push_back(st);
-      F.cgamma[1].push_back(hGamma_[c]);
+      F.cgamma[1].push_back(hGamma_.get()[c]);
       if (!(st & ST_TRI_VALID)) F.stats.n_tri_invalid_prune++;
       if (st & ST_GATE_PASS) { F.stats.n_gate_pass_prune++; ++feature_updates_; }
     }
@@ -2026,8 +1911,8 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       if (b >= 0) F.clones.erase(F.clones.begin() + b);
       F.clones.erase(F.clones.begin() + a);
     }
-    std::memcpy(F.imu_mirror.data(), hImu_ + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
-    std::memcpy(F.clone_mirror.data(), hClones_ + (size_t)fi * Ncap_ * CL_STRIDE,
+    std::memcpy(F.imu_mirror.data(), hImu_.get() + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
+    std::memcpy(F.clone_mirror.data(), hClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE,
                 (size_t)Ncap_ * CL_STRIDE * sizeof(double));
   }
   g_sp.mark(11);
@@ -2052,25 +1937,20 @@ void Batch::hybrid_queue_gather(std::vector<Track*>& tracks) {
   }
   const size_t n = tracks.size();
   if (n == 0) return;
-  if (n > hb.gather_cap) {             // (the previous gather was consumed behind a synchronisation)
-    cudaFree(hb.dGather);
-    cudaFreeHost(hb.hGather);
-    hb.gather_cap = n * 2;
-    note_growth("hybrid gather (device + pinned)", hb.gather_cap * 6 * sizeof(double));
-    CK(cudaMalloc(&hb.dGather, hb.gather_cap * 6 * sizeof(double)));
-    CK(cudaMallocHost(&hb.hGather, hb.gather_cap * 6 * sizeof(double)));
-  }
+  // (the previous gather was consumed behind a synchronisation)
+  CKA(hb.dGather.grow(n * 6, n * 2 * 6, "hybrid gather"));
+  CKA(hb.hGather.grow(n * 6, n * 2 * 6, "hybrid gather (pinned)"));
   bool okp = true;
   const int* d_f = hb.put(filt.data(), n, stream_, &okp);
   const int* d_s = hb.put(slots.data(), n, stream_, &okp);
   if (!okp) { ok_ = false; err_ = "hybrid upload arena exhausted"; tracks.clear(); return; }
-  launch_hybrid_gather(d_f, d_s, (int)n, dFpos_, dFidp_, Fcap_, hb.dGather, stream_);
+  launch_hybrid_gather(d_f, d_s, (int)n, dFpos_.get(), dFidp_.get(), Fcap_, hb.dGather.get(), stream_);
   ++launches_;
-  CK(cudaMemcpyAsync(hb.hGather, hb.dGather, n * 6 * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  CK(cudaMemcpyAsync(hb.hGather.get(), hb.dGather.get(), n * 6 * sizeof(double), cudaMemcpyDeviceToHost, stream_));
 }
 
 void Batch::hybrid_apply_gather(const std::vector<Track*>& tracks) {
-  const double* g = hyb_->hGather;
+  const double* g = hyb_->hGather.get();
   for (size_t k = 0; k < tracks.size(); ++k) {
     Track& tr = *tracks[k];
     for (int q = 0; q < 3; ++q) tr.mpos[q] = g[6 * k + q];
@@ -2116,7 +1996,7 @@ int Batch::get_state(int i, OrcvioState* out) {
   out->dim = ORCVIO_LEG + 6 * out->n_clones + (int)F.feature_states.size();
   out->n_map_features = (int)F.map_server.size();
   double c9[81];
-  CK(cudaMemcpy2D(c9, 9 * sizeof(double), dP_ + (size_t)i * ldp_ * ldp_, ldp_ * sizeof(double),
+  CK(cudaMemcpy2D(c9, 9 * sizeof(double), dP_.get() + (size_t)i * ldp_ * ldp_, ldp_ * sizeof(double),
                   9 * sizeof(double), 9, cudaMemcpyDeviceToHost));
   // getPpose :3000-3015: [[P_pp, P_po],[P_op, P_oo]]
   for (int a = 0; a < 3; ++a)
@@ -2137,7 +2017,7 @@ int Batch::get_cov(int i, double* P, int cap, int* D) {
   if (!P) return ORCVIO_OK;
   if (cap < d * d) return ORCVIO_ERR_ARG;
   // device is row-major with ld; P is symmetric so the column-major view is identical
-  CK(cudaMemcpy2D(P, d * sizeof(double), dP_ + (size_t)i * ldp_ * ldp_, ldp_ * sizeof(double),
+  CK(cudaMemcpy2D(P, d * sizeof(double), dP_.get() + (size_t)i * ldp_ * ldp_, ldp_ * sizeof(double),
                   d * sizeof(double), d, cudaMemcpyDeviceToHost));
   return ORCVIO_OK;
 }
@@ -2147,8 +2027,8 @@ int Batch::get_map_points(int i, long long* ids, double* xyz, int cap) {
   FilterHost& F = f_[i];
   std::vector<double> fp((size_t)Fcap_ * FP_STRIDE);
   std::vector<long long> fg(Fcap_);
-  CK(cudaMemcpy(fp.data(), dFpos_ + (size_t)i * Fcap_ * FP_STRIDE, fp.size() * sizeof(double), cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(fg.data(), dFgen_ + (size_t)i * Fcap_, fg.size() * sizeof(long long), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(fp.data(), dFpos_.get() + (size_t)i * Fcap_ * FP_STRIDE, fp.size() * sizeof(double), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(fg.data(), dFgen_.get() + (size_t)i * Fcap_, fg.size() * sizeof(long long), cudaMemcpyDeviceToHost));
   int n = 0;
   for (auto& kv : F.map_server) {
     if (n >= cap) break;
@@ -2178,7 +2058,7 @@ int Batch::set_cov(int i, const double* P, int D) {
         for (int c = 0; c < D; ++c)
           if (P[(size_t)r * D + c] != 0.0 || P[(size_t)c * D + r] != 0.0) return ORCVIO_ERR_ARG;
   }
-  CK(cudaMemcpy2D(dP_ + (size_t)i * ldp_ * ldp_, ldp_ * sizeof(double), P, D * sizeof(double),
+  CK(cudaMemcpy2D(dP_.get() + (size_t)i * ldp_ * ldp_, ldp_ * sizeof(double), P, D * sizeof(double),
                   D * sizeof(double), D, cudaMemcpyHostToDevice));
   return ORCVIO_OK;
 }
@@ -2189,7 +2069,7 @@ void Batch::override_noise(double sigma2, double chi2_p) {
   if (chi2_p != p_.chi_square_threshold_feat) {
     p_.chi_square_threshold_feat = chi2_p;
     for (int i = 1; i < 500; ++i) chi2_host_[i] = chi2_quantile(chi2_p, i);
-    CK(cudaMemcpy(dChi2_, chi2_host_.data(), 500 * sizeof(double), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(dChi2_.get(), chi2_host_.data(), 500 * sizeof(double), cudaMemcpyHostToDevice));
   }
 }
 
@@ -2203,13 +2083,11 @@ struct Batch::SnapState {
   std::vector<int> sblk, eblk;     // first / last clone block per feature
   int N = 0, D = 0, n_feat = 0, nobs_total = 0;
   bool has_positions = false;
-  double *dP0 = nullptr, *dCl0 = nullptr, *dIm0 = nullptr, *dPos0 = nullptr;   // pristine window
-  long long* dGen0 = nullptr;
-  size_t pos_cap = 0;
-  double *hP0 = nullptr, *hCl0 = nullptr, *hIm0 = nullptr;                      // pinned staging
-  double* hOut = nullptr;          // pinned download buffer (P, dx, clones)
-  size_t hout_cap = 0;
-  FilterWork* hFw = nullptr; FilterWork* dFw = nullptr;   // (N, D) record for the early prior launch
+  DeviceBuf<double> dP0, dCl0, dIm0, dPos0;     // pristine window
+  DeviceBuf<long long> dGen0;
+  PinnedBuf<double> hP0, hCl0, hIm0;            // staging
+  PinnedBuf<double> hOut;          // download buffer (P, dx, clones)
+  PinnedBuf<FilterWork> hFw; DeviceBuf<FilterWork> dFw;   // (N, D) record for the early prior launch
   bool prior_early = false;
   bool tri_early = false;          // k_triangulate (direct mode) already queued by snapshot_prepare
   std::vector<int> rowoff_f, hblkoff_f, small_f, large_f;   // per feature (caller's order): offsets, size classes
@@ -2228,16 +2106,7 @@ struct Batch::SnapState {
     plain_runs = 0;
     graph_replays = 0;
   }
-  ~SnapState() {
-    drop_graph();
-    cudaFree(dFw);
-    if (hFw) cudaFreeHost(hFw);
-    cudaFree(dP0); cudaFree(dCl0); cudaFree(dIm0); cudaFree(dPos0); cudaFree(dGen0);
-    if (hP0) cudaFreeHost(hP0);
-    if (hCl0) cudaFreeHost(hCl0);
-    if (hIm0) cudaFreeHost(hIm0);
-    if (hOut) cudaFreeHost(hOut);
-  }
+  ~SnapState() { drop_graph(); }
 };
 
 void Batch::SnapDeleter::operator()(SnapState* p) const { delete p; }
@@ -2249,16 +2118,15 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   if (!snap_) {
     snap_.reset(new SnapState());
     SnapState& S = *snap_;
-    CK(cudaMalloc(&S.dP0, (size_t)ldp_ * ldp_ * sizeof(double)));
-    CK(cudaMalloc(&S.dCl0, (size_t)Ncap_ * CL_STRIDE * sizeof(double)));
-    CK(cudaMalloc(&S.dIm0, IM_STRIDE * sizeof(double)));
-    CK(cudaMallocHost(&S.hP0, (size_t)ldp_ * ldp_ * sizeof(double)));
-    CK(cudaMallocHost(&S.hCl0, (size_t)Ncap_ * CL_STRIDE * sizeof(double)));
-    CK(cudaMallocHost(&S.hIm0, IM_STRIDE * sizeof(double)));
-    S.hout_cap = (size_t)ldp_ * ldp_ + ldp_ + (size_t)Ncap_ * CL_STRIDE;
-    CK(cudaMallocHost(&S.hOut, S.hout_cap * sizeof(double)));
-    CK(cudaMallocHost(&S.hFw, sizeof(FilterWork)));
-    CK(cudaMalloc(&S.dFw, sizeof(FilterWork)));
+    CKA(S.dP0.alloc((size_t)ldp_ * ldp_));
+    CKA(S.dCl0.alloc((size_t)Ncap_ * CL_STRIDE));
+    CKA(S.dIm0.alloc(IM_STRIDE));
+    CKA(S.hP0.alloc((size_t)ldp_ * ldp_));
+    CKA(S.hCl0.alloc((size_t)Ncap_ * CL_STRIDE));
+    CKA(S.hIm0.alloc(IM_STRIDE));
+    CKA(S.hOut.alloc((size_t)ldp_ * ldp_ + ldp_ + (size_t)Ncap_ * CL_STRIDE));
+    CKA(S.hFw.alloc(1));
+    CKA(S.dFw.alloc(1));
   }
   SnapState& S = *snap_;
   S.drop_graph();                  // new work lists: the captured chain no longer matches
@@ -2266,10 +2134,9 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   if (io.n_feat > Fcap_) {
     // grow the feature tables of this (single filter) batch
     CK(cudaStreamSynchronize(stream_));
-    cudaFree(dFpos_); cudaFree(dFgen_);
     Fcap_ = io.n_feat + 1024;
-    CK(cudaMalloc(&dFpos_, (size_t)B_ * Fcap_ * FP_STRIDE * sizeof(double)));
-    CK(cudaMalloc(&dFgen_, (size_t)B_ * Fcap_ * sizeof(long long)));
+    CKA(dFpos_.alloc((size_t)B_ * Fcap_ * FP_STRIDE));
+    CKA(dFgen_.alloc((size_t)B_ * Fcap_));
   }
   const int D = ORCVIO_LEG + 6 * N;
   S.N = N; S.D = D; S.n_feat = io.n_feat;
@@ -2298,8 +2165,9 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   const bool early_tri = io.early_prior && (io.stages & 1) && (io.stages & 2) && !io.positions_in && !io.iters &&
                          !io.cost && nF > 0;
   w.obs_preuploaded = early_tri;
-  blob_.ensure_pinned(4096 + (size_t)std::max(nF, 1) * (sizeof(Cand) + sizeof(Tile) + 2 * sizeof(int)) +
-                      sizeof(FilterWork) * B_ + (early_tri ? 0 : (size_t)nobs_total * 20));
+  const size_t blob_bytes = 4096 + (size_t)std::max(nF, 1) * (sizeof(Cand) + sizeof(Tile) + 2 * sizeof(int)) +
+                            sizeof(FilterWork) * B_ + (early_tri ? 0 : (size_t)nobs_total * 20);
+  CKA(blob_.pinned.grow(blob_bytes, blob_bytes * 2 + 4096, "pinned blob"));     // ahead of time: nothing to preserve
   S.list_err = ORCVIO_OK;
   S.scan_done.store(0, std::memory_order_relaxed);
   S.lists_done.store(0, std::memory_order_relaxed);
@@ -2387,25 +2255,17 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
     e_fo = blob_early_.reserve(sizeof(int) * (size_t)(nF + 1));
     e_oc = blob_early_.reserve(sizeof(int) * (size_t)nobs_total);
     e_oz = blob_early_.reserve(sizeof(double) * 2 * (size_t)nobs_total);
-    std::memcpy(blob_early_.pinned + e_fo, io.feat_off, sizeof(int) * (size_t)(nF + 1));
-    std::memcpy(blob_early_.pinned + e_oc, io.obs_clone, sizeof(int) * (size_t)nobs_total);
-    std::memcpy(blob_early_.pinned + e_oz, io.obs_z, sizeof(double) * 2 * (size_t)nobs_total);
-    if (blob_early_.used > blob_early_.dev_cap) {
-      if (blob_early_.dev) cudaFree(blob_early_.dev);
-      blob_early_.dev_cap = blob_early_.used * 2 + 4096;
-      CK(cudaMalloc(&blob_early_.dev, blob_early_.dev_cap));
-    }
-    if ((size_t)nF > statusf_cap_) {
-      if (dStatusF_) cudaFree(dStatusF_);
-      statusf_cap_ = (size_t)nF * 2 + 1024;
-      CK(cudaMalloc(&dStatusF_, statusf_cap_ * sizeof(int)));
-    }
-    CK(cudaMemcpyAsync(blob_early_.dev, blob_early_.pinned, blob_early_.used, cudaMemcpyHostToDevice, stream_));
+    char* pe = blob_early_.pinned.get();
+    std::memcpy(pe + e_fo, io.feat_off, sizeof(int) * (size_t)(nF + 1));
+    std::memcpy(pe + e_oc, io.obs_clone, sizeof(int) * (size_t)nobs_total);
+    std::memcpy(pe + e_oz, io.obs_z, sizeof(double) * 2 * (size_t)nobs_total);
+    CKA(dStatusF_.grow(nF, (size_t)nF * 2 + 1024, "status by feature"));
+    CK(blob_early_.upload(stream_));
     g_hp.mark("obs_up");
   }
   // ---- host staging of the window
-  double* cl = S.hCl0;
-  double* im = S.hIm0;
+  double* cl = S.hCl0.get();
+  double* im = S.hIm0.get();
   std::memset(cl, 0, (size_t)Ncap_ * CL_STRIDE * sizeof(double));
   std::memset(im, 0, IM_STRIDE * sizeof(double));
   double Rbc[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, tcb[3] = {0, 0, 0};
@@ -2434,8 +2294,8 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   // imu record: current state = newest clone (only used by the state increment)
   for (int k = 0; k < 9; ++k) im[IM_R + k] = cl[(size_t)(N - 1) * CL_STRIDE + CL_R + k];
   for (int k = 0; k < 3; ++k) im[IM_P + k] = cl[(size_t)(N - 1) * CL_STRIDE + CL_P + k];
-  CK(cudaMemcpyAsync(S.dCl0, S.hCl0, (size_t)Ncap_ * CL_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
-  CK(cudaMemcpyAsync(S.dIm0, S.hIm0, IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
+  CK(cudaMemcpyAsync(S.dCl0.get(), S.hCl0.get(), (size_t)Ncap_ * CL_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
+  CK(cudaMemcpyAsync(S.dIm0.get(), S.hIm0.get(), IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
   FilterHost& F = f_[0];
   F.clones.clear();
   for (int c = 0; c < N; ++c) F.clones.push_back(CloneMeta{c, (double)c, 0.0});
@@ -2453,19 +2313,19 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   S.tri_early = false;
   if (early_tri) {
     // the window the kernels work on (snapshot_execute skips these restores for this run)
-    CK(cudaMemcpyAsync(dClones_, S.dCl0, (size_t)Ncap_ * CL_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
-    CK(cudaMemcpyAsync(dImu_, S.dIm0, IM_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
-    CK(cudaMemsetAsync(dFgen_, 0xFF, (size_t)Fcap_ * sizeof(long long), stream_));
-    w.pre_dOc = (const int*)(blob_early_.dev + e_oc);
-    w.pre_dOz = (const double*)(blob_early_.dev + e_oz);
+    CK(cudaMemcpyAsync(dClones_.get(), S.dCl0.get(), (size_t)Ncap_ * CL_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+    CK(cudaMemcpyAsync(dImu_.get(), S.dIm0.get(), IM_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+    CK(cudaMemsetAsync(dFgen_.get(), 0xFF, (size_t)Fcap_ * sizeof(long long), stream_));
+    w.pre_dOc = (const int*)(blob_early_.dev.get() + e_oc);
+    w.pre_dOz = (const double*)(blob_early_.dev.get() + e_oz);
     TriArgs ta{};
     ta.cand = nullptr; ta.n_cand = nF;
-    ta.clones = dClones_; ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    ta.fpos = dFpos_; ta.fgen = dFgen_; ta.fcap = Fcap_;
+    ta.clones = dClones_.get(); ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+    ta.fpos = dFpos_.get(); ta.fgen = dFgen_.get(); ta.fcap = Fcap_;
     ta.obs_clone = w.pre_dOc; ta.obs_z = w.pre_dOz;
     ta.cfg = tricfg_;
-    ta.status = dStatusF_;
-    ta.feat_off = (const int*)(blob_early_.dev + e_fo);
+    ta.status = dStatusF_.get();
+    ta.feat_off = (const int*)(blob_early_.dev.get() + e_fo);
     ta.direct_n_clones = N; ta.direct_n_obs = nobs_total;
     launch_triangulate(ta, stream_);
     ++launches_;
@@ -2493,30 +2353,30 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   // P: the caller's matrix is column-major and symmetric, the device copy row-major with ld
   if (io.P_in) {
     for (int i = 0; i < D; ++i) {
-      std::memcpy(S.hP0 + (size_t)i * ldp_, io.P_in + (size_t)i * D, D * sizeof(double));
-      for (int j = D; j < ldp_; ++j) S.hP0[(size_t)i * ldp_ + j] = 0.0;
+      std::memcpy(S.hP0.get() + (size_t)i * ldp_, io.P_in + (size_t)i * D, D * sizeof(double));
+      for (int j = D; j < ldp_; ++j) S.hP0.get()[(size_t)i * ldp_ + j] = 0.0;
     }
-    for (int i = D; i < ldp_; ++i) std::memset(S.hP0 + (size_t)i * ldp_, 0, ldp_ * sizeof(double));
+    for (int i = D; i < ldp_; ++i) std::memset(S.hP0.get() + (size_t)i * ldp_, 0, ldp_ * sizeof(double));
   } else {
-    std::memset(S.hP0, 0, (size_t)ldp_ * ldp_ * sizeof(double));
+    std::memset(S.hP0.get(), 0, (size_t)ldp_ * ldp_ * sizeof(double));
   }
   g_hp.mark("stageP");
   // when the early triangulation is already queued on stream_, P goes up on the side stream: the prior factor
   // (which forks off the P upload) must not wait for k_triangulate
   cudaStream_t sp = S.tri_early ? stream_up_ : stream_;
-  CK(cudaMemcpyAsync(S.dP0, S.hP0, (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyHostToDevice, sp));
+  CK(cudaMemcpyAsync(S.dP0.get(), S.hP0.get(), (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyHostToDevice, sp));
   S.prior_early = false;
   if ((io.stages & 4) && io.early_prior) {
     // The prior factor needs only P: put P in place and start k_chol_prior on the second stream now, so it
     // runs while the host is still building and uploading this frame's work lists.
-    S.hFw[0] = FilterWork{};
-    S.hFw[0].N = N; S.hFw[0].D = D; S.hFw[0].active = 1;
-    CK(cudaMemcpyAsync(S.dFw, S.hFw, sizeof(FilterWork), cudaMemcpyHostToDevice, sp));
-    CK(cudaMemcpyAsync(dP_, S.dP0, (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyDeviceToDevice, sp));
+    S.hFw.get()[0] = FilterWork{};
+    S.hFw.get()[0].N = N; S.hFw.get()[0].D = D; S.hFw.get()[0].active = 1;
+    CK(cudaMemcpyAsync(S.dFw.get(), S.hFw.get(), sizeof(FilterWork), cudaMemcpyHostToDevice, sp));
+    CK(cudaMemcpyAsync(dP_.get(), S.dP0.get(), (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyDeviceToDevice, sp));
     CK(cudaEventRecord(ev_fork_, sp));
     InfoBufs ib{};
-    ib.Ls = dLs_; ib.ls_done = ev_ls_;
-    launch_info_prior(upd_args(S.dFw), ib, N, stream2_, ev_fork_, ev_join_);
+    ib.Ls = dLs_.get(); ib.ls_done = ev_ls_;
+    launch_info_prior(upd_args(S.dFw.get()), ib, N, stream2_, ev_fork_, ev_join_);
     launches_ += 2;
     S.prior_early = true;
   }
@@ -2533,11 +2393,7 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
     // offsets and size classes come out of the validation scan, so nothing of it waits for the sorted lists
     if (!io.raw_Hx) {
       ensure_scratch(std::max(nF, 1), std::max<size_t>(w.hblk_total, 1), std::max<size_t>(w.rows_total, 1));
-      if ((size_t)nF > gammaf_cap_) {
-        if (dGammaF_) cudaFree(dGammaF_);
-        gammaf_cap_ = (size_t)nF * 2 + 1024;
-        CK(cudaMalloc(&dGammaF_, gammaf_cap_ * sizeof(double)));
-      }
+      CKA(dGammaF_.grow(nF, (size_t)nF * 2 + 1024, "gamma by feature"));
       blob_early2_.reset();
       const size_t e_ro = blob_early2_.reserve(sizeof(int) * (size_t)nF);
       const size_t e_ho = blob_early2_.reserve(sizeof(int) * (size_t)nF);
@@ -2545,41 +2401,37 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
       const size_t e_eb = blob_early2_.reserve(sizeof(int) * (size_t)nF);
       const size_t e_sm = blob_early2_.reserve(sizeof(int) * std::max<size_t>(S.small_f.size(), 1));
       const size_t e_lg = blob_early2_.reserve(sizeof(int) * std::max<size_t>(S.large_f.size(), 1));
-      std::memcpy(blob_early2_.pinned + e_ro, S.rowoff_f.data(), sizeof(int) * (size_t)nF);
-      std::memcpy(blob_early2_.pinned + e_ho, S.hblkoff_f.data(), sizeof(int) * (size_t)nF);
-      std::memcpy(blob_early2_.pinned + e_sb, S.sblk.data(), sizeof(int) * (size_t)nF);
-      std::memcpy(blob_early2_.pinned + e_eb, S.eblk.data(), sizeof(int) * (size_t)nF);
-      if (!S.small_f.empty()) std::memcpy(blob_early2_.pinned + e_sm, S.small_f.data(), sizeof(int) * S.small_f.size());
-      if (!S.large_f.empty()) std::memcpy(blob_early2_.pinned + e_lg, S.large_f.data(), sizeof(int) * S.large_f.size());
-      if (blob_early2_.used > blob_early2_.dev_cap) {
-        if (blob_early2_.dev) cudaFree(blob_early2_.dev);
-        blob_early2_.dev_cap = blob_early2_.used * 2 + 4096;
-        CK(cudaMalloc(&blob_early2_.dev, blob_early2_.dev_cap));
-      }
-      CK(cudaMemcpyAsync(blob_early2_.dev, blob_early2_.pinned, blob_early2_.used, cudaMemcpyHostToDevice, stream_));
+      char* pe2 = blob_early2_.pinned.get();
+      std::memcpy(pe2 + e_ro, S.rowoff_f.data(), sizeof(int) * (size_t)nF);
+      std::memcpy(pe2 + e_ho, S.hblkoff_f.data(), sizeof(int) * (size_t)nF);
+      std::memcpy(pe2 + e_sb, S.sblk.data(), sizeof(int) * (size_t)nF);
+      std::memcpy(pe2 + e_eb, S.eblk.data(), sizeof(int) * (size_t)nF);
+      if (!S.small_f.empty()) std::memcpy(pe2 + e_sm, S.small_f.data(), sizeof(int) * S.small_f.size());
+      if (!S.large_f.empty()) std::memcpy(pe2 + e_lg, S.large_f.data(), sizeof(int) * S.large_f.size());
+      CK(blob_early2_.upload(stream_));
       JacArgs ja{};
       ja.cand = nullptr;
-      ja.clones = dClones_; ja.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-      ja.imu = dImu_; ja.fpos = dFpos_; ja.fcap = Fcap_;
-      ja.P = dP_; ja.p_stride = (size_t)ldp_ * ldp_; ja.ldp = ldp_;
+      ja.clones = dClones_.get(); ja.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+      ja.imu = dImu_.get(); ja.fpos = dFpos_.get(); ja.fcap = Fcap_;
+      ja.P = dP_.get(); ja.p_stride = (size_t)ldp_ * ldp_; ja.ldp = ldp_;
       ja.obs_clone = w.pre_dOc; ja.obs_z = w.pre_dOz;
-      ja.flags = flags_; ja.sigma2 = p_.feature_observation_noise; ja.chi2 = dChi2_;
-      ja.status = dStatusF_; ja.gamma = dGammaF_;
-      ja.hblk = dHblk_; ja.rblk = dRblk_;
-      ja.feat_off = (const int*)(blob_early_.dev + e_fo);
-      ja.rowoff_f = (const int*)(blob_early2_.dev + e_ro);
-      ja.hblkoff_f = (const int*)(blob_early2_.dev + e_ho);
+      ja.flags = flags_; ja.sigma2 = p_.feature_observation_noise; ja.chi2 = dChi2_.get();
+      ja.status = dStatusF_.get(); ja.gamma = dGammaF_.get();
+      ja.hblk = dHblk_.get(); ja.rblk = dRblk_.get();
+      ja.feat_off = (const int*)(blob_early_.dev.get() + e_fo);
+      ja.rowoff_f = (const int*)(blob_early2_.dev.get() + e_ro);
+      ja.hblkoff_f = (const int*)(blob_early2_.dev.get() + e_ho);
       JacArgs js = ja, jl = ja;
-      js.cand_list = (const int*)(blob_early2_.dev + e_sm); js.n_list = (int)S.small_f.size();
-      jl.cand_list = (const int*)(blob_early2_.dev + e_lg); jl.n_list = (int)S.large_f.size();
-      if (!S.prior_early) CK(cudaMemcpyAsync(dP_, S.dP0, (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+      js.cand_list = (const int*)(blob_early2_.dev.get() + e_sm); js.n_list = (int)S.small_f.size();
+      jl.cand_list = (const int*)(blob_early2_.dev.get() + e_lg); jl.n_list = (int)S.large_f.size();
+      if (!S.prior_early) CK(cudaMemcpyAsync(dP_.get(), S.dP0.get(), (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
       launch_jac_gate(js, jl, stream_);
       launches_ += (js.n_list > 0) + (jl.n_list > 0);
       S.jac_early = true;
       // the A-form kernel reads the same per-feature arrays (+ the sorted order): no candidate record is uploaded
       dir_feat_off_ = ja.feat_off; dir_rowoff_ = ja.rowoff_f; dir_hblkoff_ = ja.hblkoff_f;
-      dir_sblk_ = (const int*)(blob_early2_.dev + e_sb);
-      dir_eblk_ = (const int*)(blob_early2_.dev + e_eb);
+      dir_sblk_ = (const int*)(blob_early2_.dev.get() + e_sb);
+      dir_eblk_ = (const int*)(blob_early2_.dev.get() + e_eb);
       w.cands_stay_on_host = true;
     }
     g_hp.mark("jac_early");
@@ -2591,20 +2443,16 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
 
   S.has_positions = io.positions_in != nullptr;
   if (S.has_positions) {
-    if ((size_t)Fcap_ > S.pos_cap) {
-      cudaFree(S.dPos0); cudaFree(S.dGen0);
-      S.pos_cap = Fcap_;
-      CK(cudaMalloc(&S.dPos0, S.pos_cap * FP_STRIDE * sizeof(double)));
-      CK(cudaMalloc(&S.dGen0, S.pos_cap * sizeof(long long)));
-    }
+    CKA(S.dPos0.grow((size_t)Fcap_ * FP_STRIDE, (size_t)Fcap_ * FP_STRIDE, "given positions"));
+    CKA(S.dGen0.grow(Fcap_, Fcap_, "given positions"));
     std::vector<double> pos_in((size_t)Fcap_ * FP_STRIDE, 0.0);
     for (int f = 0; f < io.n_feat; ++f)
       for (int k = 0; k < 3; ++k) pos_in[(size_t)f * FP_STRIDE + k] = io.positions_in[3 * (size_t)f + k];
     // mark every slot initialised with its own generation so the kernels use the given positions
     std::vector<long long> gens(Fcap_, -1);
     for (int f = 0; f < io.n_feat; ++f) gens[f] = f + 1;
-    CK(cudaMemcpy(S.dPos0, pos_in.data(), pos_in.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(S.dGen0, gens.data(), gens.size() * sizeof(long long), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(S.dPos0.get(), pos_in.data(), pos_in.size() * sizeof(double), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(S.dGen0.get(), gens.data(), gens.size() * sizeof(long long), cudaMemcpyHostToDevice));
   }
   want_iters_ = io.iters || io.cost;
   want_raw_ = io.raw_Hx != nullptr;
@@ -2619,7 +2467,7 @@ int Batch::snapshot_prepare(const SnapshotIO& io) {
   g_hp.mark("stage_blob");
   if (skip_tri_ && nC > 0) {
     std::vector<int> st(nC, ST_TRI_VALID);
-    CK(cudaMemcpy(dStatus_, st.data(), sizeof(int) * nC, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(dStatus_.get(), st.data(), sizeof(int) * nC, cudaMemcpyHostToDevice));
   }
   return ok_ ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
@@ -2683,20 +2531,20 @@ int Batch::snapshot_execute(bool download) {
 int Batch::snapshot_execute_plain(bool download, bool prior_in_flight) {
   SnapState& S = *snap_;
   if (!prior_in_flight && !(S.tri_early && S.jac_early))
-    CK(cudaMemcpyAsync(dP_, S.dP0, (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+    CK(cudaMemcpyAsync(dP_.get(), S.dP0.get(), (size_t)ldp_ * ldp_ * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
   tri_done_early_ = S.tri_early;                    // window restored and k_triangulate started by snapshot_prepare
   jac_done_early_ = S.tri_early && S.jac_early;
   S.by_feature = jac_done_early_;
   S.tri_early = false;
   S.jac_early = false;
   if (!tri_done_early_) {
-    CK(cudaMemcpyAsync(dClones_, S.dCl0, (size_t)Ncap_ * CL_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
-    CK(cudaMemcpyAsync(dImu_, S.dIm0, IM_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+    CK(cudaMemcpyAsync(dClones_.get(), S.dCl0.get(), (size_t)Ncap_ * CL_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+    CK(cudaMemcpyAsync(dImu_.get(), S.dIm0.get(), IM_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
     if (S.has_positions) {
-      CK(cudaMemcpyAsync(dFpos_, S.dPos0, (size_t)Fcap_ * FP_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
-      CK(cudaMemcpyAsync(dFgen_, S.dGen0, (size_t)Fcap_ * sizeof(long long), cudaMemcpyDeviceToDevice, stream_));
+      CK(cudaMemcpyAsync(dFpos_.get(), S.dPos0.get(), (size_t)Fcap_ * FP_STRIDE * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
+      CK(cudaMemcpyAsync(dFgen_.get(), S.dGen0.get(), (size_t)Fcap_ * sizeof(long long), cudaMemcpyDeviceToDevice, stream_));
     } else {
-      CK(cudaMemsetAsync(dFgen_, 0xFF, (size_t)Fcap_ * sizeof(long long), stream_));
+      CK(cudaMemsetAsync(dFgen_.get(), 0xFF, (size_t)Fcap_ * sizeof(long long), stream_));
     }
   }
   launch_phase(S.w, download, prior_in_flight);
@@ -2709,26 +2557,26 @@ int Batch::snapshot_fetch(const SnapshotIO& io) {
   SnapState& S = *snap_;
   const int N = S.N, D = S.D, nC = (int)S.w.cands.size();
   // queue every download on the stream, then one synchronisation
-  double* hP = S.hOut;
+  double* hP = S.hOut.get();
   double* hDx = hP + (size_t)ldp_ * ldp_;
   double* hCl = hDx + ldp_;
-  if (io.P_out) CK(cudaMemcpyAsync(hP, dP_, (size_t)D * ldp_ * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-  else if (io.P_lead9) CK(cudaMemcpyAsync(hP, dP_, (size_t)9 * ldp_ * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-  if (io.delta_x) CK(cudaMemcpyAsync(hDx, dDx_, ldp_ * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-  if (io.clone_out) CK(cudaMemcpyAsync(hCl, dClones_, (size_t)N * CL_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  if (io.P_out) CK(cudaMemcpyAsync(hP, dP_.get(), (size_t)D * ldp_ * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  else if (io.P_lead9) CK(cudaMemcpyAsync(hP, dP_.get(), (size_t)9 * ldp_ * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  if (io.delta_x) CK(cudaMemcpyAsync(hDx, dDx_.get(), ldp_ * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  if (io.clone_out) CK(cudaMemcpyAsync(hCl, dClones_.get(), (size_t)N * CL_STRIDE * sizeof(double), cudaMemcpyDeviceToHost, stream_));
   CK(cudaStreamSynchronize(stream_));
   g_hp.mark("gpu_wait");
   if (io.status || io.gamma)
     for (int c = 0; c < nC; ++c) {
       const int f = S.by_feature ? c : S.order[c];
-      if (io.status) io.status[f] = hStatus_[c];
-      if (io.gamma) io.gamma[f] = hGamma_[c];
+      if (io.status) io.status[f] = hStatus_.get()[c];
+      if (io.gamma) io.gamma[f] = hGamma_.get()[c];
     }
   if (io.iters || io.cost) {
     std::vector<int> it(2 * (size_t)nC);
     std::vector<double> cs(nC);
-    CK(cudaMemcpy(it.data(), dIters_, it.size() * sizeof(int), cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(cs.data(), dCost_, cs.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(it.data(), dIters_.get(), it.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(cs.data(), dCost_.get(), cs.size() * sizeof(double), cudaMemcpyDeviceToHost));
     for (int c = 0; c < nC; ++c) {
       if (io.iters) { io.iters[2 * S.order[c]] = it[2 * c]; io.iters[2 * S.order[c] + 1] = it[2 * c + 1]; }
       if (io.cost) io.cost[S.order[c]] = cs[c];
@@ -2736,16 +2584,16 @@ int Batch::snapshot_fetch(const SnapshotIO& io) {
   }
   if (io.positions) {
     std::vector<double> fp((size_t)S.n_feat * FP_STRIDE);
-    CK(cudaMemcpy(fp.data(), dFpos_, fp.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(fp.data(), dFpos_.get(), fp.size() * sizeof(double), cudaMemcpyDeviceToHost));
     for (int f = 0; f < S.n_feat; ++f)
       for (int k = 0; k < 3; ++k) io.positions[3 * (size_t)f + k] = fp[(size_t)f * FP_STRIDE + k];
   }
   if (io.raw_Hx) {
     const size_t no = (size_t)S.nobs_total;
-    CK(cudaMemcpy(io.raw_Hx, dRawHx_, no * 12 * sizeof(double), cudaMemcpyDeviceToHost));
-    if (io.raw_He) CK(cudaMemcpy(io.raw_He, dRawHe_, no * 12 * sizeof(double), cudaMemcpyDeviceToHost));
-    if (io.raw_Hf) CK(cudaMemcpy(io.raw_Hf, dRawHf_, no * 6 * sizeof(double), cudaMemcpyDeviceToHost));
-    if (io.raw_r) CK(cudaMemcpy(io.raw_r, dRawR_, no * 2 * sizeof(double), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(io.raw_Hx, dRawHx_.get(), no * 12 * sizeof(double), cudaMemcpyDeviceToHost));
+    if (io.raw_He) CK(cudaMemcpy(io.raw_He, dRawHe_.get(), no * 12 * sizeof(double), cudaMemcpyDeviceToHost));
+    if (io.raw_Hf) CK(cudaMemcpy(io.raw_Hf, dRawHf_.get(), no * 6 * sizeof(double), cudaMemcpyDeviceToHost));
+    if (io.raw_r) CK(cudaMemcpy(io.raw_r, dRawR_.get(), no * 2 * sizeof(double), cudaMemcpyDeviceToHost));
   }
   if (io.P_lead9)
     for (int i = 0; i < 9; ++i) std::memcpy(io.P_lead9 + 9 * i, hP + (size_t)i * ldp_, 9 * sizeof(double));
@@ -2769,8 +2617,8 @@ int Batch::snapshot_fetch_last(const SnapshotIO& io) {
   const SnapState& S = *snap_;
   const int nC = (int)S.w.cands.size();
   if (nC > 0 && (io.status || io.gamma)) {
-    CK(cudaMemcpyAsync(hStatus_, S.by_feature ? dStatusF_ : dStatus_, sizeof(int) * nC, cudaMemcpyDeviceToHost, stream_));
-    CK(cudaMemcpyAsync(hGamma_, S.by_feature ? dGammaF_ : dGamma_, sizeof(double) * nC, cudaMemcpyDeviceToHost, stream_));
+    CK(cudaMemcpyAsync(hStatus_.get(), S.by_feature ? dStatusF_.get() : dStatus_.get(), sizeof(int) * nC, cudaMemcpyDeviceToHost, stream_));
+    CK(cudaMemcpyAsync(hGamma_.get(), S.by_feature ? dGammaF_.get() : dGamma_.get(), sizeof(double) * nC, cudaMemcpyDeviceToHost, stream_));
   }
   return snapshot_fetch(io);
 }

@@ -15,6 +15,7 @@
 
 #include "../../include/orcvio_b200.h"
 #include "config.h"
+#include "devmem.h"
 #include "kernels.h"
 
 namespace ob {
@@ -111,39 +112,28 @@ struct FilterHost {
 };
 
 struct Blob {                 // one pinned host blob + device twin, carved into sections
-  char* dev = nullptr;
-  size_t dev_cap = 0;
-  char* pinned = nullptr;     // sections are written in place: no pageable staging copy
-  size_t pinned_cap = 0;
+  DeviceBuf<char> dev;
+  PinnedBuf<char> pinned;     // sections are written in place: no pageable staging copy
   size_t used = 0;
   size_t reserve(size_t bytes) {
-    size_t off = (used + 255) & ~size_t(255);
-    const size_t old_used = used;
-    used = off + bytes;
-    if (used > pinned_cap) {
-      char* np = nullptr;
-      const size_t ncap = used * 2 + 4096;
-      if (getenv("ORCVIO_HOST_PROF") && atoi(getenv("ORCVIO_HOST_PROF")) == 3)
-        fprintf(stderr, "[replay prof] growth: pinned blob -> %.1f MB\n", ncap / 1048576.0);
-      if (cudaMallocHost(&np, ncap) != cudaSuccess) { used = old_used; return 0; }
-      if (pinned) {
-        if (old_used) std::memcpy(np, pinned, old_used);
-        cudaFreeHost(pinned);
-      }
-      pinned = np;
-      pinned_cap = ncap;
+    const size_t off = (used + 255) & ~size_t(255);
+    if (off + bytes > pinned.size()) {      // the sections written so far are kept
+      PinnedBuf<char> np;
+      const size_t ncap = (off + bytes) * 2 + 4096;
+      note_growth("pinned blob", ncap);
+      if (!np.alloc(ncap)) return 0;
+      if (used) std::memcpy(np.get(), pinned.get(), used);
+      pinned = std::move(np);
     }
+    used = off + bytes;
     return off;
   }
   void reset() { used = 0; }
-  void ensure_pinned(size_t bytes) {      // grow the pinned half ahead of time (contents are not preserved)
-    if (bytes <= pinned_cap) return;
-    char* np = nullptr;
-    const size_t ncap = bytes * 2 + 4096;
-    if (cudaMallocHost(&np, ncap) != cudaSuccess) return;
-    if (pinned) cudaFreeHost(pinned);
-    pinned = np;
-    pinned_cap = ncap;
+  // grows the device twin (contents are not preserved) and queues the copy of the used part
+  cudaError_t upload(cudaStream_t s) {
+    if (used == 0) return cudaSuccess;
+    if (!dev.grow(used, used * 2 + 4096, "work-list blob")) return cudaErrorMemoryAllocation;
+    return cudaMemcpyAsync(dev.get(), pinned.get(), used, cudaMemcpyHostToDevice, s);
   }
 };
 
@@ -247,13 +237,13 @@ class Batch {
  private:
   friend struct CApi;
   bool ok_ = false;
-  double* hDiag_ = nullptr;      // pinned: the 15 diagonal entries of the initial covariance
+  PinnedBuf<double> hDiag_;      // the 15 diagonal entries of the initial covariance
   std::string err_;
   Params p_;
   int B_ = 0, Ncap_ = 0, ldp_ = 0, Fcap_ = 0, ldr_ = 0, ldt_ = 0, dev_ = 0;
   int Emax_ = 0, nmax_ = 0;            // EKF-SLAM feature states (hybrid mode); window columns 6 Ncap + Emax
   bool hybrid_ = false;
-  double* dFidp_ = nullptr;            // inverse-depth records by feature slot
+  DeviceBuf<double> dFidp_;            // inverse-depth records by feature slot
   struct HybridBufs;
   struct HybridDeleter { void operator()(HybridBufs* p) const; };
   std::unique_ptr<HybridBufs, HybridDeleter> hyb_;
@@ -261,49 +251,41 @@ class Batch {
   std::vector<FilterHost> f_;
   cudaStream_t stream_ = nullptr, stream2_ = nullptr;
   cudaEvent_t ev_fork_ = nullptr, ev_join_ = nullptr, ev_ls_ = nullptr;
-  double *dAmat_ = nullptr, *dPart_ = nullptr;
-  size_t amat_cap_ = 0, part_cap_ = 0;
-  double* dLs_ = nullptr;
-  int *dTileRows_ = nullptr, *dFilterRows_ = nullptr;
-  unsigned int* dSyrkCnt_ = nullptr;   // split-K arrival counters of k_syrk
+  DeviceBuf<double> dAmat_, dPart_;
+  DeviceBuf<double> dLs_;
+  DeviceBuf<int> dTileRows_, dFilterRows_;
+  DeviceBuf<unsigned int> dSyrkCnt_;   // split-K arrival counters of k_syrk
   int n_sm_ = 148;
   float last_syrk_us_ = 0.f, last_prior_us_ = 0.f;
-  size_t tilerows_cap_ = 0;
   cudaEvent_t ev_[16];
   // device state
-  double *dP_ = nullptr, *dImu_ = nullptr, *dClones_ = nullptr, *dFpos_ = nullptr;
-  long long* dFgen_ = nullptr;
-  double *dT_ = nullptr, *dS_ = nullptr, *dYv_ = nullptr, *dDx_ = nullptr;
-  double* dChi2_ = nullptr;
+  DeviceBuf<double> dP_, dImu_, dClones_, dFpos_;
+  DeviceBuf<long long> dFgen_;
+  DeviceBuf<double> dT_, dS_, dYv_, dDx_;
+  DeviceBuf<double> dChi2_;
   // growable device scratch
-  double *dHblk_ = nullptr, *dRblk_ = nullptr;
-  size_t hblk_cap_ = 0, rblk_cap_ = 0;
-  int* dStatus_ = nullptr;
-  double* dGamma_ = nullptr;
-  size_t cand_cap_ = 0;
+  DeviceBuf<double> dHblk_, dRblk_;
+  DeviceBuf<int> dStatus_;
+  DeviceBuf<double> dGamma_;
   Blob blob_;
   Blob blob_early_;                    // feat_off + observation pools of the end-to-end call, uploaded ahead
-  int* dTriDone_ = nullptr;            // per-candidate completion flags of k_triangulate (epoch-stamped)
-  size_t tridone_cap_ = 0;
+  DeviceBuf<int> dTriDone_;            // per-candidate completion flags of k_triangulate (epoch-stamped)
   int tri_epoch_ = 0;
   bool graph_capturing_ = false;
-  int* dStatusF_ = nullptr;            // triangulation status by feature slot (early direct-mode pass)
-  size_t statusf_cap_ = 0;
+  DeviceBuf<int> dStatusF_;            // triangulation status by feature slot (early direct-mode pass)
   bool tri_done_early_ = false, jac_done_early_ = false;
   cudaStream_t stream_up_ = nullptr;   // side stream of the work-list upload when kernels are already queued
   cudaEvent_t ev_up_ = nullptr, ev_p_ = nullptr;
   bool upload_on_side_stream_ = false;
   Blob blob_early2_;                   // per-feature offsets / size-class lists of the early Jacobian pass
-  double* dGammaF_ = nullptr;          // gamma by feature slot (early direct-mode pass)
+  DeviceBuf<double> dGammaF_;          // gamma by feature slot (early direct-mode pass)
   const int *dir_feat_off_ = nullptr, *dir_rowoff_ = nullptr, *dir_hblkoff_ = nullptr, *dir_sblk_ = nullptr,
             *dir_eblk_ = nullptr;      // device views of the per-feature arrays of the direct-mode passes
-  size_t gammaf_cap_ = 0;
   std::shared_ptr<class HostWorker> worker_;   // helper thread of the end-to-end frame call (batch.cu)
   // pinned download buffers
-  int* hStatus_ = nullptr;
-  double* hGamma_ = nullptr;
-  size_t hcand_cap_ = 0;
-  double *hImu_ = nullptr, *hClones_ = nullptr, *hDx_ = nullptr;
+  PinnedBuf<int> hStatus_;
+  PinnedBuf<double> hGamma_;
+  PinnedBuf<double> hImu_, hClones_, hDx_;
   TriCfg tricfg_{};
   long long feature_updates_ = 0, launches_ = 0;
   double gpu_ms_ = 0;
@@ -311,14 +293,14 @@ class Batch {
   PhaseTimes pt_;
   std::vector<double> chi2_host_;
   std::vector<double> chi2_zupt_host_;     // chi_squared_table_zupt (p = 0.95, :482-493)
-  int* dZuptDec_ = nullptr; double* dZuptInfo_ = nullptr;
-  double* dCovHist_ = nullptr;         // replay with covariance capture: n_filters x n_frames x 225
-  size_t covhist_cap_ = 0;
-  int* hZuptDec_ = nullptr; double* hZuptInfo_ = nullptr;
+  DeviceBuf<int> dZuptDec_; DeviceBuf<double> dZuptInfo_;
+  DeviceBuf<double> dCovHist_;         // replay with covariance capture: n_filters x n_frames x 225
+  PinnedBuf<int> hZuptDec_; PinnedBuf<double> hZuptInfo_;
 
   void prereserve();
   void upload_blob();
   void ensure_scratch(size_t n_cand, size_t hblk, size_t rblk);
+  cudaError_t grow_update_scratch(size_t need_a, size_t need_p);
   void run_phase(PhaseWork& w, int phase);
   void stage_phase(PhaseWork& w);
   void stage_pack(PhaseWork& w);
@@ -332,8 +314,8 @@ class Batch {
   struct SnapState;
   struct SnapDeleter { void operator()(SnapState* p) const; };
   std::unique_ptr<SnapState, SnapDeleter> snap_;
-  int* dIters_ = nullptr; double* dCost_ = nullptr; size_t iters_cap_ = 0;
-  double *dRawHx_ = nullptr, *dRawHe_ = nullptr, *dRawHf_ = nullptr, *dRawR_ = nullptr; size_t raw_cap_ = 0;
+  DeviceBuf<int> dIters_; DeviceBuf<double> dCost_;
+  DeviceBuf<double> dRawHx_, dRawHe_, dRawHf_, dRawR_;
   bool want_iters_ = false, want_raw_ = false, skip_tri_ = false, skip_update_ = false, skip_jac_ = false;
   void download_mirrors();
   void init_filter_device(int i);

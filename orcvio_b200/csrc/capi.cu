@@ -85,6 +85,12 @@ int orcvio_set_device(int device) {
   return ORCVIO_OK;
 }
 
+int orcvio_device_bytes_held(long long* device, long long* pinned) {
+  if (device) *device = bytes_held()[0].load();
+  if (pinned) *pinned = bytes_held()[1].load();
+  return ORCVIO_OK;
+}
+
 const char* orcvio_version(void) { return "orcvio_b200 0.1 (sm_100a)"; }
 
 double orcvio_chi2_quantile(double p, int dof) { return chi2_quantile(p, dof); }

@@ -20,6 +20,7 @@
 #include <cmath>
 
 #include "../../include/orcvio_b200.h"
+#include "devmem.h"
 #include "kernels.h"
 
 namespace ob {
@@ -224,16 +225,12 @@ int nees_summary(const double* nees8, int n_traj, int n_frames, double* summary9
   if (n_traj < 1 || n_frames < 1 || !nees8 || !summary9) return ORCVIO_ERR_ARG;
   if (!have_device()) return ORCVIO_ERR_NO_DEVICE;
   const size_t nr = (size_t)n_traj * n_frames * 8, ns = (size_t)n_frames * 9;
-  double *dN = nullptr, *dS = nullptr;
-  if (cudaMalloc(&dN, nr * sizeof(double)) != cudaSuccess || cudaMalloc(&dS, ns * sizeof(double)) != cudaSuccess) {
-    cudaFree(dN); cudaFree(dS);
-    return ORCVIO_ERR_CUDA;
-  }
-  cudaMemcpy(dN, nees8, nr * sizeof(double), cudaMemcpyHostToDevice);
-  k_nees_summary<<<n_frames, SUM_THREADS>>>(dN, n_traj, n_frames, dS);
+  DeviceBuf<double> dN, dS;
+  if (!dN.alloc(nr) || !dS.alloc(ns)) return ORCVIO_ERR_CUDA;
+  cudaMemcpy(dN.get(), nees8, nr * sizeof(double), cudaMemcpyHostToDevice);
+  k_nees_summary<<<n_frames, SUM_THREADS>>>(dN.get(), n_traj, n_frames, dS.get());
   check_launch("k_nees_summary");
-  const cudaError_t e = cudaMemcpy(summary9, dS, ns * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dN); cudaFree(dS);
+  const cudaError_t e = cudaMemcpy(summary9, dS.get(), ns * sizeof(double), cudaMemcpyDeviceToHost);
   return e == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -243,25 +240,21 @@ int trajectory_nees(const double* est17, const double* gt17, const double* cov15
   if (!have_device()) return ORCVIO_ERR_NO_DEVICE;
   const long long n = (long long)n_traj * n_frames;
   const size_t ns = summary9 ? (size_t)n_frames * 9 : 0;
-  double *dE = nullptr, *dG = nullptr, *dC = nullptr, *dO = nullptr, *dS = nullptr;
-  if (cudaMalloc(&dE, n * 17 * sizeof(double)) != cudaSuccess || cudaMalloc(&dG, n * 17 * sizeof(double)) != cudaSuccess ||
-      cudaMalloc(&dC, n * 225 * sizeof(double)) != cudaSuccess || cudaMalloc(&dO, n * 8 * sizeof(double)) != cudaSuccess ||
-      (ns && cudaMalloc(&dS, ns * sizeof(double)) != cudaSuccess)) {
-    cudaFree(dE); cudaFree(dG); cudaFree(dC); cudaFree(dO); cudaFree(dS);
+  DeviceBuf<double> dE, dG, dC, dO, dS;
+  if (!dE.alloc(n * 17) || !dG.alloc(n * 17) || !dC.alloc(n * 225) || !dO.alloc(n * 8) || !dS.alloc(ns))
     return ORCVIO_ERR_CUDA;
-  }
-  cudaMemcpy(dE, est17, n * 17 * sizeof(double), cudaMemcpyHostToDevice);
-  cudaMemcpy(dG, gt17, n * 17 * sizeof(double), cudaMemcpyHostToDevice);
-  cudaMemcpy(dC, cov15, n * 225 * sizeof(double), cudaMemcpyHostToDevice);
-  k_nees<<<(unsigned)((n + NEES_WARPS - 1) / NEES_WARPS), NEES_WARPS * 32>>>(dE, dG, dC, n, (flags & 3) != 0, dO);
+  cudaMemcpy(dE.get(), est17, n * 17 * sizeof(double), cudaMemcpyHostToDevice);
+  cudaMemcpy(dG.get(), gt17, n * 17 * sizeof(double), cudaMemcpyHostToDevice);
+  cudaMemcpy(dC.get(), cov15, n * 225 * sizeof(double), cudaMemcpyHostToDevice);
+  k_nees<<<(unsigned)((n + NEES_WARPS - 1) / NEES_WARPS), NEES_WARPS * 32>>>(dE.get(), dG.get(), dC.get(), n,
+                                                                          (flags & 3) != 0, dO.get());
   check_launch("k_nees");
   if (ns) {
-    k_nees_summary<<<n_frames, SUM_THREADS>>>(dO, n_traj, n_frames, dS);
+    k_nees_summary<<<n_frames, SUM_THREADS>>>(dO.get(), n_traj, n_frames, dS.get());
     check_launch("k_nees_summary");
   }
-  cudaError_t e = cudaMemcpy(nees8, dO, n * 8 * sizeof(double), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && ns) e = cudaMemcpy(summary9, dS, ns * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dE); cudaFree(dG); cudaFree(dC); cudaFree(dO); cudaFree(dS);
+  cudaError_t e = cudaMemcpy(nees8, dO.get(), n * 8 * sizeof(double), cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess && ns) e = cudaMemcpy(summary9, dS.get(), ns * sizeof(double), cudaMemcpyDeviceToHost);
   return e == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 

@@ -15,6 +15,7 @@
 
 #include "../../include/orcvio_b200.h"
 #include "config.h"
+#include "devmem.h"
 #include "kernels.h"
 #include "ekf_math.cuh"
 
@@ -326,19 +327,13 @@ __global__ void k_ekf_drop_block(const double* Pin, int D, int c0, int w, double
 }
 
 namespace {
-struct Dev {
-  void* p = nullptr;
-  ~Dev() { if (p) cudaFree(p); }
-  template <class T>
-  bool put(const T* h, size_t n) {
-    if (cudaMalloc(&p, std::max<size_t>(n, 1) * sizeof(T)) != cudaSuccess) return false;
-    return n == 0 || cudaMemcpy(p, h, n * sizeof(T), cudaMemcpyHostToDevice) == cudaSuccess;
-  }
-  template <class T>
-  bool make(size_t n) { return cudaMalloc(&p, std::max<size_t>(n, 1) * sizeof(T)) == cudaSuccess; }
-  template <class T>
-  T* as() { return (T*)p; }
-};
+// (at least one element, so that an empty array still has a device address)
+template <class T>
+bool make(DeviceBuf<T>& d, size_t n) { return d.alloc(std::max<size_t>(n, 1)); }
+template <class T>
+bool put(DeviceBuf<T>& d, const T* h, size_t n) {
+  return make(d, n) && (n == 0 || cudaMemcpy(d.get(), h, n * sizeof(T), cudaMemcpyHostToDevice) == cudaSuccess);
+}
 
 std::vector<double> clone_records(const double* clone_R, const double* clone_p, int N) {
   std::vector<double> cl((size_t)N * CL_STRIDE, 0.0);
@@ -372,23 +367,24 @@ extern "C" int orcvio_ekf_measurement_jacobians(const double* clone_R, const dou
   }
   if (n_obs == 0) return ORCVIO_OK;
   const std::vector<double> cl = clone_records(clone_R, clone_p, n_clones);
-  Dev dcl, dR, dt, dan, drho, dfan, dpos, dof, doc, doz, dHf, dHa, dHx, dHe, dr;
-  bool ok = dcl.put(cl.data(), cl.size()) && dR.put(R_b2c, 9) && dt.put(t_c_b, 3) && dan.put(anchor, n_feat) &&
-            drho.put(inv_depth, n_feat) && dfan.put(f_an, 2 * (size_t)n_feat) && dpos.put(positions, 3 * (size_t)n_feat) &&
-            dof.put(obs_feat.data(), n_obs) && doc.put(obs_clone, n_obs) && doz.put(obs_z, 2 * (size_t)n_obs) &&
-            dHf.make<double>(2 * (size_t)n_obs) && dHa.make<double>(12 * (size_t)n_obs) &&
-            dHx.make<double>(12 * (size_t)n_obs) && dHe.make<double>(12 * (size_t)n_obs) && dr.make<double>(2 * (size_t)n_obs);
+  DeviceBuf<double> dcl, dR, dt, drho, dfan, dpos, doz, dHf, dHa, dHx, dHe, dr;
+  DeviceBuf<int> dan, dof, doc;
+  bool ok = put(dcl, cl.data(), cl.size()) && put(dR, R_b2c, 9) && put(dt, t_c_b, 3) && put(dan, anchor, n_feat) &&
+            put(drho, inv_depth, n_feat) && put(dfan, f_an, 2 * (size_t)n_feat) && put(dpos, positions, 3 * (size_t)n_feat) &&
+            put(dof, obs_feat.data(), n_obs) && put(doc, obs_clone, n_obs) && put(doz, obs_z, 2 * (size_t)n_obs) &&
+            make(dHf, 2 * (size_t)n_obs) && make(dHa, 12 * (size_t)n_obs) &&
+            make(dHx, 12 * (size_t)n_obs) && make(dHe, 12 * (size_t)n_obs) && make(dr, 2 * (size_t)n_obs);
   if (!ok) return ORCVIO_ERR_CUDA;
-  EkfArgs a{dcl.as<double>(), dR.as<double>(), dt.as<double>(), dan.as<int>(), drho.as<double>(), dfan.as<double>(),
-            dpos.as<double>(), dof.as<int>(), doc.as<int>(), doz.as<double>(), n_obs, dHf.as<double>(), dHa.as<double>(),
-            dHx.as<double>(), dHe.as<double>(), dr.as<double>()};
+  EkfArgs a{dcl.get(), dR.get(), dt.get(), dan.get(), drho.get(), dfan.get(),
+            dpos.get(), dof.get(), doc.get(), doz.get(), n_obs, dHf.get(), dHa.get(),
+            dHx.get(), dHe.get(), dr.get()};
   k_ekf_jac<<<(n_obs + 127) / 128, 128>>>(a);
   check_launch("k_ekf_jac");
-  ok = cudaMemcpy(H_f, dHf.p, 2 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(H_a, dHa.p, 12 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(H_x, dHx.p, 12 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(H_e, dHe.p, 12 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(r, dr.p, 2 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess;
+  ok = cudaMemcpy(H_f, dHf.get(), 2 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(H_a, dHa.get(), 12 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(H_x, dHx.get(), 12 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(H_e, dHe.get(), 12 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(r, dr.get(), 2 * (size_t)n_obs * 8, cudaMemcpyDeviceToHost) == cudaSuccess;
   return ok ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -405,21 +401,22 @@ extern "C" int orcvio_ekf_feature_rows(const double* clone_R, const double* clon
     if (anchor[f] < 0 || anchor[f] >= n_clones || !(inv_depth[f] != 0.0)) return ORCVIO_ERR_ARG;
   if (n_feat == 0) return ORCVIO_OK;
   const std::vector<double> cl = clone_records(clone_R, clone_p, n_clones);
-  Dev dcl, dR, dt, dan, drho, dfan, dpos, dz, dP, dH, dr, dg, dp;
-  bool ok = dcl.put(cl.data(), cl.size()) && dR.put(R_b2c, 9) && dt.put(t_c_b, 3) && dan.put(anchor, n_feat) &&
-            drho.put(inv_depth, n_feat) && dfan.put(f_an, 2 * (size_t)n_feat) && dpos.put(positions, 3 * (size_t)n_feat) &&
-            dz.put(z_cur, 2 * (size_t)n_feat) && dP.put(P, (size_t)D * D) && dH.make<double>((size_t)2 * n_feat * D) &&
-            dr.make<double>(2 * (size_t)n_feat) && dg.make<double>(n_feat) && dp.make<int>(n_feat);
+  DeviceBuf<double> dcl, dR, dt, drho, dfan, dpos, dz, dP, dH, dr, dg;
+  DeviceBuf<int> dan, dp;
+  bool ok = put(dcl, cl.data(), cl.size()) && put(dR, R_b2c, 9) && put(dt, t_c_b, 3) && put(dan, anchor, n_feat) &&
+            put(drho, inv_depth, n_feat) && put(dfan, f_an, 2 * (size_t)n_feat) && put(dpos, positions, 3 * (size_t)n_feat) &&
+            put(dz, z_cur, 2 * (size_t)n_feat) && put(dP, P, (size_t)D * D) && make(dH, (size_t)2 * n_feat * D) &&
+            make(dr, 2 * (size_t)n_feat) && make(dg, n_feat) && make(dp, n_feat);
   if (!ok) return ORCVIO_ERR_CUDA;
-  EkfRowArgs a{dcl.as<double>(), dR.as<double>(), dt.as<double>(), n_clones, n_feat, dan.as<int>(), drho.as<double>(),
-               dfan.as<double>(), dpos.as<double>(), dz.as<double>(), dP.as<double>(), D, noise_var,
-               chi2_quantile(chi2_p, 2), dH.as<double>(), dr.as<double>(), dg.as<double>(), dp.as<int>()};
+  EkfRowArgs a{dcl.get(), dR.get(), dt.get(), n_clones, n_feat, dan.get(), drho.get(),
+               dfan.get(), dpos.get(), dz.get(), dP.get(), D, noise_var,
+               chi2_quantile(chi2_p, 2), dH.get(), dr.get(), dg.get(), dp.get()};
   k_ekf_rows<<<(n_feat + 63) / 64, 64>>>(a);
   check_launch("k_ekf_rows");
-  ok = cudaMemcpy(H, dH.p, (size_t)2 * n_feat * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(r, dr.p, 2 * (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(gamma, dg.p, (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(pass, dp.p, (size_t)n_feat * 4, cudaMemcpyDeviceToHost) == cudaSuccess;
+  ok = cudaMemcpy(H, dH.get(), (size_t)2 * n_feat * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(r, dr.get(), 2 * (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(gamma, dg.get(), (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(pass, dp.get(), (size_t)n_feat * 4, cudaMemcpyDeviceToHost) == cudaSuccess;
   return ok ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -435,20 +432,20 @@ extern "C" int orcvio_ekf_update_feature_cov(double* P, int D, const double* clo
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return ORCVIO_ERR_NO_DEVICE;
   const std::vector<double> cl = clone_records(clone_R, clone_p, n_clones);
-  Dev dcl, dR, dt, dP, dJ;
-  bool ok = dcl.put(cl.data(), cl.size()) && dR.put(R_b2c, 9) && dt.put(t_c_b, 3) && dP.put(P, (size_t)D * D) &&
-            dJ.make<double>(D);
+  DeviceBuf<double> dcl, dR, dt, dP, dJ;
+  bool ok = put(dcl, cl.data(), cl.size()) && put(dR, R_b2c, 9) && put(dt, t_c_b, 3) && put(dP, P, (size_t)D * D) &&
+            make(dJ, D);
   if (!ok) return ORCVIO_ERR_CUDA;
   ReanchorArgs a{};
-  a.clones = dcl.as<double>(); a.Rbc = dR.as<double>(); a.tcb = dt.as<double>(); a.N = n_clones;
+  a.clones = dcl.get(); a.Rbc = dR.get(); a.tcb = dt.get(); a.N = n_clones;
   a.feat_idx = feat_idx; a.old_idx = old_idx; a.new_idx = new_idx;
   for (int k = 0; k < 3; ++k) a.pw[k] = p_w[k];
   a.rho_new = inv_depth_new;
-  a.P = dP.as<double>(); a.D = D; a.J_out = dJ.as<double>();
+  a.P = dP.get(); a.D = D; a.J_out = dJ.get();
   k_ekf_reanchor<<<1, 256, 2 * (size_t)D * sizeof(double)>>>(a);
   check_launch("k_ekf_reanchor");
-  ok = cudaMemcpy(P, dP.p, (size_t)D * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       (!J_out || cudaMemcpy(J_out, dJ.p, (size_t)D * 8, cudaMemcpyDeviceToHost) == cudaSuccess);
+  ok = cudaMemcpy(P, dP.get(), (size_t)D * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       (!J_out || cudaMemcpy(J_out, dJ.get(), (size_t)D * 8, cudaMemcpyDeviceToHost) == cudaSuccess);
   return ok ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -458,12 +455,12 @@ extern "C" int orcvio_ekf_remove_feature_cov(const double* P, int D, int n_clone
   if (n_clones < 1 || E < 1 || feat_idx < 0 || feat_idx >= E) return ORCVIO_ERR_ARG;
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return ORCVIO_ERR_NO_DEVICE;
-  Dev dP, dO;
+  DeviceBuf<double> dP, dO;
   const int Dn = D - 1;
-  if (!dP.put(P, (size_t)D * D) || !dO.make<double>((size_t)Dn * Dn)) return ORCVIO_ERR_CUDA;
-  k_ekf_drop_state<<<(Dn * Dn + 255) / 256, 256>>>(dP.as<double>(), D, ORCVIO_LEG + 6 * n_clones + feat_idx, dO.as<double>());
+  if (!put(dP, P, (size_t)D * D) || !make(dO, (size_t)Dn * Dn)) return ORCVIO_ERR_CUDA;
+  k_ekf_drop_state<<<(Dn * Dn + 255) / 256, 256>>>(dP.get(), D, ORCVIO_LEG + 6 * n_clones + feat_idx, dO.get());
   check_launch("k_ekf_drop_state");
-  return cudaMemcpy(P_out, dO.p, (size_t)Dn * Dn * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
+  return cudaMemcpy(P_out, dO.get(), (size_t)Dn * Dn * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
 extern "C" int orcvio_ekf_new_feature_rows(const double* clone_R, const double* clone_p, int n_clones,
@@ -492,27 +489,28 @@ extern "C" int orcvio_ekf_new_feature_rows(const double* clone_R, const double* 
   if (n_feat == 0) return ORCVIO_OK;
   const int n_obs = feat_off[n_feat], n_ho = row_off[n_feat];
   const std::vector<double> cl = clone_records(clone_R, clone_p, n_clones);
-  Dev dcl, dR, dt, dan, drho, dfan, dpos, dfo, doc, doz, dro, dH1, dh2, dr1, dHo, dr, dsc;
-  bool ok = dcl.put(cl.data(), cl.size()) && dR.put(R_b2c, 9) && dt.put(t_c_b, 3) && dan.put(anchor, n_feat) &&
-            drho.put(inv_depth, n_feat) && dfan.put(f_an, 2 * (size_t)n_feat) && dpos.put(positions, 3 * (size_t)n_feat) &&
-            dfo.put(feat_off, n_feat + 1) && doc.put(obs_clone, n_obs) && doz.put(obs_z, 2 * (size_t)n_obs) &&
-            dro.put(row_off.data(), n_feat + 1) && dH1.make<double>((size_t)n_feat * D) && dh2.make<double>(n_feat) &&
-            dr1.make<double>(n_feat) && dHo.make<double>((size_t)n_ho * D) && dr.make<double>(n_ho) &&
-            dsc.make<double>((size_t)n_feat * 64 * D);
+  DeviceBuf<double> dcl, dR, dt, drho, dfan, dpos, doz, dH1, dh2, dr1, dHo, dr, dsc;
+  DeviceBuf<int> dan, dfo, doc, dro;
+  bool ok = put(dcl, cl.data(), cl.size()) && put(dR, R_b2c, 9) && put(dt, t_c_b, 3) && put(dan, anchor, n_feat) &&
+            put(drho, inv_depth, n_feat) && put(dfan, f_an, 2 * (size_t)n_feat) && put(dpos, positions, 3 * (size_t)n_feat) &&
+            put(dfo, feat_off, n_feat + 1) && put(doc, obs_clone, n_obs) && put(doz, obs_z, 2 * (size_t)n_obs) &&
+            put(dro, row_off.data(), n_feat + 1) && make(dH1, (size_t)n_feat * D) && make(dh2, n_feat) &&
+            make(dr1, n_feat) && make(dHo, (size_t)n_ho * D) && make(dr, n_ho) &&
+            make(dsc, (size_t)n_feat * 64 * D);
   if (!ok) return ORCVIO_ERR_CUDA;
-  cudaMemset(dH1.p, 0, (size_t)n_feat * D * 8);
-  cudaMemset(dh2.p, 0, (size_t)n_feat * 8);
-  cudaMemset(dr1.p, 0, (size_t)n_feat * 8);
-  EkfNewArgs a{dcl.as<double>(), dR.as<double>(), dt.as<double>(), n_clones, D, dan.as<int>(), drho.as<double>(),
-               dfan.as<double>(), dpos.as<double>(), dfo.as<int>(), doc.as<int>(), doz.as<double>(), dro.as<int>(),
-               dH1.as<double>(), dh2.as<double>(), dr1.as<double>(), dHo.as<double>(), dr.as<double>(), dsc.as<double>()};
+  cudaMemset(dH1.get(), 0, (size_t)n_feat * D * 8);
+  cudaMemset(dh2.get(), 0, (size_t)n_feat * 8);
+  cudaMemset(dr1.get(), 0, (size_t)n_feat * 8);
+  EkfNewArgs a{dcl.get(), dR.get(), dt.get(), n_clones, D, dan.get(), drho.get(),
+               dfan.get(), dpos.get(), dfo.get(), doc.get(), doz.get(), dro.get(),
+               dH1.get(), dh2.get(), dr1.get(), dHo.get(), dr.get(), dsc.get()};
   k_ekf_new_rows<<<n_feat, 128>>>(a);
   check_launch("k_ekf_new_rows");
-  ok = cudaMemcpy(H_1, dH1.p, (size_t)n_feat * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(h_2, dh2.p, (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(r_1, dr1.p, (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       (n_ho == 0 || (cudaMemcpy(H_o, dHo.p, (size_t)n_ho * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-                      cudaMemcpy(r_o, dr.p, (size_t)n_ho * 8, cudaMemcpyDeviceToHost) == cudaSuccess));
+  ok = cudaMemcpy(H_1, dH1.get(), (size_t)n_feat * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(h_2, dh2.get(), (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(r_1, dr1.get(), (size_t)n_feat * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       (n_ho == 0 || (cudaMemcpy(H_o, dHo.get(), (size_t)n_ho * D * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+                      cudaMemcpy(r_o, dr.get(), (size_t)n_ho * 8, cudaMemcpyDeviceToHost) == cudaSuccess));
   return ok ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -525,19 +523,19 @@ extern "C" int orcvio_ekf_delayed_init(const double* P, int D, const double* dx_
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return ORCVIO_ERR_NO_DEVICE;
   const int Da = D + n_new;
-  Dev dP, ddx, dH1, dh2, dr1, dn, dxn, dPa;
-  bool ok = dP.put(P, (size_t)D * D) && ddx.put(dx_leg, D) && dH1.put(H_1, (size_t)n_new * D) && dh2.put(h_2, n_new) &&
-            dr1.put(r_1, n_new) && dn.make<double>((size_t)n_new * D) && dxn.make<double>(n_new) &&
-            dPa.make<double>((size_t)Da * Da);
+  DeviceBuf<double> dP, ddx, dH1, dh2, dr1, dn, dxn, dPa;
+  bool ok = put(dP, P, (size_t)D * D) && put(ddx, dx_leg, D) && put(dH1, H_1, (size_t)n_new * D) && put(dh2, h_2, n_new) &&
+            put(dr1, r_1, n_new) && make(dn, (size_t)n_new * D) && make(dxn, n_new) &&
+            make(dPa, (size_t)Da * Da);
   if (!ok) return ORCVIO_ERR_CUDA;
-  EkfInitArgs a{dP.as<double>(), D, n_new, ddx.as<double>(), dH1.as<double>(), dh2.as<double>(), dr1.as<double>(),
-                noise_var, dn.as<double>(), dxn.as<double>(), dPa.as<double>()};
+  EkfInitArgs a{dP.get(), D, n_new, ddx.get(), dH1.get(), dh2.get(), dr1.get(),
+                noise_var, dn.get(), dxn.get(), dPa.get()};
   k_ekf_init_cross<<<n_new, 256, (size_t)D * sizeof(double)>>>(a);
   check_launch("k_ekf_init_cross");
   k_ekf_init_assemble<<<(int)(((size_t)Da * Da + 255) / 256), 256>>>(a);
   check_launch("k_ekf_init_assemble");
-  ok = cudaMemcpy(dx_new, dxn.p, (size_t)n_new * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
-       cudaMemcpy(P_aug, dPa.p, (size_t)Da * Da * 8, cudaMemcpyDeviceToHost) == cudaSuccess;
+  ok = cudaMemcpy(dx_new, dxn.get(), (size_t)n_new * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+       cudaMemcpy(P_aug, dPa.get(), (size_t)Da * Da * 8, cudaMemcpyDeviceToHost) == cudaSuccess;
   return ok ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -547,12 +545,12 @@ extern "C" int orcvio_ekf_augment_cov(const double* P, int D, int n_clones, doub
   if (n_clones < 0 || D < c0) return ORCVIO_ERR_ARG;
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return ORCVIO_ERR_NO_DEVICE;
-  Dev dP, dO;
+  DeviceBuf<double> dP, dO;
   const int Dn = D + 6;
-  if (!dP.put(P, (size_t)D * D) || !dO.make<double>((size_t)Dn * Dn)) return ORCVIO_ERR_CUDA;
-  k_ekf_augment<<<(int)(((size_t)Dn * Dn + 255) / 256), 256>>>(dP.as<double>(), D, c0, dO.as<double>());
+  if (!put(dP, P, (size_t)D * D) || !make(dO, (size_t)Dn * Dn)) return ORCVIO_ERR_CUDA;
+  k_ekf_augment<<<(int)(((size_t)Dn * Dn + 255) / 256), 256>>>(dP.get(), D, c0, dO.get());
   check_launch("k_ekf_augment");
-  return cudaMemcpy(P_out, dO.p, (size_t)Dn * Dn * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
+  return cudaMemcpy(P_out, dO.get(), (size_t)Dn * Dn * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
 extern "C" int orcvio_ekf_remove_clone_cov(const double* P, int D, int n_clones, int clone_idx, double* P_out) {
@@ -560,11 +558,11 @@ extern "C" int orcvio_ekf_remove_clone_cov(const double* P, int D, int n_clones,
   if (n_clones < 1 || clone_idx < 0 || clone_idx >= n_clones || D < ORCVIO_LEG + 6 * n_clones) return ORCVIO_ERR_ARG;
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) return ORCVIO_ERR_NO_DEVICE;
-  Dev dP, dO;
+  DeviceBuf<double> dP, dO;
   const int Dn = D - 6;
-  if (!dP.put(P, (size_t)D * D) || !dO.make<double>((size_t)Dn * Dn)) return ORCVIO_ERR_CUDA;
-  k_ekf_drop_block<<<(int)(((size_t)Dn * Dn + 255) / 256), 256>>>(dP.as<double>(), D, ORCVIO_LEG + 6 * clone_idx, 6,
-                                                                  dO.as<double>());
+  if (!put(dP, P, (size_t)D * D) || !make(dO, (size_t)Dn * Dn)) return ORCVIO_ERR_CUDA;
+  k_ekf_drop_block<<<(int)(((size_t)Dn * Dn + 255) / 256), 256>>>(dP.get(), D, ORCVIO_LEG + 6 * clone_idx, 6,
+                                                                  dO.get());
   check_launch("k_ekf_drop_block");
-  return cudaMemcpy(P_out, dO.p, (size_t)Dn * Dn * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
+  return cudaMemcpy(P_out, dO.get(), (size_t)Dn * Dn * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }

@@ -10,6 +10,7 @@
 // (coplanar keypoints: src/tests/test_kabsch.cpp test_planar) is completed with the cross product of the two leading
 // left vectors -- the rotation V diag(1, 1, det(V U^T)) U^T does not depend on the sign of that third vector.
 #include "../../include/orcvio_b200.h"
+#include "devmem.h"
 #include "kernels.h"
 #include "svd3.cuh"
 
@@ -85,22 +86,18 @@ int kabsch_init(const double* mean_pts, const double* world_pts, const int* off,
   if (n_obj < 1 || !mean_pts || !world_pts || !off || !wTq16 || !ok) return ORCVIO_ERR_ARG;
   const int n_pts = off[n_obj];
   if (n_pts < 0) return ORCVIO_ERR_ARG;
-  double *dA = nullptr, *dB = nullptr, *dT = nullptr;
-  int *dOff = nullptr, *dOk = nullptr;
-  const size_t nb = sizeof(double) * 3 * (size_t)std::max(n_pts, 1);
-  bool good = cudaMalloc(&dA, nb) == cudaSuccess && cudaMalloc(&dB, nb) == cudaSuccess &&
-              cudaMalloc(&dT, sizeof(double) * 16 * n_obj) == cudaSuccess &&
-              cudaMalloc(&dOff, sizeof(int) * (n_obj + 1)) == cudaSuccess && cudaMalloc(&dOk, sizeof(int) * n_obj) == cudaSuccess;
-  if (good) {
-    cudaMemcpy(dA, mean_pts, sizeof(double) * 3 * n_pts, cudaMemcpyHostToDevice);
-    cudaMemcpy(dB, world_pts, sizeof(double) * 3 * n_pts, cudaMemcpyHostToDevice);
-    cudaMemcpy(dOff, off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
-    k_kabsch<<<(n_obj + 63) / 64, 64>>>(dA, dB, dOff, n_obj, se2, dT, dOk);
-    check_launch("k_kabsch");
-    good = cudaMemcpy(wTq16, dT, sizeof(double) * 16 * n_obj, cudaMemcpyDeviceToHost) == cudaSuccess &&
-           cudaMemcpy(ok, dOk, sizeof(int) * n_obj, cudaMemcpyDeviceToHost) == cudaSuccess;
-  }
-  cudaFree(dA); cudaFree(dB); cudaFree(dT); cudaFree(dOff); cudaFree(dOk);
+  DeviceBuf<double> dA, dB, dT;
+  DeviceBuf<int> dOff, dOk;
+  const size_t np = 3 * (size_t)std::max(n_pts, 1);
+  if (!dA.alloc(np) || !dB.alloc(np) || !dT.alloc(16 * (size_t)n_obj) || !dOff.alloc(n_obj + 1) || !dOk.alloc(n_obj))
+    return ORCVIO_ERR_CUDA;
+  cudaMemcpy(dA.get(), mean_pts, sizeof(double) * 3 * n_pts, cudaMemcpyHostToDevice);
+  cudaMemcpy(dB.get(), world_pts, sizeof(double) * 3 * n_pts, cudaMemcpyHostToDevice);
+  cudaMemcpy(dOff.get(), off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
+  k_kabsch<<<(n_obj + 63) / 64, 64>>>(dA.get(), dB.get(), dOff.get(), n_obj, se2, dT.get(), dOk.get());
+  check_launch("k_kabsch");
+  const bool good = cudaMemcpy(wTq16, dT.get(), sizeof(double) * 16 * n_obj, cudaMemcpyDeviceToHost) == cudaSuccess &&
+                    cudaMemcpy(ok, dOk.get(), sizeof(int) * n_obj, cudaMemcpyDeviceToHost) == cudaSuccess;
   return good ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 

@@ -9,6 +9,7 @@
 // threads, fixed-order tree reduction.  Outputs per trajectory: mean orientation error (deg), mean position error (m),
 // position RMSE (m), final position error (m).
 #include "../../include/orcvio_b200.h"
+#include "devmem.h"
 #include "kernels.h"
 #include "svd3.cuh"
 
@@ -117,19 +118,15 @@ __global__ void __launch_bounds__(128) k_trajectory_metrics(const double* __rest
 
 int trajectory_metrics(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, double* out4) {
   if (n_traj < 1 || n_frames < 1) return ORCVIO_ERR_ARG;
-  const size_t nb = (size_t)n_traj * n_frames * 7 * sizeof(double);
-  double *dE = nullptr, *dG = nullptr, *dO = nullptr;
-  if (cudaMalloc(&dE, nb) != cudaSuccess || cudaMalloc(&dG, nb) != cudaSuccess ||
-      cudaMalloc(&dO, (size_t)n_traj * 4 * sizeof(double)) != cudaSuccess) {
-    cudaFree(dE); cudaFree(dG); cudaFree(dO);
+  const size_t np = (size_t)n_traj * n_frames * 7, nb = np * sizeof(double);
+  DeviceBuf<double> dE, dG, dO;
+  if (!dE.alloc(np) || !dG.alloc(np) || !dO.alloc((size_t)n_traj * 4))
     return ORCVIO_ERR_CUDA;
-  }
-  cudaMemcpy(dE, est_pose7, nb, cudaMemcpyHostToDevice);
-  cudaMemcpy(dG, gt_pose7, nb, cudaMemcpyHostToDevice);
-  k_trajectory_metrics<<<n_traj, 128>>>(dE, dG, n_frames, dO);
+  cudaMemcpy(dE.get(), est_pose7, nb, cudaMemcpyHostToDevice);
+  cudaMemcpy(dG.get(), gt_pose7, nb, cudaMemcpyHostToDevice);
+  k_trajectory_metrics<<<n_traj, 128>>>(dE.get(), dG.get(), n_frames, dO.get());
   check_launch("k_trajectory_metrics");
-  const cudaError_t e = cudaMemcpy(out4, dO, (size_t)n_traj * 4 * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dE); cudaFree(dG); cudaFree(dO);
+  const cudaError_t e = cudaMemcpy(out4, dO.get(), dO.bytes(), cudaMemcpyDeviceToHost);
   return e == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
@@ -257,25 +254,22 @@ __global__ void __launch_bounds__(256) k_kitti_relative_error(const double* __re
 int kitti_relative_error(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, const double* lengths,
                          int n_len, const double* scale, double* out4, double* trans_error_pct) {
   if (n_traj < 1 || n_frames < 2 || n_len < 1 || n_frames > 4096) return ORCVIO_ERR_ARG;
-  const size_t nb = (size_t)n_traj * n_frames * 7 * sizeof(double);
-  double *dE = nullptr, *dG = nullptr, *dL = nullptr, *dO = nullptr, *dS = nullptr;
+  const size_t np = (size_t)n_traj * n_frames * 7, nb = np * sizeof(double);
+  DeviceBuf<double> dE, dG, dL, dO, dS;
   const size_t no = (size_t)n_traj * n_len * 4;
-  if (cudaMalloc(&dE, nb) != cudaSuccess || cudaMalloc(&dG, nb) != cudaSuccess ||
-      cudaMalloc(&dL, n_len * sizeof(double)) != cudaSuccess || cudaMalloc(&dO, no * sizeof(double)) != cudaSuccess ||
-      cudaMalloc(&dS, n_traj * sizeof(double)) != cudaSuccess) {
-    cudaFree(dE); cudaFree(dG); cudaFree(dL); cudaFree(dO); cudaFree(dS);
+  if (!dE.alloc(np) || !dG.alloc(np) || !dL.alloc(n_len) || !dO.alloc(no) ||
+      !dS.alloc(n_traj))
     return ORCVIO_ERR_CUDA;
-  }
-  if (scale) cudaMemcpy(dS, scale, n_traj * sizeof(double), cudaMemcpyHostToDevice);
-  cudaMemcpy(dE, est_pose7, nb, cudaMemcpyHostToDevice);
-  cudaMemcpy(dG, gt_pose7, nb, cudaMemcpyHostToDevice);
-  cudaMemcpy(dL, lengths, n_len * sizeof(double), cudaMemcpyHostToDevice);
+  if (scale) cudaMemcpy(dS.get(), scale, n_traj * sizeof(double), cudaMemcpyHostToDevice);
+  cudaMemcpy(dE.get(), est_pose7, nb, cudaMemcpyHostToDevice);
+  cudaMemcpy(dG.get(), gt_pose7, nb, cudaMemcpyHostToDevice);
+  cudaMemcpy(dL.get(), lengths, n_len * sizeof(double), cudaMemcpyHostToDevice);
   const size_t smem = (size_t)n_frames * (4 * sizeof(double) + 2 * sizeof(int));
   cudaFuncSetAttribute(k_kitti_relative_error, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  k_kitti_relative_error<<<dim3(n_len, n_traj), 256, smem>>>(dE, dG, n_frames, dL, n_len, scale ? dS : nullptr, dO);
+  k_kitti_relative_error<<<dim3(n_len, n_traj), 256, smem>>>(dE.get(), dG.get(), n_frames, dL.get(), n_len,
+                                                            scale ? dS.get() : nullptr, dO.get());
   check_launch("k_kitti_relative_error");
-  const cudaError_t e = cudaMemcpy(out4, dO, no * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dE); cudaFree(dG); cudaFree(dL); cudaFree(dO); cudaFree(dS);
+  const cudaError_t e = cudaMemcpy(out4, dO.get(), no * sizeof(double), cudaMemcpyDeviceToHost);
   if (e != cudaSuccess) return ORCVIO_ERR_CUDA;
   if (trans_error_pct)                 // write_kitti_errors_to_yaml: sum of the per-length means / (valid lengths + 1e-5)
     for (int t = 0; t < n_traj; ++t) {
@@ -374,19 +368,15 @@ __global__ void __launch_bounds__(128) k_umeyama_ate(const double* __restrict__ 
 
 int umeyama_ate(const double* est_pose7, const double* gt_pose7, int n_traj, int n_frames, int known_scale, double* out15) {
   if (n_traj < 1 || n_frames < 3) return ORCVIO_ERR_ARG;
-  const size_t nb = (size_t)n_traj * n_frames * 7 * sizeof(double);
-  double *dE = nullptr, *dG = nullptr, *dO = nullptr;
-  if (cudaMalloc(&dE, nb) != cudaSuccess || cudaMalloc(&dG, nb) != cudaSuccess ||
-      cudaMalloc(&dO, (size_t)n_traj * 15 * sizeof(double)) != cudaSuccess) {
-    cudaFree(dE); cudaFree(dG); cudaFree(dO);
+  const size_t np = (size_t)n_traj * n_frames * 7, nb = np * sizeof(double);
+  DeviceBuf<double> dE, dG, dO;
+  if (!dE.alloc(np) || !dG.alloc(np) || !dO.alloc((size_t)n_traj * 15))
     return ORCVIO_ERR_CUDA;
-  }
-  cudaMemcpy(dE, est_pose7, nb, cudaMemcpyHostToDevice);
-  cudaMemcpy(dG, gt_pose7, nb, cudaMemcpyHostToDevice);
-  k_umeyama_ate<<<n_traj, 128>>>(dE, dG, n_frames, known_scale, dO);
+  cudaMemcpy(dE.get(), est_pose7, nb, cudaMemcpyHostToDevice);
+  cudaMemcpy(dG.get(), gt_pose7, nb, cudaMemcpyHostToDevice);
+  k_umeyama_ate<<<n_traj, 128>>>(dE.get(), dG.get(), n_frames, known_scale, dO.get());
   check_launch("k_umeyama_ate");
-  const cudaError_t e = cudaMemcpy(out15, dO, (size_t)n_traj * 15 * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dE); cudaFree(dG); cudaFree(dO);
+  const cudaError_t e = cudaMemcpy(out15, dO.get(), dO.bytes(), cudaMemcpyDeviceToHost);
   return e == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 

@@ -24,13 +24,6 @@ namespace ob {
 
 namespace {
 
-struct DevBuf {
-  void* p = nullptr;
-  ~DevBuf() { if (p) cudaFree(p); }
-  template <class T> T* as() { return (T*)p; }
-  cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 8); }
-};
-
 // Scratch of the calling thread for the per-object entries: ONE grow-only device block and ONE pinned host block,
 // carved by bump pointers.  The entries are called once per object and frame; a cudaMalloc / cudaFree pair per buffer
 // (about ten per call, each a device-wide synchronisation) and a blocking copy per argument were most of their time.
@@ -291,37 +284,26 @@ int Batch::object_update(int fi, const double* Hx, const double* Hf, const doubl
   FilterWork fw{};                                       // jrow0 = 0: a dense block has no staircase
   fw.N = N; fw.D = D; fw.active = 1; fw.arow0 = 0; fw.arows = prow;
   const int units = syrk_plan(fw, n_sm_).total;
-  const size_t need_a = ((size_t)prow + 16) * ldr_;
-  if (need_a > amat_cap_) {
-    if (dAmat_) cudaFree(dAmat_);
-    amat_cap_ = need_a * 2;
-    CKO(cudaMalloc(&dAmat_, amat_cap_ * sizeof(double)));
-  }
-  const size_t need_p = (size_t)units * 4096;
-  if (need_p > part_cap_) {
-    if (dPart_) cudaFree(dPart_);
-    part_cap_ = need_p * 2;
-    CKO(cudaMalloc(&dPart_, part_cap_ * sizeof(double)));
-  }
+  CKO(grow_update_scratch(((size_t)prow + 16) * ldr_, (size_t)units * 4096));
   *hFw = fw;
   CKO(cudaMemcpyAsync(dM, M, up_bytes, cudaMemcpyHostToDevice, stream_));        // M and the work record: one copy
   launch_project_dense(dM, rows, ld, odim, ld, stream_);                          // nullspace_project_inplace_svd
   const size_t r_stride = (size_t)(nmax_ + 1) * ldr_;
   UpdArgs ua{};
   ua.fw = dFw; ua.n_filters = 1;
-  ua.P = dP_ + (size_t)fi * ldp_ * ldp_; ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
+  ua.P = dP_.get() + (size_t)fi * ldp_ * ldp_; ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
   ua.r_stride = r_stride; ua.ldr = ldr_;
-  ua.T = dT_ + (size_t)fi * nmax_ * ldt_; ua.S = dS_ + (size_t)fi * r_stride;
+  ua.T = dT_.get() + (size_t)fi * nmax_ * ldt_; ua.S = dS_.get() + (size_t)fi * r_stride;
   ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
-  ua.yv = dYv_ + (size_t)fi * ldr_;
-  ua.imu = dImu_ + (size_t)fi * IM_STRIDE; ua.clones = dClones_ + (size_t)fi * Ncap_ * CL_STRIDE;
+  ua.yv = dYv_.get() + (size_t)fi * ldr_;
+  ua.imu = dImu_.get() + (size_t)fi * IM_STRIDE; ua.clones = dClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE;
   ua.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-  ua.dx = dDx_ + (size_t)fi * ldp_; ua.lddx = ldp_;
+  ua.dx = dDx_.get() + (size_t)fi * ldp_; ua.lddx = ldp_;
   ua.flags = flags_; ua.sigma2 = p_.feature_observation_noise;
   InfoBufs ib{};
-  ib.Ls = dLs_ + (size_t)fi * ORCVIO_LEG * ORCVIO_LEG; ib.Amat = dAmat_; ib.part = dPart_;
-  ib.max_units = units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_;
-  ib.tile_rows = nullptr; ib.filter_rows = dFilterRows_ + fi;
+  ib.Ls = dLs_.get() + (size_t)fi * ORCVIO_LEG * ORCVIO_LEG; ib.Amat = dAmat_.get(); ib.part = dPart_.get();
+  ib.max_units = units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_.get();
+  ib.tile_rows = nullptr; ib.filter_rows = dFilterRows_.get() + fi;
   const double* Hp = dM + (size_t)odim * ld + odim;
   launch_info_dense_factor(ua, ib, Hp, ld, prow, n, stream_);
   launches_ += 5;
@@ -346,8 +328,8 @@ int Batch::object_update(int fi, const double* Hx, const double* Hf, const doubl
   launches_ += 1;
   download_mirrors();
   CKO(cudaStreamSynchronize(stream_));
-  std::memcpy(F.imu_mirror.data(), hImu_ + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
-  std::memcpy(F.clone_mirror.data(), hClones_ + (size_t)fi * Ncap_ * CL_STRIDE,
+  std::memcpy(F.imu_mirror.data(), hImu_.get() + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
+  std::memcpy(F.clone_mirror.data(), hClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE,
               (size_t)Ncap_ * CL_STRIDE * sizeof(double));
   return done(0, 1);
 }
@@ -370,31 +352,32 @@ int Batch::propagate_standalone(double* state16, const double* bg, const double*
   }
   for (int k = 0; k < 9; ++k) im[IM_RBC + k] = (k % 4 == 0) ? 1.0 : 0.0;
   im[IM_TIME] = state16[15];
-  CKO(cudaMemcpy(dImu_, im.data(), IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice));
-  CKO(cudaMemcpy2D(dP_, ldp_ * sizeof(double), P, D * sizeof(double), D * sizeof(double), D, cudaMemcpyHostToDevice));
+  CKO(cudaMemcpy(dImu_.get(), im.data(), IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice));
+  CKO(cudaMemcpy2D(dP_.get(), ldp_ * sizeof(double), P, D * sizeof(double), D * sizeof(double), D, cudaMemcpyHostToDevice));
   std::vector<PropSample> smp(std::max(n, 1));
   for (int k = 0; k < n; ++k) {
     smp[k].t = imu[k].t;
     for (int q = 0; q < 3; ++q) { smp[k].w[q] = imu[k].gyro[q]; smp[k].a[q] = imu[k].acc[q]; }
   }
-  DevBuf dS, dOff, dD;
+  DeviceBuf<PropSample> dS;
+  DeviceBuf<int> dOff, dD;
   int off[2] = {0, n};
-  CKO(dS.alloc(sizeof(PropSample) * smp.size())); CKO(dOff.alloc(sizeof(off))); CKO(dD.alloc(sizeof(int)));
-  CKO(cudaMemcpy(dS.p, smp.data(), sizeof(PropSample) * smp.size(), cudaMemcpyHostToDevice));
-  CKO(cudaMemcpy(dOff.p, off, sizeof(off), cudaMemcpyHostToDevice));
-  CKO(cudaMemcpy(dD.p, &D, sizeof(int), cudaMemcpyHostToDevice));
+  if (!dS.alloc(smp.size()) || !dOff.alloc(2) || !dD.alloc(1)) return ORCVIO_ERR_CUDA;
+  CKO(cudaMemcpy(dS.get(), smp.data(), sizeof(PropSample) * smp.size(), cudaMemcpyHostToDevice));
+  CKO(cudaMemcpy(dOff.get(), off, sizeof(off), cudaMemcpyHostToDevice));
+  CKO(cudaMemcpy(dD.get(), &D, sizeof(int), cudaMemcpyHostToDevice));
   PropArgs pa{};
-  pa.P = dP_; pa.p_stride = (size_t)ldp_ * ldp_; pa.ldp = ldp_;
-  pa.imu = dImu_;
-  pa.samples = dS.as<PropSample>(); pa.samp_off = dOff.as<int>(); pa.D = dD.as<int>();
+  pa.P = dP_.get(); pa.p_stride = (size_t)ldp_ * ldp_; pa.ldp = ldp_;
+  pa.imu = dImu_.get();
+  pa.samples = dS.get(); pa.samp_off = dOff.get(); pa.D = dD.get();
   pa.n_filters = 1; pa.flags = flags_;
   for (int k = 0; k < 4; ++k) pa.qc[k] = noise4[k];
   launch_propagate(pa, stream_);
   ++launches_;
   CKO(cudaStreamSynchronize(stream_));
   if (launch_error_count() > 0) return ORCVIO_ERR_CUDA;
-  CKO(cudaMemcpy(im.data(), dImu_, IM_STRIDE * sizeof(double), cudaMemcpyDeviceToHost));
-  CKO(cudaMemcpy2D(P, D * sizeof(double), dP_, ldp_ * sizeof(double), D * sizeof(double), D, cudaMemcpyDeviceToHost));
+  CKO(cudaMemcpy(im.data(), dImu_.get(), IM_STRIDE * sizeof(double), cudaMemcpyDeviceToHost));
+  CKO(cudaMemcpy2D(P, D * sizeof(double), dP_.get(), ldp_ * sizeof(double), D * sizeof(double), D, cudaMemcpyDeviceToHost));
   for (int k = 0; k < 9; ++k) state16[k] = im[IM_R + k];
   for (int k = 0; k < 3; ++k) { state16[9 + k] = im[IM_V + k]; state16[12 + k] = im[IM_P + k]; }
   state16[15] = im[IM_TIME];
@@ -411,8 +394,8 @@ int Batch::dense_update(const double* P_in, int D, const double* H, const double
   const int n = D - ORCVIO_LEG;
   if (n < 1 || D > ldp_ || n > nmax_ || rows < 1) return ORCVIO_ERR_ARG;
   const int fi = 0;
-  CKO(cudaMemsetAsync(dP_, 0, (size_t)ldp_ * ldp_ * sizeof(double), stream_));
-  CKO(cudaMemcpy2DAsync(dP_, ldp_ * sizeof(double), P_in, D * sizeof(double), D * sizeof(double), D,
+  CKO(cudaMemsetAsync(dP_.get(), 0, (size_t)ldp_ * ldp_ * sizeof(double), stream_));
+  CKO(cudaMemcpy2DAsync(dP_.get(), ldp_ * sizeof(double), P_in, D * sizeof(double), D * sizeof(double), D,
                         cudaMemcpyHostToDevice, stream_));
   const int ld = n + 1;
   std::vector<double> M((size_t)rows * ld);
@@ -420,47 +403,37 @@ int Batch::dense_update(const double* P_in, int D, const double* H, const double
     for (int k = 0; k < n; ++k) M[(size_t)i * ld + k] = H[(size_t)i * D + ORCVIO_LEG + k];
     M[(size_t)i * ld + n] = r[i];
   }
-  DevBuf dM, dFw;
-  CKO(dM.alloc(M.size() * sizeof(double)));
-  CKO(cudaMemcpyAsync(dM.p, M.data(), M.size() * sizeof(double), cudaMemcpyHostToDevice, stream_));
+  DeviceBuf<double> dM;
+  DeviceBuf<FilterWork> dFw;
+  if (!dM.alloc(M.size())) return ORCVIO_ERR_CUDA;
+  CKO(cudaMemcpyAsync(dM.get(), M.data(), M.size() * sizeof(double), cudaMemcpyHostToDevice, stream_));
   FilterWork fw{};
   fw.N = 0;                                              // no clone poses behind this entry: dx is returned, not applied
   fw.D = D; fw.active = 1; fw.arow0 = 0; fw.arows = rows;
   const int units = syrk_plan(fw, n_sm_).total;
-  const size_t need_a = ((size_t)rows + 16) * ldr_;
-  if (need_a > amat_cap_) {
-    if (dAmat_) cudaFree(dAmat_);
-    amat_cap_ = need_a * 2;
-    CKO(cudaMalloc(&dAmat_, amat_cap_ * sizeof(double)));
-  }
-  const size_t need_p = (size_t)units * 4096;
-  if (need_p > part_cap_) {
-    if (dPart_) cudaFree(dPart_);
-    part_cap_ = need_p * 2;
-    CKO(cudaMalloc(&dPart_, part_cap_ * sizeof(double)));
-  }
-  CKO(dFw.alloc(sizeof(FilterWork)));
-  CKO(cudaMemcpyAsync(dFw.p, &fw, sizeof(fw), cudaMemcpyHostToDevice, stream_));
+  CKO(grow_update_scratch(((size_t)rows + 16) * ldr_, (size_t)units * 4096));
+  if (!dFw.alloc(1)) return ORCVIO_ERR_CUDA;
+  CKO(cudaMemcpyAsync(dFw.get(), &fw, sizeof(fw), cudaMemcpyHostToDevice, stream_));
   const size_t r_stride = (size_t)(nmax_ + 1) * ldr_;
   UpdArgs ua{};
-  ua.fw = dFw.as<FilterWork>(); ua.n_filters = 1;
-  ua.P = dP_; ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
+  ua.fw = dFw.get(); ua.n_filters = 1;
+  ua.P = dP_.get(); ua.p_stride = (size_t)ldp_ * ldp_; ua.ldp = ldp_;
   ua.r_stride = r_stride; ua.ldr = ldr_;
-  ua.T = dT_; ua.S = dS_; ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
-  ua.yv = dYv_;
-  ua.imu = dImu_; ua.clones = dClones_; ua.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-  ua.dx = dDx_; ua.lddx = ldp_;
+  ua.T = dT_.get(); ua.S = dS_.get(); ua.t_stride = (size_t)nmax_ * ldt_; ua.ldt = ldt_;
+  ua.yv = dYv_.get();
+  ua.imu = dImu_.get(); ua.clones = dClones_.get(); ua.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+  ua.dx = dDx_.get(); ua.lddx = ldp_;
   ua.flags = 0; ua.sigma2 = p_.feature_observation_noise;
   InfoBufs ib{};
-  ib.Ls = dLs_; ib.Amat = dAmat_; ib.part = dPart_;
-  ib.max_units = units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_;
-  ib.tile_rows = nullptr; ib.filter_rows = dFilterRows_ + fi;
-  CKO(cudaMemsetAsync(dImu_, 0, IM_STRIDE * sizeof(double), stream_));
-  launch_info_dense_factor(ua, ib, dM.as<double>(), ld, rows, n, stream_);
+  ib.Ls = dLs_.get(); ib.Amat = dAmat_.get(); ib.part = dPart_.get();
+  ib.max_units = units; ib.cta_budget = n_sm_; ib.syrk_cnt = dSyrkCnt_.get();
+  ib.tile_rows = nullptr; ib.filter_rows = dFilterRows_.get() + fi;
+  CKO(cudaMemsetAsync(dImu_.get(), 0, IM_STRIDE * sizeof(double), stream_));
+  launch_info_dense_factor(ua, ib, dM.get(), ld, rows, n, stream_);
   launch_info_dense_apply(ua, ib, n, stream_);
   launches_ += 6;
-  CKO(cudaMemcpyAsync(dx_out, dDx_, D * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-  CKO(cudaMemcpy2DAsync(P_out, D * sizeof(double), dP_, ldp_ * sizeof(double), D * sizeof(double), D,
+  CKO(cudaMemcpyAsync(dx_out, dDx_.get(), D * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+  CKO(cudaMemcpy2DAsync(P_out, D * sizeof(double), dP_.get(), ldp_ * sizeof(double), D * sizeof(double), D,
                         cudaMemcpyDeviceToHost, stream_));
   CKO(cudaStreamSynchronize(stream_));
   return launch_error_count() > 0 ? ORCVIO_ERR_CUDA : ORCVIO_OK;

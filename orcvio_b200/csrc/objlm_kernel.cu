@@ -21,6 +21,7 @@
 #include <vector>
 
 #include "../../include/orcvio_b200.h"
+#include "devmem.h"
 #include "kernels.h"
 #include "lm.h"
 #include "obj_math.cuh"
@@ -295,13 +296,6 @@ __global__ void k_kp_triangulate(const double* __restrict__ frames_wTc, const do
 }
 
 // k_kabsch lives in kabsch_kernel.cu
-struct DevBuf {
-  void* p = nullptr;
-  ~DevBuf() { if (p) cudaFree(p); }
-  bool alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 8) == cudaSuccess; }
-  template <typename T> T* as() { return static_cast<T*>(p); }
-};
-
 bool valid_obs(const double* zs, int K, int f, int k) {
   return std::isfinite(zs[((size_t)f * K + k) * 2]) && std::isfinite(zs[((size_t)f * K + k) * 2 + 1]);
 }
@@ -337,18 +331,18 @@ int object_init(int n_obj, const int* frame_off, const double* frames_wTc, const
   const int n_list = off[n_obj];
   std::vector<double> pts(3 * (size_t)std::max(n_list, 1), 0.0);
   if (n_list > 0) {
-    DevBuf dF, dZ, dOff, dList, dP;
-    if (!dF.alloc(sizeof(double) * 16 * sumT) || !dZ.alloc(sizeof(double) * 2 * K * sumT) ||
-        !dOff.alloc(sizeof(int) * (n_obj + 1)) || !dList.alloc(sizeof(int) * 3 * n_list) || !dP.alloc(sizeof(double) * 3 * n_list))
+    DeviceBuf<double> dF, dZ, dP;
+    DeviceBuf<int> dOff, dList;
+    if (!dF.alloc(16 * (size_t)sumT) || !dZ.alloc(2 * (size_t)K * sumT) || !dOff.alloc(n_obj + 1) ||
+        !dList.alloc(3 * (size_t)n_list) || !dP.alloc(3 * (size_t)n_list))
       return ORCVIO_ERR_CUDA;
-    cudaMemcpy(dF.p, frames_wTc, sizeof(double) * 16 * sumT, cudaMemcpyHostToDevice);
-    cudaMemcpy(dZ.p, zs, sizeof(double) * 2 * K * sumT, cudaMemcpyHostToDevice);
-    cudaMemcpy(dOff.p, frame_off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
-    cudaMemcpy(dList.p, list.data(), sizeof(int) * 3 * n_list, cudaMemcpyHostToDevice);
-    k_kp_triangulate<<<(n_list + 63) / 64, 64>>>(dF.as<double>(), dZ.as<double>(), dOff.as<int>(), dList.as<int>(), n_list, K,
-                                                 dP.as<double>());
+    cudaMemcpy(dF.get(), frames_wTc, sizeof(double) * 16 * sumT, cudaMemcpyHostToDevice);
+    cudaMemcpy(dZ.get(), zs, sizeof(double) * 2 * K * sumT, cudaMemcpyHostToDevice);
+    cudaMemcpy(dOff.get(), frame_off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
+    cudaMemcpy(dList.get(), list.data(), sizeof(int) * 3 * n_list, cudaMemcpyHostToDevice);
+    k_kp_triangulate<<<(n_list + 63) / 64, 64>>>(dF.get(), dZ.get(), dOff.get(), dList.get(), n_list, K, dP.get());
     check_launch("k_kp_triangulate");
-    if (cudaMemcpy(pts.data(), dP.p, sizeof(double) * 3 * n_list, cudaMemcpyDeviceToHost) != cudaSuccess) return ORCVIO_ERR_CUDA;
+    if (cudaMemcpy(pts.data(), dP.get(), sizeof(double) * 3 * n_list, cudaMemcpyDeviceToHost) != cudaSuccess) return ORCVIO_ERR_CUDA;
   }
   if (kp_world)
     for (int o = 0; o < n_obj; ++o) {
@@ -397,22 +391,23 @@ int object_lm(int n_obj, const int* frame_off, const double* frames_wTc, const d
   for (int o = 0; o < n_obj; ++o)
     if (frame_off[o + 1] <= frame_off[o]) return ORCVIO_ERR_ARG;
   const int n = 9 + 3 * K, xdim = 19 + 3 * K, odim = 1 + n + n * n;
-  DevBuf dF, dZ, dB, dOff, dReq, dX, dMean, dShape, dOut;
-  if (!dF.alloc(sizeof(double) * 16 * sumT) || !dZ.alloc(sizeof(double) * 2 * K * sumT) || !dB.alloc(sizeof(double) * 4 * sumT) ||
-      !dOff.alloc(sizeof(int) * (n_obj + 1)) || !dReq.alloc(sizeof(int) * n_obj) || !dX.alloc(sizeof(double) * xdim * n_obj) ||
-      !dMean.alloc(sizeof(double) * 3 * K) || !dShape.alloc(sizeof(double) * 3) || !dOut.alloc(sizeof(double) * odim * n_obj))
+  DeviceBuf<double> dF, dZ, dB, dX, dMean, dShape, dOut;
+  DeviceBuf<int> dOff, dReq;
+  if (!dF.alloc(16 * (size_t)sumT) || !dZ.alloc(2 * (size_t)K * sumT) || !dB.alloc(4 * (size_t)sumT) ||
+      !dOff.alloc(n_obj + 1) || !dReq.alloc(n_obj) || !dX.alloc((size_t)xdim * n_obj) || !dMean.alloc(3 * (size_t)K) ||
+      !dShape.alloc(3) || !dOut.alloc((size_t)odim * n_obj))
     return ORCVIO_ERR_CUDA;
-  cudaMemcpy(dF.p, frames_wTc, sizeof(double) * 16 * sumT, cudaMemcpyHostToDevice);
-  cudaMemcpy(dZ.p, zs, sizeof(double) * 2 * K * sumT, cudaMemcpyHostToDevice);
-  cudaMemcpy(dB.p, zb, sizeof(double) * 4 * sumT, cudaMemcpyHostToDevice);
-  cudaMemcpy(dOff.p, frame_off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
-  cudaMemcpy(dMean.p, kps_mean, sizeof(double) * 3 * K, cudaMemcpyHostToDevice);
-  cudaMemcpy(dShape.p, mean_shape, sizeof(double) * 3, cudaMemcpyHostToDevice);
+  cudaMemcpy(dF.get(), frames_wTc, sizeof(double) * 16 * sumT, cudaMemcpyHostToDevice);
+  cudaMemcpy(dZ.get(), zs, sizeof(double) * 2 * K * sumT, cudaMemcpyHostToDevice);
+  cudaMemcpy(dB.get(), zb, sizeof(double) * 4 * sumT, cudaMemcpyHostToDevice);
+  cudaMemcpy(dOff.get(), frame_off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
+  cudaMemcpy(dMean.get(), kps_mean, sizeof(double) * 3 * K, cudaMemcpyHostToDevice);
+  cudaMemcpy(dShape.get(), mean_shape, sizeof(double) * 3, cudaMemcpyHostToDevice);
   ObjLmArgs a{};
-  a.frames_wTc = dF.as<double>(); a.zs = dZ.as<double>(); a.zb = dB.as<double>(); a.frame_off = dOff.as<int>();
-  a.req_obj = dReq.as<int>(); a.xs = dX.as<double>(); a.kps_mean = dMean.as<double>(); a.mean_shape = dShape.as<double>();
+  a.frames_wTc = dF.get(); a.zs = dZ.get(); a.zb = dB.get(); a.frame_off = dOff.get();
+  a.req_obj = dReq.get(); a.xs = dX.get(); a.kps_mean = dMean.get(); a.mean_shape = dShape.get();
   for (int i = 0; i < 4; ++i) a.w[i] = weights4[i];
-  a.K = K; a.flags = flags; a.out = dOut.as<double>();
+  a.K = K; a.flags = flags; a.out = dOut.get();
 
   // LMObjectState operator+ (always a left retraction) and scaled_norm (a sum of block norms)
   PlusFn plus = [K](const std::vector<double>& x, const double* dx, std::vector<double>& out) {
@@ -462,12 +457,12 @@ int object_lm(int n_obj, const int* frame_off, const double* frames_wTc, const d
       }
     if (req.empty()) break;
     const int nr = (int)req.size();
-    cudaMemcpy(dReq.p, req.data(), sizeof(int) * nr, cudaMemcpyHostToDevice);
-    cudaMemcpy(dX.p, xs.data(), sizeof(double) * xdim * nr, cudaMemcpyHostToDevice);
+    cudaMemcpy(dReq.get(), req.data(), sizeof(int) * nr, cudaMemcpyHostToDevice);
+    cudaMemcpy(dX.get(), xs.data(), sizeof(double) * xdim * nr, cudaMemcpyHostToDevice);
     k_object_lm_eval<<<nr, LM_SLOTS * LM_LANES>>>(a);
     check_launch("k_object_lm_eval");
     out.resize((size_t)odim * nr);
-    if (cudaMemcpy(out.data(), dOut.p, sizeof(double) * odim * nr, cudaMemcpyDeviceToHost) != cudaSuccess) return ORCVIO_ERR_CUDA;
+    if (cudaMemcpy(out.data(), dOut.get(), sizeof(double) * odim * nr, cudaMemcpyDeviceToHost) != cudaSuccess) return ORCVIO_ERR_CUDA;
     for (int i = 0; i < nr; ++i) {
       const double* r = out.data() + (size_t)odim * i;
       solvers[req[i]].feed(r[0], r + 1 + n, r + 1);
@@ -502,29 +497,30 @@ int object_lm_eval(int n_obj, const int* frame_off, const double* frames_wTc, co
   if (K < 1 || K + 4 > LM_SLOTS) return ORCVIO_ERR_ARG;
   const int sumT = frame_off[n_obj];
   const int n = 9 + 3 * K, xdim = 19 + 3 * K, odim = 1 + n + n * n;
-  DevBuf dF, dZ, dB, dOff, dReq, dX, dMean, dShape, dOut;
-  if (!dF.alloc(sizeof(double) * 16 * sumT) || !dZ.alloc(sizeof(double) * 2 * K * sumT) || !dB.alloc(sizeof(double) * 4 * sumT) ||
-      !dOff.alloc(sizeof(int) * (n_obj + 1)) || !dReq.alloc(sizeof(int) * n_obj) || !dX.alloc(sizeof(double) * xdim * n_obj) ||
-      !dMean.alloc(sizeof(double) * 3 * K) || !dShape.alloc(sizeof(double) * 3) || !dOut.alloc(sizeof(double) * odim * n_obj))
+  DeviceBuf<double> dF, dZ, dB, dX, dMean, dShape, dOut;
+  DeviceBuf<int> dOff, dReq;
+  if (!dF.alloc(16 * (size_t)sumT) || !dZ.alloc(2 * (size_t)K * sumT) || !dB.alloc(4 * (size_t)sumT) ||
+      !dOff.alloc(n_obj + 1) || !dReq.alloc(n_obj) || !dX.alloc((size_t)xdim * n_obj) || !dMean.alloc(3 * (size_t)K) ||
+      !dShape.alloc(3) || !dOut.alloc((size_t)odim * n_obj))
     return ORCVIO_ERR_CUDA;
   std::vector<int> req(n_obj);
   for (int o = 0; o < n_obj; ++o) req[o] = o;
-  cudaMemcpy(dF.p, frames_wTc, sizeof(double) * 16 * sumT, cudaMemcpyHostToDevice);
-  cudaMemcpy(dZ.p, zs, sizeof(double) * 2 * K * sumT, cudaMemcpyHostToDevice);
-  cudaMemcpy(dB.p, zb, sizeof(double) * 4 * sumT, cudaMemcpyHostToDevice);
-  cudaMemcpy(dOff.p, frame_off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
-  cudaMemcpy(dMean.p, kps_mean, sizeof(double) * 3 * K, cudaMemcpyHostToDevice);
-  cudaMemcpy(dShape.p, mean_shape, sizeof(double) * 3, cudaMemcpyHostToDevice);
-  cudaMemcpy(dReq.p, req.data(), sizeof(int) * n_obj, cudaMemcpyHostToDevice);
-  cudaMemcpy(dX.p, xs, sizeof(double) * xdim * n_obj, cudaMemcpyHostToDevice);
+  cudaMemcpy(dF.get(), frames_wTc, sizeof(double) * 16 * sumT, cudaMemcpyHostToDevice);
+  cudaMemcpy(dZ.get(), zs, sizeof(double) * 2 * K * sumT, cudaMemcpyHostToDevice);
+  cudaMemcpy(dB.get(), zb, sizeof(double) * 4 * sumT, cudaMemcpyHostToDevice);
+  cudaMemcpy(dOff.get(), frame_off, sizeof(int) * (n_obj + 1), cudaMemcpyHostToDevice);
+  cudaMemcpy(dMean.get(), kps_mean, sizeof(double) * 3 * K, cudaMemcpyHostToDevice);
+  cudaMemcpy(dShape.get(), mean_shape, sizeof(double) * 3, cudaMemcpyHostToDevice);
+  cudaMemcpy(dReq.get(), req.data(), sizeof(int) * n_obj, cudaMemcpyHostToDevice);
+  cudaMemcpy(dX.get(), xs, sizeof(double) * xdim * n_obj, cudaMemcpyHostToDevice);
   ObjLmArgs a{};
-  a.frames_wTc = dF.as<double>(); a.zs = dZ.as<double>(); a.zb = dB.as<double>(); a.frame_off = dOff.as<int>();
-  a.req_obj = dReq.as<int>(); a.xs = dX.as<double>(); a.kps_mean = dMean.as<double>(); a.mean_shape = dShape.as<double>();
+  a.frames_wTc = dF.get(); a.zs = dZ.get(); a.zb = dB.get(); a.frame_off = dOff.get();
+  a.req_obj = dReq.get(); a.xs = dX.get(); a.kps_mean = dMean.get(); a.mean_shape = dShape.get();
   for (int i = 0; i < 4; ++i) a.w[i] = weights4[i];
-  a.K = K; a.flags = flags; a.out = dOut.as<double>();
+  a.K = K; a.flags = flags; a.out = dOut.get();
   k_object_lm_eval<<<n_obj, LM_SLOTS * LM_LANES>>>(a);
   check_launch("k_object_lm_eval");
-  return cudaMemcpy(out, dOut.p, sizeof(double) * odim * n_obj, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
+  return cudaMemcpy(out, dOut.get(), sizeof(double) * odim * n_obj, cudaMemcpyDeviceToHost) == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
 // the two known-answer problems of src/tests/test_levenberg_marquardt.cpp through the same driver (host only)

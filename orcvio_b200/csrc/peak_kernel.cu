@@ -2,6 +2,7 @@
 // dependent-chain-free DFMA throughput and mma.sync m8n8k4 f64 (DMMA) throughput.
 #include <cuda_runtime.h>
 #include "../../include/orcvio_b200.h"
+#include "devmem.h"
 #include "kernels.h"
 #include "chol.cuh"
 
@@ -210,64 +211,58 @@ extern "C" int orcvio_chol_probe(int m, int nx, const double* A, const double* X
   using namespace ob;
   if (m < 1 || m > ORCVIO_LEG + 6 * ORCVIO_MAX_OBS || nx < 0 || m + nx > CHOL_MAXR - 8 ||
       chol_smem_doubles(m, nx) * sizeof(double) > 225 * 1024) return ORCVIO_ERR_ARG;
-  double *dA = nullptr, *dX = nullptr, *dL = nullptr, *dXs = nullptr;
-  long long* dprof = nullptr;
   const size_t nA = (size_t)m * m, nX = (size_t)std::max(nx, 1) * m;
-  if (cudaMalloc(&dA, nA * 8) != cudaSuccess) return ORCVIO_ERR_NO_DEVICE;
-  cudaMalloc(&dX, nX * 8);
-  cudaMalloc(&dL, nA * 8);
-  cudaMalloc(&dXs, nX * 8);
-  cudaMalloc(&dprof, 64 * 8 * sizeof(long long));
-  cudaMemcpy(dA, A, nA * 8, cudaMemcpyHostToDevice);
-  if (nx > 0) cudaMemcpy(dX, X, (size_t)nx * m * 8, cudaMemcpyHostToDevice);
-  cudaMemset(dL, 0, nA * 8);
-  cudaMemset(dprof, 0, 64 * 8 * sizeof(long long));
+  DeviceBuf<double> dA, dX, dL, dXs;
+  DeviceBuf<long long> dprof;
+  if (!dA.alloc(nA)) return ORCVIO_ERR_NO_DEVICE;
+  if (!dX.alloc(nX) || !dL.alloc(nA) || !dXs.alloc(nX) || !dprof.alloc(64 * 8)) return ORCVIO_ERR_CUDA;
+  cudaMemcpy(dA.get(), A, nA * 8, cudaMemcpyHostToDevice);
+  if (nx > 0) cudaMemcpy(dX.get(), X, (size_t)nx * m * 8, cudaMemcpyHostToDevice);
+  cudaMemset(dL.get(), 0, nA * 8);
+  cudaMemset(dprof.get(), 0, 64 * 8 * sizeof(long long));
   const size_t smem = chol_smem_doubles(m, nx) * sizeof(double);
   auto kp = k_chol_probe<true>;
   auto kf = k_chol_probe<false>;
   cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024);
   cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024);
-  kp<<<1, CHOL_THREADS, smem>>>(dA, dX, m, nx, dL, dXs, dprof);
+  kp<<<1, CHOL_THREADS, smem>>>(dA.get(), dX.get(), m, nx, dL.get(), dXs.get(), dprof.get());
   cudaEvent_t e0, e1;
   cudaEventCreate(&e0);
   cudaEventCreate(&e1);
-  kf<<<1, CHOL_THREADS, smem>>>(dA, dX, m, nx, dL, dXs, dprof);
+  kf<<<1, CHOL_THREADS, smem>>>(dA.get(), dX.get(), m, nx, dL.get(), dXs.get(), dprof.get());
   cudaEventRecord(e0);
-  for (int r = 0; r < reps; ++r) kf<<<1, CHOL_THREADS, smem>>>(dA, dX, m, nx, dL, dXs, dprof);
+  for (int r = 0; r < reps; ++r) kf<<<1, CHOL_THREADS, smem>>>(dA.get(), dX.get(), m, nx, dL.get(), dXs.get(), dprof.get());
   cudaEventRecord(e1);
   cudaEventSynchronize(e1);
   float ms = 0;
   cudaEventElapsedTime(&ms, e0, e1);
   if (us) *us = 1e3f * ms / std::max(reps, 1);
-  cudaMemcpy(L, dL, nA * 8, cudaMemcpyDeviceToHost);
-  if (nx > 0) cudaMemcpy(Xs, dXs, (size_t)nx * m * 8, cudaMemcpyDeviceToHost);
-  if (prof) cudaMemcpy(prof, dprof, 64 * 8 * sizeof(long long), cudaMemcpyDeviceToHost);
+  cudaMemcpy(L, dL.get(), nA * 8, cudaMemcpyDeviceToHost);
+  if (nx > 0) cudaMemcpy(Xs, dXs.get(), (size_t)nx * m * 8, cudaMemcpyDeviceToHost);
+  if (prof) cudaMemcpy(prof, dprof.get(), 64 * 8 * sizeof(long long), cudaMemcpyDeviceToHost);
   cudaEventDestroy(e0);
   cudaEventDestroy(e1);
-  cudaFree(dA); cudaFree(dX); cudaFree(dL); cudaFree(dXs); cudaFree(dprof);
   return cudaGetLastError() == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
 extern "C" int orcvio_latency_probe(double* cycles7) {
-  double* out = nullptr;
-  if (cudaMalloc(&out, 8 * sizeof(double)) != cudaSuccess) return ORCVIO_ERR_NO_DEVICE;
-  k_latency<<<1, 512>>>(out, 0.25);
-  k_latency<<<1, 512>>>(out, 0.25);
+  ob::DeviceBuf<double> out;
+  if (!out.alloc(8)) return ORCVIO_ERR_NO_DEVICE;
+  k_latency<<<1, 512>>>(out.get(), 0.25);
+  k_latency<<<1, 512>>>(out.get(), 0.25);
   double h[8];
-  cudaMemcpy(h, out, sizeof(h), cudaMemcpyDeviceToHost);
-  cudaFree(out);
+  cudaMemcpy(h, out.get(), sizeof(h), cudaMemcpyDeviceToHost);
   for (int i = 0; i < 7; ++i) cycles7[i] = h[i];
   return cudaGetLastError() == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
 
 extern "C" int orcvio_latency_probe1(double* cycles10) {
-  double* out = nullptr;
-  if (cudaMalloc(&out, 16 * sizeof(double)) != cudaSuccess) return ORCVIO_ERR_NO_DEVICE;
-  k_latency1<<<1, 64>>>(out, 0.25);
-  k_latency1<<<1, 64>>>(out, 0.25);
+  ob::DeviceBuf<double> out;
+  if (!out.alloc(16)) return ORCVIO_ERR_NO_DEVICE;
+  k_latency1<<<1, 64>>>(out.get(), 0.25);
+  k_latency1<<<1, 64>>>(out.get(), 0.25);
   double h[16];
-  cudaMemcpy(h, out, sizeof(h), cudaMemcpyDeviceToHost);
-  cudaFree(out);
+  cudaMemcpy(h, out.get(), sizeof(h), cudaMemcpyDeviceToHost);
   for (int i = 0; i < 10; ++i) cycles10[i] = h[i];
   return cudaGetLastError() == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
@@ -277,15 +272,15 @@ extern "C" int orcvio_fp64_peak(double* dfma_tflops, double* dmma_tflops) {
   if (cudaGetDevice(&dev) != cudaSuccess) return ORCVIO_ERR_NO_DEVICE;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int blocks = sms * 8, threads = 256, iters = 8192;
-  double* out = nullptr;
-  if (cudaMalloc(&out, (size_t)blocks * threads * sizeof(double)) != cudaSuccess) return ORCVIO_ERR_CUDA;
+  ob::DeviceBuf<double> out;
+  if (!out.alloc((size_t)blocks * threads)) return ORCVIO_ERR_CUDA;
   cudaEvent_t e0, e1;
   cudaEventCreate(&e0);
   cudaEventCreate(&e1);
   float ms = 0;
   for (int rep = 0; rep < 2; ++rep) {
     cudaEventRecord(e0);
-    k_dfma_peak<<<blocks, threads>>>(out, iters, 1.0);
+    k_dfma_peak<<<blocks, threads>>>(out.get(), iters, 1.0);
     cudaEventRecord(e1);
     cudaEventSynchronize(e1);
     cudaEventElapsedTime(&ms, e0, e1);
@@ -293,7 +288,7 @@ extern "C" int orcvio_fp64_peak(double* dfma_tflops, double* dmma_tflops) {
   if (dfma_tflops) *dfma_tflops = 2.0 * 8 * iters * (double)blocks * threads / (ms * 1e-3) / 1e12;
   for (int rep = 0; rep < 2; ++rep) {
     cudaEventRecord(e0);
-    k_dmma_peak<<<blocks, threads>>>(out, iters, 1.0);
+    k_dmma_peak<<<blocks, threads>>>(out.get(), iters, 1.0);
     cudaEventRecord(e1);
     cudaEventSynchronize(e1);
     cudaEventElapsedTime(&ms, e0, e1);
@@ -302,6 +297,5 @@ extern "C" int orcvio_fp64_peak(double* dfma_tflops, double* dmma_tflops) {
   if (dmma_tflops) *dmma_tflops = 512.0 * 4 * iters * (double)blocks * (threads / 32) / (ms * 1e-3) / 1e12;
   cudaEventDestroy(e0);
   cudaEventDestroy(e1);
-  cudaFree(out);
   return cudaGetLastError() == cudaSuccess ? ORCVIO_OK : ORCVIO_ERR_CUDA;
 }
