@@ -90,6 +90,38 @@ struct Batch::PhaseWork {
   }
 };
 
+struct CandBuild {
+  Cand c;
+  long long id;
+  int kind;
+};
+
+// Per-frame state of process_ptrs, handed from one step of processFeatures to the next.
+struct Batch::FrameWork {
+  std::vector<PropSample> samples;               // batchImuProcessing, CSR by samp_off
+  std::vector<int> samp_off, N, E, D;            // clones (-1: not in the frame), feature states, dimension
+  PhaseWork A, B;                                // the updates of removeLostFeatures / pruneImuStateBuffer
+  std::vector<std::vector<CandBuild>> lost;      // per filter: the lost / tracked-long candidates of phase A
+  // hybrid mode (:2283-2323): tracked-long features whose grid cell had room when the walk started.  Whether such a
+  // feature becomes an EKF-SLAM feature depends on the triangulation outcome of the ones before it (cells fill up in
+  // id order), so initializeInvParamPosition runs speculatively for all of them into a scratch table; the host then
+  // replays the reference's sequential decision and commits the ones that took the branch.
+  struct PossRec { Track* tr; int code; int spec; long long spec_gen; };
+  std::vector<std::vector<PossRec>> poss;
+  std::vector<std::map<int, int>> cells;         // per filter: EKF-SLAM features by grid cell
+  std::vector<std::vector<Track*>> news;         // per filter: this frame's new EKF-SLAM features
+  PhaseWork spec;                                // candidates of the speculative triangulation
+  std::vector<CommitRec> commits;
+  bool hyb_ok = true;                            // false: upload arena exhausted or an anchor outside the window
+  std::vector<Track*> gather_tracks;             // tracks behind the last queued host-mirror gather
+  std::vector<int> rm_idx;                       // pruneImuStateBuffer: the 2 removed clones of a filter, -1 = none
+  std::vector<ReanchorRec> reanchor;
+  std::vector<int> reanchor_off;
+  explicit FrameWork(int B)
+      : samp_off(B + 1, 0), N(B, -1), E(B, 0), D(B, 0), lost(B), poss(B), cells(B), news(B), rm_idx(2 * (size_t)B, -1),
+        reanchor_off(B + 1, 0) {}
+};
+
 // Device / pinned buffers of the hybrid MSCKF / EKF-SLAM mode (allocated only when max_features_in_one_grid > 0).
 struct Batch::HybridBufs {
   DeviceBuf<double> dSpecPos;          // scratch position table of the speculative initializeInvParamPosition pass
@@ -372,18 +404,6 @@ void Batch::download_mirrors() {
 // ---------------------------------------------------------------------------------------
 // Build tiles for the candidates [c0, c1) of one filter (already sorted by s_blk).
 static void build_tiles(Batch::PhaseWork& w, int fi, int c0, int c1);
-
-struct CandBuild {
-  Cand c;
-  long long id;
-  int kind;
-};
-
-void Batch::run_phase(PhaseWork& w, int phase) {
-  stage_phase(w);
-  launch_phase(w, true);
-  (void)phase;
-}
 
 // Pack the work lists of one phase into the pinned blob and upload them (one H2D copy).
 // Host half of the staging: carve the pinned blob and copy the work lists into it (no CUDA call as long as the
@@ -721,6 +741,27 @@ static void build_tiles(Batch::PhaseWork& w, int fi, int c0, int c1) {
       if (6 * w.tiles[t].c1_blk >= SY_TILE * J) fw.jrow0[J] = std::min(fw.jrow0[J], w.tiles[t].arow - fw.arow0);
 }
 
+// Append one candidate with the offsets of its rows (none when tri_only); returns its index.
+static int push_candidate(Batch::PhaseWork& w, int fi, const CandBuild& x, std::vector<CandInfo>& info_out,
+                          bool tri_only) {
+  Cand c = x.c;
+  c.filter = fi;
+  const int r = tri_only ? 0 : std::max(2 * c.jac_m - 3, 0);
+  c.row_off = (int)w.rows_total;
+  c.hblk_off = (int)w.hblk_total;
+  w.rows_total += (size_t)r;
+  w.hblk_total += (size_t)r * 6 * (c.e_blk - c.s_blk + 1);
+  const int idx = (int)w.cands.size();
+  if (!tri_only) {
+    w.own_wmax_blk = std::max(w.own_wmax_blk, c.e_blk - c.s_blk + 1);
+    if (c.jac_m <= 8) w.small_list.push_back(idx);
+    else w.large_list.push_back(idx);
+  }
+  w.cands.push_back(c);
+  info_out.push_back(CandInfo{x.id, x.kind});
+  return idx;
+}
+
 // Append one filter's candidates (sorted by first clone, then id) to the phase work list.
 static void append_candidates(Batch::PhaseWork& w, int fi, std::vector<CandBuild>& cb,
                               std::vector<CandInfo>& info_out, bool tri_only = false) {
@@ -729,23 +770,7 @@ static void append_candidates(Batch::PhaseWork& w, int fi, std::vector<CandBuild
     return a.id < b.id;
   });
   const int c0 = (int)w.cands.size();
-  for (auto& x : cb) {
-    Cand c = x.c;
-    c.filter = fi;
-    const int r = tri_only ? 0 : 2 * c.jac_m - 3;
-    c.row_off = (int)w.rows_total;
-    c.hblk_off = (int)w.hblk_total;
-    w.rows_total += (size_t)std::max(r, 0);
-    w.hblk_total += (size_t)std::max(r, 0) * 6 * (c.e_blk - c.s_blk + 1);
-    const int idx = (int)w.cands.size();
-    if (!tri_only) {
-      w.own_wmax_blk = std::max(w.own_wmax_blk, c.e_blk - c.s_blk + 1);
-      if (c.jac_m <= 8) w.small_list.push_back(idx);
-      else w.large_list.push_back(idx);
-    }
-    w.cands.push_back(c);
-    info_out.push_back(CandInfo{x.id, x.kind});
-  }
+  for (const CandBuild& x : cb) push_candidate(w, fi, x, info_out, tri_only);
   if (!tri_only) build_tiles(w, fi, c0, (int)w.cands.size());
 }
 
@@ -942,33 +967,15 @@ int Batch::replay(int n_frames, const double* t_img, const OrcvioFeature* const*
 }
 
 
+// processFeatures :500-661, host side: the reference's steps in its order.
 int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, const int* nfeat,
                         const OrcvioImu* const* imup, const int* nimu_v, int* imu_used, int* published) {
   if (!ok_) return ORCVIO_ERR_CUDA;
   g_sp.start();
   cudaSetDevice(dev_);                // the current device is per host thread (replays run on worker threads)
-  const int L = ORCVIO_LEG;
-  // Capacity is checked before anything is touched: a frame either runs on every filter or leaves all of them as
-  // they were (a failure in the middle of the per-filter loop would leave host bookkeeping and device state apart).
-  if (!p_.prediction_only_flag)
-    for (int fi = 0; fi < B_; ++fi) {
-      const FilterHost& F = f_[fi];
-      const OrcvioFeature* ft = featp[fi];
-      const int nf = nfeat[fi];
-      if ((size_t)nf <= F.free_slots.size()) continue;     // even if every feature is new there is room
-      size_t fresh = 0;
-      for (int k = 0; k < nf; ++k) fresh += F.find_track((long long)ft[k].id) ? 0 : 1;
-      if (fresh > F.free_slots.size()) {
-        std::fprintf(stderr, "[orcvio_b200] feature table full (capacity %d live tracks per filter, filter %d needs %zu more)\n",
-                     Fcap_, fi, fresh - F.free_slots.size());
-        return ORCVIO_ERR_CAPACITY;
-      }
-    }
+  if (!p_.prediction_only_flag && !check_feature_capacity(featp, nfeat)) return ORCVIO_ERR_CAPACITY;
   g_sp.mark(0);
-  // ---------------------------------------------------------------- A: propagation inputs
-  std::vector<PropSample> samples;
-  std::vector<int> samp_off(B_ + 1, 0), Dvec(B_, 0), Nvec(B_, 0), Evec(B_, 0);
-  bool need_imu_upload = false;
+  FrameWork fr(B_);
   for (int fi = 0; fi < B_; ++fi) {
     FilterHost& F = f_[fi];
     F.active = false;
@@ -981,397 +988,353 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     F.log_new_ok.clear(); F.log_ekf_gamma.clear(); F.log_new_gamma.clear(); F.log_reanchor.clear();
     published[fi] = 0;
     imu_used[fi] = 0;
-    samp_off[fi + 1] = (int)samples.size();
-    const OrcvioImu* im = imup[fi];
-    const int nimu = nimu_v[fi];
-    const double ti = t_img[fi];
-    if (!F.first_features) {   // :504-510
-      if (nimu > 0 && (im[0].t - ti - p_.td <= 0.0)) F.first_features = true;
-      else continue;
-    }
-    int prefix = 0;
-    if (!F.gravity_set) {      // :513-563, initial_use_gt branch only
-      if (!F.has_init) continue;
-      int useful = 0;
-      for (int k = 0; k < nimu; ++k) {
-        if (im[k].t > F.init_t) break;
-        ++useful;
-      }
-      if (useful >= nimu) --useful;
-      if (useful < 0) continue;
-      init_filter_device(fi);
-      double* hm = hImu_.get() + (size_t)fi * IM_STRIDE;
-      for (int k = 0; k < 3; ++k) {
-        hm[IM_GOLD + k] = im[useful].gyro[k];
-        hm[IM_AOLD + k] = im[useful].acc[k];
-      }
-      CK(cudaMemcpyAsync(dImu_.get() + (size_t)fi * IM_STRIDE, hm, IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
-      need_imu_upload = true;
-      prefix = useful;
-      F.gravity_set = true;
-      F.imu_time = F.init_t;
-      F.take_off_stamp = F.init_t;
-      F.last_zupt_time = F.init_t;       // :556
-    }
-    // batchImuProcessing :664-724
-    const double bound = ti + p_.td;
-    int used = 0;
-    double dt = 0.0;
-    for (int k = prefix; k < nimu; ++k) {
-      const double t = im[k].t;
-      if (t <= F.imu_time) { ++used; continue; }
-      if (t - bound > p_.imu_img_timeTh) break;
-      PropSample s;
-      s.t = t;
-      for (int q = 0; q < 3; ++q) { s.w[q] = im[k].gyro[q]; s.a[q] = im[k].acc[q]; }
-      samples.push_back(s);
-      dt = t - bound;
-      F.imu_time = t;
-      ++used;
-    }
-    samp_off[fi + 1] = (int)samples.size();
-    F.state_id = F.next_state_id++;
-    F.dt = dt;
-    imu_used[fi] = prefix + used;
-    Nvec[fi] = (int)F.clones.size();
-    Evec[fi] = (int)F.feature_states.size();
-    Dvec[fi] = L + 6 * Nvec[fi] + Evec[fi];
-    F.active = true;
+    const bool in_frame = batch_imu_processing(fr, fi, imup[fi], nimu_v[fi], t_img[fi], &imu_used[fi]);
+    fr.samp_off[fi + 1] = (int)fr.samples.size();
+    if (!in_frame) continue;
     published[fi] = 1;
-
-    // addFeatureObservations :1016-1068
-    if (!p_.prediction_only_flag) {
-      const OrcvioFeature* ft = featp[fi];
-      const int nf = nfeat[fi];
-      const long long sid = F.state_id;
-      const int curr_feature_num = (int)F.map_server.size();
-      int tracked = 0;
-      for (int k = 0; k < nf; ++k) {
-        const OrcvioFeature& m = ft[k];
-        const long long id = (long long)m.id;
-        Track* found = F.find_track(id);
-        if (!found) {
-          if (F.free_slots.empty()) {      // (cannot happen after the pre-pass; if it does the batch is unusable)
-            std::fprintf(stderr, "[orcvio_b200] feature table full (capacity %d)\n", Fcap_);
-            ok_ = false;
-            err_ = "feature table overflow in the middle of a frame";
-            return ORCVIO_ERR_CAPACITY;
-          }
-          Track tr;
-          tr.id = id;
-          tr.slot = F.free_slots.back();
-          F.free_slots.pop_back();
-          tr.gen = F.next_gen++;
-          bool have_prev = false;
-          double dt_prev = 0.0;
-          if (!(m.u_init == -1 && m.v_init == -1)) {
-            for (const auto& c : F.clones)
-              if (c.id == sid - 1) { have_prev = true; dt_prev = c.dt; }
-          }
-          if (have_prev) {
-            Obs o{};
-            o.sid = sid - 1;
-            o.z[0] = m.u_init + m.u_init_vel * dt_prev;
-            o.z[1] = m.v_init + m.v_init_vel * dt_prev;
-            o.vel[0] = m.u_init_vel; o.vel[1] = m.v_init_vel;
-            tr.obs.push_back(o);
-          }
-          Obs o{};
-          o.sid = sid;
-          o.z[0] = m.u + m.u_vel * dt;
-          o.z[1] = m.v + m.v_vel * dt;
-          o.vel[0] = m.u_vel; o.vel[1] = m.v_vel;
-          tr.obs.push_back(o);
-          tr.touch();
-          F.add_track(std::move(tr));
-        } else {
-          Obs o{};
-          o.sid = sid;
-          o.z[0] = m.u + m.u_vel * dt;
-          o.z[1] = m.v + m.v_vel * dt;
-          o.vel[0] = m.u_vel; o.vel[1] = m.v_vel;
-          Track& tr = *found;
-          if (!tr.obs.empty() && tr.obs.back().sid == sid) tr.obs.back() = o;
-          else tr.obs.push_back(o);
-          tr.touch();
-          ++tracked;
-          if (p_.if_ZUPT_valid && p_.if_use_feature_zupt_flag) {     // :1052-1058
-            // (the observations are in ascending state-id order and end with this frame's: the previous frame's, if
-            // there is one, is the one before it)
-            if (tr.obs.size() >= 2 && tr.obs[tr.obs.size() - 2].sid == sid - 1) {
-              const Obs& po = tr.obs[tr.obs.size() - 2];
-              const double du = m.u - po.z[0], dv = m.v - po.z[1];
-              F.coarse_feature_dis.push_back(std::sqrt(du * du + dv * dv));
-            }
-          }
-        }
-      }
-      F.tracking_rate = (double)tracked / (double)curr_feature_num;   // 0/0 -> NaN like the reference
-    }
+    if (!p_.prediction_only_flag && !add_feature_observations(fi, featp[fi], nfeat[fi])) return ORCVIO_ERR_CAPACITY;
     // stateAugmentation bookkeeping :937-961
     F.cur_window_timestamps.push_back(F.imu_time);
     F.clones.push_back(CloneMeta{F.state_id, F.imu_time, F.dt});
   }
-  (void)need_imu_upload;
   g_sp.mark(1);
+  propagate_and_augment(fr);
+  if (!remove_lost_features(fr)) return ORCVIO_ERR_CUDA;
+  apply_lost_results(fr);
+  if (!prune_imu_state_buffer(fr)) return ORCVIO_ERR_CUDA;
+  g_sp.done(B_);
+  return ok_ ? ORCVIO_OK : ORCVIO_ERR_CUDA;
+}
 
-  // ---------------------------------------------------------------- B: propagate + augment
-  {
-    blob_.reset();
-    const size_t o_s = blob_.reserve(sizeof(PropSample) * std::max<size_t>(samples.size(), 1));
-    const size_t o_o = blob_.reserve(sizeof(int) * (B_ + 1));
-    const size_t o_d = blob_.reserve(sizeof(int) * B_);
-    const size_t o_n = blob_.reserve(sizeof(int) * B_);
-    const size_t o_e = blob_.reserve(sizeof(int) * B_);
-    char* h = blob_.pinned.get();
-    std::memcpy(h + o_e, Evec.data(), sizeof(int) * B_);
-    if (!samples.empty()) std::memcpy(h + o_s, samples.data(), sizeof(PropSample) * samples.size());
-    std::memcpy(h + o_o, samp_off.data(), sizeof(int) * (B_ + 1));
-    std::memcpy(h + o_d, Dvec.data(), sizeof(int) * B_);
-    // augmentation only for active filters: N = -1 disables
-    std::vector<int> Naug(B_);
-    for (int fi = 0; fi < B_; ++fi) Naug[fi] = f_[fi].active ? Nvec[fi] : -1;
-    std::memcpy(h + o_n, Naug.data(), sizeof(int) * B_);
-    // ZUPT (:583-592): the feature test (checkZUPTFeat :3081-3125) is a host decision on the sorted
-    // track displacements; the IMU test (checkZUPTIMU) needs P and runs inside k_zupt.
-    size_t o_zm = 0, o_zn = 0, o_zc = 0;
-    bool any_zupt = false;
-    if (p_.if_ZUPT_valid) {
-      std::vector<int> zmode(B_, 0), zN(B_, -1);
-      std::vector<double> zchk(B_, 0.0);
-      for (int fi = 0; fi < B_; ++fi) {
-        FilterHost& F = f_[fi];
-        F.if_zupt = false;
-        if (!F.active) continue;
-        zN[fi] = Nvec[fi] + 1;
-        if (p_.if_use_feature_zupt_flag) {
-          std::vector<double>& d = F.coarse_feature_dis;
-          if (d.size() >= 20) {
-            // (the reference sorts and reads element size - 9: the same order statistic without the full sort)
-            std::nth_element(d.begin(), d.end() - 9, d.end());
-            if (d[d.size() - 9] < p_.zupt_max_feature_dis) zmode[fi] = 1;
-          }
-          d.clear();
-        } else {
-          const int cnt = samp_off[fi + 1] - samp_off[fi];
-          if (cnt >= 2) {
-            zmode[fi] = 2;
-            const int dof = 6 * (cnt - 1);
-            zchk[fi] = dof < 500 ? chi2_zupt_host_[dof] : chi2_quantile(0.95, dof);
-          }
-        }
-        any_zupt |= zmode[fi] != 0;
-      }
-      o_zm = blob_.reserve(sizeof(int) * B_);
-      o_zn = blob_.reserve(sizeof(int) * B_);
-      o_zc = blob_.reserve(sizeof(double) * B_);
-      h = blob_.pinned.get();
-      std::memcpy(h + o_zm, zmode.data(), sizeof(int) * B_);
-      std::memcpy(h + o_zn, zN.data(), sizeof(int) * B_);
-      std::memcpy(h + o_zc, zchk.data(), sizeof(double) * B_);
-    }
-    upload_blob();
-    if (profiling_) CK(cudaEventRecord(ev_[6], stream_));
-    PropArgs pa{};
-    pa.P = dP_.get(); pa.p_stride = (size_t)ldp_ * ldp_; pa.ldp = ldp_;
-    pa.imu = dImu_.get();
-    pa.samples = (const PropSample*)(blob_.dev.get() + o_s);
-    pa.samp_off = (const int*)(blob_.dev.get() + o_o);
-    pa.D = (const int*)(blob_.dev.get() + o_d);
-    pa.n_filters = B_; pa.flags = flags_;
-    pa.qc[0] = p_.imu_gyro_noise; pa.qc[1] = p_.imu_acc_noise;
-    pa.qc[2] = p_.imu_gyro_bias_noise; pa.qc[3] = p_.imu_acc_bias_noise;
-    launch_propagate(pa, stream_);
-    AugArgs aa{};
-    aa.P = dP_.get(); aa.p_stride = pa.p_stride; aa.ldp = ldp_;
-    aa.imu = dImu_.get(); aa.clones = dClones_.get(); aa.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    aa.N = (const int*)(blob_.dev.get() + o_n); aa.n_filters = B_;
-    aa.E = hybrid_ ? (const int*)(blob_.dev.get() + o_e) : nullptr;
-    launch_augment(aa, stream_);
-    launches_ += 2;
-    if (any_zupt) {
-      ZuptArgs za{};
-      za.P = dP_.get(); za.p_stride = pa.p_stride; za.ldp = ldp_;
-      za.imu = dImu_.get(); za.clones = dClones_.get(); za.clone_stride = aa.clone_stride;
-      za.samples = pa.samples; za.samp_off = pa.samp_off;
-      za.N = (const int*)(blob_.dev.get() + o_zn);
-      za.mode = (const int*)(blob_.dev.get() + o_zm);
-      za.chi2_check = (const double*)(blob_.dev.get() + o_zc);
-      za.decision = dZuptDec_.get(); za.info = dZuptInfo_.get();
-      za.dx = dDx_.get(); za.lddx = ldp_;
-      za.n_filters = B_; za.flags = flags_;
-      za.noise_v = p_.zupt_noise_v; za.noise_p = p_.zupt_noise_p; za.noise_q = p_.zupt_noise_q;
-      launch_zupt(za, stream_);
-      ++launches_;
-      CK(cudaMemcpyAsync(hZuptDec_.get(), dZuptDec_.get(), sizeof(int) * B_, cudaMemcpyDeviceToHost, stream_));
-      CK(cudaMemcpyAsync(hZuptInfo_.get(), dZuptInfo_.get(), sizeof(double) * 2 * B_, cudaMemcpyDeviceToHost, stream_));
-    }
-    if (profiling_) {
-      CK(cudaEventRecord(ev_[7], stream_));
-    }
-    // the blob is reused by the next phase: wait for the upload + kernels reading it
-    g_sp.mark(2);
-    CK(cudaStreamSynchronize(stream_));
-    g_sp.mark(3);
-    if (profiling_) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, ev_[6], ev_[7]);
-      pt_.prop += ms; pt_.n_prop++;
-    }
-    if (any_zupt) {
-      for (int fi = 0; fi < B_; ++fi) {
-        FilterHost& F = f_[fi];
-        if (!F.active) continue;
-        F.if_zupt = hZuptDec_.get()[fi] != 0;
-        F.zupt_chi2 = hZuptInfo_.get()[2 * fi];
-        F.zupt_vnorm = hZuptInfo_.get()[2 * fi + 1];
-        F.stats.zupt = F.if_zupt ? 1 : 0;
-        F.stats.zupt_chi2 = F.zupt_chi2;
-        F.stats.zupt_vnorm = F.zupt_vnorm;
-        if (F.if_zupt) {
-          F.last_zupt_time = F.imu_time;                 // :3451
-          // checkZUPTFeat :3104-3115 / checkZUPTIMU :3304-3315: a stationary frame drops every EKF-SLAM feature; the
-          // update itself only touched the leading 22 + 6N block, the feature rows / columns are simply abandoned
-          for (long long id : F.feature_states) {
-            Track& tr = *F.find_track(id);
-            tr.in_state = tr.ekf_feature = tr.initialized = false;
-            tr.gen = F.next_gen++;                       // the device slot no longer counts as initialised
-          }
-          F.feature_states.clear();
-        }
-      }
-    }
-  }
-
-  // ---------------------------------------------------------------- C: removeLostFeatures
-  PhaseWork wA;
-  wA.fw.assign(B_, FilterWork{});
-  wA.cand_begin.assign(B_ + 1, 0);
-  if (hybrid_) { wA.hyb_phase = 0; wA.hw.assign(B_, HybWork{}); }
-  // state id -> index in the window.  The window does not change between augmentation (above) and the end of the frame,
-  // and its ids span a few dozen consecutive values: one small table per filter instead of a search per observation.
-  std::vector<std::vector<short>> clone_lut(B_);
+// Capacity is checked before anything is touched: a frame either runs on every filter or leaves all of them as they
+// were (a failure in the middle of the per-filter loop would leave host bookkeeping and device state apart).
+bool Batch::check_feature_capacity(const OrcvioFeature* const* featp, const int* nfeat) const {
   for (int fi = 0; fi < B_; ++fi) {
     const FilterHost& F = f_[fi];
-    if (!F.active || F.clones.empty()) continue;
-    const long long base = F.clones.front().id, span = F.clones.back().id - base + 1;
-    if (span > 4096) continue;                             // (never seen: falls back to the search)
-    clone_lut[fi].assign((size_t)span, (short)-1);
-    for (int k = 0; k < (int)F.clones.size(); ++k) clone_lut[fi][(size_t)(F.clones[k].id - base)] = (short)k;
+    const OrcvioFeature* ft = featp[fi];
+    const int nf = nfeat[fi];
+    if ((size_t)nf <= F.free_slots.size()) continue;     // even if every feature is new there is room
+    size_t fresh = 0;
+    for (int k = 0; k < nf; ++k) fresh += F.find_track((long long)ft[k].id) ? 0 : 1;
+    if (fresh > F.free_slots.size()) {
+      std::fprintf(stderr, "[orcvio_b200] feature table full (capacity %d live tracks per filter, filter %d needs %zu more)\n",
+                   Fcap_, fi, fresh - F.free_slots.size());
+      return false;
+    }
   }
-  const FilterHost* f_base = f_.data();
-  auto clone_index_of = [&clone_lut, f_base](const FilterHost& F, long long sid) {
-    const std::vector<short>& lut = clone_lut[&F - f_base];
-    if (!lut.empty()) {
-      const long long off = sid - F.clones.front().id;
-      return (off >= 0 && off < (long long)lut.size()) ? (int)lut[(size_t)off] : -1;
+  return true;
+}
+
+// batchImuProcessing :664-724 behind the first-frame checks :504-563.  False: filter fi sits this frame out.
+bool Batch::batch_imu_processing(FrameWork& fr, int fi, const OrcvioImu* im, int nimu, double ti, int* imu_used) {
+  FilterHost& F = f_[fi];
+  if (!F.first_features) {   // :504-510
+    if (nimu > 0 && (im[0].t - ti - p_.td <= 0.0)) F.first_features = true;
+    else return false;
+  }
+  int prefix = 0;
+  if (!F.gravity_set) {      // :513-563, initial_use_gt branch only
+    if (!F.has_init) return false;
+    int useful = 0;
+    for (int k = 0; k < nimu; ++k) {
+      if (im[k].t > F.init_t) break;
+      ++useful;
     }
-    for (int k = (int)F.clones.size() - 1; k >= 0; --k)
-      if (F.clones[k].id == sid) return k;
-    return -1;
-  };
-  // one candidate record + its observations in the pools of w (lost / tracked-long feature of removeLostFeatures)
-  auto make_cand = [&](PhaseWork& w, const FilterHost& F, const Track& tr, bool tracked_now, int kind, int flags) {
-    CandBuild x{};
-    x.id = tr.id;
-    x.kind = kind;
-    Cand& c = x.c;
-    c.slot = tr.slot;
-    c.gen = tr.gen;
-    c.flags = flags;
-    c.jac_off = c.tri_off = (int)w.obs_clone.size();
-    int s_blk = 1 << 30, e_blk = -1, cnt = 0;
-    for (const Obs& o : tr.obs) {
-      const int ci = clone_index_of(F, o.sid);
-      if (ci < 0) continue;
-      w.obs_clone.push_back(ci);
-      w.obs_z.push_back(o.z[0]);
-      w.obs_z.push_back(o.z[1]);
-      s_blk = std::min(s_blk, ci);
-      e_blk = std::max(e_blk, ci);
-      ++cnt;
+    if (useful >= nimu) --useful;
+    if (useful < 0) return false;
+    init_filter_device(fi);
+    double* hm = hImu_.get() + (size_t)fi * IM_STRIDE;
+    for (int k = 0; k < 3; ++k) {
+      hm[IM_GOLD + k] = im[useful].gyro[k];
+      hm[IM_AOLD + k] = im[useful].acc[k];
     }
-    c.jac_m = cnt;
-    c.tri_m = tracked_now ? cnt - 1 : cnt;   // initializePosition skips the current frame (:414)
-    c.s_blk = s_blk;
-    c.e_blk = e_blk;
-    c.cm_first_clone = w.obs_clone[c.jac_off];
-    c.cm_last_clone = w.obs_clone[c.jac_off + (tracked_now ? cnt - 2 : cnt - 1)];
-    c.cm_zu = w.obs_z[2 * (size_t)c.jac_off];
-    c.cm_zv = w.obs_z[2 * (size_t)c.jac_off + 1];
-    return x;
-  };
-  std::vector<std::vector<CandBuild>> cbs(B_);
-  // hybrid mode (:2283-2323): tracked-long features whose grid cell had room when the walk started.  Whether such a
-  // feature becomes an EKF-SLAM feature depends on the triangulation outcome of the ones before it (cells fill up in
-  // id order), so initializeInvParamPosition runs speculatively for all of them into a scratch table; the host then
-  // replays the reference's sequential decision and commits the ones that took the branch.
-  struct PossRec { Track* tr; int code; int spec; long long spec_gen; };
-  std::vector<std::vector<PossRec>> poss(B_);
-  std::vector<std::map<int, int>> cells(B_);
-  std::vector<std::vector<Track*>> news(B_);
-  PhaseWork wS;
-  HybridBufs* hb = hyb_.get();
-  bool hyb_ok = true;
-  if (hybrid_) {
-    hb->used = 0;                          // the stream is idle (synchronised at the end of section B)
-    std::vector<int> newidx, Dold(B_, 0);
-    bool any_compact = false;
-    for (int fi = 0; fi < B_; ++fi) {
-      FilterHost& F = f_[fi];
-      if (!F.active || F.feature_states.empty()) continue;
-      // features of the state: tracked now -> a 2-row update; lost -> dropped (:2210-2232, rmLostFeaturesCov :3776-3828)
-      const int base = L + 6 * (int)F.clones.size(), E0 = (int)F.feature_states.size();
-      std::vector<long long> kept;
-      std::vector<int> map_e(E0, -1);
-      for (int i = 0; i < E0; ++i) {
-        Track& tr = *F.find_track(F.feature_states[i]);
-        if (!tr.obs.empty() && tr.obs.back().sid == F.state_id) {
-          map_e[i] = (int)kept.size();
-          kept.push_back(tr.id);
-        } else {
-          const long long lost_id = tr.id;
-          F.log_ekf_lost.push_back(lost_id);
-          F.free_slots.push_back(tr.slot);
-          F.erase_track(lost_id);
+    CK(cudaMemcpyAsync(dImu_.get() + (size_t)fi * IM_STRIDE, hm, IM_STRIDE * sizeof(double), cudaMemcpyHostToDevice, stream_));
+    prefix = useful;
+    F.gravity_set = true;
+    F.imu_time = F.init_t;
+    F.take_off_stamp = F.init_t;
+    F.last_zupt_time = F.init_t;       // :556
+  }
+  const double bound = ti + p_.td;
+  int used = 0;
+  double dt = 0.0;
+  for (int k = prefix; k < nimu; ++k) {
+    const double t = im[k].t;
+    if (t <= F.imu_time) { ++used; continue; }
+    if (t - bound > p_.imu_img_timeTh) break;
+    PropSample s;
+    s.t = t;
+    for (int q = 0; q < 3; ++q) { s.w[q] = im[k].gyro[q]; s.a[q] = im[k].acc[q]; }
+    fr.samples.push_back(s);
+    dt = t - bound;
+    F.imu_time = t;
+    ++used;
+  }
+  F.state_id = F.next_state_id++;
+  F.dt = dt;
+  *imu_used = prefix + used;
+  fr.N[fi] = (int)F.clones.size();
+  fr.E[fi] = (int)F.feature_states.size();
+  fr.D[fi] = ORCVIO_LEG + 6 * fr.N[fi] + fr.E[fi];
+  F.active = true;
+  return true;
+}
+
+static Obs make_obs(long long sid, double u, double v, double u_vel, double v_vel, double dt) {
+  Obs o{};
+  o.sid = sid;
+  o.z[0] = u + u_vel * dt;
+  o.z[1] = v + v_vel * dt;
+  o.vel[0] = u_vel; o.vel[1] = v_vel;
+  return o;
+}
+
+// addFeatureObservations :1016-1068 of filter fi.  False: the feature table overflowed (the batch is unusable).
+bool Batch::add_feature_observations(int fi, const OrcvioFeature* ft, int nf) {
+  FilterHost& F = f_[fi];
+  const long long sid = F.state_id;
+  const double dt = F.dt;
+  const int curr_feature_num = (int)F.map_server.size();
+  int tracked = 0;
+  for (int k = 0; k < nf; ++k) {
+    const OrcvioFeature& m = ft[k];
+    const long long id = (long long)m.id;
+    Track* found = F.find_track(id);
+    if (!found) {
+      if (F.free_slots.empty()) {      // (cannot happen after the pre-pass; if it does the batch is unusable)
+        std::fprintf(stderr, "[orcvio_b200] feature table full (capacity %d)\n", Fcap_);
+        ok_ = false;
+        err_ = "feature table overflow in the middle of a frame";
+        return false;
+      }
+      Track tr;
+      tr.id = id;
+      tr.slot = F.free_slots.back();
+      F.free_slots.pop_back();
+      tr.gen = F.next_gen++;
+      bool have_prev = false;
+      double dt_prev = 0.0;
+      if (!(m.u_init == -1 && m.v_init == -1)) {
+        for (const auto& c : F.clones)
+          if (c.id == sid - 1) { have_prev = true; dt_prev = c.dt; }
+      }
+      if (have_prev) tr.obs.push_back(make_obs(sid - 1, m.u_init, m.v_init, m.u_init_vel, m.v_init_vel, dt_prev));
+      tr.obs.push_back(make_obs(sid, m.u, m.v, m.u_vel, m.v_vel, dt));
+      tr.touch();
+      F.add_track(std::move(tr));
+    } else {
+      const Obs o = make_obs(sid, m.u, m.v, m.u_vel, m.v_vel, dt);
+      Track& tr = *found;
+      if (!tr.obs.empty() && tr.obs.back().sid == sid) tr.obs.back() = o;
+      else tr.obs.push_back(o);
+      tr.touch();
+      ++tracked;
+      if (p_.if_ZUPT_valid && p_.if_use_feature_zupt_flag) {     // :1052-1058
+        // (the observations are in ascending state-id order and end with this frame's: the previous frame's, if
+        // there is one, is the one before it)
+        if (tr.obs.size() >= 2 && tr.obs[tr.obs.size() - 2].sid == sid - 1) {
+          const Obs& po = tr.obs[tr.obs.size() - 2];
+          const double du = m.u - po.z[0], dv = m.v - po.z[1];
+          F.coarse_feature_dis.push_back(std::sqrt(du * du + dv * dv));
         }
       }
-      if ((int)kept.size() != E0) {
-        if (newidx.empty()) newidx.assign((size_t)B_ * ldp_, -1);
-        int* ni = newidx.data() + (size_t)fi * ldp_;
-        for (int j = 0; j < base; ++j) ni[j] = j;
-        for (int i = 0; i < E0; ++i) ni[base + i] = map_e[i] < 0 ? -1 : base + map_e[i];
-        Dold[fi] = base + E0;
-        any_compact = true;
-        F.feature_states = kept;
-      }
-    }
-    if (any_compact) {
-      const int* d_ni = hb->put(newidx.data(), newidx.size(), stream_, &hyb_ok);
-      const int* d_do = hb->put(Dold.data(), Dold.size(), stream_, &hyb_ok);
-      if (hyb_ok) { launch_compact_cov(dP_.get(), (size_t)ldp_ * ldp_, ldp_, d_ni, d_do, B_, stream_); ++launches_; }
     }
   }
-  auto grid_code = [&](const Track& tr) {   // :2286-2289 / :3841-3845 (the casts truncate toward zero)
-    const double* z = tr.obs.back().z;
-    const int row = (int)((z[1] - p_.y_min) / p_.grid_height);
-    const int col = (int)((z[0] - p_.x_min) / p_.grid_width);
-    return row * p_.grid_cols + col;
-  };
+  F.tracking_rate = (double)tracked / (double)curr_feature_num;   // 0/0 -> NaN like the reference
+  return true;
+}
+
+// k_propagate, k_augment and the ZUPT of :583-592 (k_zupt) for every active filter, then the ZUPT decisions.
+void Batch::propagate_and_augment(FrameWork& fr) {
+  blob_.reset();
+  const size_t o_s = blob_.reserve(sizeof(PropSample) * std::max<size_t>(fr.samples.size(), 1));
+  const size_t o_o = blob_.reserve(sizeof(int) * (B_ + 1));
+  const size_t o_d = blob_.reserve(sizeof(int) * B_);
+  const size_t o_n = blob_.reserve(sizeof(int) * B_);
+  const size_t o_e = blob_.reserve(sizeof(int) * B_);
+  char* h = blob_.pinned.get();
+  std::memcpy(h + o_e, fr.E.data(), sizeof(int) * B_);
+  if (!fr.samples.empty()) std::memcpy(h + o_s, fr.samples.data(), sizeof(PropSample) * fr.samples.size());
+  std::memcpy(h + o_o, fr.samp_off.data(), sizeof(int) * (B_ + 1));
+  std::memcpy(h + o_d, fr.D.data(), sizeof(int) * B_);
+  std::memcpy(h + o_n, fr.N.data(), sizeof(int) * B_);     // augmentation only for active filters: N = -1 disables
+  // ZUPT (:583-592): the feature test (checkZUPTFeat :3081-3125) is a host decision on the sorted
+  // track displacements; the IMU test (checkZUPTIMU) needs P and runs inside k_zupt.
+  size_t o_zm = 0, o_zn = 0, o_zc = 0;
+  bool any_zupt = false;
+  if (p_.if_ZUPT_valid) {
+    std::vector<int> zmode(B_, 0), zN(B_, -1);
+    std::vector<double> zchk(B_, 0.0);
+    for (int fi = 0; fi < B_; ++fi) {
+      FilterHost& F = f_[fi];
+      F.if_zupt = false;
+      if (!F.active) continue;
+      zN[fi] = fr.N[fi] + 1;
+      if (p_.if_use_feature_zupt_flag) {
+        std::vector<double>& d = F.coarse_feature_dis;
+        if (d.size() >= 20) {
+          // (the reference sorts and reads element size - 9: the same order statistic without the full sort)
+          std::nth_element(d.begin(), d.end() - 9, d.end());
+          if (d[d.size() - 9] < p_.zupt_max_feature_dis) zmode[fi] = 1;
+        }
+        d.clear();
+      } else {
+        const int cnt = fr.samp_off[fi + 1] - fr.samp_off[fi];
+        if (cnt >= 2) {
+          zmode[fi] = 2;
+          const int dof = 6 * (cnt - 1);
+          zchk[fi] = dof < 500 ? chi2_zupt_host_[dof] : chi2_quantile(0.95, dof);
+        }
+      }
+      any_zupt |= zmode[fi] != 0;
+    }
+    o_zm = blob_.reserve(sizeof(int) * B_);
+    o_zn = blob_.reserve(sizeof(int) * B_);
+    o_zc = blob_.reserve(sizeof(double) * B_);
+    h = blob_.pinned.get();
+    std::memcpy(h + o_zm, zmode.data(), sizeof(int) * B_);
+    std::memcpy(h + o_zn, zN.data(), sizeof(int) * B_);
+    std::memcpy(h + o_zc, zchk.data(), sizeof(double) * B_);
+  }
+  upload_blob();
+  if (profiling_) CK(cudaEventRecord(ev_[6], stream_));
+  PropArgs pa{};
+  pa.P = dP_.get(); pa.p_stride = (size_t)ldp_ * ldp_; pa.ldp = ldp_;
+  pa.imu = dImu_.get();
+  pa.samples = (const PropSample*)(blob_.dev.get() + o_s);
+  pa.samp_off = (const int*)(blob_.dev.get() + o_o);
+  pa.D = (const int*)(blob_.dev.get() + o_d);
+  pa.n_filters = B_; pa.flags = flags_;
+  pa.qc[0] = p_.imu_gyro_noise; pa.qc[1] = p_.imu_acc_noise;
+  pa.qc[2] = p_.imu_gyro_bias_noise; pa.qc[3] = p_.imu_acc_bias_noise;
+  launch_propagate(pa, stream_);
+  AugArgs aa{};
+  aa.P = dP_.get(); aa.p_stride = pa.p_stride; aa.ldp = ldp_;
+  aa.imu = dImu_.get(); aa.clones = dClones_.get(); aa.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+  aa.N = (const int*)(blob_.dev.get() + o_n); aa.n_filters = B_;
+  aa.E = hybrid_ ? (const int*)(blob_.dev.get() + o_e) : nullptr;
+  launch_augment(aa, stream_);
+  launches_ += 2;
+  if (any_zupt) {
+    ZuptArgs za{};
+    za.P = dP_.get(); za.p_stride = pa.p_stride; za.ldp = ldp_;
+    za.imu = dImu_.get(); za.clones = dClones_.get(); za.clone_stride = aa.clone_stride;
+    za.samples = pa.samples; za.samp_off = pa.samp_off;
+    za.N = (const int*)(blob_.dev.get() + o_zn);
+    za.mode = (const int*)(blob_.dev.get() + o_zm);
+    za.chi2_check = (const double*)(blob_.dev.get() + o_zc);
+    za.decision = dZuptDec_.get(); za.info = dZuptInfo_.get();
+    za.dx = dDx_.get(); za.lddx = ldp_;
+    za.n_filters = B_; za.flags = flags_;
+    za.noise_v = p_.zupt_noise_v; za.noise_p = p_.zupt_noise_p; za.noise_q = p_.zupt_noise_q;
+    launch_zupt(za, stream_);
+    ++launches_;
+    CK(cudaMemcpyAsync(hZuptDec_.get(), dZuptDec_.get(), sizeof(int) * B_, cudaMemcpyDeviceToHost, stream_));
+    CK(cudaMemcpyAsync(hZuptInfo_.get(), dZuptInfo_.get(), sizeof(double) * 2 * B_, cudaMemcpyDeviceToHost, stream_));
+  }
+  if (profiling_) {
+    CK(cudaEventRecord(ev_[7], stream_));
+  }
+  // the blob is reused by the next phase: wait for the upload + kernels reading it
+  g_sp.mark(2);
+  CK(cudaStreamSynchronize(stream_));
+  g_sp.mark(3);
+  if (profiling_) {
+    float ms = 0;
+    cudaEventElapsedTime(&ms, ev_[6], ev_[7]);
+    pt_.prop += ms; pt_.n_prop++;
+  }
+  if (!any_zupt) return;
   for (int fi = 0; fi < B_; ++fi) {
     FilterHost& F = f_[fi];
-    FilterWork& fw = wA.fw[fi];
-    fw.N = (int)F.clones.size();
-    fw.D = L + 6 * fw.N + (int)F.feature_states.size();
-    fw.active = 0;
     if (!F.active) continue;
-    wA.maxN = std::max(wA.maxN, fw.N);
+    F.if_zupt = hZuptDec_.get()[fi] != 0;
+    F.stats.zupt = F.if_zupt ? 1 : 0;
+    F.stats.zupt_chi2 = hZuptInfo_.get()[2 * fi];
+    F.stats.zupt_vnorm = hZuptInfo_.get()[2 * fi + 1];
+    if (F.if_zupt) {
+      F.last_zupt_time = F.imu_time;                 // :3451
+      // checkZUPTFeat :3104-3115 / checkZUPTIMU :3304-3315: a stationary frame drops every EKF-SLAM feature; the
+      // update itself only touched the leading 22 + 6N block, the feature rows / columns are simply abandoned
+      for (long long id : F.feature_states) {
+        Track& tr = *F.find_track(id);
+        tr.in_state = tr.ekf_feature = tr.initialized = false;
+        tr.gen = F.next_gen++;                       // the device slot no longer counts as initialised
+      }
+      F.feature_states.clear();
+    }
+  }
+}
+
+// Empty work lists of one update phase, the filter sizes from the window and the state.
+void Batch::begin_phase(PhaseWork& w, int hyb_phase) {
+  w.fw.assign(B_, FilterWork{});
+  w.cand_begin.assign(B_ + 1, 0);
+  if (hybrid_) { w.hyb_phase = hyb_phase; w.hw.assign(B_, HybWork{}); }
+  for (int fi = 0; fi < B_; ++fi) {
+    FilterWork& fw = w.fw[fi];
+    fw.N = (int)f_[fi].clones.size();
+    fw.D = ORCVIO_LEG + 6 * fw.N + (int)f_[fi].feature_states.size();
+  }
+}
+
+// One candidate record + its observations in the pools of w (lost / tracked-long feature of removeLostFeatures).
+static CandBuild lost_candidate(Batch::PhaseWork& w, const FilterHost& F, const Track& tr, bool tracked_now, int kind,
+                                int flags) {
+  CandBuild x{};
+  x.id = tr.id;
+  x.kind = kind;
+  Cand& c = x.c;
+  c.slot = tr.slot;
+  c.gen = tr.gen;
+  c.flags = flags;
+  c.jac_off = c.tri_off = (int)w.obs_clone.size();
+  int s_blk = 1 << 30, e_blk = -1, cnt = 0;
+  for (const Obs& o : tr.obs) {
+    const int ci = F.clone_index(o.sid);
+    if (ci < 0) continue;
+    w.obs_clone.push_back(ci);
+    w.obs_z.push_back(o.z[0]);
+    w.obs_z.push_back(o.z[1]);
+    s_blk = std::min(s_blk, ci);
+    e_blk = std::max(e_blk, ci);
+    ++cnt;
+  }
+  c.jac_m = cnt;
+  c.tri_m = tracked_now ? cnt - 1 : cnt;   // initializePosition skips the current frame (:414)
+  c.s_blk = s_blk;
+  c.e_blk = e_blk;
+  c.cm_first_clone = w.obs_clone[c.jac_off];
+  c.cm_last_clone = w.obs_clone[c.jac_off + (tracked_now ? cnt - 2 : cnt - 1)];
+  c.cm_zu = w.obs_z[2 * (size_t)c.jac_off];
+  c.cm_zv = w.obs_z[2 * (size_t)c.jac_off + 1];
+  return x;
+}
+
+// Grid cell of a track's newest observation, :2286-2289 / :3841-3845 (the casts truncate toward zero).
+static int grid_code(const Params& p, const Track& tr) {
+  const double* z = tr.obs.back().z;
+  const int row = (int)((z[1] - p.y_min) / p.grid_height);
+  const int col = (int)((z[0] - p.x_min) / p.grid_width);
+  return row * p.grid_cols + col;
+}
+
+// removeLostFeatures :2196-2579 up to the read-back of phase A.  False: the hybrid bookkeeping failed (err_).
+bool Batch::remove_lost_features(FrameWork& fr) {
+  PhaseWork& A = fr.A;
+  for (FilterHost& F : f_) F.index_clones();
+  if (hybrid_) compact_feature_states(fr);
+  begin_phase(A, 0);
+  for (int fi = 0; fi < B_; ++fi) {           // :2234-2289: the walk over the map server
+    FilterHost& F = f_[fi];
+    if (!F.active) continue;
+    A.maxN = std::max(A.maxN, A.fw[fi].N);
     const long long cur = F.state_id;
-    std::vector<CandBuild>& cb = cbs[fi];
+    std::vector<CandBuild>& cb = fr.lost[fi];
     std::vector<long long> invalid;
     bool ekf_open = false;
     if (hybrid_) {
-      for (long long id : F.feature_states) cells[fi][grid_code(*F.find_track(id))]++;   // updateGridMap :3831-3850
+      for (long long id : F.feature_states) fr.cells[fi][grid_code(p_, *F.find_track(id))]++;   // updateGridMap :3831-3850
       ekf_open = (F.imu_time - F.last_zupt_time > 5) && (int)F.feature_states.size() < Emax_;
     }
     for (auto& kv : F.map_server) {
@@ -1384,26 +1347,25 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       } else {
         if (!(nobs >= p_.max_track_len)) continue;
         if (ekf_open) {
-          const int code = grid_code(tr);
-          auto it = cells[fi].find(code);
-          if ((it == cells[fi].end() ? 0 : it->second) < p_.max_features) {
-            PossRec pr{&tr, code, -1, 0};
+          const int code = grid_code(p_, tr);
+          auto it = fr.cells[fi].find(code);
+          if ((it == fr.cells[fi].end() ? 0 : it->second) < p_.max_features) {
+            FrameWork::PossRec pr{&tr, code, -1, 0};
             if (!tr.ekf_feature) {
               // is_initialized = false (:2296): a fresh serial, so the kernel starts from the two-view guess
               pr.spec_gen = F.next_gen++;
-              Track probe = tr;
-              probe.gen = pr.spec_gen;
-              CandBuild x = make_cand(wS, F, probe, true, 1, 0);
+              CandBuild x = lost_candidate(fr.spec, F, tr, true, 1, 0);
+              x.c.gen = pr.spec_gen;
               x.c.filter = fi;
-              pr.spec = (int)wS.cands.size();
-              wS.cands.push_back(x.c);
+              pr.spec = (int)fr.spec.cands.size();
+              fr.spec.cands.push_back(x.c);
             }
-            poss[fi].push_back(pr);
+            fr.poss[fi].push_back(pr);
             continue;
           }
         }
       }
-      cb.push_back(make_cand(wA, F, tr, tracked_now, tracked_now ? 1 : 0, 0));
+      cb.push_back(lost_candidate(A, F, tr, tracked_now, tracked_now ? 1 : 0, 0));
     }
     for (long long id : invalid) {
       F.free_slots.push_back(F.find_track(id)->slot);
@@ -1411,154 +1373,34 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
     }
   }
   g_sp.mark(4);
-  std::vector<CommitRec> commits;
-  if (hybrid_ && !wS.cands.empty()) {
-    const size_t nS = wS.cands.size();
-    const size_t cap = nS * 2 + 64;
-    CKA(hb->dFinal.grow(nS * 3, cap * 3, "speculative triangulation"));
-    CKA(hb->dSpecStatus.grow(nS, cap, "speculative triangulation"));
-    CKA(hb->hSpecStatus.grow(nS, cap, "speculative triangulation (pinned)"));
-    TriArgs ta{};
-    ta.cand = hb->put(wS.cands.data(), nS, stream_, &hyb_ok); ta.n_cand = (int)nS;
-    ta.clones = dClones_.get(); ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    ta.fpos = hb->dSpecPos.get(); ta.fgen = hb->dSpecGen.get(); ta.fcap = Fcap_;
-    ta.obs_clone = hb->put(wS.obs_clone.data(), wS.obs_clone.size(), stream_, &hyb_ok);
-    ta.obs_z = hb->put(wS.obs_z.data(), wS.obs_z.size(), stream_, &hyb_ok);
-    ta.cfg = tricfg_;
-    ta.status = hb->dSpecStatus.get();
-    ta.final_pos = hb->dFinal.get();
-    if (hyb_ok) {
-      launch_triangulate(ta, stream_);
-      ++launches_;
-      CK(cudaMemcpyAsync(hb->hSpecStatus.get(), hb->dSpecStatus.get(), nS * sizeof(int), cudaMemcpyDeviceToHost, stream_));
-      CK(cudaStreamSynchronize(stream_));
-    }
-  }
+  if (hybrid_ && !fr.spec.cands.empty()) speculative_triangulation(fr);
   g_sp.mark(5);
-  for (int fi = 0; fi < B_; ++fi) {
-    FilterHost& F = f_[fi];
-    wA.cand_begin[fi] = (int)wA.cands.size();
-    FilterWork& fw = wA.fw[fi];
-    if (!F.active) continue;
-    std::vector<CandBuild>& cb = cbs[fi];
-    const int E = (int)F.feature_states.size();
-    if (hybrid_) {
-      // the reference's sequential grid decision (:2291-2323), now that every triangulation outcome is known
-      int n_new = 0;
-      for (PossRec& pr : poss[fi]) {
-        Track& tr = *pr.tr;
-        int& cell = cells[fi][pr.code];
-        if (!(cell < p_.max_features && E + n_new < Emax_)) {       // no room any more: an MSCKF feature
-          cb.push_back(make_cand(wA, F, tr, true, 1, 0));
-          continue;
-        }
-        if (!tr.ekf_feature) {
-          tr.gen = pr.spec_gen;                                      // is_initialized = false
-          tr.initialized = false;
-          if (!(hb->hSpecStatus.get()[pr.spec] & ST_TRI_VALID)) continue;  // checkMotion / triangulation failed (:2297-2303)
-          tr.ekf_feature = true;
-          tr.initialized = true;
-          for (int k = (int)tr.obs.size() - 1; k >= 0; --k)          // anchor = the last camera used (feature.hpp:536)
-            if (tr.obs[k].sid != F.state_id && clone_index_of(F, tr.obs[k].sid) >= 0) { tr.id_anchor = tr.obs[k].sid; break; }
-          commits.push_back(CommitRec{pr.spec, fi * Fcap_ + tr.slot, tr.gen});
-        }
-        news[fi].push_back(&tr);
-        ++cell;
-        ++n_new;
-      }
-    }
-    F.stats.n_candidates_lost = (int)cb.size();
-    if (cb.empty() && E == 0 && news[fi].empty()) continue;
-    if (F.if_zupt) {
-      // :2564-2569: under ZUPT the candidates are still initialised (and the failures erased) but
-      // no Jacobian is stacked and no update runs
-      append_candidates(wA, fi, cb, F.cinfo[0], true);
-      continue;
-    }
-    fw.active = 1;
-    wA.any_active = true;
-    append_candidates(wA, fi, cb, F.cinfo[0]);
-    if (hybrid_) {
-      HybWork& hw = wA.hw[fi];
-      hw.N = fw.N; hw.E = E; hw.active = 1;
-      hw.feat_begin = (int)wA.hfeats.size();
-      for (long long id : F.feature_states) {
-        const Track& tr = *F.find_track(id);
-        HybFeat hf{};
-        hf.slot = tr.slot;
-        hf.anchor = clone_index_of(F, tr.id_anchor);
-        hf.zu = tr.obs.back().z[0];
-        hf.zv = tr.obs.back().z[1];
-        if (hf.anchor < 0) { hyb_ok = false; hf.anchor = 0; }
-        wA.hfeats.push_back(hf);
-      }
-      hw.feat_end = (int)wA.hfeats.size();
-      hw.new_begin = (int)wA.hnews.size();
-      int nd = 2 * E;
-      for (Track* trp : news[fi]) {
-        // its MSCKF rows over every observation only decide the gate (:2365-2370); they are not stacked
-        CandBuild x = make_cand(wA, F, *trp, true, 3, CAND_GATE_ONLY);
-        Cand c = x.c;
-        c.filter = fi;
-        const int r = std::max(2 * c.jac_m - 3, 0);
-        c.row_off = (int)wA.rows_total;
-        c.hblk_off = (int)wA.hblk_total;
-        wA.rows_total += (size_t)r;
-        wA.hblk_total += (size_t)r * 6 * (c.e_blk - c.s_blk + 1);
-        wA.own_wmax_blk = std::max(wA.own_wmax_blk, c.e_blk - c.s_blk + 1);
-        const int idx = (int)wA.cands.size();
-        (c.jac_m <= 8 ? wA.small_list : wA.large_list).push_back(idx);
-        wA.cands.push_back(c);
-        F.cinfo[0].push_back(CandInfo{x.id, 3});
-        HybNew hn{};
-        hn.slot = trp->slot;
-        hn.anchor = clone_index_of(F, trp->id_anchor);
-        hn.cand = idx;
-        hn.obs_off = c.jac_off;
-        hn.obs_m = c.jac_m;
-        hn.row_off = nd - 2 * E;
-        if (hn.anchor < 0) { hyb_ok = false; hn.anchor = 0; }
-        nd += 2 * (c.jac_m - 1) - 1;
-        wA.hnews.push_back(hn);
-      }
-      hw.new_end = (int)wA.hnews.size();
-      hw.dense_off = (int)wA.dense_total;
-      hw.n_dense = nd;
-      hw.arow_dense = fw.arows;
-      fw.dense_rows = nd;
-      for (int J = 0; J < SY_MAXT; ++J) fw.jrow0[J] = std::min(fw.jrow0[J], fw.arows);
-      fw.arows += nd;
-      wA.arows_total += (size_t)nd;
-      wA.dense_total += (size_t)nd;
-      wA.max_dense = std::max(wA.max_dense, nd);
-      wA.maxE = std::max(wA.maxE, E);
-    }
-  }
-  wA.cand_begin[B_] = (int)wA.cands.size();
-  if (hybrid_ && !commits.empty()) {
-    const CommitRec* d_rec = hb->put(commits.data(), commits.size(), stream_, &hyb_ok);
-    if (hyb_ok) {
-      launch_hybrid_commit(d_rec, (int)commits.size(), hb->dFinal.get(), hb->dSpecPos.get(), dFpos_.get(), dFgen_.get(), dFidp_.get(), stream_);
+  for (int fi = 0; fi < B_; ++fi) stage_lost_features(fr, fi);
+  A.cand_begin[B_] = (int)A.cands.size();
+  HybridBufs* hb = hyb_.get();
+  if (hybrid_ && !fr.commits.empty()) {
+    const CommitRec* d_rec = hb->put(fr.commits.data(), fr.commits.size(), stream_, &fr.hyb_ok);
+    if (fr.hyb_ok) {
+      launch_hybrid_commit(d_rec, (int)fr.commits.size(), hb->dFinal.get(), hb->dSpecPos.get(), dFpos_.get(), dFgen_.get(), dFidp_.get(), stream_);
       ++launches_;
     }
   }
-  if (!hyb_ok) { ok_ = false; err_ = "hybrid bookkeeping failed (upload arena / anchor outside the window)"; return ORCVIO_ERR_CUDA; }
-  cudaEvent_t* e = ev_;
+  if (!fr.hyb_ok) { ok_ = false; err_ = "hybrid bookkeeping failed (upload arena / anchor outside the window)"; return false; }
   g_sp.mark(6);
-  run_phase(wA, 0);
-  std::vector<Track*> gather_tracks;
+  stage_phase(A);
+  launch_phase(A, true);
   if (hybrid_) {
     for (int fi = 0; fi < B_; ++fi) {       // the features whose host mirror the prune phase may need
       FilterHost& F = f_[fi];
       F.ekf_watch.clear();
       if (!F.active) continue;
       F.ekf_watch = F.feature_states;
-      for (Track* trp : news[fi]) F.ekf_watch.push_back(trp->id);
+      for (Track* trp : fr.news[fi]) F.ekf_watch.push_back(trp->id);
     }
-    hybrid_queue_gather(gather_tracks);
-    if (!wA.hfeats.empty()) {
-      CK(cudaMemcpyAsync(hb->hEkfPass.get(), hb->dEkfPass.get(), wA.hfeats.size() * sizeof(int), cudaMemcpyDeviceToHost, stream_));
-      CK(cudaMemcpyAsync(hb->hEkfGamma.get(), hb->dEkfGamma.get(), wA.hfeats.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+    hybrid_queue_gather(fr.gather_tracks);
+    if (!A.hfeats.empty()) {
+      CK(cudaMemcpyAsync(hb->hEkfPass.get(), hb->dEkfPass.get(), A.hfeats.size() * sizeof(int), cudaMemcpyDeviceToHost, stream_));
+      CK(cudaMemcpyAsync(hb->hEkfGamma.get(), hb->dEkfGamma.get(), A.hfeats.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
     }
   }
   download_mirrors();
@@ -1566,123 +1408,225 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
   CK(cudaStreamSynchronize(stream_));
   g_sp.mark(8);
   if (hybrid_) {
-    hybrid_apply_gather(gather_tracks);
+    hybrid_apply_gather(fr.gather_tracks);
     hb->used = 0;
   }
-  auto account = [&](bool had_update) {
-    if (!profiling_) return;
-    float ms = 0;
-    cudaEventElapsedTime(&ms, e[0], e[1]); pt_.tri += ms; pt_.n_tri++;
-    cudaEventElapsedTime(&ms, e[1], e[2]); pt_.jac += ms; pt_.n_jac++;
-    if (had_update) {
-      cudaEventElapsedTime(&ms, e[2], e[3]); pt_.qr_tiles += ms; pt_.n_qr_tiles++;
-      cudaEventElapsedTime(&ms, e[3], e[4]); pt_.qr_chain += ms; pt_.n_qr_chain++;
-      cudaEventElapsedTime(&ms, e[4], e[5]); pt_.update += ms; pt_.n_update++;
-    }
-  };
-  account(wA.any_active);
+  account_phase(A.any_active);
+  return true;
+}
 
-  // ---------------------------------------------------------------- E: post-process A, prune
-  PhaseWork wB;
-  wB.fw.assign(B_, FilterWork{});
-  wB.cand_begin.assign(B_ + 1, 0);
-  if (hybrid_) { wB.hyb_phase = 1; wB.hw.assign(B_, HybWork{}); }
-  std::vector<int> rm_idx(2 * (size_t)B_, -1), Nbefore(B_, 0), Ebefore(B_, 0);
-  std::vector<ReanchorRec> reanchor;
-  std::vector<int> reanchor_off(B_ + 1, 0);
-  // pruneImuStateBuffer :2665-2773: an EKF-SLAM feature (of the state, or initialised and waiting outside it) whose anchor
-  // clone is about to leave the window moves to a new anchor (getNewAnchorId :3892-3950) before anything else happens
-  auto reanchor_tracks = [&](int fi, FilterHost& F, const long long* rm_ids, int n_rm) {
-    if (F.ekf_watch.empty()) return;
-    std::vector<long long> ids = F.ekf_watch;
-    std::sort(ids.begin(), ids.end());
-    auto removed = [&](long long sid) {
-      for (int q = 0; q < n_rm; ++q) if (rm_ids[q] == sid) return true;
-      return false;
-    };
-    for (long long id : ids) {
-      Track* trp = F.find_track(id);
-      if (!trp) continue;
-      Track& tr = *trp;
-      if (!tr.ekf_feature || !tr.initialized || !removed(tr.id_anchor)) continue;
-      bool anchor_observed = false;
-      for (const Obs& o : tr.obs) anchor_observed |= (o.sid == tr.id_anchor);
-      if (!anchor_observed) continue;                   // `involved` holds only clones the feature was seen from
-      // getNewAnchorId: the observing clone (the two newest and the removed ones excluded) whose stored observation is
-      // closest to the reprojection of the feature; the newest clone when there is none
-      const int n = (int)F.clones.size();
-      long long new_id = F.clones.back().id;
-      if (n > 2) {
-        double min_dis = 99999.0;
-        long long best = -1;
-        for (int k = 0; k < n - 2; ++k) {
-          const long long sid = F.clones[k].id;
-          if (removed(sid)) continue;
-          const Obs* ob = nullptr;
-          for (const Obs& o : tr.obs) if (o.sid == sid) ob = &o;
-          if (!ob) continue;
-          const double* c = F.clone_mirror.data() + (size_t)k * CL_STRIDE;
-          const double d[3] = {tr.mpos[0] - c[CL_PC], tr.mpos[1] - c[CL_PC + 1], tr.mpos[2] - c[CL_PC + 2]};
-          double pn[3];
-          m3_inv_vec(c + CL_RC, d, pn);
-          const double du = pn[0] / pn[2] - ob->z[0], dv = pn[1] / pn[2] - ob->z[1];
-          const double dis = std::sqrt(du * du + dv * dv);
-          if (min_dis > dis) { min_dis = dis; best = sid; }
-        }
-        if (best >= 0) new_id = best;
-      }
-      ReanchorRec rc{};
-      rc.filter = fi;
-      rc.slot = tr.slot;
-      rc.col = -1;
-      if (tr.in_state)
-        for (int i = 0; i < (int)F.feature_states.size(); ++i)
-          if (F.feature_states[i] == id) rc.col = i;
-      rc.old_idx = clone_index_of(F, tr.id_anchor);
-      rc.new_idx = clone_index_of(F, new_id);
-      if (!tr.in_state) {
-        // :2762-2764: obs_anchor <- the stored observation in the new anchor (operator[] default-constructs it)
-        const Obs* ob = nullptr;
-        for (const Obs& o : tr.obs) if (o.sid == new_id) ob = &o;
-        if (!ob) {
-          Obs z{};
-          z.sid = new_id;
-          auto pos = std::lower_bound(tr.obs.begin(), tr.obs.end(), new_id,
-                                      [](const Obs& o, long long sid) { return o.sid < sid; });
-          ob = &*tr.obs.insert(pos, z);
-          tr.touch();
-        }
-        rc.zu = ob->z[0];
-        rc.zv = ob->z[1];
-      } else {
-        F.log_reanchor.push_back(id);
-        F.log_reanchor.push_back(tr.id_anchor);
-        F.log_reanchor.push_back(new_id);
-      }
-      tr.id_anchor = new_id;
-      reanchor.push_back(rc);
-    }
-  };
+// features of the state: tracked now -> a 2-row update; lost -> dropped (:2210-2232, rmLostFeaturesCov :3776-3828)
+void Batch::compact_feature_states(FrameWork& fr) {
+  HybridBufs* hb = hyb_.get();
+  hb->used = 0;                          // the stream is idle (synchronised at the end of propagate_and_augment)
+  std::vector<int> newidx, Dold(B_, 0);
+  bool any_compact = false;
   for (int fi = 0; fi < B_; ++fi) {
     FilterHost& F = f_[fi];
-    wB.cand_begin[fi] = (int)wB.cands.size();
-    reanchor_off[fi] = (int)reanchor.size();
-    FilterWork& fw = wB.fw[fi];
-    fw.N = (int)F.clones.size();
-    fw.D = L + 6 * fw.N + (int)F.feature_states.size();
-    fw.active = 0;
-    Nbefore[fi] = fw.N;
-    if (!F.active) { Ebefore[fi] = (int)F.feature_states.size(); continue; }
-    std::memcpy(F.imu_mirror.data(), hImu_.get() + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
-    std::memcpy(F.clone_mirror.data(), hClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE,
-                (size_t)Ncap_ * CL_STRIDE * sizeof(double));
-    // results of phase A
-    const int c0 = wA.cand_begin[fi], c1 = wA.cand_begin[fi + 1];
+    if (!F.active || F.feature_states.empty()) continue;
+    const int base = ORCVIO_LEG + 6 * (int)F.clones.size(), E0 = (int)F.feature_states.size();
+    std::vector<long long> kept;
+    std::vector<int> map_e(E0, -1);
+    for (int i = 0; i < E0; ++i) {
+      Track& tr = *F.find_track(F.feature_states[i]);
+      if (!tr.obs.empty() && tr.obs.back().sid == F.state_id) {
+        map_e[i] = (int)kept.size();
+        kept.push_back(tr.id);
+      } else {
+        const long long lost_id = tr.id;
+        F.log_ekf_lost.push_back(lost_id);
+        F.free_slots.push_back(tr.slot);
+        F.erase_track(lost_id);
+      }
+    }
+    if ((int)kept.size() != E0) {
+      if (newidx.empty()) newidx.assign((size_t)B_ * ldp_, -1);
+      int* ni = newidx.data() + (size_t)fi * ldp_;
+      for (int j = 0; j < base; ++j) ni[j] = j;
+      for (int i = 0; i < E0; ++i) ni[base + i] = map_e[i] < 0 ? -1 : base + map_e[i];
+      Dold[fi] = base + E0;
+      any_compact = true;
+      F.feature_states = kept;
+    }
+  }
+  if (any_compact) {
+    const int* d_ni = hb->put(newidx.data(), newidx.size(), stream_, &fr.hyb_ok);
+    const int* d_do = hb->put(Dold.data(), Dold.size(), stream_, &fr.hyb_ok);
+    if (fr.hyb_ok) { launch_compact_cov(dP_.get(), (size_t)ldp_ * ldp_, ldp_, d_ni, d_do, B_, stream_); ++launches_; }
+  }
+}
+
+// initializeInvParamPosition of every FrameWork::PossRec into the scratch position table, waited for.
+void Batch::speculative_triangulation(FrameWork& fr) {
+  HybridBufs* hb = hyb_.get();
+  const size_t nS = fr.spec.cands.size();
+  const size_t cap = nS * 2 + 64;
+  CKA(hb->dFinal.grow(nS * 3, cap * 3, "speculative triangulation"));
+  CKA(hb->dSpecStatus.grow(nS, cap, "speculative triangulation"));
+  CKA(hb->hSpecStatus.grow(nS, cap, "speculative triangulation (pinned)"));
+  TriArgs ta{};
+  ta.cand = hb->put(fr.spec.cands.data(), nS, stream_, &fr.hyb_ok); ta.n_cand = (int)nS;
+  ta.clones = dClones_.get(); ta.clone_stride = (size_t)Ncap_ * CL_STRIDE;
+  ta.fpos = hb->dSpecPos.get(); ta.fgen = hb->dSpecGen.get(); ta.fcap = Fcap_;
+  ta.obs_clone = hb->put(fr.spec.obs_clone.data(), fr.spec.obs_clone.size(), stream_, &fr.hyb_ok);
+  ta.obs_z = hb->put(fr.spec.obs_z.data(), fr.spec.obs_z.size(), stream_, &fr.hyb_ok);
+  ta.cfg = tricfg_;
+  ta.status = hb->dSpecStatus.get();
+  ta.final_pos = hb->dFinal.get();
+  if (fr.hyb_ok) {
+    launch_triangulate(ta, stream_);
+    ++launches_;
+    CK(cudaMemcpyAsync(hb->hSpecStatus.get(), hb->dSpecStatus.get(), nS * sizeof(int), cudaMemcpyDeviceToHost, stream_));
+    CK(cudaStreamSynchronize(stream_));
+  }
+}
+
+// the reference's sequential grid decision (:2291-2323), now that every triangulation outcome is known
+void Batch::decide_grid_cells(FrameWork& fr, int fi) {
+  FilterHost& F = f_[fi];
+  const int E = (int)F.feature_states.size();
+  int n_new = 0;
+  for (FrameWork::PossRec& pr : fr.poss[fi]) {
+    Track& tr = *pr.tr;
+    int& cell = fr.cells[fi][pr.code];
+    if (!(cell < p_.max_features && E + n_new < Emax_)) {       // no room any more: an MSCKF feature
+      fr.lost[fi].push_back(lost_candidate(fr.A, F, tr, true, 1, 0));
+      continue;
+    }
+    if (!tr.ekf_feature) {
+      tr.gen = pr.spec_gen;                                      // is_initialized = false
+      tr.initialized = false;
+      if (!(hyb_->hSpecStatus.get()[pr.spec] & ST_TRI_VALID)) continue;  // checkMotion / triangulation failed (:2297-2303)
+      tr.ekf_feature = true;
+      tr.initialized = true;
+      for (int k = (int)tr.obs.size() - 1; k >= 0; --k)          // anchor = the last camera used (feature.hpp:536)
+        if (tr.obs[k].sid != F.state_id && F.clone_index(tr.obs[k].sid) >= 0) { tr.id_anchor = tr.obs[k].sid; break; }
+      fr.commits.push_back(CommitRec{pr.spec, fi * Fcap_ + tr.slot, tr.gen});
+    }
+    fr.news[fi].push_back(&tr);
+    ++cell;
+    ++n_new;
+  }
+}
+
+// Phase A work of filter fi: its lost / tracked-long candidates and, hybrid, the dense rows of the EKF-SLAM features.
+void Batch::stage_lost_features(FrameWork& fr, int fi) {
+  FilterHost& F = f_[fi];
+  PhaseWork& A = fr.A;
+  A.cand_begin[fi] = (int)A.cands.size();
+  if (!F.active) return;
+  std::vector<CandBuild>& cb = fr.lost[fi];
+  if (hybrid_) decide_grid_cells(fr, fi);
+  F.stats.n_candidates_lost = (int)cb.size();
+  if (cb.empty() && F.feature_states.empty() && fr.news[fi].empty()) return;
+  if (F.if_zupt) {
+    // :2564-2569: under ZUPT the candidates are still initialised (and the failures erased) but
+    // no Jacobian is stacked and no update runs
+    append_candidates(A, fi, cb, F.cinfo[0], true);
+    return;
+  }
+  FilterWork& fw = A.fw[fi];
+  fw.active = 1;
+  A.any_active = true;
+  append_candidates(A, fi, cb, F.cinfo[0]);
+  if (!hybrid_) return;
+  // the 2-row updates of the features of the state, the new EKF-SLAM features behind their gate-only candidates
+  HybWork& hw = A.hw[fi];
+  const int E = (int)F.feature_states.size();
+  push_hyb_feats(A, fi, 1, true, &fr.hyb_ok);
+  hw.new_begin = (int)A.hnews.size();
+  int nd = 2 * E;
+  for (Track* trp : fr.news[fi]) {
+    // its MSCKF rows over every observation only decide the gate (:2365-2370); they are not stacked
+    const CandBuild x = lost_candidate(A, F, *trp, true, 3, CAND_GATE_ONLY);
+    HybNew hn{};
+    hn.slot = trp->slot;
+    hn.anchor = F.clone_index(trp->id_anchor);
+    hn.cand = push_candidate(A, fi, x, F.cinfo[0], false);
+    hn.obs_off = x.c.jac_off;
+    hn.obs_m = x.c.jac_m;
+    hn.row_off = nd - 2 * E;
+    if (hn.anchor < 0) { fr.hyb_ok = false; hn.anchor = 0; }
+    nd += 2 * (x.c.jac_m - 1) - 1;
+    A.hnews.push_back(hn);
+  }
+  hw.new_end = (int)A.hnews.size();
+  hw.dense_off = (int)A.dense_total;
+  hw.n_dense = nd;
+  hw.arow_dense = fw.arows;
+  fw.dense_rows = nd;
+  for (int J = 0; J < SY_MAXT; ++J) fw.jrow0[J] = std::min(fw.jrow0[J], fw.arows);
+  fw.arows += nd;
+  A.arows_total += (size_t)nd;
+  A.dense_total += (size_t)nd;
+  A.max_dense = std::max(A.max_dense, nd);
+  A.maxE = std::max(A.maxE, E);
+}
+
+// HybWork of filter fi and a HybFeat per feature of its state; with_obs: its newest observation (phase B leaves it 0).
+void Batch::push_hyb_feats(PhaseWork& w, int fi, int active, bool with_obs, bool* ok) {
+  const FilterHost& F = f_[fi];
+  HybWork& hw = w.hw[fi];
+  hw.N = w.fw[fi].N; hw.E = (int)F.feature_states.size(); hw.active = active;
+  hw.feat_begin = (int)w.hfeats.size();
+  for (long long id : F.feature_states) {
+    const Track& tr = *F.find_track(id);
+    HybFeat hf{};
+    hf.slot = tr.slot;
+    hf.anchor = F.clone_index(tr.id_anchor);
+    if (with_obs) {
+      hf.zu = tr.obs.back().z[0];
+      hf.zv = tr.obs.back().z[1];
+    }
+    if (hf.anchor < 0) { *ok = false; hf.anchor = 0; }
+    w.hfeats.push_back(hf);
+  }
+  hw.feat_end = (int)w.hfeats.size();
+}
+
+// status / gamma of candidate c of phase ph into F's log and, when counted, the frame stats; returns the status
+int Batch::take_result(FilterHost& F, int ph, int c, bool counted) {
+  const int st = hStatus_.get()[c];
+  F.cstatus[ph].push_back(st);
+  F.cgamma[ph].push_back(hGamma_.get()[c]);
+  if (counted) {
+    if (!(st & ST_TRI_VALID)) ++(ph ? F.stats.n_tri_invalid_prune : F.stats.n_tri_invalid_lost);
+    if (st & ST_GATE_PASS) { ++(ph ? F.stats.n_gate_pass_prune : F.stats.n_gate_pass_lost); ++feature_updates_; }
+  }
+  return st;
+}
+
+void Batch::refresh_mirrors(int fi) {
+  FilterHost& F = f_[fi];
+  std::memcpy(F.imu_mirror.data(), hImu_.get() + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
+  std::memcpy(F.clone_mirror.data(), hClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE,
+              (size_t)Ncap_ * CL_STRIDE * sizeof(double));
+}
+
+// stage times of the phase just read back (set_profiling)
+void Batch::account_phase(bool had_update) {
+  if (!profiling_) return;
+  float ms = 0;
+  cudaEventElapsedTime(&ms, ev_[0], ev_[1]); pt_.tri += ms; pt_.n_tri++;
+  cudaEventElapsedTime(&ms, ev_[1], ev_[2]); pt_.jac += ms; pt_.n_jac++;
+  if (had_update) {
+    cudaEventElapsedTime(&ms, ev_[2], ev_[3]); pt_.qr_tiles += ms; pt_.n_qr_tiles++;
+    cudaEventElapsedTime(&ms, ev_[3], ev_[4]); pt_.qr_chain += ms; pt_.n_qr_chain++;
+    cudaEventElapsedTime(&ms, ev_[4], ev_[5]); pt_.update += ms; pt_.n_update++;
+  }
+}
+
+// Results of phase A (:2371-2411, :2564-2576).  Each filter only touches its own records.
+void Batch::apply_lost_results(const FrameWork& fr) {
+  const PhaseWork& A = fr.A;
+  for (int fi = 0; fi < B_; ++fi) {
+    FilterHost& F = f_[fi];
+    if (!F.active) continue;
+    refresh_mirrors(fi);
+    const int c0 = A.cand_begin[fi], c1 = A.cand_begin[fi + 1];
     for (int c = c0; c < c1; ++c) {
-      const int st = hStatus_.get()[c];
       const CandInfo& ci = F.cinfo[0][c - c0];
-      F.cstatus[0].push_back(st);
-      F.cgamma[0].push_back(hGamma_.get()[c]);
+      const int st = take_result(F, 0, c, ci.kind != 3);
       if (ci.kind == 3) {
         // candidate EKF-SLAM feature: in the state iff its MSCKF rows passed the gate (:2371-2411); a rejected one
         // keeps its inverse-depth record and waits outside the state
@@ -1697,8 +1641,6 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
         }
         continue;
       }
-      if (!(st & ST_TRI_VALID)) F.stats.n_tri_invalid_lost++;
-      if (st & ST_GATE_PASS) { F.stats.n_gate_pass_lost++; ++feature_updates_; }
       // lost features are always erased (:2572-2576); tracked-long ones only when they were
       // initialised and therefore used (:2310-2319)
       if (ci.kind == 0 || (st & ST_TRI_VALID)) {
@@ -1708,201 +1650,259 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
         }
       }
     }
-    if (hybrid_ && wA.hw[fi].active) {
-      const HybWork& hw = wA.hw[fi];
+    if (hybrid_ && A.hw[fi].active) {
+      const HybWork& hw = A.hw[fi];
       for (int i = 0; i < hw.E; ++i) {
         F.log_ekf_ids.push_back(F.feature_states[i]);
-        F.log_ekf_pass.push_back(hb->hEkfPass.get()[hw.feat_begin + i]);
-        F.log_ekf_gamma.push_back(hb->hEkfGamma.get()[hw.feat_begin + i]);
-        if (hb->hEkfPass.get()[hw.feat_begin + i]) ++feature_updates_;
+        F.log_ekf_pass.push_back(hyb_->hEkfPass.get()[hw.feat_begin + i]);
+        F.log_ekf_gamma.push_back(hyb_->hEkfGamma.get()[hw.feat_begin + i]);
+        if (hyb_->hEkfPass.get()[hw.feat_begin + i]) ++feature_updates_;
       }
     }
-    fw.D = L + 6 * fw.N + (int)F.feature_states.size();
-    Ebefore[fi] = (int)F.feature_states.size();
-    wB.maxE = std::max(wB.maxE, Ebefore[fi]);
-    auto fill_hw = [&]() {              // features of the state with their (possibly new) anchors
-      if (!hybrid_) return;
-      HybWork& hw = wB.hw[fi];
-      hw.N = fw.N; hw.E = Ebefore[fi]; hw.active = fw.active;
-      hw.feat_begin = (int)wB.hfeats.size();
-      for (long long id : F.feature_states) {
-        const Track& tr = *F.find_track(id);
-        HybFeat hf{};
-        hf.slot = tr.slot;
-        hf.anchor = clone_index_of(F, tr.id_anchor);
-        if (hf.anchor < 0) { hyb_ok = false; hf.anchor = 0; }
-        wB.hfeats.push_back(hf);
-      }
-      hw.feat_end = (int)wB.hfeats.size();
-      hw.new_begin = hw.new_end = 0;
-    };
-    // pruneImuStateBuffer :2629-2959
-    if (F.if_zupt) {
-      // :2633-2639: a stationary frame drops the previous clone (id - 1) and uses nothing
-      const int n = (int)F.clones.size();
-      if (n < 2) { fill_hw(); continue; }
-      rm_idx[2 * fi] = n - 2;
-      const long long rm_id = F.clones[n - 2].id;
-      F.stats.n_removed_clones = 1;
-      F.stats.removed_ids[0] = rm_id;
-      if (hybrid_) reanchor_tracks(fi, F, &rm_id, 1);
-      for (auto& kv : F.map_server) {
-        Track& tr = kv.second;
-        if (tr.first_sid > rm_id || tr.last_sid < rm_id) continue;     // (ascending ids: it cannot hold the clone)
-        tr.obs.erase(std::remove_if(tr.obs.begin(), tr.obs.end(), [&](const Obs& o) { return o.sid == rm_id; }),
-                     tr.obs.end());
+  }
+}
+
+// findRedundantImuStates :2582-2626: the two clone indices to remove, ascending
+void Batch::find_redundant_imu_states(const FilterHost& F, int rm[2]) const {
+  const int n = (int)F.clones.size();
+  int key_i = n - 4, st_i = key_i + 1, first_i = 0;
+  const double* key = F.clone_mirror.data() + (size_t)key_i * CL_STRIDE;
+  for (int r = 0; r < 2; ++r) {
+    const double* c = F.clone_mirror.data() + (size_t)st_i * CL_STRIDE;
+    const double dx = c[CL_PC] - key[CL_PC], dy = c[CL_PC + 1] - key[CL_PC + 1], dz = c[CL_PC + 2] - key[CL_PC + 2];
+    const double distance = std::sqrt((dx * dx + dy * dy) + dz * dz);
+    double Rr[9];
+    m3_Tmul(c + CL_RC, key + CL_RC, Rr);      // rotation = R_cam^T ; rotation * key_rotation
+    const double angle = angle_axis_angle(Rr);
+    if (angle < p_.rotation_threshold && distance < p_.translation_threshold &&
+        F.tracking_rate > p_.tracking_rate_threshold) {
+      rm[r] = st_i;
+      ++st_i;
+    } else {
+      rm[r] = first_i;
+      ++first_i;
+      st_i -= 2;
+    }
+  }
+  if (rm[0] > rm[1]) std::swap(rm[0], rm[1]);
+}
+
+// getNewAnchorId :3892-3950: the observing clone (the two newest and the removed ones excluded) whose stored observation
+// is closest to the reprojection of the feature; the newest clone when there is none.
+static long long get_new_anchor_id(const FilterHost& F, const Track& tr, const long long* rm_ids, int n_rm) {
+  const int n = (int)F.clones.size();
+  long long new_id = F.clones.back().id;
+  if (n > 2) {
+    double min_dis = 99999.0;
+    long long best = -1;
+    for (int k = 0; k < n - 2; ++k) {
+      const long long sid = F.clones[k].id;
+      if (std::count(rm_ids, rm_ids + n_rm, sid)) continue;
+      const Obs* ob = nullptr;
+      for (const Obs& o : tr.obs) if (o.sid == sid) ob = &o;
+      if (!ob) continue;
+      const double* c = F.clone_mirror.data() + (size_t)k * CL_STRIDE;
+      const double d[3] = {tr.mpos[0] - c[CL_PC], tr.mpos[1] - c[CL_PC + 1], tr.mpos[2] - c[CL_PC + 2]};
+      double pn[3];
+      m3_inv_vec(c + CL_RC, d, pn);
+      const double du = pn[0] / pn[2] - ob->z[0], dv = pn[1] / pn[2] - ob->z[1];
+      const double dis = std::sqrt(du * du + dv * dv);
+      if (min_dis > dis) { min_dis = dis; best = sid; }
+    }
+    if (best >= 0) new_id = best;
+  }
+  return new_id;
+}
+
+// pruneImuStateBuffer :2665-2773: an EKF-SLAM feature (of the state, or initialised and waiting outside it) whose anchor
+// clone is about to leave the window moves to a new anchor before anything else happens.
+void Batch::reanchor_tracks(FrameWork& fr, int fi, const long long* rm_ids, int n_rm) {
+  FilterHost& F = f_[fi];
+  if (F.ekf_watch.empty()) return;
+  std::vector<long long> ids = F.ekf_watch;
+  std::sort(ids.begin(), ids.end());
+  for (long long id : ids) {
+    Track* trp = F.find_track(id);
+    if (!trp) continue;
+    Track& tr = *trp;
+    if (!tr.ekf_feature || !tr.initialized || !std::count(rm_ids, rm_ids + n_rm, tr.id_anchor)) continue;
+    bool anchor_observed = false;
+    for (const Obs& o : tr.obs) anchor_observed |= (o.sid == tr.id_anchor);
+    if (!anchor_observed) continue;                   // `involved` holds only clones the feature was seen from
+    const long long new_id = get_new_anchor_id(F, tr, rm_ids, n_rm);
+    ReanchorRec rc{};
+    rc.filter = fi;
+    rc.slot = tr.slot;
+    rc.col = -1;
+    if (tr.in_state)
+      for (int i = 0; i < (int)F.feature_states.size(); ++i)
+        if (F.feature_states[i] == id) rc.col = i;
+    rc.old_idx = F.clone_index(tr.id_anchor);
+    rc.new_idx = F.clone_index(new_id);
+    if (!tr.in_state) {
+      // :2762-2764: obs_anchor <- the stored observation in the new anchor (operator[] default-constructs it)
+      const Obs* ob = nullptr;
+      for (const Obs& o : tr.obs) if (o.sid == new_id) ob = &o;
+      if (!ob) {
+        Obs z{};
+        z.sid = new_id;
+        auto pos = std::lower_bound(tr.obs.begin(), tr.obs.end(), new_id,
+                                    [](const Obs& o, long long sid) { return o.sid < sid; });
+        ob = &*tr.obs.insert(pos, z);
         tr.touch();
       }
-      fill_hw();
-      continue;
+      rc.zu = ob->z[0];
+      rc.zv = ob->z[1];
+    } else {
+      F.log_reanchor.push_back(id);
+      F.log_reanchor.push_back(tr.id_anchor);
+      F.log_reanchor.push_back(new_id);
     }
-    if ((int)F.clones.size() < p_.sw_size) { fill_hw(); continue; }
-    wB.maxN = std::max(wB.maxN, fw.N);
-    // findRedundantImuStates :2582-2626
-    const int n = (int)F.clones.size();
-    int key_i = n - 4, st_i = key_i + 1, first_i = 0;
-    const double* key = F.clone_mirror.data() + (size_t)key_i * CL_STRIDE;
-    int rm[2];
-    for (int r = 0; r < 2; ++r) {
-      const double* c = F.clone_mirror.data() + (size_t)st_i * CL_STRIDE;
-      const double dx = c[CL_PC] - key[CL_PC], dy = c[CL_PC + 1] - key[CL_PC + 1], dz = c[CL_PC + 2] - key[CL_PC + 2];
-      const double distance = std::sqrt((dx * dx + dy * dy) + dz * dz);
-      double Rr[9];
-      m3_Tmul(c + CL_RC, key + CL_RC, Rr);      // rotation = R_cam^T ; rotation * key_rotation
-      const double angle = angle_axis_angle(Rr);
-      if (angle < p_.rotation_threshold && distance < p_.translation_threshold &&
-          F.tracking_rate > p_.tracking_rate_threshold) {
-        rm[r] = st_i;
-        ++st_i;
-      } else {
-        rm[r] = first_i;
-        ++first_i;
-        st_i -= 2;
-      }
-    }
-    if (rm[0] > rm[1]) std::swap(rm[0], rm[1]);
-    rm_idx[2 * fi] = rm[0];
-    rm_idx[2 * fi + 1] = rm[1];
-    const long long rm_id0 = F.clones[rm[0]].id, rm_id1 = F.clones[rm[1]].id;
-    F.stats.n_removed_clones = 2;
-    F.stats.removed_ids[0] = rm_id0;
-    F.stats.removed_ids[1] = rm_id1;
-    const long long cur = F.state_id;
-    if (hybrid_) {
-      const long long rms[2] = {rm_id0, rm_id1};
-      reanchor_tracks(fi, F, rms, 2);
-    }
-    std::vector<CandBuild> cb;
-    auto clone_index = [&](long long sid) { return clone_index_of(F, sid); };
-    for (auto& kv : F.map_server) {
-      Track& tr = kv.second;
-      if (tr.first_sid > rm_id1 || tr.last_sid < rm_id0) continue;     // (rm_id0 < rm_id1: neither clone observed it)
-      int inv0 = -1, inv1 = -1;
-      for (int k = 0; k < (int)tr.obs.size(); ++k) {
-        if (tr.obs[k].sid == rm_id0) inv0 = k;
-        if (tr.obs[k].sid == rm_id1) inv1 = k;
-      }
-      if (inv0 < 0 && inv1 < 0) continue;
-      // (:2776: EKF-SLAM features never contribute MSCKF rows here)
-      if (inv0 >= 0 && inv1 >= 0 && !tr.in_state && !tr.ekf_feature) {
-        const int nobs = (int)tr.obs.size();
-        const bool tracked = tr.obs.back().sid == cur;
-        CandBuild x{};
-        x.id = tr.id;
-        x.kind = 2;
-        Cand& c = x.c;
-        c.slot = tr.slot;
-        c.gen = tr.gen;
-        c.flags = 0;
-        c.tri_off = (int)wB.obs_clone.size();
-        for (const Obs& o : tr.obs) {            // initializePosition_AssignAnchor: all obs
-          wB.obs_clone.push_back(clone_index(o.sid));
-          wB.obs_z.push_back(o.z[0]);
-          wB.obs_z.push_back(o.z[1]);
-        }
-        c.tri_m = nobs;
-        c.jac_off = (int)wB.obs_clone.size();
-        const int ks[2] = {inv0, inv1};
-        for (int q = 0; q < 2; ++q) {
-          wB.obs_clone.push_back(clone_index(tr.obs[ks[q]].sid));
-          wB.obs_z.push_back(tr.obs[ks[q]].z[0]);
-          wB.obs_z.push_back(tr.obs[ks[q]].z[1]);
-        }
-        c.jac_m = 2;
-        c.s_blk = rm[0];
-        c.e_blk = rm[1];
-        c.cm_first_clone = wB.obs_clone[c.tri_off];
-        c.cm_last_clone = wB.obs_clone[c.tri_off + (tracked ? nobs - 2 : nobs - 1)];
-        c.cm_zu = tr.obs[0].z[0];
-        c.cm_zv = tr.obs[0].z[1];
-        cb.push_back(x);
-      }
-      // erase the observations of the removed clones (:2842-2844)
-      tr.obs.erase(std::remove_if(tr.obs.begin(), tr.obs.end(),
-                                  [&](const Obs& o) { return o.sid == rm_id0 || o.sid == rm_id1; }),
-                   tr.obs.end());
-      tr.touch();
-    }
-    F.stats.n_candidates_prune = (int)cb.size();
-    if (!cb.empty()) {
-      fw.active = 1;
-      wB.any_active = true;
-      append_candidates(wB, fi, cb, F.cinfo[1]);
-    }
-    fill_hw();
+    tr.id_anchor = new_id;
+    fr.reanchor.push_back(rc);
   }
-  wB.cand_begin[B_] = (int)wB.cands.size();
-  reanchor_off[B_] = (int)reanchor.size();
-  wB.extra_ints = rm_idx;
-  wB.extra_ints.insert(wB.extra_ints.end(), Nbefore.begin(), Nbefore.end());
-  wB.extra_ints.insert(wB.extra_ints.end(), Ebefore.begin(), Ebefore.end());
-  if (!hyb_ok) { ok_ = false; err_ = "hybrid bookkeeping failed (anchor outside the window)"; return ORCVIO_ERR_CUDA; }
+}
+
+// prune candidate (:2776-2839): rows from the observations obs[inv0], obs[inv1] by the removed clones rm[0] < rm[1]
+static CandBuild prune_candidate(Batch::PhaseWork& w, const FilterHost& F, const Track& tr, int inv0, int inv1,
+                                 const int rm[2]) {
+  const int nobs = (int)tr.obs.size();
+  const bool tracked = tr.obs.back().sid == F.state_id;
+  CandBuild x{};
+  x.id = tr.id;
+  x.kind = 2;
+  Cand& c = x.c;
+  c.slot = tr.slot;
+  c.gen = tr.gen;
+  c.flags = 0;
+  c.tri_off = (int)w.obs_clone.size();
+  for (const Obs& o : tr.obs) {            // initializePosition_AssignAnchor: all obs
+    w.obs_clone.push_back(F.clone_index(o.sid));
+    w.obs_z.push_back(o.z[0]);
+    w.obs_z.push_back(o.z[1]);
+  }
+  c.tri_m = nobs;
+  c.jac_off = (int)w.obs_clone.size();
+  const int ks[2] = {inv0, inv1};
+  for (int q = 0; q < 2; ++q) {
+    w.obs_clone.push_back(F.clone_index(tr.obs[ks[q]].sid));
+    w.obs_z.push_back(tr.obs[ks[q]].z[0]);
+    w.obs_z.push_back(tr.obs[ks[q]].z[1]);
+  }
+  c.jac_m = 2;
+  c.s_blk = rm[0];
+  c.e_blk = rm[1];
+  c.cm_first_clone = w.obs_clone[c.tri_off];
+  c.cm_last_clone = w.obs_clone[c.tri_off + (tracked ? nobs - 2 : nobs - 1)];
+  c.cm_zu = tr.obs[0].z[0];
+  c.cm_zv = tr.obs[0].z[1];
+  return x;
+}
+
+// pruneImuStateBuffer :2629-2873 of filter fi, up to the update
+void Batch::prune_filter(FrameWork& fr, int fi) {
+  FilterHost& F = f_[fi];
+  PhaseWork& w = fr.B;
+  const int n = (int)F.clones.size();
+  int* rm = &fr.rm_idx[2 * fi];
+  if (F.if_zupt) {
+    // :2633-2639: a stationary frame drops the previous clone (id - 1) and uses nothing
+    if (n < 2) return;
+    rm[0] = n - 2;
+  } else {
+    if (n < p_.sw_size) return;
+    w.maxN = std::max(w.maxN, w.fw[fi].N);
+    find_redundant_imu_states(F, rm);
+  }
+  const int n_rm = F.if_zupt ? 1 : 2;
+  const long long rm_ids[2] = {F.clones[rm[0]].id, F.clones[rm[n_rm - 1]].id};
+  F.stats.n_removed_clones = n_rm;
+  for (int q = 0; q < n_rm; ++q) F.stats.removed_ids[q] = rm_ids[q];
+  if (hybrid_) reanchor_tracks(fr, fi, rm_ids, n_rm);
+  std::vector<CandBuild> cb;
+  for (auto& kv : F.map_server) {
+    Track& tr = kv.second;
+    if (tr.first_sid > rm_ids[1] || tr.last_sid < rm_ids[0]) continue;   // (ascending ids: it cannot hold the clones)
+    int inv0 = -1, inv1 = -1;
+    for (int k = 0; k < (int)tr.obs.size(); ++k) {
+      if (tr.obs[k].sid == rm_ids[0]) inv0 = k;
+      if (tr.obs[k].sid == rm_ids[1]) inv1 = k;
+    }
+    if (inv0 < 0 && inv1 < 0) continue;
+    // (:2776: EKF-SLAM features never contribute MSCKF rows here)
+    if (!F.if_zupt && inv0 >= 0 && inv1 >= 0 && !tr.in_state && !tr.ekf_feature)
+      cb.push_back(prune_candidate(w, F, tr, inv0, inv1, rm));
+    // erase the observations of the removed clones (:2842-2844)
+    tr.obs.erase(std::remove_if(tr.obs.begin(), tr.obs.end(),
+                                [&](const Obs& o) { return o.sid == rm_ids[0] || o.sid == rm_ids[1]; }),
+                 tr.obs.end());
+    tr.touch();
+  }
+  F.stats.n_candidates_prune = (int)cb.size();
+  if (!cb.empty()) {
+    w.fw[fi].active = 1;
+    w.any_active = true;
+    append_candidates(w, fi, cb, F.cinfo[1]);
+  }
+}
+
+// pruneImuStateBuffer :2629-2959: phase B, k_reanchor, k_remove.  False: the hybrid bookkeeping failed (err_).
+bool Batch::prune_imu_state_buffer(FrameWork& fr) {
+  PhaseWork& B = fr.B;
+  begin_phase(B, 1);
+  for (int fi = 0; fi < B_; ++fi) {
+    FilterHost& F = f_[fi];
+    B.cand_begin[fi] = (int)B.cands.size();
+    fr.reanchor_off[fi] = (int)fr.reanchor.size();
+    if (!F.active) continue;
+    B.maxE = std::max(B.maxE, (int)F.feature_states.size());
+    prune_filter(fr, fi);
+    if (hybrid_) push_hyb_feats(B, fi, B.fw[fi].active, false, &fr.hyb_ok);   // anchors after the changes
+  }
+  B.cand_begin[B_] = (int)B.cands.size();
+  fr.reanchor_off[B_] = (int)fr.reanchor.size();
+  B.extra_ints = fr.rm_idx;                     // k_remove: the removed clones, then N and E before the removal
+  for (const FilterWork& fw : B.fw) B.extra_ints.push_back(fw.N);
+  for (const FilterHost& F : f_) B.extra_ints.push_back((int)F.feature_states.size());
+  if (!fr.hyb_ok) { ok_ = false; err_ = "hybrid bookkeeping failed (anchor outside the window)"; return false; }
   g_sp.mark(9);
-  stage_phase(wB);
-  if (hybrid_ && !reanchor.empty()) {
-    const ReanchorRec* d_rec = hb->put(reanchor.data(), reanchor.size(), stream_, &hyb_ok);
-    const int* d_off = hb->put(reanchor_off.data(), reanchor_off.size(), stream_, &hyb_ok);
-    if (hyb_ok) {
-      launch_reanchor(d_rec, d_off, B_, wB.dHw, dClones_.get(), (size_t)Ncap_ * CL_STRIDE, dImu_.get(), dFpos_.get(), dFidp_.get(), Fcap_, dP_.get(),
+  stage_phase(B);
+  if (hybrid_ && !fr.reanchor.empty()) {
+    const ReanchorRec* d_rec = hyb_->put(fr.reanchor.data(), fr.reanchor.size(), stream_, &fr.hyb_ok);
+    const int* d_off = hyb_->put(fr.reanchor_off.data(), fr.reanchor_off.size(), stream_, &fr.hyb_ok);
+    if (fr.hyb_ok) {
+      launch_reanchor(d_rec, d_off, B_, B.dHw, dClones_.get(), (size_t)Ncap_ * CL_STRIDE, dImu_.get(), dFpos_.get(), dFidp_.get(), Fcap_, dP_.get(),
                       (size_t)ldp_ * ldp_, ldp_, stream_);
       ++launches_;
     }
   }
-  launch_phase(wB, true);
-  // remove the pruned clones from P / clone array (:2875-2956)
+  launch_phase(B, true);
   bool any_rm = false;
-  for (int v : rm_idx) any_rm |= (v >= 0);
+  for (int v : fr.rm_idx) any_rm |= (v >= 0);
   if (any_rm) {
     RemoveArgs ra{};
     ra.P = dP_.get(); ra.p_stride = (size_t)ldp_ * ldp_; ra.ldp = ldp_;
     ra.clones = dClones_.get(); ra.clone_stride = (size_t)Ncap_ * CL_STRIDE;
-    ra.rm = wB.d_extra; ra.N = wB.d_extra + 2 * B_; ra.n_filters = B_;
-    ra.E = hybrid_ ? wB.d_extra + 3 * B_ : nullptr;
+    ra.rm = B.d_extra; ra.N = B.d_extra + 2 * B_; ra.n_filters = B_;
+    ra.E = hybrid_ ? B.d_extra + 3 * B_ : nullptr;
     launch_remove(ra, stream_);
     ++launches_;
   }
-  if (hybrid_) hybrid_queue_gather(gather_tracks);
+  if (hybrid_) hybrid_queue_gather(fr.gather_tracks);
   download_mirrors();
   g_sp.mark(10);
   CK(cudaStreamSynchronize(stream_));
   if (hybrid_) {
-    hybrid_apply_gather(gather_tracks);
-    if (!hyb_ok) { ok_ = false; err_ = "hybrid upload arena exhausted"; }
+    hybrid_apply_gather(fr.gather_tracks);
+    if (!fr.hyb_ok) { ok_ = false; err_ = "hybrid upload arena exhausted"; }
   }
-  account(wB.any_active);
+  account_phase(B.any_active);
   for (int fi = 0; fi < B_; ++fi) {
     FilterHost& F = f_[fi];
     if (!F.active) continue;
-    const int c0 = wB.cand_begin[fi], c1 = wB.cand_begin[fi + 1];
-    for (int c = c0; c < c1; ++c) {
-      const int st = hStatus_.get()[c];
-      F.cstatus[1].push_back(st);
-      F.cgamma[1].push_back(hGamma_.get()[c]);
-      if (!(st & ST_TRI_VALID)) F.stats.n_tri_invalid_prune++;
-      if (st & ST_GATE_PASS) { F.stats.n_gate_pass_prune++; ++feature_updates_; }
-    }
-    if (rm_idx[2 * fi] >= 0) {
-      const int a = rm_idx[2 * fi], b = rm_idx[2 * fi + 1];
+    for (int c = B.cand_begin[fi]; c < B.cand_begin[fi + 1]; ++c) take_result(F, 1, c, true);
+    const int a = fr.rm_idx[2 * fi], b = fr.rm_idx[2 * fi + 1];
+    if (a >= 0) {
       const double ta = F.clones[a].time, tb = b >= 0 ? F.clones[b].time : ta;
       F.cur_window_timestamps.erase(
           std::remove_if(F.cur_window_timestamps.begin(), F.cur_window_timestamps.end(),
@@ -1911,13 +1911,10 @@ int Batch::process_ptrs(const double* t_img, const OrcvioFeature* const* featp, 
       if (b >= 0) F.clones.erase(F.clones.begin() + b);
       F.clones.erase(F.clones.begin() + a);
     }
-    std::memcpy(F.imu_mirror.data(), hImu_.get() + (size_t)fi * IM_STRIDE, IM_STRIDE * sizeof(double));
-    std::memcpy(F.clone_mirror.data(), hClones_.get() + (size_t)fi * Ncap_ * CL_STRIDE,
-                (size_t)Ncap_ * CL_STRIDE * sizeof(double));
+    refresh_mirrors(fi);
   }
   g_sp.mark(11);
-  g_sp.done(B_);
-  return ok_ ? ORCVIO_OK : ORCVIO_ERR_CUDA;
+  return true;
 }
 
 void Batch::hybrid_queue_gather(std::vector<Track*>& tracks) {

@@ -74,6 +74,26 @@ struct FilterHost {
     map_server.erase(id);
   }
   std::vector<CloneMeta> clones;
+  // state id -> index in the window.  The window does not change between augmentation and the end of a frame, and its
+  // ids span a few dozen consecutive values: one small table per filter instead of a search per observation.
+  std::vector<short> clone_lut;        // empty: clone_index searches the window
+  void index_clones() {                // every frame, for every filter (a filter outside the frame gets the search)
+    clone_lut.clear();
+    if (!active || clones.empty()) return;
+    const long long base = clones.front().id, span = clones.back().id - base + 1;
+    if (span > 4096) return;                             // (never seen: falls back to the search)
+    clone_lut.assign((size_t)span, (short)-1);
+    for (int k = 0; k < (int)clones.size(); ++k) clone_lut[(size_t)(clones[k].id - base)] = (short)k;
+  }
+  int clone_index(long long sid) const {   // -1: not in the window
+    if (!clone_lut.empty()) {
+      const long long off = sid - clones.front().id;
+      return (off >= 0 && off < (long long)clone_lut.size()) ? (int)clone_lut[(size_t)off] : -1;
+    }
+    for (int k = (int)clones.size() - 1; k >= 0; --k)
+      if (clones[k].id == sid) return k;
+    return -1;
+  }
   std::vector<int> free_slots;
   long long next_state_id = 0;
   long long next_gen = 1;
@@ -88,7 +108,6 @@ struct FilterHost {
   bool active = false;        // took part in the current frame
   bool if_zupt = false;
   std::vector<double> coarse_feature_dis;   // checkZUPTFeat input, filled by addFeatureObservations (:1052-1058)
-  double zupt_chi2 = 0.0, zupt_vnorm = 0.0;  // checkZUPTIMU diagnostics of the last frame
   std::vector<double> imu_mirror;      // IM_STRIDE
   std::vector<double> clone_mirror;    // Ncap * CL_STRIDE
   std::vector<double> cur_window_timestamps;
@@ -301,7 +320,6 @@ class Batch {
   void upload_blob();
   void ensure_scratch(size_t n_cand, size_t hblk, size_t rblk);
   cudaError_t grow_update_scratch(size_t need_a, size_t need_p);
-  void run_phase(PhaseWork& w, int phase);
   void stage_phase(PhaseWork& w);
   void stage_pack(PhaseWork& w);
   void stage_upload(PhaseWork& w);
@@ -319,6 +337,28 @@ class Batch {
   bool want_iters_ = false, want_raw_ = false, skip_tri_ = false, skip_update_ = false, skip_jac_ = false;
   void download_mirrors();
   void init_filter_device(int i);
+  // processFeatures (process_ptrs), one method per step of the reference (batch.cu)
+  struct FrameWork;
+  bool check_feature_capacity(const OrcvioFeature* const* feats, const int* n_feats) const;
+  bool batch_imu_processing(FrameWork& fr, int fi, const OrcvioImu* imu, int n_imu, double t_img, int* imu_used);
+  bool add_feature_observations(int fi, const OrcvioFeature* feats, int n_feats);
+  void propagate_and_augment(FrameWork& fr);
+  bool remove_lost_features(FrameWork& fr);
+  void compact_feature_states(FrameWork& fr);
+  void speculative_triangulation(FrameWork& fr);
+  void decide_grid_cells(FrameWork& fr, int fi);
+  void stage_lost_features(FrameWork& fr, int fi);
+  void apply_lost_results(const FrameWork& fr);
+  void find_redundant_imu_states(const FilterHost& F, int rm[2]) const;
+  void reanchor_tracks(FrameWork& fr, int fi, const long long* rm_ids, int n_rm);
+  void prune_filter(FrameWork& fr, int fi);
+  bool prune_imu_state_buffer(FrameWork& fr);
+  // shared by the two update phases
+  void begin_phase(PhaseWork& w, int hyb_phase);
+  void push_hyb_feats(PhaseWork& w, int fi, int active, bool with_obs, bool* ok);
+  int take_result(FilterHost& F, int ph, int c, bool counted);
+  void refresh_mirrors(int fi);
+  void account_phase(bool had_update);
 };
 
 void rotation_to_quat_xyzw(const double* R, double* q);
